@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- packet-steps/sec of the SWRaytracing hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--single-process]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--single-process] [--dump-outputs DIR]
 
 HEADLINE (value, e2e, roofline of the one JSON line) = BASELINE.json configs[3], the configuration its target sentence is
 quoted on: **C4** -- two-layer-type flow on a 512^2 spectral grid (L = 20, mean shear), two stored frames blended on the
@@ -22,6 +22,9 @@ host cores.  ``--impl reference`` times that CPU port alone on the same config.
 
 ``--single-process``: the N GPUs are driven by ONE process through a multi-device handle (swrt_params.ngpu = N, in-library
 sharding + NCCL) instead of one torchrun rank per GPU.
+
+``--dump-outputs DIR``: after the timed steps, the headline's packet state and omega histogram as left by its last timed
+step go to DIR/*.npy.  Inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -77,10 +80,22 @@ def parse():
     ap.add_argument("--single-process", action="store_true", help="drive --gpus N devices from this one process (multi-device handle)")
     ap.add_argument("--mode", default="spectral", choices=["spectral", "nufft", "lagrange6"],
                     help="evaluation mode of the HEADLINE legs (value, e2e, roofline); default = the dense DMMA contraction")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline's last timed step computed to DIR/<name>.npy (float64): the packet state "
+                         f"x, y, k, l (a fixed, seeded sample of {DUMP_MAX_PACKETS} packets when there are more) and omega_hist")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "swrt":
+        ap.error("--dump-outputs writes the GPU arm's outputs")
+    if args.dump_outputs and not args.single_process and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs needs the whole ensemble in one process (use --single-process for several GPUs)")
+    return args
 
 
 TOTALS = {"C2": 65536, "C3": 1048576, "C4": 16777216, "C5": 4194304}
+DUMP_MAX_PACKETS = 1 << 20          # 4 float64 arrays of this length = 32 MiB of --dump-outputs
+DUMP_SEED = 0
 GRID = {"C1": 64, "C2": 128, "C3": 256, "C4": 512, "C5": 256}
 SCHEME = {"C5": "rk4_xka"}
 
@@ -376,9 +391,10 @@ def make_engine(S, W, w, mode, ctx, mtiles=0):
     return eng
 
 
-def measure(ctx, name, total_packets, sub, steps, warmup, mode_name, peaks, headline=False):
+def measure(ctx, name, total_packets, sub, steps, warmup, mode_name, peaks, headline=False, dump=False):
     """time one workload on this process's shard: device-resident `value`, end-to-end `e2e` (pinned + pageable host buffers
-    through swrt_step_host), the dominant kernel's roofline.  Returns the dict that goes into the JSON line."""
+    through swrt_step_host), the dominant kernel's roofline.  Returns the dict that goes into the JSON line; with `dump`,
+    also (under "_outputs") what the last timed device-resident step left: packet state and omega histogram."""
     import swraytracing_b200 as S
     from swraytracing_b200 import workloads as W
     from swraytracing_b200.distributed import ShardedEnsemble, shard_range
@@ -441,6 +457,14 @@ def measure(ctx, name, total_packets, sub, steps, warmup, mode_name, peaks, head
     total_ms = ctx.max_over_ranks(float(np.sum(step_ms)))
     value = n_total * sub * steps / (total_ms * 1e-3)
     hist_total = int(np.asarray(last_counts[0]).sum())
+    outputs = None
+    if dump:
+        # read before the legs below step the same packets further
+        state = eng.get_packets()
+        if n > DUMP_MAX_PACKETS:
+            pick = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_MAX_PACKETS, replace=False))
+            state = [a[pick] for a in state]
+        outputs = dict(zip("xykl", state), omega_hist=np.asarray(last_counts[0], dtype=np.float64))
 
     # dominant-kernel time: re-time the packet kernel(s) alone with the handle's own event pair
     k_ms, nl = [], 1
@@ -553,6 +577,7 @@ def measure(ctx, name, total_packets, sub, steps, warmup, mode_name, peaks, head
         res["shard_bit_identical"] = shard_ok
     res["_w"] = w
     res["_sub"] = sub
+    res["_outputs"] = outputs
     eng.close()
     return res
 
@@ -591,13 +616,19 @@ def main():
 
     name = args.workload
     sub = args.substeps or SUBSTEPS.get(name, 16)
-    head = measure(ctx, name, args.packets, sub, args.steps, args.warmup, args.mode, peaks, headline=True)
+    head = measure(ctx, name, args.packets, sub, args.steps, args.warmup, args.mode, peaks, headline=True, dump=bool(args.dump_outputs))
     w = head.pop("_w"); head.pop("_sub")
+    outputs = head.pop("_outputs")
+    if outputs is not None:
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for key, arr in outputs.items():
+            np.save(out_dir / f"{key}.npy", arr)
 
     configs = {}
     for cname in [c for c in args.configs.split(",") if c and c != name]:
         r = measure(ctx, cname, 0, SUBSTEPS.get(cname, 16), args.side_steps, 3, args.mode, peaks)
-        r.pop("_w"); r.pop("_sub")
+        r.pop("_w"); r.pop("_sub"); r.pop("_outputs")
         configs[cname] = r
 
     side = {}

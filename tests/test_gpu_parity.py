@@ -1266,6 +1266,44 @@ def test_bench_gpu_arm_prints_one_contract_line():
     assert d["histogram_total"] <= 9472
 
 
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: the packets and omega histogram after warm-up + --steps bench steps, equal to the same
+    steps driven through the Engine directly; the same arguments give the same files, one more step gives other ones"""
+    import os, subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = dict(os.environ)
+    for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK"):
+        env.pop(k, None)
+    n, warmup = 9472, 3
+
+    def bench(steps, tag):
+        out = tmp_path / tag
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(steps), "--warmup", str(warmup),
+                            "--packets", str(n), "--configs", "", "--no-side-modes", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, env=env, timeout=900, cwd=root)
+        assert r.returncode == 0, r.stderr[-3000:]
+        files = sorted(out.glob("*.npy"))
+        assert [f.stem for f in files] == ["k", "l", "omega_hist", "x", "y"]
+        assert sum(f.stat().st_size for f in files) <= 64 << 20
+        return {f.stem: np.load(f) for f in files}
+
+    w = W.make_workload("C4", n_packets=n)
+    edges = np.linspace(0.0, float(np.sqrt(w.f ** 2 + w.gH * 4 * (w.k ** 2 + w.l ** 2).max())), 300)
+    with S.Engine(w.nx, w.L, w.f, w.gH, S.MODE_SPECTRAL) as e:
+        e.set_flow_spectral(w.psik, slot=0, u_mean=w.u_mean); e.set_flow_spectral(w.psik2, slot=1, u_mean=w.u_mean)
+        e.set_packets(w.x, w.y, w.k, w.l)
+        want = {}
+        for total in range(1, warmup + 3):
+            e.step(S.SCHEME_LEAPFROG, w.dt / 2, 2, 0.25, 0.5)            # one C4 bench step: two time-centred sub-steps
+            if total - warmup in (1, 2):
+                want[total - warmup] = dict(zip("xykl", e.get_packets()), omega_hist=e.hist_omega(edges).astype(np.float64))
+    one, again, two = bench(1, "one"), bench(1, "again"), bench(2, "two")
+    for name in one:
+        assert one[name].dtype == np.float64 and np.array_equal(one[name], again[name]), name
+        assert np.array_equal(one[name], want[1][name]) and np.array_equal(two[name], want[2][name]), name
+    assert not np.array_equal(one["x"], two["x"]) and one["omega_hist"].sum() == n
+
+
 def test_nufft_gradients_at_and_next_to_grid_nodes():
     """A packet on a grid node (or within rounding of one: x = i*dx) puts a stencil node at the very end of the NUFFT kernel's
     support, where the analytic derivative phi' = -phi beta z / sqrt(1 - z^2) is singular; before the end node was dropped

@@ -3,7 +3,7 @@
 1. Language semantics: known MATLAB behaviours (column-major linear indexing, ``end``, growth on assignment, implicit expansion,
    value semantics, white space inside brackets, transpose vs quote, ``nargin`` / ``nargout``, nested functions sharing the
    parent workspace, closures, classdef with inheritance and method dispatch, command syntax, ``fread`` / ``fwrite``).
-2. Against numbers REAL MATLAB produced and the reference still holds (needs ``/root/reference``; skipped on the GPU box):
+2. Against numbers REAL MATLAB produced and the reference still holds (needs a checkout of it in ``SWRT_REFERENCE_DIR``):
    the unmodified ``qg_flow_ray_trace/qgsw_raytrace.m`` run under minimat prints the header lines MATLAB R2020b printed into
    the shipped SLURM logs, its ``pv_time`` stream lands within 2 ulps of the stored one, the unmodified ``rsw/k2g.m`` /
    ``fulspec.m`` reproduce the grid fields stored in ``rsw/matlab.mat``, and the unmodified solver ``rsw/swk.m`` run for 300
@@ -27,8 +27,10 @@ sys.path.insert(0, str(ROOT / "tests" / "golden"))
 
 from oracle.minimat import Interp, MatlabError, MStruct, MCell      # noqa: E402
 
-REF = Path("/root/reference")
-needs_ref = pytest.mark.skipif(not (REF / "ode_symplectic.m").exists(), reason="the reference checkout is not on this machine")
+# a checkout of the original MATLAB project (ndefilippis/SWRaytracing), which this repository does not carry
+REF = Path(os.environ.get("SWRT_REFERENCE_DIR", "")).absolute()
+HAVE_REF = bool(os.environ.get("SWRT_REFERENCE_DIR")) and (REF / "ode_symplectic.m").exists()
+needs_ref = pytest.mark.skipif(not HAVE_REF, reason="set SWRT_REFERENCE_DIR to a checkout of the original MATLAB project")
 GOLD = ROOT / "tests" / "golden"
 
 
