@@ -229,7 +229,9 @@ int swrt_set_flow_from_qg2(swrt_handle* h, int slot, swrt_qg2* q);
 /* number of kernel launches issued by this handle since creation / since the last reset        */
 int64_t swrt_launch_count(swrt_handle* h, int reset);
 /* milliseconds spent in the dominant kernel of the most recent swrt_step / swrt_eval call,
- * measured with CUDA events on the handle's stream; nlaunch receives how many launches         */
+ * measured with CUDA events on the handle's stream; nlaunch receives how many packet-stepping
+ * runs it made: one per dense-kernel launch, one per anchored leapfrog run (whose drift, sort,
+ * K1 and K2 launches of every sub-step are all inside the timed bracket and in swrt_launch_count) */
 double  swrt_last_kernel_ms(swrt_handle* h, int* nlaunch);
 /* executed real fp64 flops (spectral) or gathered bytes (Lagrange) per packet per evaluation   */
 double  swrt_work_per_eval(const swrt_handle* h, int nplanes);

@@ -18,6 +18,7 @@
 #include "spectral_common.cuh"
 #include <cstdio>
 #include <cstdlib>
+#include <cmath>
 
 namespace swrt {
 
@@ -252,6 +253,82 @@ size_t spectral_smem_bytes(const PackGeom& g) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// per-row epilogue pieces shared by the dense kernel and the anchored step kernel (same arithmetic in both)
+// ------------------------------------------------------------------------------------------------
+// stage 2 of one pass: F_c += Re[e^{i ky ty} G_c(ky)] for this lane's ky of every group, then advance the y twiddles
+template <int NPL, int G, bool PSI, int NF>
+__device__ __forceinline__ void stage2_pass(const double (&acc)[NPL * G][2], Cplx (&ytw)[G], const Cplx yrot, double& kyd,
+                                            double (&F)[NF]) {
+#pragma unroll
+    for (int gg = 0; gg < G; gg++) {
+        const double cy = ytw[gg].re, sy = ytw[gg].im;
+        if constexpr (PSI) {
+            const double ky = kyd + (double)(4 * gg);
+            const double g0r = acc[0 * G + gg][0], g0i = acc[0 * G + gg][1];
+            const double g1r = acc[1 * G + gg][0], g1i = acc[1 * G + gg][1];
+            const double g2r = acc[2 * G + gg][0], g2i = acc[2 * G + gg][1];
+            const double a0 = fma(g0r, cy, -g0i * sy), b0 = fma(g0i, cy, g0r * sy);
+            const double a1 = fma(g1r, cy, -g1i * sy), b1 = fma(g1i, cy, g1r * sy);
+            const double a2 = fma(g2r, cy, -g2i * sy);
+            F[0] = fma(ky, b0, F[0]);          // u  / kap
+            F[1] += a1;                        // v  / kap
+            F[2] = fma(ky, b1, F[2]);          // ux / kap^2
+            F[3] = fma(ky * ky, a0, F[3]);     // uy / kap^2
+            F[4] += a2;                        // vx / kap^2
+        } else {
+#pragma unroll
+            for (int c = 0; c < NPL; c++) {
+                F[c] = fma(acc[c * G + gg][0], cy, F[c]);
+                F[c] = fma(-acc[c * G + gg][1], sy, F[c]);
+            }
+        }
+        ytw[gg] = cmul(ytw[gg], yrot);
+    }
+    kyd += (double)(4 * G);
+}
+
+// quad reduction (the 4 lanes of a quad hold 4 interleaved ky subsets) and, for psi-hat stacks, the six planes
+template <bool PSI, int NPL, int NF>
+__device__ __forceinline__ void finish_planes(double (&F)[NF], const SpecArgs& a, int ev) {
+#pragma unroll
+    for (int c = 0; c < (PSI ? 5 : NPL); c++) {
+        double v = F[c];
+        v += __shfl_xor_sync(0xffffffffu, v, 1);
+        v += __shfl_xor_sync(0xffffffffu, v, 2);
+        F[c] = v;
+    }
+    if constexpr (PSI) {
+        const double kap = a.kappa, kap2 = a.kappa * a.kappa;
+        // mean shear of the blended frame (grid_U.m:11; interpolate_U.m:19-23), every rounding pinned
+        const double al = __dadd_rn(a.alpha0, __dmul_rn((double)(a.j0 + ev), a.dalpha));
+        const double um = __dadd_rn(__dmul_rn(__dsub_rn(1.0, al), a.u_mean0), __dmul_rn(al, a.u_mean1));
+        F[0] = fma(kap, F[0], um);
+        F[1] = kap * F[1];
+        F[2] = kap2 * F[2];
+        F[3] = kap2 * F[3];
+        F[4] = kap2 * F[4];
+        F[5] = -F[2];
+    }
+}
+
+// phi2(dt): x += dt*U(x1); k -= dt*(grad U)^T k with the OLD k (ode_symplectic.m:18-21); then phi1(dt/2) with the new k
+template <int NF>
+__device__ __forceinline__ void leapfrog_kick(const double (&F)[NF], const SpecArgs& a, double& px, double& py, double& pk,
+                                              double& pl, double& hcx, double& hcy) {
+    const double u = F[0], v = F[1], ux = F[2], uy = F[3], vx = F[4], vy = F[5];
+    px = px + a.dt * u;
+    py = py + a.dt * v;
+    const double k0 = pk, l0 = pl;
+    pk = k0 - a.dt * (ux * k0 + vx * l0);
+    pl = l0 - a.dt * (uy * k0 + vy * l0);
+    // (explicit un-fused mul/add so that a fused run of n steps and n single-step
+    // launches produce bit-identical states)
+    half_drift(pk, pl, a.f2, a.gH, __dmul_rn(__dmul_rn(0.5, a.dt), a.gH), hcx, hcy);
+    px = __dadd_rn(px, hcx);
+    py = __dadd_rn(py, hcy);
+}
+
+// ------------------------------------------------------------------------------------------------
 // the contraction kernel
 // ------------------------------------------------------------------------------------------------
 // PSI = true: the stack holds the three psi-hat moment planes N0 = psi, N1 = i kx psi, N2 = -kx^2 psi
@@ -261,6 +338,10 @@ size_t spectral_smem_bytes(const PackGeom& g) {
 // ATAB: 0 = x twiddles rotated in registers inside the k-loop; 1 = tabulated once per step in shared memory; 2 = tabulated
 // once per step in a per-CTA global scratch (L2-resident; grids whose table does not fit in shared memory), read back
 // with plain loads one unrolled body ahead -- in both table forms the k-loop holds no fp64 instruction but the DMMAs.
+// MODE SPEC_ANCHOR (K1 of the anchored leapfrog, DESIGN.md section 3e): a row is (occupied anchor, expansion order r) instead
+// of a packet.  A warp's 8 rows are 2 anchors x 4 orders of one parity (a.parity): r = 2*(row & 3) + parity, so that one
+// stack serves the CTA (even orders: the normal stack; odd orders: the S/D-swapped one).  The twiddle table carries
+// (kx/kmax)^r e^{i kx t_a}; the epilogue writes i^r/r! * the pass's accumulators as K2's B fragments instead of stage 2.
 template <int NPL, int G, int MT, int MODE, bool PSI, int ATAB>
 __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(const SpecArgs a) {
     static_assert(!ATAB || MT == 1, "the twiddle table is laid out for one m-tile per warp");
@@ -270,6 +351,8 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     constexpr int HALF_NT = NT / 2;
     constexpr int TILE_P = kConsumerWarps * 8 * MT;
     static_assert(NT % 2 == 0, "n-tiles are fetched in pairs");
+    constexpr bool ANC = MODE == SPEC_ANCHOR;
+    static_assert(!ANC || (PSI && MT == 1 && ATAB == 2), "the anchor contraction runs on psi-hat stacks with the global table");
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const PackGeom& g = a.g;
@@ -284,7 +367,9 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     double* sA;
     if constexpr (ATAB == 2) sA = a.twid + ((size_t)blockIdx.x * kConsumerWarps + warp) * g.ksteps * 32 + lane;
     else sA = reinterpret_cast<double*>(smem_raw + (size_t)nstages * chunk_bytes + 128) + (size_t)warp * g.ksteps * 32 + lane;
-    const long long ntiles = (a.n + TILE_P - 1) / TILE_P;
+    const long long nocc = ANC ? (long long)*a.anc_nocc : 0;
+    const long long nrows = ANC ? 4 * nocc : a.n;
+    const long long ntiles = (nrows + TILE_P - 1) / TILE_P;
     const int nevals = (MODE == SPEC_LEAPFROG) ? a.nsteps : 1;
 
     if (threadIdx.x == 0) {
@@ -367,10 +452,17 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         long long prow[MT];
         double px[MT], py[MT], pk[MT], pl[MT];
+        int anc_id = 0;                     // SPEC_ANCHOR: this row's anchor
 #pragma unroll
         for (int mt = 0; mt < MT; mt++) {
             long long r = tile * TILE_P + (long long)warp * 8 * MT + mt * 8 + quad_row;
             prow[mt] = r;
+            if constexpr (ANC) {
+                const long long slot = (r >> 2) < nocc ? (r >> 2) : nocc - 1;
+                anc_id = a.anc_list[slot];
+                px[mt] = py[mt] = pk[mt] = pl[mt] = 0.0;
+                continue;
+            }
             long long rc = r < a.n ? r : a.n - 1;
             if (MODE == SPEC_LEAPFROG) { px[mt] = a.x[rc]; py[mt] = a.y[rc]; pk[mt] = a.k[rc]; pl[mt] = a.l[rc]; }
             else { px[mt] = a.xin[rc]; py[mt] = a.yin[rc]; pk[mt] = 0; pl[mt] = 0; }
@@ -403,7 +495,7 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
             double F[MT][NF];
             double kyd[MT];                     // PSI: this lane's ky of group 0 in the current pass (as double)
 #pragma unroll
-            for (int mt = 0; mt < MT; mt++) {
+            for (int mt = 0; mt < (ANC ? 0 : MT); mt++) {
                 double s1, c1;
                 sincospi(reduced_turns(px[mt], a.dx, a.nxd, a.inv_nx), &s1, &c1);
                 double er = kx0 ? c1 : 1.0, ei = kx0 ? s1 : 0.0;
@@ -440,7 +532,25 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
                 kyd[mt] = (double)jq;
             }
 
-            if constexpr (ATAB) {
+            if constexpr (ANC) {
+                // A element of this lane: (kx/kmax)^r * (cos | sin)(pi kx t_a), kx = 2s + kx0.  t_a = (id + 1/2) * anc_h is a
+                // dyadic rational with few bits, so kx * t_a is exact and sincospi gives each twiddle to the last bit or so.
+                const int r = 2 * (quad_row & 3) + a.parity;
+                const double ta = ((double)anc_id + 0.5) * a.anc_h;
+                for (int s = 0; s < g.ksteps; s++) {
+                    const int kx = 2 * s + kx0;
+                    double v = 0.0;
+                    if (kx <= g.kmax) {
+                        double sn, cs;
+                        sincospi((double)kx * ta, &sn, &cs);
+                        const double w = (double)kx / (double)g.kmax;
+                        double wr = 1.0;
+                        for (int i = 0; i < r; i++) wr *= w;
+                        v = wr * (odd ? sn : cs);
+                    }
+                    sA[s * 32] = v;
+                }
+            } else if constexpr (ATAB) {
                 // the same two recurrences the in-loop rotation runs, tabulated once per step for all passes
                 double ap = ep0[0], aq = eq0[0], bp = ep1[0], bq = eq1[0];
                 for (int s = 0; s < g.ksteps; s += 2) {
@@ -524,78 +634,40 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
                     stage = nstage; phase = nphase;
                     ++ci;
                 }
-                // ---- stage 2: F_c += Gr*cos(ky ty) - Gi*sin(ky ty) for this lane's ky ----------
+                if constexpr (ANC) {
+                    // K2's B fragments of this pass: H'_r = i^r / r! * H~_r.  Real column 2jq (re) and 2jq+1 (im) of n-tile t
+                    // go to the B lane (column * 4 + r % 4) of k-step r / 4, in the dense stack's [pass][kstep][tp][lane][2] order.
+                    if (prow[0] < nrows) {
+                        const int r = 2 * (quad_row & 3) + a.parity;
+                        double fact = 1.0;
+                        for (int i = 2; i <= r; i++) fact *= (double)i;
+                        double* blk = a.hexp + (size_t)anc_id * a.anc_block + (size_t)pass * 2 * NT * 32;
+                        const int ks = r >> 2, krow = r & 3;
 #pragma unroll
-                for (int mt = 0; mt < MT; mt++) {
-#pragma unroll
-                    for (int gg = 0; gg < G; gg++) {
-                        const double cy = ytw[mt][gg].re, sy = ytw[mt][gg].im;
-                        if constexpr (PSI) {
-                            const double ky = kyd[mt] + (double)(4 * gg);
-                            const double g0r = acc[mt][0 * G + gg][0], g0i = acc[mt][0 * G + gg][1];
-                            const double g1r = acc[mt][1 * G + gg][0], g1i = acc[mt][1 * G + gg][1];
-                            const double g2r = acc[mt][2 * G + gg][0], g2i = acc[mt][2 * G + gg][1];
-                            const double a0 = fma(g0r, cy, -g0i * sy), b0 = fma(g0i, cy, g0r * sy);
-                            const double a1 = fma(g1r, cy, -g1i * sy), b1 = fma(g1i, cy, g1r * sy);
-                            const double a2 = fma(g2r, cy, -g2i * sy);
-                            F[mt][0] = fma(ky, b0, F[mt][0]);          // u  / kap
-                            F[mt][1] += a1;                            // v  / kap
-                            F[mt][2] = fma(ky, b1, F[mt][2]);          // ux / kap^2
-                            F[mt][3] = fma(ky * ky, a0, F[mt][3]);     // uy / kap^2
-                            F[mt][4] += a2;                            // vx / kap^2
-                        } else {
-#pragma unroll
-                            for (int c = 0; c < NPL; c++) {
-                                F[mt][c] = fma(acc[mt][c * G + gg][0], cy, F[mt][c]);
-                                F[mt][c] = fma(-acc[mt][c * G + gg][1], sy, F[mt][c]);
-                            }
+                        for (int t = 0; t < NT; t++) {
+                            const double re = acc[0][t][0] / fact, im = acc[0][t][1] / fact;
+                            const double hr = (r & 3) == 0 ? re : ((r & 3) == 1 ? -im : ((r & 3) == 2 ? -re : im));
+                            const double hi = (r & 3) == 0 ? im : ((r & 3) == 1 ? re : ((r & 3) == 2 ? -im : -re));
+                            double* dst = blk + ((size_t)(ks * HALF_NT + (t >> 1)) * 32) * 2 + (t & 1);
+                            dst[((2 * jq) * 4 + krow) * 2] = hr;
+                            dst[((2 * jq + 1) * 4 + krow) * 2] = hi;
                         }
-                        ytw[mt][gg] = cmul(ytw[mt][gg], yrot[mt]);
                     }
-                    kyd[mt] += (double)(4 * G);
+                } else {
+                    // ---- stage 2: F_c += Gr*cos(ky ty) - Gi*sin(ky ty) for this lane's ky ----------
+#pragma unroll
+                    for (int mt = 0; mt < MT; mt++) stage2_pass<NPL, G, PSI, NF>(acc[mt], ytw[mt], yrot[mt], kyd[mt], F[mt]);
                 }
             }
+            if constexpr (ANC) continue;
+            else {
             // ---- quad reduction: the 4 lanes of a quad hold 4 interleaved ky subsets ----------
 #pragma unroll
-            for (int mt = 0; mt < MT; mt++) {
-#pragma unroll
-                for (int c = 0; c < (PSI ? 5 : NPL); c++) {
-                    double v = F[mt][c];
-                    v += __shfl_xor_sync(0xffffffffu, v, 1);
-                    v += __shfl_xor_sync(0xffffffffu, v, 2);
-                    F[mt][c] = v;
-                }
-                if constexpr (PSI) {
-                    const double kap = a.kappa, kap2 = a.kappa * a.kappa;
-                    // mean shear of the blended frame (grid_U.m:11; interpolate_U.m:19-23), every rounding pinned
-                    const double al = __dadd_rn(a.alpha0, __dmul_rn((double)(a.j0 + ev), a.dalpha));
-                    const double um = __dadd_rn(__dmul_rn(__dsub_rn(1.0, al), a.u_mean0), __dmul_rn(al, a.u_mean1));
-                    F[mt][0] = fma(kap, F[mt][0], um);
-                    F[mt][1] = kap * F[mt][1];
-                    F[mt][2] = kap2 * F[mt][2];
-                    F[mt][3] = kap2 * F[mt][3];
-                    F[mt][4] = kap2 * F[mt][4];
-                    F[mt][5] = -F[mt][2];
-                }
-            }
+            for (int mt = 0; mt < MT; mt++) finish_planes<PSI, NPL, NF>(F[mt], a, ev);
             if (MODE == SPEC_LEAPFROG) {
                 if constexpr (NF >= 6) {
 #pragma unroll
-                    for (int mt = 0; mt < MT; mt++) {
-                        // phi2(dt): x += dt*U(x1); k -= dt*(grad U)^T k with the OLD k (ode_symplectic.m:18-21)
-                        const double u = F[mt][0], v = F[mt][1], ux = F[mt][2], uy = F[mt][3], vx = F[mt][4], vy = F[mt][5];
-                        px[mt] = px[mt] + a.dt * u;
-                        py[mt] = py[mt] + a.dt * v;
-                        const double k0 = pk[mt], l0 = pl[mt];
-                        pk[mt] = k0 - a.dt * (ux * k0 + vx * l0);
-                        pl[mt] = l0 - a.dt * (uy * k0 + vy * l0);
-                        // phi1(dt/2) with the new k
-                        // (explicit un-fused mul/add so that a fused run of n steps and n single-step
-                        // launches produce bit-identical states)
-                        half_drift(pk[mt], pl[mt], a.f2, a.gH, __dmul_rn(__dmul_rn(0.5, a.dt), a.gH), hcx[mt], hcy[mt]);
-                        px[mt] = __dadd_rn(px[mt], hcx[mt]);
-                        py[mt] = __dadd_rn(py[mt], hcy[mt]);
-                    }
+                    for (int mt = 0; mt < MT; mt++) leapfrog_kick<NF>(F[mt], a, px[mt], py[mt], pk[mt], pl[mt], hcx[mt], hcy[mt]);
                 }
             } else {
                 if (jq == 0) {
@@ -608,6 +680,7 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
                         }
                     }
                 }
+            }
             }
         }
         if (MODE == SPEC_LEAPFROG) {
@@ -674,6 +747,216 @@ cudaError_t launch_spectral(const SpecArgs& a, int mode, int mtiles, int num_sms
     SWRT_INST(1, 24, 1) SWRT_INST(1, 12, 2)
 #undef SWRT_INST
     return cudaErrorInvalidValue;
+}
+
+// ================================================================================================
+// anchored leapfrog (DESIGN.md section 3e): per sub-step  drift + key -> counting sort -> K1 (SPEC_ANCHOR) -> K2
+// ================================================================================================
+// Anchor cells of 2^-m turns, m the smallest with (pi kmax 2^-m)^R / R! <= 2^-53 (the truncation bound of the expansion
+// relative to sum |B|).  Grids from 256^2 to 512^2: below, a cell holds too few packets to pay for its K1 rows (C2 at
+// 128^2 is at break-even); above, an anchor's H' block (npass * 12 KB) no longer fits two CTAs per SM.
+int anchor_log2_cells(int nx) {
+    if (nx < 256 || nx > 512 || (nx & (nx - 1))) return 0;
+    const double kmax = nx / 2 - 1;
+    double fact = 1.0;
+    for (int i = 2; i <= kAnchorOrders; i++) fact *= i;
+    for (int m = 8; m < 30; m++)
+        if (std::pow(M_PI * kmax * std::ldexp(1.0, -m), kAnchorOrders) / fact <= std::ldexp(1.0, -53)) return m;
+    return 0;
+}
+
+cudaError_t launch_spectral_anchor(const SpecArgs& a, int max_rows, int num_sms, cudaStream_t st) {
+    if (a.g.npl != 3 || a.g.G != 8 || a.g.atab != 2 || !a.twid || !a.psi) return cudaErrorInvalidValue;
+    SpecArgs b = a;
+    b.n = max_rows;                   // grid sizing only: the kernel reads the row count from anc_nocc
+    return launch_inst2<3, 8, 1, SPEC_ANCHOR, true, 2>(b, num_sms, st);
+}
+
+// S/D-swapped stack for the odd expansion orders: in [[Sr Si],[-Di Dr]] the element (Er/Ei row, re/im column) is replaced
+// by the one of [[Dr Di],[-Si Sr]], which is the element of the partner lane (k row ^ 1, n column ^ 1), negated when
+// row and column parity differ.  Exact, so blending and swapping commute.
+__global__ void stack_swap_kernel(const double* __restrict__ in, double* __restrict__ out, size_t n) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    for (; i < n; i += stride) {
+        const int lane = (int)((i >> 1) & 31);
+        const bool same = (lane & 1) == ((lane >> 2) & 1);
+        const double v = in[i ^ (size_t)10];        // lane ^ 5
+        out[i] = same ? v : -v;
+    }
+}
+void launch_stack_swap(const double* in, double* out, size_t n, cudaStream_t st) {
+    size_t nb = (n + 255) / 256;
+    if (nb > 148 * 16) nb = 148 * 16;
+    stack_swap_kernel<<<(unsigned)nb, 256, 0, st>>>(in, out, n);
+}
+
+// first half drift (the dense kernel's arithmetic) and the anchor key; rank = position inside the anchor (atomic order:
+// results do not depend on it)
+__global__ void anchor_key_kernel(double* __restrict__ x, double* __restrict__ y, const double* __restrict__ k,
+                                  const double* __restrict__ l, long long n, double dx, double nxd, double inv_nx, double f2,
+                                  double gH, double dt, double inv_h, int nanchors, unsigned long long* __restrict__ cnt,
+                                  int* __restrict__ key, unsigned long long* __restrict__ rank) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double hx, hy;
+    half_drift(k[i], l[i], f2, gH, __dmul_rn(__dmul_rn(0.5, dt), gH), hx, hy);
+    const double xi = __dadd_rn(x[i], hx);
+    x[i] = xi;
+    y[i] = __dadd_rn(y[i], hy);
+    int c = (int)floor(reduced_turns(xi, dx, nxd, inv_nx) * inv_h);
+    c = c < 0 ? 0 : (c >= nanchors ? nanchors - 1 : c);
+    key[i] = c;
+    rank[i] = atomicAdd(&cnt[c], 1ULL);
+}
+void launch_anchor_key(double* x, double* y, const double* k, const double* l, long long n, double dx, double nxd, double inv_nx,
+                       double f2, double gH, double dt, double inv_h, int nanchors, unsigned long long* cnt, int* key,
+                       unsigned long long* rank, cudaStream_t st) {
+    anchor_key_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, y, k, l, n, dx, nxd, inv_nx, f2, gH, dt, inv_h, nanchors, cnt,
+                                                                  key, rank);
+}
+
+// exclusive scan of the anchor counts and the compacted list of occupied anchors (one CTA; at most 2^15 anchors)
+__global__ void __launch_bounds__(1024) anchor_scan_kernel(const unsigned long long* __restrict__ cnt, unsigned long long* __restrict__ off,
+                                                           int* __restrict__ occ, int* __restrict__ nocc, int nanchors) {
+    __shared__ unsigned long long sc[1024];
+    __shared__ int so[1024];
+    const int t = threadIdx.x;
+    const int per = (nanchors + 1023) / 1024;
+    const int lo = t * per, hi = (lo + per < nanchors) ? lo + per : nanchors;
+    unsigned long long c = 0; int o = 0;
+    for (int i = lo; i < hi; i++) { c += cnt[i]; o += cnt[i] != 0; }
+    sc[t] = c; so[t] = o;
+    __syncthreads();
+    for (int d = 1; d < 1024; d <<= 1) {
+        const unsigned long long vc = t >= d ? sc[t - d] : 0;
+        const int vo = t >= d ? so[t - d] : 0;
+        __syncthreads();
+        sc[t] += vc; so[t] += vo;
+        __syncthreads();
+    }
+    unsigned long long base = t ? sc[t - 1] : 0;
+    int ob = t ? so[t - 1] : 0;
+    for (int i = lo; i < hi; i++) {
+        off[i] = base;
+        base += cnt[i];
+        if (cnt[i]) occ[ob++] = i;
+    }
+    if (t == 1023) *nocc = so[1023];
+}
+void launch_anchor_scan(const unsigned long long* cnt, unsigned long long* off, int* occ, int* nocc, int nanchors, cudaStream_t st) {
+    anchor_scan_kernel<<<1, 1024, 0, st>>>(cnt, off, occ, nocc, nanchors);
+}
+
+__global__ void anchor_scatter_kernel(const int* __restrict__ key, const unsigned long long* __restrict__ rank,
+                                      const unsigned long long* __restrict__ off, long long* __restrict__ perm, long long n) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) perm[off[key[i]] + rank[i]] = i;
+}
+void launch_anchor_scatter(const int* key, const unsigned long long* rank, const unsigned long long* off, long long* perm, long long n,
+                           cudaStream_t st) {
+    anchor_scatter_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(key, rank, off, perm, n);
+}
+
+// K2: one CTA per anchor.  The anchor's H' block (8 orders x 2 nky x 3 planes, in K2's B-fragment order) is bulk-copied into
+// shared memory; each warp takes 8-packet groups of the anchor: A = [z^0 .. z^7] of its 8 packets (two k-steps of m8n8k4),
+// per ky pass 2 x NT DMMAs give G = sum_r z^r H'_r, then the dense kernel's stage 2, quad reduction, kick and half drift.
+// A packet's result depends on its own state and its anchor's H' only: grouping, order and padding do not change a bit.
+template <int G>
+__global__ void __launch_bounds__(kAncWarps * 32, 2) anchored_step_kernel(const SpecArgs a) {
+    constexpr int NPL = 3, NT = NPL * G, HALF_NT = NT / 2, NF = 6;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const int anc = blockIdx.x;
+    const unsigned long long cnt = a.anc_cnt[anc];
+    if (cnt == 0) return;
+    const unsigned long long off = a.anc_off[anc];
+    const uint32_t block_bytes = (uint32_t)(a.anc_block * 8);
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + block_bytes);
+    if (threadIdx.x == 0) {
+        mbar_init(bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        mbar_expect_tx(bar, block_bytes);
+        const unsigned char* src = reinterpret_cast<const unsigned char*>(a.hexp + (size_t)anc * a.anc_block);
+        for (uint32_t o = 0; o < block_bytes; o += 32768) {
+            const uint32_t b = block_bytes - o < 32768 ? block_bytes - o : 32768;
+            bulk_g2s(smem_raw + o, src + o, b, bar);
+        }
+    }
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int quad_row = lane >> 2, jq = lane & 3;
+    const double ta = ((double)anc + 0.5) * a.anc_h;
+    const long long ngroups = (long long)((cnt + 7) / 8);
+    bool waited = false;
+    for (long long gi = warp; gi < ngroups; gi += kAncWarps) {
+        long long row = gi * 8 + quad_row;
+        const bool valid = row < (long long)cnt;
+        if (!valid) row = (long long)cnt - 1;
+        const long long p = a.anc_perm[off + row];
+        double px = a.x[p], py = a.y[p], pk = a.k[p], pl = a.l[p];     // x, y after the first half drift
+        // A fragments: z^jq (k-step 0) and z^(4 + jq) (k-step 1)
+        const double z = a.zscale * (reduced_turns(px, a.dx, a.nxd, a.inv_nx) - ta);
+        const double z2 = z * z;
+        const double zj = jq == 0 ? 1.0 : (jq == 1 ? z : (jq == 2 ? z2 : z2 * z));
+        const double a0 = zj, a1 = zj * (z2 * z2);
+        // y twiddles exactly as the dense kernel forms them
+        Cplx ytw[G], yrot;
+        double F[NF], kyd;
+        {
+            double sy, cy;
+            sincospi(reduced_turns(py, a.dx, a.nxd, a.inv_nx), &sy, &cy);
+            Cplx e1{cy, sy};
+            Cplx e2 = cmul(e1, e1);
+            Cplx e3 = cmul(e2, e1);
+            Cplx e4 = cmul(e2, e2);
+            Cplx cur = jq == 0 ? Cplx{1.0, 0.0} : (jq == 1 ? e1 : (jq == 2 ? e2 : e3));
+#pragma unroll
+            for (int gg = 0; gg < G; gg++) {
+                ytw[gg] = cur;
+                cur = cmul(cur, e4);
+            }
+            yrot = cpow<G>(e4);
+#pragma unroll
+            for (int c = 0; c < NF; c++) F[c] = 0.0;
+            kyd = (double)jq;
+        }
+        if (!waited) { mbar_wait(bar, 0); waited = true; }
+        for (int pass = 0; pass < a.g.npass; pass++) {
+            double acc[NT][2];
+#pragma unroll
+            for (int t = 0; t < NT; t++) { acc[t][0] = 0.0; acc[t][1] = 0.0; }
+            const double2* sB = reinterpret_cast<const double2*>(smem_raw) + (size_t)pass * 2 * HALF_NT * 32 + lane;
+#pragma unroll
+            for (int ks = 0; ks < 2; ks++) {
+                const double av = ks ? a1 : a0;
+#pragma unroll
+                for (int tp = 0; tp < HALF_NT; tp++) {
+                    const double2 b = sB[(ks * HALF_NT + tp) * 32];
+                    dmma884(acc[2 * tp][0], acc[2 * tp][1], av, b.x);
+                    dmma884(acc[2 * tp + 1][0], acc[2 * tp + 1][1], av, b.y);
+                }
+            }
+            stage2_pass<NPL, G, true, NF>(acc, ytw, yrot, kyd, F);
+        }
+        finish_planes<true, NPL, NF>(F, a, a.ev);
+        double hcx, hcy;
+        leapfrog_kick<NF>(F, a, px, py, pk, pl, hcx, hcy);
+        if (valid && jq == 0) { a.x[p] = px; a.y[p] = py; a.k[p] = pk; a.l[p] = pl; }
+    }
+    if (!waited) mbar_wait(bar, 0);       // the bulk copy must land before the CTA exits
+}
+
+cudaError_t launch_anchored_step(const SpecArgs& a, int nanchors, cudaStream_t st) {
+    if (a.g.npl != 3 || a.g.G != 8 || !a.psi) return cudaErrorInvalidValue;
+    const size_t smem = a.anc_block * 8 + 16;
+    auto kern = anchored_step_kernel<8>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<nanchors, kAncWarps * 32, smem, st>>>(a);
+    return cudaGetLastError();
 }
 
 }  // namespace swrt
