@@ -162,6 +162,15 @@ int swrt_bs23_accept(swrt_handle* h);
  * SW_zero_background_raytracing.m:73-78): y(t + s*hstep) = y + hstep * [f1 f2 f3 f4] * BI * [s; s^2; s^3],
  * BI = [1 -4/3 5/9; 0 1 -2/3; 0 4/3 -8/9; 0 -1 1].  Call between attempt and accept; s in (0, 1].     */
 int swrt_bs23_interp(swrt_handle* h, double hstep, double s, double* x, double* y, double* k, double* l);
+/* [~, Y] = ode23(odefun, tspan, [x;y;k;l]) on the resident packets (qgsw_raytrace.m:143-150,
+ * SW_zero_background_raytracing.m:73-78) in one call, the step-size controller on the device: the decisions of
+ * reference_api.ode23 (MATLAB's ode23 with MaxStep 0.1*|tf - t0|).  alpha = t/tmax (tmax = 0: steady flow, slot 0).
+ * ntspan >= 2; when ntspan > 2, Y (ntspan x 4 x n, host, may be NULL) receives the state at every tspan entry (ntrp23
+ * dense output).  stats[0..3] = accepted steps, rejected steps, RHS evaluations, host waits.  h_trace (may be NULL)
+ * receives up to h_cap accepted step sizes.  SWRT_ERR_STATE when the step size falls below 16*eps(t) (a packet blew
+ * up; the message names t); the packets are then those of the last accepted step.                               */
+int swrt_ode23(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol, double* Y,
+               int64_t stats[4], double* h_trace, int h_cap);
 
 /* ---- diagnostics -------------------------------------------------------------------------- */
 /* histcounts(omega, edges) (analysis/load_data.m:39-47): counts[nedges-1], bin i = [e_i,e_i+1),

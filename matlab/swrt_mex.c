@@ -296,6 +296,16 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         need(nrhs, 4, "'bs23_interp', h, hstep, s");
         double* o[4]; for (int i = 0; i < 4; i++) o[i] = outv(plhs, i, n);
         if (swrt_bs23_interp(h, mxGetScalar(prhs[2]), mxGetScalar(prhs[3]), o[0], o[1], o[2], o[3])) fail(h, cmd);
+    } else if (!strcmp(cmd, "ode23")) {               /* [stats, Y] = (h, tspan, tmax, rtol, atol)  -- whole solve, controller on the device */
+        need(nrhs, 6, "'ode23', h, tspan, tmax, rtol, atol");
+        int nt = (int)mxGetNumberOfElements(prhs[2]);
+        int64_t st[4];
+        double* Y = NULL;
+        if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix((size_t)n, nt > 2 ? (size_t)4 * nt : 0, mxREAL); if (nt > 2) Y = mxGetPr(plhs[1]); }
+        /* Y is n x (4*numel(tspan)): reshape(Y, n, 4, []) gives the state [x y k l] of every packet at every tspan entry */
+        if (swrt_ode23(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), Y, st, NULL, 0)) fail(h, cmd);
+        plhs[0] = mxCreateDoubleMatrix(1, 4, mxREAL);
+        for (int i = 0; i < 4; i++) mxGetPr(plhs[0])[i] = (double)st[i];
     } else if (!strcmp(cmd, "hist_omega")) {          /* counts = (h, kind, alpha, edges) */
         need(nrhs, 5, "'hist_omega', h, kind, alpha, edges");
         int ne = (int)mxGetNumberOfElements(prhs[4]);

@@ -17,10 +17,8 @@ __global__ void fill_kernel(double* p, double v, long long n) {
 // odefun: dxdt = U + Cg*k/sqrt(f^2 + Cg^2 |k|^2), dkdt = -(grad U)^T k
 struct E6 { const double* p[6]; };
 // cgfac = Cg (qgsw_raytrace.m:262) or gH (SW_zero_background_raytracing.m:182-184)
-__global__ void rhs_kernel(long long n, const double* __restrict__ k, const double* __restrict__ l, E6 e, double f,
-                           double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+__device__ __forceinline__ void rhs_at(long long i, const double* __restrict__ k, const double* __restrict__ l, const E6& e,
+                                       double f, double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt) {
     const double kk = k[i], ll = l[i];
     // every product and sum rounded on its own (no FMA contraction): with the LAGRANGE6 evaluation in front, odefun is then
     // the reference's double arithmetic operation for operation (qgsw_raytrace.m:262-263)
@@ -29,6 +27,18 @@ __global__ void rhs_kernel(long long n, const double* __restrict__ k, const doub
     if (dydt) dydt[i] = __dadd_rn(e.p[1][i], __dmul_rn(cgfac, ll) / w);
     if (dkdt) dkdt[i] = -__dadd_rn(__dmul_rn(e.p[2][i], kk), __dmul_rn(e.p[4][i], ll));
     if (dldt) dldt[i] = -__dadd_rn(__dmul_rn(e.p[3][i], kk), __dmul_rn(e.p[5][i], ll));
+}
+__global__ void rhs_kernel(long long n, const double* __restrict__ k, const double* __restrict__ l, E6 e, double f,
+                           double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    rhs_at(i, k, l, e, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
+}
+__global__ void rhs_dev_kernel(const Ode23Ctl* ctl, long long n, const double* __restrict__ k, const double* __restrict__ l, E6 e,
+                               double f, double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || ode23_idle(ctl)) return;
+    rhs_at(i, k, l, e, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
 }
 
 __global__ void omega_kernel(long long n, const double* __restrict__ k, const double* __restrict__ l,
@@ -211,9 +221,7 @@ __global__ void diag_final_kernel(int nblocks, const double* __restrict__ part, 
 }
 // ---- Bogacki-Shampine 3(2) building blocks (MATLAB ode23, called by qgsw_raytrace.m:149) ----------
 // stage state: yt = y + h*(b1 f1 + b2 f2 + b3 f3) for the four components x,y,k,l
-__global__ void bs23_stage_kernel(Bs23Args a, double hb1, double hb2, double hb3) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n) return;
+__device__ __forceinline__ void bs23_stage_at(const Bs23Args& a, long long i, double hb1, double hb2, double hb3) {
 #pragma unroll
     for (int c = 0; c < 4; c++) {
         // y + f*hB(:,j), hB = h*B, accumulated column by column with every product and sum rounded on its own
@@ -223,9 +231,23 @@ __global__ void bs23_stage_kernel(Bs23Args a, double hb1, double hb2, double hb3
         a.yt[c][i] = __dadd_rn(a.y[c][i], acc);
     }
 }
+__global__ void bs23_stage_kernel(Bs23Args a, double hb1, double hb2, double hb3) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    bs23_stage_at(a, i, hb1, hb2, hb3);
+}
+// the same stages with h from the controller: hB(:,stage) as swrt_bs23_attempt forms it on the host
+__global__ void bs23_stage_dev_kernel(Bs23Args a, const Ode23Ctl* ctl, int stage) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n || ode23_idle(ctl)) return;
+    const double h = ctl->h;
+    if (stage == 0) bs23_stage_at(a, i, __dmul_rn(h, 0.5), 0.0, 0.0);
+    else if (stage == 1) bs23_stage_at(a, i, 0.0, __dmul_rn(h, 0.75), 0.0);
+    else bs23_stage_at(a, i, __dmul_rn(h, 2.0 / 9.0), __dmul_rn(h, 1.0 / 3.0), __dmul_rn(h, 4.0 / 9.0));
+}
 // err = max_i |(f*E)_i| / max(max(|y_i|,|ynew_i|), threshold)   (without the absh factor);
 // mode 1: rh = max_i |f1_i| / max(|y_i|, threshold) for the initial step size
-__global__ void __launch_bounds__(256) bs23_norm_kernel(Bs23Args a, int mode, double thr, unsigned long long* out) {
+__device__ __forceinline__ void bs23_norm_body(const Bs23Args& a, int mode, double thr, unsigned long long* out) {
     const double E1 = -5.0 / 72.0, E2 = 1.0 / 12.0, E3 = 1.0 / 9.0, E4 = -1.0 / 8.0;
     double m = 0.0;
     long long stride = (long long)gridDim.x * blockDim.x;
@@ -256,6 +278,13 @@ __global__ void __launch_bounds__(256) bs23_norm_kernel(Bs23Args a, int mode, do
         atomicMax(out, (unsigned long long)__double_as_longlong(v));     // non-negative doubles order like their bit patterns
     }
 }
+__global__ void __launch_bounds__(256) bs23_norm_kernel(Bs23Args a, int mode, double thr, unsigned long long* out) {
+    bs23_norm_body(a, mode, thr, out);
+}
+__global__ void __launch_bounds__(256) bs23_norm_dev_kernel(Bs23Args a, const Ode23Ctl* ctl, double thr, unsigned long long* out) {
+    if (ode23_idle(ctl)) return;
+    bs23_norm_body(a, 0, thr, out);
+}
 __global__ void bs23_accept_kernel(Bs23Args a) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n) return;
@@ -272,7 +301,145 @@ __global__ void bs23_interp_kernel(Bs23Args a, Bs23Interp q) {
         q.out[c][i] = __dadd_rn(a.y[c][i], __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(a.f[0][c][i], q.w[0]), __dmul_rn(a.f[1][c][i], q.w[1])),
                                                                __dmul_rn(a.f[2][c][i], q.w[2])), __dmul_rn(a.f[3][c][i], q.w[3])));
 }
+
+// ---- swrt_ode23: the step-size controller of reference_api.ode23 in device memory ------------------------------------
+// Every scalar operation is rounded on its own, in the host controller's order; Python's min / max are restated with their
+// argument order (min(a, b) keeps a unless b < a), which decides what a NaN operand yields.
+__device__ __forceinline__ double py_min(double a, double b) { return b < a ? b : a; }
+__device__ __forceinline__ double py_max(double a, double b) { return b > a ? b : a; }
+__device__ __forceinline__ double eps16(double t) {          // 16 * eps(t) = 16 * np.spacing(abs(t))
+    t = fabs(t);
+    return __dmul_rn(16.0, __dsub_rn(nextafter(t, __longlong_as_double(0x7ff0000000000000LL)), t));
+}
+__device__ __forceinline__ double ode23_alpha(const Ode23Ctl* c, double tt) { return c->tmax != 0.0 ? __ddiv_rn(tt, c->tmax) : 0.0; }
+// the attempt from t with step h: tnew and the alphas of the three new RHS evaluations
+__device__ void ode23_set_attempt(Ode23Ctl* c) {
+    c->tnew = c->last ? c->tfinal : __dadd_rn(c->t, c->h);
+    c->al[0] = ode23_alpha(c, __dadd_rn(c->t, __dmul_rn(0.5, c->h)));
+    c->al[1] = ode23_alpha(c, __dadd_rn(c->t, __dmul_rn(0.75, c->h)));
+    c->al[2] = ode23_alpha(c, c->tnew);
+}
+// head of the host controller's outer loop: hmin, the MaxStep clamp and the 1.1 stretch onto tfinal
+__device__ void ode23_new_step(Ode23Ctl* c) {
+    c->hmin = eps16(c->t);
+    c->absh = py_min(c->hmax, py_max(c->hmin, c->absh));
+    c->h = c->absh;
+    c->last = 0;
+    if (__dmul_rn(1.1, c->absh) >= fabs(__dsub_rn(c->tfinal, c->t))) {
+        c->h = __dsub_rn(c->tfinal, c->t);
+        c->absh = fabs(c->h);
+        c->last = 1;
+    }
+    c->nofailed = 1;
+    ode23_set_attempt(c);
+}
+__device__ __forceinline__ double take_norm(unsigned long long* norm) {
+    const double v = __longlong_as_double((long long)*norm);
+    *norm = 0ull;                              // ready for the next attempt's atomicMax
+    return v;
+}
+// after f1 and the scale norm of swrt_bs23_begin: the initial step (rh, htspan rule, hmin) and the first attempt
+__global__ void ode23_init_kernel(Ode23Ctl* c, unsigned long long* norm) {
+    const double rh = __ddiv_rn(take_norm(norm), c->rh_den);
+    c->nfevals = 1;
+    c->hmin = eps16(c->t);
+    double absh = py_min(c->hmax, c->htspan);
+    if (__dmul_rn(absh, rh) > 1.0) absh = __ddiv_rn(1.0, rh);
+    c->absh = py_max(absh, c->hmin);
+    c->nxt = c->nxt_end = 1;
+    ode23_new_step(c);
+}
+// after an attempt's norm: accept or reject, the next h and stage alphas; the dense rows the accepted step passes
+__global__ void ode23_control_kernel(Ode23Ctl* c, unsigned long long* norm) {
+    const double nrm = take_norm(norm);
+    c->accepted = 0;
+    c->nxt = c->nxt_end;
+    if (c->done || c->status) return;
+    const double err = __dmul_rn(c->absh, nrm);
+    c->err = err;
+    c->nfevals += 3;
+    if (!(err <= c->rtol)) {                   // also catches NaN
+        c->nfailed++;
+        if (c->absh <= c->hmin) { c->status = 1; return; }
+        if (c->nofailed) {
+            c->nofailed = 0;
+            c->absh = isfinite(err) ? py_max(c->hmin, __dmul_rn(c->absh, py_max(0.5, __dmul_rn(0.8, pow_third(__ddiv_rn(c->rtol, err))))))
+                                    : py_max(c->hmin, __dmul_rn(0.5, c->absh));
+        } else {
+            c->absh = py_max(c->hmin, __dmul_rn(0.5, c->absh));
+        }
+        c->h = c->absh;
+        c->last = 0;
+        ode23_set_attempt(c);
+        return;
+    }
+    if (c->htrace && c->nsteps < c->hcap) c->htrace[c->nsteps] = c->h;
+    c->nsteps++;
+    c->accepted = 1;
+    c->t_acc = c->t; c->h_acc = c->h;
+    if (c->ntspan > 2) {
+        int j = c->nxt;
+        while (j < c->ntspan && __dsub_rn(c->tnew, c->tspan[j]) >= 0.0) j++;
+        c->nxt_end = j;
+    }
+    if (c->nofailed) {
+        const double temp = __dmul_rn(1.25, pow_third(__ddiv_rn(err, c->rtol)));
+        c->absh = temp > 0.2 ? __ddiv_rn(c->absh, temp) : __dmul_rn(5.0, c->absh);
+    }
+    c->t = c->tnew;
+    if (c->last) c->done = 1;
+    else ode23_new_step(c);
+}
+// ntrp23 rows of the accepted step: s == 1 gives ynew itself, the weights are formed as swrt_bs23_interp forms them
+__global__ void bs23_interp_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n || !ctl->accepted) return;
+    const double t0 = ctl->t_acc, h = ctl->h_acc, tnew = ctl->t;
+    for (int j = ctl->nxt; j < ctl->nxt_end; j++) {
+        const double tj = ctl->tspan[j];
+        const double s = tj == tnew ? 1.0 : __ddiv_rn(__dsub_rn(tj, t0), h);
+        double* row = ctl->yout + (size_t)j * 4 * a.n;
+        if (s == 1.0) {
+#pragma unroll
+            for (int c = 0; c < 4; c++) row[(size_t)c * a.n + i] = a.yt[c][i];
+            continue;
+        }
+        const double s2 = __dmul_rn(s, s), s3 = __dmul_rn(s2, s);
+        const double w0 = __dmul_rn(h, __dadd_rn(__dsub_rn(s, __dmul_rn(4.0 / 3.0, s2)), __dmul_rn(5.0 / 9.0, s3)));
+        const double w1 = __dmul_rn(h, __dsub_rn(s2, __dmul_rn(2.0 / 3.0, s3)));
+        const double w2 = __dmul_rn(h, __dsub_rn(__dmul_rn(4.0 / 3.0, s2), __dmul_rn(8.0 / 9.0, s3)));
+        const double w3 = __dmul_rn(h, __dadd_rn(-s2, s3));
+#pragma unroll
+        for (int c = 0; c < 4; c++)
+            row[(size_t)c * a.n + i] = __dadd_rn(a.y[c][i], __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(a.f[0][c][i], w0), __dmul_rn(a.f[1][c][i], w1)),
+                                                                             __dmul_rn(a.f[2][c][i], w2)), __dmul_rn(a.f[3][c][i], w3)));
+    }
+}
+// y <- ynew, f1 <- f4 (first same as last), predicated on the controller's decision
+__global__ void bs23_accept_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n || !ctl->accepted) return;
+#pragma unroll
+    for (int c = 0; c < 4; c++) { a.y[c][i] = a.yt[c][i]; a.f[0][c][i] = a.f[3][c][i]; }
+}
 }  // namespace
+
+// x^p with p = 1/3 rounded to double, correctly rounded (ties aside), which is what glibc's pow returns in all but
+// vanishingly rare cases: CUDA's pow (2 ulp) gives the candidates, and the one whose cube lies nearest to x^(3p) in
+// double-double arithmetic wins.  3p = 1 - 2^-54 exactly, so x^(3p) = x - 2^-54 x ln(x) to far below an ulp.
+__host__ __device__ double pow_third(double x) {
+    const double r = pow(x, 1.0 / 3.0);
+    if (!(x > 0.0) || !isfinite(x) || !isfinite(r) || r == 0.0) return r;
+    const double Xl = -(x * log(x)) * 0x1p-54;
+    double c = nextafter(nextafter(r, 0.0), 0.0), best = r, bestd = -1.0;
+    for (int q = 0; q < 5; q++, c = nextafter(c, 2.0 * c)) {
+        const double c2 = c * c, c2l = fma(c, c, -c2);
+        const double c3 = c2 * c, c3l = fma(c2, c, -c3) + c2l * c;
+        const double d = fabs((c3 - x) + (c3l - Xl));          // c3 - x is exact (Sterbenz)
+        if (bestd < 0.0 || d < bestd) { bestd = d; best = c; }
+    }
+    return best;
+}
 
 void launch_bs23_interp(const Bs23Args& a, const double w[4], double* const out[4], cudaStream_t st) {
     Bs23Interp q;
@@ -291,6 +458,29 @@ void launch_bs23_norm(const Bs23Args& a, int mode, double thr, unsigned long lon
 }
 void launch_bs23_accept(const Bs23Args& a, cudaStream_t st) {
     if (a.n > 0) bs23_accept_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a);
+}
+void launch_bs23_stage_dev(const Bs23Args& a, const Ode23Ctl* ctl, int stage, cudaStream_t st) {
+    if (a.n > 0) bs23_stage_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl, stage);
+}
+void launch_rhs_dev(const Ode23Ctl* ctl, long long n, const double* k, const double* l, const double* const* e6, double f,
+                    double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt, cudaStream_t st) {
+    E6 e; for (int i = 0; i < 6; i++) e.p[i] = e6[i];
+    if (n > 0) rhs_dev_kernel<<<nblk(n, 256), 256, 0, st>>>(ctl, n, k, l, e, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
+}
+// the norm word is zeroed by the controller kernel that consumes it (and by swrt_bs23_begin's launch before the solve)
+void launch_bs23_norm_dev(const Bs23Args& a, const Ode23Ctl* ctl, double thr, unsigned long long* out, cudaStream_t st) {
+    if (a.n <= 0) return;
+    unsigned nb = nblk(a.n, 256 * 4);
+    if (nb > 148 * 8) nb = 148 * 8;
+    bs23_norm_dev_kernel<<<nb, 256, 0, st>>>(a, ctl, thr, out);
+}
+void launch_ode23_init(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st) { ode23_init_kernel<<<1, 1, 0, st>>>(ctl, norm); }
+void launch_ode23_control(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st) { ode23_control_kernel<<<1, 1, 0, st>>>(ctl, norm); }
+void launch_bs23_interp_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st) {
+    if (a.n > 0) bs23_interp_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl);
+}
+void launch_bs23_accept_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st) {
+    if (a.n > 0) bs23_accept_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl);
 }
 
 void launch_fill(double* p, double v, long long n, cudaStream_t st) {

@@ -160,6 +160,28 @@ __global__ void __launch_bounds__(kBlock) nufft_eval_kernel(const NufftArgs a) {
     }
 }
 
+// swrt_ode23's evaluation of the six planes: the fine grid active_nufft_grid picks for the controller's alpha (frame 0,
+// frame 1 or the blend that axpby_dev_kernel wrote); nothing to do once the solve is done
+__global__ void __launch_bounds__(kBlock) nufft_eval_dev_kernel(const NufftArgs a, const Ode23Sel sel) {
+    if (ode23_idle(sel.ctl)) return;
+    const double al = sel.ctl->al[sel.stage];
+    const double2* grid = a.grid;
+    if (al == 1.0 && sel.frame1) grid = static_cast<const double2*>(sel.frame1);
+    else if (al != 0.0 && sel.blend) grid = static_cast<const double2*>(sel.blend);
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long p = t >> LPP_SHIFT;
+    const int lane = threadIdx.x & 31, q = lane & (LPP - 1), qb = lane & ~(LPP - 1);
+    const long long pc = p < a.n ? p : a.n - 1;
+    double F[7];
+    nufft_eval6<false>(grid, nullptr, a.nf, a.beta, a.dscale, reduced_coord(a.xin[pc], a.dx, a.nxd),
+                       reduced_coord(a.yin[pc], a.dx, a.nxd), q, qb, F);
+    if (p < a.n && q == 0) {
+#pragma unroll
+        for (int c = 0; c < 6; c++)
+            if (a.out[c]) a.out[c][p] = F[c];
+    }
+}
+
 // ode_symplectic.m:13-21,33-37 with the six planes from the NUFFT evaluation at x1
 #ifndef SWRT_NUFFT_MINB
 #define SWRT_NUFFT_MINB 5     /* 96 registers: 4 / 5 / 6 / 8 blocks per SM give 1.75 / 1.84 / 1.70 / 1.15e9 packet-steps/s at C3 */
@@ -314,6 +336,11 @@ cudaError_t launch_nufft_eval(const NufftArgs& a, cudaStream_t st) {
     if (a.n <= 0) return cudaSuccess;
     if (a.hgrid) nufft_eval_kernel<true><<<(unsigned)(((long long)LPP * a.n + kBlock - 1) / kBlock), kBlock, 0, st>>>(a);
     else nufft_eval_kernel<false><<<(unsigned)(((long long)LPP * a.n + kBlock - 1) / kBlock), kBlock, 0, st>>>(a);
+    return cudaGetLastError();
+}
+cudaError_t launch_nufft_eval_dev(const NufftArgs& a, const Ode23Sel& sel, cudaStream_t st) {
+    if (a.n <= 0) return cudaSuccess;
+    nufft_eval_dev_kernel<<<(unsigned)(((long long)LPP * a.n + kBlock - 1) / kBlock), kBlock, 0, st>>>(a, sel);
     return cudaGetLastError();
 }
 cudaError_t launch_nufft_leapfrog(const NufftArgs& a, cudaStream_t st) {

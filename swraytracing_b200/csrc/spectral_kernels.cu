@@ -160,6 +160,24 @@ void launch_axpby_multi(double* out, const double* a, const double* b, double al
     if (nb > 148 * 16) nb = 148 * 16;
     axpby_multi_kernel<<<(unsigned)nb, bs, 0, st>>>(out, a, b, alpha0, dalpha, j0, m, n);
 }
+// the blend above at the ode23 controller's alpha (weights 1 - al, al as the host forms them); alpha 0 and 1 read a frame
+// directly (as active_stack does), so nothing is blended then, nor once the solve is done
+__global__ void axpby_dev_kernel(double* __restrict__ out, const double* __restrict__ a, const double* __restrict__ b,
+                                 const Ode23Ctl* ctl, int stage, size_t n) {
+    if (ode23_idle(ctl)) return;
+    const double al = ctl->al[stage];
+    if (al == 0.0 || al == 1.0) return;
+    const double wa = __dsub_rn(1.0, al);
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    size_t stride = (size_t)gridDim.x * blockDim.x;
+    for (; i < n; i += stride) out[i] = fma(wa, a[i], __dmul_rn(al, b[i]));
+}
+void launch_axpby_dev(double* out, const double* a, const double* b, const Ode23Ctl* ctl, int stage, size_t n, cudaStream_t st) {
+    int bs = 256;
+    size_t nb = (n + bs - 1) / bs;
+    if (nb > 148 * 16) nb = 148 * 16;
+    axpby_dev_kernel<<<(unsigned)nb, bs, 0, st>>>(out, a, b, ctl, stage, n);
+}
 void launch_axpby(double* out, const double* a, const double* b, double wa, double wb, size_t n, cudaStream_t st) {
     int bs = 256;
     size_t nb = (n + bs - 1) / bs;
@@ -288,7 +306,7 @@ __device__ __forceinline__ void stage2_pass(const double (&acc)[NPL * G][2], Cpl
 }
 
 // quad reduction (the 4 lanes of a quad hold 4 interleaved ky subsets) and, for psi-hat stacks, the six planes
-template <bool PSI, int NPL, int NF>
+template <bool PSI, int NPL, int NF, bool DEV = false>
 __device__ __forceinline__ void finish_planes(double (&F)[NF], const SpecArgs& a, int ev) {
 #pragma unroll
     for (int c = 0; c < (PSI ? 5 : NPL); c++) {
@@ -300,7 +318,7 @@ __device__ __forceinline__ void finish_planes(double (&F)[NF], const SpecArgs& a
     if constexpr (PSI) {
         const double kap = a.kappa, kap2 = a.kappa * a.kappa;
         // mean shear of the blended frame (grid_U.m:11; interpolate_U.m:19-23), every rounding pinned
-        const double al = __dadd_rn(a.alpha0, __dmul_rn((double)(a.j0 + ev), a.dalpha));
+        const double al = DEV ? a.sel.ctl->al[a.sel.stage] : __dadd_rn(a.alpha0, __dmul_rn((double)(a.j0 + ev), a.dalpha));
         const double um = __dadd_rn(__dmul_rn(__dsub_rn(1.0, al), a.u_mean0), __dmul_rn(al, a.u_mean1));
         F[0] = fma(kap, F[0], um);
         F[1] = kap * F[1];
@@ -371,6 +389,14 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     const long long nrows = ANC ? 4 * nocc : a.n;
     const long long ntiles = (nrows + TILE_P - 1) / TILE_P;
     const int nevals = (MODE == SPEC_LEAPFROG) ? a.nsteps : 1;
+    // SPEC_EVAL_DEV (swrt_ode23): the stack the host would pick for the controller's alpha; nothing to do once it is done
+    const double* stack = a.stack;
+    if constexpr (MODE == SPEC_EVAL_DEV) {
+        if (ode23_idle(a.sel.ctl)) return;
+        const double al = a.sel.ctl->al[a.sel.stage];
+        if (al == 1.0 && a.sel.frame1) stack = static_cast<const double*>(a.sel.frame1);
+        else if (al != 0.0 && a.sel.blend) stack = static_cast<const double*>(a.sel.blend);
+    }
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < nstages; s++) {
@@ -405,7 +431,7 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     auto producer_issue = [&]() {          // lane 0 only; issues chunk pj
         if (p_it > 0) mbar_wait(&empty_bar[p_st], (uint32_t)((p_it - 1) & 1));
         mbar_expect_tx(&full_bar[p_st], chunk_bytes);
-        bulk_g2s(smem_raw + (size_t)p_st * chunk_bytes, a.stack + (size_t)p_src * g.chunk_doubles, chunk_bytes, &full_bar[p_st]);
+        bulk_g2s(smem_raw + (size_t)p_st * chunk_bytes, stack + (size_t)p_src * g.chunk_doubles, chunk_bytes, &full_bar[p_st]);
     };
     auto producer_advance = [&]() {        // all lanes (uniform): pj += kConsumerWarps
         pj += kConsumerWarps;
@@ -663,7 +689,7 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
             else {
             // ---- quad reduction: the 4 lanes of a quad hold 4 interleaved ky subsets ----------
 #pragma unroll
-            for (int mt = 0; mt < MT; mt++) finish_planes<PSI, NPL, NF>(F[mt], a, ev);
+            for (int mt = 0; mt < MT; mt++) finish_planes<PSI, NPL, NF, MODE == SPEC_EVAL_DEV>(F[mt], a, ev);
             if (MODE == SPEC_LEAPFROG) {
                 if constexpr (NF >= 6) {
 #pragma unroll
@@ -733,6 +759,13 @@ static cudaError_t dispatch_mode(const SpecArgs& a, int mode, int num_sms, cudaS
         else return cudaErrorInvalidValue;
     }
     return launch_inst<NPL, G, MT, SPEC_EVAL, false>(a, num_sms, st);
+}
+
+// swrt_ode23's evaluations: the six planes (or the psi-hat moment planes) with one m-tile, alpha from the controller
+cudaError_t launch_spectral_eval_dev(const SpecArgs& a, int num_sms, cudaStream_t st) {
+    if (a.psi && a.g.npl == 3 && a.g.G == 8) return launch_inst<3, 8, 1, SPEC_EVAL_DEV, true>(a, num_sms, st);
+    if (!a.psi && a.g.npl == 6 && a.g.G == 4) return launch_inst<6, 4, 1, SPEC_EVAL_DEV, false>(a, num_sms, st);
+    return cudaErrorInvalidValue;
 }
 
 cudaError_t launch_spectral(const SpecArgs& a, int mode, int mtiles, int num_sms, cudaStream_t st) {

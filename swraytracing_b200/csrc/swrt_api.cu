@@ -84,6 +84,9 @@ struct swrt_handle {
     double* bs_f[4][4] = {};
     unsigned long long* bs_norm_dev = nullptr;
     bool bs_ready = false;
+    Ode23Ctl* ode_ctl = nullptr;          // swrt_ode23: the controller state on the device ...
+    Ode23Ctl* ode_host = nullptr;         // ... and its pinned host image (set-up and read-back)
+    cudaEvent_t ode_ev = nullptr;
     double* edges_dev = nullptr; int edges_cap = 0;
     std::vector<double> edges_host;       // what edges_dev currently holds
     unsigned long long* counts_dev = nullptr; int counts_cap = 0;
@@ -698,6 +701,9 @@ int swrt_destroy(swrt_handle* h) {
     dfree(h->diag_dev); dfree(h->edges_dev); dfree(h->counts_dev); dfree(h->bs_norm_dev);
     for (auto& p : h->bs_yt) dfree(p);
     for (auto& row : h->bs_f) for (auto& p : row) dfree(p);
+    dfree(h->ode_ctl);
+    if (h->ode_host) cudaFreeHost(h->ode_host);
+    if (h->ode_ev) cudaEventDestroy(h->ode_ev);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
     if (h->hist_ev) cudaEventDestroy(h->hist_ev);
@@ -1910,3 +1916,4 @@ int swrt_spectral_geometry(int nx, int nplanes, int mtiles, int64_t out[10]) {
 }  // extern "C"
 
 #include "swrt_group.inc"     // multi-device handles: sharding + in-library NCCL
+#include "swrt_ode23.inc"     // swrt_ode23: a whole ode23 solve with the controller on the device

@@ -44,6 +44,40 @@ struct PackGeom {
     int plane_ids[kMaxPlanes];   // which of the 7 source planes each stack plane is
 };
 
+// ---------------------------------------------------------------------------------------------
+// swrt_ode23: a whole ode23 solve with the step-size controller in device memory (DESIGN.md section 11).  The stage,
+// evaluation, norm, interp and accept kernels of an attempt read h, the stage alphas and `done` from here; a single-thread
+// controller kernel after each attempt's norm makes reference_api.ode23's decisions.  Queued attempts after the last
+// one (or after a failure) exit at once.
+// ---------------------------------------------------------------------------------------------
+struct Ode23Ctl {
+    // per solve (set by the host before the first attempt)
+    double tfinal, rtol, hmax, tmax, rh_den, htspan;   // rh_den = 0.8 * rtol^(1/3); htspan = |tspan(2) - tspan(1)|
+    const double* tspan; int ntspan;                   // device copy of tspan (dense output when ntspan > 2)
+    double* yout;                                      // ntspan x 4 x n rows (dense output) or null
+    double* htrace; int hcap;                          // accepted step sizes (optional)
+    // controller state
+    double t, absh, h, tnew, hmin, err;
+    double al[3];                                      // RHS alphas of stages 2..4 (t + h/2, t + 3h/4, tnew)
+    double t_acc, h_acc;                               // t and h of the attempt just accepted (dense output)
+    int last;                                          // this attempt lands on tfinal (the host controller's `done`)
+    int nofailed;
+    int accepted;                                      // the attempt just decided was accepted: interp and accept run
+    int done;                                          // the solve is complete
+    int status;                                        // 0, or 1 = step size below hmin (t holds where)
+    int nxt, nxt_end;                                  // dense rows [nxt, nxt_end) are written after this attempt
+    long long nsteps, nfailed, nfevals;
+};
+// a pointer-argument evaluation: the frame is chosen on the device from ctl->al[stage] as the host picks it for a value
+// alpha (alpha == 0: frame 0, alpha == 1: frame 1, else the blend); frame1 / blend may be null for a steady flow
+struct Ode23Sel {
+    const Ode23Ctl* ctl;
+    int stage;
+    const void* frame1;
+    const void* blend;
+};
+__device__ __forceinline__ bool ode23_idle(const Ode23Ctl* c) { return c->done || c->status; }
+
 PackGeom make_geom(int nx, int npl, const int* plane_ids, int mtiles, int twiddle_pref = 0);
 
 // one source slot: complex planes on the device, [plane][ky][kx+kmax] as double2 (kx fastest)
@@ -91,9 +125,10 @@ struct SpecArgs {
     double anc_h;                         // anchor cell width in the reduced coordinate t of reduced_turns (t in [0, 2))
     double zscale;                        // pi * kmax: z = zscale * (t - t_anchor)
     int ev;                               // anchored_step_kernel: sub-step index j of the run (mean-shear blend weight)
+    Ode23Sel sel;                         // SPEC_EVAL_DEV: stack and alpha chosen from the ode23 controller
 };
 
-enum SpecMode { SPEC_EVAL = 0, SPEC_LEAPFROG = 1, SPEC_ANCHOR = 2 };
+enum SpecMode { SPEC_EVAL = 0, SPEC_LEAPFROG = 1, SPEC_ANCHOR = 2, SPEC_EVAL_DEV = 3 };
 
 // anchored leapfrog: expansion order, anchor geometry and the kernels around K1 (SPEC_ANCHOR) and K2
 constexpr int kAnchorOrders = 8;        // R: Taylor orders of e^{i kx delta} kept per anchor (two DMMA k-steps)
@@ -225,5 +260,22 @@ void launch_bs23_stage(const Bs23Args& a, double hb1, double hb2, double hb3, cu
 void launch_bs23_norm(const Bs23Args& a, int mode, double thr, unsigned long long* out, cudaStream_t st);
 void launch_bs23_accept(const Bs23Args& a, cudaStream_t st);
 void launch_bs23_interp(const Bs23Args& a, const double w[4], double* const out[4], cudaStream_t st);
+
+
+void launch_bs23_stage_dev(const Bs23Args& a, const Ode23Ctl* ctl, int stage, cudaStream_t st);
+void launch_rhs_dev(const Ode23Ctl* ctl, long long n, const double* k, const double* l, const double* const* e6, double f,
+                    double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt, cudaStream_t st);
+void launch_bs23_norm_dev(const Bs23Args& a, const Ode23Ctl* ctl, double thr, unsigned long long* out, cudaStream_t st);
+void launch_ode23_init(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st);
+void launch_ode23_control(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st);
+void launch_bs23_interp_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st);
+void launch_bs23_accept_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st);
+// out = (1 - al)*a + al*b with al = ctl->al[stage], skipped when al is 0 or 1 (the evaluation then reads a frame itself)
+void launch_axpby_dev(double* out, const double* a, const double* b, const Ode23Ctl* ctl, int stage, size_t n, cudaStream_t st);
+cudaError_t launch_spectral_eval_dev(const SpecArgs& a, int num_sms, cudaStream_t st);     // a.sel set
+cudaError_t launch_nufft_eval_dev(const NufftArgs& a, const Ode23Sel& sel, cudaStream_t st);
+cudaError_t launch_lagrange_eval_dev(const LagArgs& a, const Ode23Ctl* ctl, int stage, cudaStream_t st);
+// (rtol/err)^(1/3) as glibc's correctly rounded-in-practice pow gives it (host and device, misc_kernels.cu)
+__host__ __device__ double pow_third(double x);
 
 }  // namespace swrt

@@ -50,8 +50,9 @@ def initial_q(X, Y, a_g, K_d2, rs, k_min=5, k_max=8, ring=False):
 def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_days, U_g, f, Cg, *, outdir="data",
                   integrator="ode23", mode=MODE_SPECTRAL, r_drag=0.1, beta=0.0, force_strength=0.1, max_steps=None,
                   seed=146, device=0, log=print, leapfrog_substeps=4):
-    """qgsw_raytrace.m:1-180 on the device.  ``integrator``: 'ode23' (the reference) or 'leapfrog' (the fused
-    symplectic stepper with time-centred frame blending).  ``max_steps`` truncates the run (tests)."""
+    """qgsw_raytrace.m:1-180 on the device.  ``integrator``: 'ode23' (the reference), 'ode23_device' (the same solve
+    with the controller on the device, swrt_ode23) or 'leapfrog' (the fused symplectic stepper with time-centred frame
+    blending).  ``max_steps`` truncates the run (tests)."""
     L = 2 * np.pi
     dx = L / nx
     xg = matlab_linspace(-L / 2, L / 2, nx)
@@ -111,8 +112,8 @@ def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_da
         t += dt
         if Npackets > 0 and t > packet_delay:
             qg.to_flow(eng, 1)                                         # background_flow2 = grid_U(qk), :142
-            if integrator == "ode23":
-                st = ode23(eng, [0.0, dt], dt)                         # :143-150
+            if integrator in ("ode23", "ode23_device"):
+                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device")      # :143-150
                 stats["ode23_steps"] += st["nsteps"]; stats["ode23_failed"] += st["nfailed"]
             else:
                 m = leapfrog_substeps
@@ -216,11 +217,12 @@ def symplectic_full_fourier(q=None, *, nx=None, f=None, Cg=None, run_log_file=No
 
 
 def SW_zero_background_raytracing(q=None, *, nx=None, f=None, Cg=None, run_log_file=None, pv=None, frame=2000, Nparticles=10,
-                                  Tend=None, rtol=1e-6, atol=1e-7, mode=MODE_SPECTRAL, seed=123, device=0):
+                                  Tend=None, rtol=1e-6, atol=1e-7, mode=MODE_SPECTRAL, seed=123, device=0, integrator="ode23"):
     """SW_zero_background_raytracing.m:1-132 (BASELINE config 1): the same frozen frame and packet ring, integrated
     by ``ode23`` with RelTol 1e-6 / AbsTol 1e-7 and output requested at ``t_hist = dt*(0:Nsteps)`` (:70-78), RHS
     ``dx/dt = U + gH k/omega`` (:134-145,182-184).  ``q = zeros`` is the "zero background" of the file name
-    (the hint on :28-29).  Returns dict(t_hist, solver_x, solver_k, solver_error, w, Omega_0, U0, Fr, dt, stats)."""
+    (the hint on :28-29).  ``integrator='ode23_device'`` runs the solve with the controller on the device (swrt_ode23).
+    Returns dict(t_hist, solver_x, solver_k, solver_error, w, Omega_0, U0, Fr, dt, stats)."""
     from .engine import FLAG_RHS_GH
     from .reference_api import ode23
     if run_log_file is not None:
@@ -242,7 +244,7 @@ def SW_zero_background_raytracing(q=None, *, nx=None, f=None, Cg=None, run_log_f
     eng = Engine(nx, L, f, gH, mode, device, flags=FLAG_RHS_GH)
     eng.set_flow_spectral(scheme.psik)
     eng.set_packets(x[0, 0], x[0, 1], k[0, 0], k[0, 1])
-    stats = ode23(eng, t_hist, None, rtol=rtol, atol=atol)             # steady flow: one slot, alpha = 0
+    stats = ode23(eng, t_hist, None, rtol=rtol, atol=atol, on_device=integrator == "ode23_device")   # steady flow: slot 0
     Y = stats.pop("Y")
     eng.close()
     solver_x, solver_k = Y[:, 0:2, :], Y[:, 2:4, :]
@@ -383,7 +385,8 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
                         leapfrog_substeps=4):
     """qg_flow_ray_trace/qg2layersw_raytrace.m:1-247 (BASELINE config 4) on the device: two-layer QG with mean shear on
     L = 20, adaptive dt (:156-165), AB3 + integrating factor, packets advected through the TOP layer's
-    ``grid_U`` frames (:187-196) by ode23 over [0, dt], packet frames every 25 steps.  ``k_max`` (30 in the reference)
+    ``grid_U`` frames (:187-196) by ode23 over [0, dt] ('ode23_device': controller on the device), packet frames every
+    25 steps.  ``k_max`` (30 in the reference)
     and ``max_steps`` exist for tests."""
     L = 20.0
     dx = L / nx
@@ -452,8 +455,8 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
         t = t + dt
         if advect:
             qg.to_flow(eng, 1)                                         # background_flow2 = grid_U(qk(:,:,:,1)), :188
-            if integrator == "ode23":
-                st = ode23(eng, [0.0, dt], dt)
+            if integrator in ("ode23", "ode23_device"):
+                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device")
                 stats["ode23_steps"] += st["nsteps"]; stats["ode23_failed"] += st["nfailed"]
             else:
                 m = leapfrog_substeps

@@ -63,6 +63,7 @@ SIGNATURES = {
     "swrt_bs23_attempt": (C.c_int, [C.c_void_p, C.c_double, _dp, C.c_double, _dp]),
     "swrt_bs23_accept": (C.c_int, [C.c_void_p]),
     "swrt_bs23_interp": (C.c_int, [C.c_void_p, C.c_double, C.c_double] + [_dp] * 4),
+    "swrt_ode23": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int64), _dp, C.c_int]),
     "swrt_hist_omega_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_launch": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_wait": (C.c_int, [C.c_void_p]),
@@ -329,6 +330,26 @@ class Engine:
         out = [np.empty(self.n) for _ in range(4)]
         self._check(self.lib.swrt_bs23_interp(self._h, float(hstep), float(s), *[_ptr(o) for o in out]))
         return tuple(out)
+
+    def ode23(self, tspan, tmax, rtol=1e-3, atol=1e-6, *, trace=0):
+        """a whole ``[~, Y] = ode23(ray_ode, tspan, y0)`` solve in one call (swrt_ode23): the decisions of
+        ``reference_api.ode23`` made by a controller in device memory, the host waiting a few times per solve instead of
+        twice per attempt.  ``tmax`` None / 0 = steady flow.  Returns the same dict as ``reference_api.ode23`` (``Y`` when
+        ``tspan`` has more than two entries) plus ``host_waits``, and ``h`` (the first ``trace`` accepted step sizes)
+        when ``trace`` > 0.  A step size below hmin raises SwrtError (SWRT_ERR_STATE) naming t."""
+        ts = _f64(tspan)
+        dense = ts.size > 2
+        Y = np.empty((ts.size, 4, self.n)) if dense else None
+        st = (C.c_int64 * 4)()
+        hs = np.empty(max(int(trace), 0))
+        self._check(self.lib.swrt_ode23(self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol),
+                                        _ptr(Y) if dense else None, st, _ptr(hs) if trace > 0 else None, int(hs.size)))
+        out = {"nsteps": st[0], "nfailed": st[1], "nfevals": st[2], "t": float(ts[-1]), "host_waits": st[3]}
+        if dense:
+            out["Y"] = Y
+        if trace > 0:
+            out["h"] = hs[:min(st[0], hs.size)].copy()
+        return out
 
     # -- diagnostics --
     def hist_omega(self, edges, kind=HIST_INTRINSIC, alpha=0.0, counts=None):

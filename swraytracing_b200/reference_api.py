@@ -297,7 +297,7 @@ def omega(k, f, gH):
 # ode23 -- the production drivers' integrator (qgsw_raytrace.m:149, qg2layersw_raytrace.m:195)
 # ------------------------------------------------------------------------------------------------
 
-def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None):
+def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=False):
     """``[~, Y] = ode23(ray_ode, [0 dt], y0)`` for the packets resident in ``target`` (an Engine):
     MATLAB's ode23 = Bogacki-Shampine 3(2) pair with first-same-as-last, restated from its published
     description (Shampine & Reichelt, "The MATLAB ODE Suite", SIAM J. Sci. Comput. 18, 1997; MATLAB
@@ -315,7 +315,12 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None):
     ``min(hmax, |tspan(2)-tspan(1)|, 1/rh)``, which for a dense ``tspan`` is bounded by the first output interval.
 
     One deliberate deviation: a non-finite error estimate (a packet that blew up) REJECTS the step here and, at ``hmin``,
-    raises; MATLAB's ``if err > rtol`` is false for NaN, so it would accept the step and carry NaNs on silently."""
+    raises; MATLAB's ``if err > rtol`` is false for NaN, so it would accept the step and carry NaNs on silently.
+
+    ``on_device=True`` (single-process callers, no ``reduce_max``) runs the same solve as one ``Engine.ode23`` call, the
+    controller in device memory (swrt_ode23); the returned dict then also holds ``host_waits``."""
+    if on_device and reduce_max is None:
+        return target.ode23(tspan, tmax, rtol, atol)
     red = reduce_max if reduce_max is not None else (lambda v: v)
     al = (lambda tt: tt / tmax) if tmax else (lambda tt: 0.0)       # tmax=None: steady flow, slot 0 only
     tspan = np.asarray(tspan, dtype=np.float64)
