@@ -171,6 +171,16 @@ int swrt_bs23_interp(swrt_handle* h, double hstep, double s, double* x, double* 
  * up; the message names t); the packets are then those of the last accepted step.                               */
 int swrt_ode23(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol, double* Y,
                int64_t stats[4], double* h_trace, int h_cap);
+/* [~, Y] = ode23(odefun_i, tspan, y_i) for every packet i on its own: packet i advances exactly as swrt_ode23 advances an
+ * ensemble holding packet i alone (its own error norm, initial step, rejections and dense output), so a packet's result
+ * does not depend on the other packets, their number or the sharding.  Y as in swrt_ode23 (ntspan x 4 x n, may be NULL;
+ * the rows after a stopped packet's t_end are NaN).
+ * pstat (may be NULL): n x 3 int32, column-major = accepted steps, rejected steps, status (0 reached tfinal, 1 step size
+ * fell below 16*eps(t)); t_end (may be NULL): tfinal, or the t at which the packet stopped (it keeps its last accepted
+ * state).  stats[0..4] = accepted steps, rejected steps and RHS evaluations summed over packets, packets that stopped,
+ * host waits.  A stopped packet is not an error: SWRT_OK is returned.                                               */
+int swrt_ode23_packets(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol, double* Y,
+                       int32_t* pstat, double* t_end, int64_t stats[5]);
 
 /* ---- diagnostics -------------------------------------------------------------------------- */
 /* histcounts(omega, edges) (analysis/load_data.m:39-47): counts[nedges-1], bin i = [e_i,e_i+1),

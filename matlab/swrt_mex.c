@@ -306,6 +306,24 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (swrt_ode23(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), Y, st, NULL, 0)) fail(h, cmd);
         plhs[0] = mxCreateDoubleMatrix(1, 4, mxREAL);
         for (int i = 0; i < 4; i++) mxGetPr(plhs[0])[i] = (double)st[i];
+    } else if (!strcmp(cmd, "ode23_packets")) {       /* [stats, Y, pstat, t_end] = (h, tspan, tmax, rtol, atol)  -- one controller per packet */
+        need(nrhs, 6, "'ode23_packets', h, tspan, tmax, rtol, atol");
+        int nt = (int)mxGetNumberOfElements(prhs[2]);
+        int64_t st[5];
+        double *Y = NULL, *t_end = NULL;
+        if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix((size_t)n, nt > 2 ? (size_t)4 * nt : 0, mxREAL); if (nt > 2) Y = mxGetPr(plhs[1]); }
+        /* pstat: n x 3 = accepted steps, rejected steps, status (0 reached tfinal, 1 stopped); t_end: n x 1 */
+        int32_t* ps = nlhs > 2 ? (int32_t*)mxCalloc((size_t)3 * (n > 0 ? n : 1), sizeof(int32_t)) : NULL;
+        if (nlhs > 3) t_end = outv(plhs, 3, n);
+        if (swrt_ode23_packets(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), Y, ps, t_end, st))
+            fail(h, cmd);
+        plhs[0] = mxCreateDoubleMatrix(1, 5, mxREAL);
+        for (int i = 0; i < 5; i++) mxGetPr(plhs[0])[i] = (double)st[i];
+        if (ps) {
+            plhs[2] = mxCreateDoubleMatrix((size_t)n, 3, mxREAL);
+            for (size_t i = 0; i < 3 * n; i++) mxGetPr(plhs[2])[i] = (double)ps[i];
+            mxFree(ps);
+        }
     } else if (!strcmp(cmd, "hist_omega")) {          /* counts = (h, kind, alpha, edges) */
         need(nrhs, 5, "'hist_omega', h, kind, alpha, edges");
         int ne = (int)mxGetNumberOfElements(prhs[4]);

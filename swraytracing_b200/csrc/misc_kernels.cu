@@ -237,34 +237,39 @@ __global__ void bs23_stage_kernel(Bs23Args a, double hb1, double hb2, double hb3
     bs23_stage_at(a, i, hb1, hb2, hb3);
 }
 // the same stages with h from the controller: hB(:,stage) as swrt_bs23_attempt forms it on the host
-__global__ void bs23_stage_dev_kernel(Bs23Args a, const Ode23Ctl* ctl, int stage) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n || ode23_idle(ctl)) return;
-    const double h = ctl->h;
+__device__ __forceinline__ void bs23_stage_h(const Bs23Args& a, long long i, int stage, double h) {
     if (stage == 0) bs23_stage_at(a, i, __dmul_rn(h, 0.5), 0.0, 0.0);
     else if (stage == 1) bs23_stage_at(a, i, 0.0, __dmul_rn(h, 0.75), 0.0);
     else bs23_stage_at(a, i, __dmul_rn(h, 2.0 / 9.0), __dmul_rn(h, 1.0 / 3.0), __dmul_rn(h, 4.0 / 9.0));
 }
+__global__ void bs23_stage_dev_kernel(Bs23Args a, const Ode23Ctl* ctl, int stage) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n || ode23_idle(ctl)) return;
+    bs23_stage_h(a, i, stage, ctl->h);
+}
 // err = max_i |(f*E)_i| / max(max(|y_i|,|ynew_i|), threshold)   (without the absh factor);
 // mode 1: rh = max_i |f1_i| / max(|y_i|, threshold) for the initial step size
-__device__ __forceinline__ void bs23_norm_body(const Bs23Args& a, int mode, double thr, unsigned long long* out) {
+// packet i's four ratios folded into the running max m
+__device__ __forceinline__ double bs23_norm_packet(const Bs23Args& a, long long i, int mode, double thr, double m) {
     const double E1 = -5.0 / 72.0, E2 = 1.0 / 12.0, E3 = 1.0 / 9.0, E4 = -1.0 / 8.0;
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        double num, den;
+        if (mode == 1) { num = fabs(a.f[0][c][i]); den = fmax(fabs(a.y[c][i]), thr); }
+        else {
+            num = fabs(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(a.f[0][c][i], E1), __dmul_rn(a.f[1][c][i], E2)),
+                                          __dmul_rn(a.f[2][c][i], E3)), __dmul_rn(a.f[3][c][i], E4)));
+            den = fmax(fmax(fabs(a.y[c][i]), fabs(a.yt[c][i])), thr);
+        }
+        const double r = num / den;
+        m = (r > m || r != r) ? r : m;              // NaN propagates (a blown-up packet fails the step)
+    }
+    return m;
+}
+__device__ __forceinline__ void bs23_norm_body(const Bs23Args& a, int mode, double thr, unsigned long long* out) {
     double m = 0.0;
     long long stride = (long long)gridDim.x * blockDim.x;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += stride) {
-#pragma unroll
-        for (int c = 0; c < 4; c++) {
-            double num, den;
-            if (mode == 1) { num = fabs(a.f[0][c][i]); den = fmax(fabs(a.y[c][i]), thr); }
-            else {
-                num = fabs(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(a.f[0][c][i], E1), __dmul_rn(a.f[1][c][i], E2)),
-                                              __dmul_rn(a.f[2][c][i], E3)), __dmul_rn(a.f[3][c][i], E4)));
-                den = fmax(fmax(fabs(a.y[c][i]), fabs(a.yt[c][i])), thr);
-            }
-            const double r = num / den;
-            m = (r > m || r != r) ? r : m;          // NaN propagates (a blown-up packet fails the step)
-        }
-    }
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += stride) m = bs23_norm_packet(a, i, mode, thr, m);
     __shared__ double sh[256];
     sh[threadIdx.x] = m;
     __syncthreads();
@@ -311,94 +316,98 @@ __device__ __forceinline__ double eps16(double t) {          // 16 * eps(t) = 16
     t = fabs(t);
     return __dmul_rn(16.0, __dsub_rn(nextafter(t, __longlong_as_double(0x7ff0000000000000LL)), t));
 }
-__device__ __forceinline__ double ode23_alpha(const Ode23Ctl* c, double tt) { return c->tmax != 0.0 ? __ddiv_rn(tt, c->tmax) : 0.0; }
+__device__ __forceinline__ double ode23_alpha(const Ode23Ctl& c, double tt) { return c.tmax != 0.0 ? __ddiv_rn(tt, c.tmax) : 0.0; }
+// The rules below act on one controller state: swrt_ode23's Ode23Ctl in device memory, or a packet's state loaded into a
+// local Ode23Ctl by swrt_ode23_packets' kernels.  One copy of the rules keeps the two solves' decisions the same.
 // the attempt from t with step h: tnew and the alphas of the three new RHS evaluations
-__device__ void ode23_set_attempt(Ode23Ctl* c) {
-    c->tnew = c->last ? c->tfinal : __dadd_rn(c->t, c->h);
-    c->al[0] = ode23_alpha(c, __dadd_rn(c->t, __dmul_rn(0.5, c->h)));
-    c->al[1] = ode23_alpha(c, __dadd_rn(c->t, __dmul_rn(0.75, c->h)));
-    c->al[2] = ode23_alpha(c, c->tnew);
+__device__ __forceinline__ void ode23_set_attempt(Ode23Ctl& c) {
+    c.tnew = c.last ? c.tfinal : __dadd_rn(c.t, c.h);
+    c.al[0] = ode23_alpha(c, __dadd_rn(c.t, __dmul_rn(0.5, c.h)));
+    c.al[1] = ode23_alpha(c, __dadd_rn(c.t, __dmul_rn(0.75, c.h)));
+    c.al[2] = ode23_alpha(c, c.tnew);
 }
 // head of the host controller's outer loop: hmin, the MaxStep clamp and the 1.1 stretch onto tfinal
-__device__ void ode23_new_step(Ode23Ctl* c) {
-    c->hmin = eps16(c->t);
-    c->absh = py_min(c->hmax, py_max(c->hmin, c->absh));
-    c->h = c->absh;
-    c->last = 0;
-    if (__dmul_rn(1.1, c->absh) >= fabs(__dsub_rn(c->tfinal, c->t))) {
-        c->h = __dsub_rn(c->tfinal, c->t);
-        c->absh = fabs(c->h);
-        c->last = 1;
+__device__ __forceinline__ void ode23_new_step(Ode23Ctl& c) {
+    c.hmin = eps16(c.t);
+    c.absh = py_min(c.hmax, py_max(c.hmin, c.absh));
+    c.h = c.absh;
+    c.last = 0;
+    if (__dmul_rn(1.1, c.absh) >= fabs(__dsub_rn(c.tfinal, c.t))) {
+        c.h = __dsub_rn(c.tfinal, c.t);
+        c.absh = fabs(c.h);
+        c.last = 1;
     }
-    c->nofailed = 1;
+    c.nofailed = 1;
     ode23_set_attempt(c);
+}
+// after f1 and the scale norm: the initial step (rh, htspan rule, hmin) and the first attempt
+__device__ __forceinline__ void ode23_init(Ode23Ctl& c, double nrm) {
+    const double rh = __ddiv_rn(nrm, c.rh_den);
+    c.nfevals = 1;
+    c.hmin = eps16(c.t);
+    double absh = py_min(c.hmax, c.htspan);
+    if (__dmul_rn(absh, rh) > 1.0) absh = __ddiv_rn(1.0, rh);
+    c.absh = py_max(absh, c.hmin);
+    c.nxt = c.nxt_end = 1;
+    ode23_new_step(c);
+}
+// after an attempt's norm: accept or reject, the next h and stage alphas; the dense rows [nxt, nxt_end) the accepted
+// step passes
+__device__ __forceinline__ void ode23_control(Ode23Ctl& c, double nrm) {
+    c.accepted = 0;
+    c.nxt = c.nxt_end;
+    if (c.done || c.status) return;
+    const double err = __dmul_rn(c.absh, nrm);
+    c.err = err;
+    c.nfevals += 3;
+    if (!(err <= c.rtol)) {                    // also catches NaN
+        c.nfailed++;
+        if (c.absh <= c.hmin) { c.status = 1; return; }
+        if (c.nofailed) {
+            c.nofailed = 0;
+            c.absh = isfinite(err) ? py_max(c.hmin, __dmul_rn(c.absh, py_max(0.5, __dmul_rn(0.8, pow_third(__ddiv_rn(c.rtol, err))))))
+                                   : py_max(c.hmin, __dmul_rn(0.5, c.absh));
+        } else {
+            c.absh = py_max(c.hmin, __dmul_rn(0.5, c.absh));
+        }
+        c.h = c.absh;
+        c.last = 0;
+        ode23_set_attempt(c);
+        return;
+    }
+    if (c.htrace && c.nsteps < c.hcap) c.htrace[c.nsteps] = c.h;
+    c.nsteps++;
+    c.accepted = 1;
+    c.t_acc = c.t; c.h_acc = c.h;
+    if (c.ntspan > 2) {
+        int j = c.nxt;
+        while (j < c.ntspan && __dsub_rn(c.tnew, c.tspan[j]) >= 0.0) j++;
+        c.nxt_end = j;
+    }
+    if (c.nofailed) {
+        const double temp = __dmul_rn(1.25, pow_third(__ddiv_rn(err, c.rtol)));
+        c.absh = temp > 0.2 ? __ddiv_rn(c.absh, temp) : __dmul_rn(5.0, c.absh);
+    }
+    c.t = c.tnew;
+    if (c.last) c.done = 1;
+    else ode23_new_step(c);
 }
 __device__ __forceinline__ double take_norm(unsigned long long* norm) {
     const double v = __longlong_as_double((long long)*norm);
     *norm = 0ull;                              // ready for the next attempt's atomicMax
     return v;
 }
-// after f1 and the scale norm of swrt_bs23_begin: the initial step (rh, htspan rule, hmin) and the first attempt
-__global__ void ode23_init_kernel(Ode23Ctl* c, unsigned long long* norm) {
-    const double rh = __ddiv_rn(take_norm(norm), c->rh_den);
-    c->nfevals = 1;
-    c->hmin = eps16(c->t);
-    double absh = py_min(c->hmax, c->htspan);
-    if (__dmul_rn(absh, rh) > 1.0) absh = __ddiv_rn(1.0, rh);
-    c->absh = py_max(absh, c->hmin);
-    c->nxt = c->nxt_end = 1;
-    ode23_new_step(c);
-}
-// after an attempt's norm: accept or reject, the next h and stage alphas; the dense rows the accepted step passes
-__global__ void ode23_control_kernel(Ode23Ctl* c, unsigned long long* norm) {
-    const double nrm = take_norm(norm);
-    c->accepted = 0;
-    c->nxt = c->nxt_end;
-    if (c->done || c->status) return;
-    const double err = __dmul_rn(c->absh, nrm);
-    c->err = err;
-    c->nfevals += 3;
-    if (!(err <= c->rtol)) {                   // also catches NaN
-        c->nfailed++;
-        if (c->absh <= c->hmin) { c->status = 1; return; }
-        if (c->nofailed) {
-            c->nofailed = 0;
-            c->absh = isfinite(err) ? py_max(c->hmin, __dmul_rn(c->absh, py_max(0.5, __dmul_rn(0.8, pow_third(__ddiv_rn(c->rtol, err))))))
-                                    : py_max(c->hmin, __dmul_rn(0.5, c->absh));
-        } else {
-            c->absh = py_max(c->hmin, __dmul_rn(0.5, c->absh));
-        }
-        c->h = c->absh;
-        c->last = 0;
-        ode23_set_attempt(c);
-        return;
-    }
-    if (c->htrace && c->nsteps < c->hcap) c->htrace[c->nsteps] = c->h;
-    c->nsteps++;
-    c->accepted = 1;
-    c->t_acc = c->t; c->h_acc = c->h;
-    if (c->ntspan > 2) {
-        int j = c->nxt;
-        while (j < c->ntspan && __dsub_rn(c->tnew, c->tspan[j]) >= 0.0) j++;
-        c->nxt_end = j;
-    }
-    if (c->nofailed) {
-        const double temp = __dmul_rn(1.25, pow_third(__ddiv_rn(err, c->rtol)));
-        c->absh = temp > 0.2 ? __ddiv_rn(c->absh, temp) : __dmul_rn(5.0, c->absh);
-    }
-    c->t = c->tnew;
-    if (c->last) c->done = 1;
-    else ode23_new_step(c);
-}
-// ntrp23 rows of the accepted step: s == 1 gives ynew itself, the weights are formed as swrt_bs23_interp forms them
-__global__ void bs23_interp_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n || !ctl->accepted) return;
-    const double t0 = ctl->t_acc, h = ctl->h_acc, tnew = ctl->t;
-    for (int j = ctl->nxt; j < ctl->nxt_end; j++) {
-        const double tj = ctl->tspan[j];
+// after f1 and the scale norm of swrt_bs23_begin
+__global__ void ode23_init_kernel(Ode23Ctl* c, unsigned long long* norm) { ode23_init(*c, take_norm(norm)); }
+__global__ void ode23_control_kernel(Ode23Ctl* c, unsigned long long* norm) { ode23_control(*c, take_norm(norm)); }
+// ntrp23 rows [c.nxt, c.nxt_end) of packet i after the accepted step: s == 1 gives ynew itself, the weights are formed as
+// swrt_bs23_interp forms them
+__device__ __forceinline__ void bs23_rows_at(const Bs23Args& a, long long i, const Ode23Ctl& c) {
+    const double t0 = c.t_acc, h = c.h_acc, tnew = c.t;
+    for (int j = c.nxt; j < c.nxt_end; j++) {
+        const double tj = c.tspan[j];
         const double s = tj == tnew ? 1.0 : __ddiv_rn(__dsub_rn(tj, t0), h);
-        double* row = ctl->yout + (size_t)j * 4 * a.n;
+        double* row = c.yout + (size_t)j * 4 * a.n;
         if (s == 1.0) {
 #pragma unroll
             for (int c = 0; c < 4; c++) row[(size_t)c * a.n + i] = a.yt[c][i];
@@ -415,12 +424,106 @@ __global__ void bs23_interp_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
                                                                              __dmul_rn(a.f[2][c][i], w2)), __dmul_rn(a.f[3][c][i], w3)));
     }
 }
+__global__ void bs23_interp_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n || !ctl->accepted) return;
+    bs23_rows_at(a, i, *ctl);
+}
 // y <- ynew, f1 <- f4 (first same as last), predicated on the controller's decision
+__device__ __forceinline__ void bs23_accept_at(const Bs23Args& a, long long i) {
+#pragma unroll
+    for (int c = 0; c < 4; c++) { a.y[c][i] = a.yt[c][i]; a.f[0][c][i] = a.f[3][c][i]; }
+}
 __global__ void bs23_accept_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n || !ctl->accepted) return;
+    bs23_accept_at(a, i);
+}
+
+// ---- swrt_ode23_packets: the same rules, one controller per packet ---------------------------------------------------
+__device__ __forceinline__ void pkt_load(const Ode23Pkt& s, long long i, long long n, Ode23Ctl& c) {
+    c.t = s.t[i]; c.absh = s.absh[i]; c.h = s.h[i]; c.hmin = s.hmin[i]; c.tnew = s.tnew[i];
+    c.t_acc = s.t_acc[i]; c.h_acc = s.h_acc[i];
 #pragma unroll
-    for (int c = 0; c < 4; c++) { a.y[c][i] = a.yt[c][i]; a.f[0][c][i] = a.f[3][c][i]; }
+    for (int q = 0; q < 3; q++) c.al[q] = s.al[q][i];
+    const int fl = s.flags[i];
+    c.last = (fl & kPktLast) != 0; c.nofailed = (fl & kPktNofailed) != 0; c.done = (fl & kPktDone) != 0;
+    c.status = (fl & kPktStopped) != 0;
+    c.nsteps = s.cnt[i]; c.nfailed = s.cnt[n + i];
+    c.nxt = c.nxt_end = s.nxt[i];
+}
+__device__ __forceinline__ void pkt_store(const Ode23Pkt& s, long long i, long long n, const Ode23Ctl& c) {
+    s.t[i] = c.t; s.absh[i] = c.absh; s.h[i] = c.h; s.hmin[i] = c.hmin; s.tnew[i] = c.tnew;
+    s.t_acc[i] = c.t_acc; s.h_acc[i] = c.h_acc;
+#pragma unroll
+    for (int q = 0; q < 3; q++) s.al[q][i] = c.al[q];
+    s.flags[i] = (c.last ? kPktLast : 0) | (c.nofailed ? kPktNofailed : 0) | (c.done ? kPktDone : 0) | (c.status ? kPktStopped : 0);
+    s.cnt[i] = (int)c.nsteps; s.cnt[n + i] = (int)c.nfailed; s.cnt[2 * n + i] = c.status;
+    s.nxt[i] = c.nxt_end;
+}
+// the error norm of packet i alone, as bs23_norm_body and its atomicMax deliver it for a one-packet ensemble
+__device__ __forceinline__ double pkt_norm(const Bs23Args& a, long long i, int mode, double thr) {
+    const double m = bs23_norm_packet(a, i, mode, thr, 0.0);
+    return m != m ? __longlong_as_double(0x7ff0000000000000LL) : m;
+}
+__global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    ode23_init(c, pkt_norm(a, i, 1, thr));
+    pkt_store(s, i, a.n, c);
+}
+__global__ void bs23_stage_pkt_kernel(Bs23Args a, Ode23Pkt s, int stage) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n || ode23_pkt_idle(s, i)) return;
+    bs23_stage_h(a, i, stage, s.h[i]);
+}
+// two: the planes come from two evaluations, e at alpha 0 and e1 at alpha 1; between the frames they are blended at the
+// packet's alpha, in place in e (packet i's entries are this thread's own scratch)
+__global__ void rhs_pkt_kernel(Ode23Pkt s, int stage, long long n, const double* __restrict__ k, const double* __restrict__ l,
+                               E6 e, E6 e1, bool two, double f, double gH, double cgfac, double* dxdt, double* dydt,
+                               double* dkdt, double* dldt) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || ode23_pkt_idle(s, i)) return;
+    const double al = two ? ode23_pkt_alpha(s, stage)[i] : 0.0;
+    E6 src;
+#pragma unroll
+    for (int c = 0; c < 6; c++) {
+        src.p[c] = al == 1.0 ? e1.p[c] : e.p[c];
+        if (al != 0.0 && al != 1.0)
+            const_cast<double*>(e.p[c])[i] = __dadd_rn(__dmul_rn(__dsub_rn(1.0, al), e.p[c][i]), __dmul_rn(al, e1.p[c][i]));
+    }
+    rhs_at(i, k, l, src, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
+}
+// after a round's three stages: each unfinished packet's norm, its controller, its dense rows and its predicated accept.
+// Block-reduced into the report pair of this round: the packets still unfinished and the attempts the slowest of them
+// needs; the other pair is cleared for the next round.
+__global__ void __launch_bounds__(256) ode23_pkt_decide_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, int round) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    int open = 0, batch = 0;
+    if (i < a.n && !ode23_pkt_idle(s, i)) {
+        pkt_load(s, i, a.n, c);
+        ode23_control(c, pkt_norm(a, i, 0, thr));
+        if (c.accepted) {
+            if (c.ntspan > 2) bs23_rows_at(a, i, c);
+            bs23_accept_at(a, i);
+        }
+        pkt_store(s, i, a.n, c);
+        if (!c.done && !c.status) { open = 1; batch = ode23_batch_estimate(c.tfinal, c.t, c.absh, c.hmax); }
+    }
+    __shared__ int sh_open[8], sh_batch[8];
+    for (int o = 16; o > 0; o >>= 1) {
+        open += __shfl_xor_sync(0xffffffffu, open, o);
+        batch = max(batch, __shfl_xor_sync(0xffffffffu, batch, o));
+    }
+    const int w = threadIdx.x >> 5;
+    if ((threadIdx.x & 31) == 0) { sh_open[w] = open; sh_batch[w] = batch; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int q = 1; q < 8; q++) { open += sh_open[q]; batch = max(batch, sh_batch[q]); }
+        int* rep = s.report + 2 * (round & 1);
+        if (open) { atomicAdd(rep, open); atomicMax(rep + 1, batch); }
+        if (blockIdx.x == 0) { int* nxt = s.report + 2 * ((round + 1) & 1); nxt[0] = 0; nxt[1] = 0; }
+    }
 }
 }  // namespace
 
@@ -481,6 +584,22 @@ void launch_bs23_interp_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t
 }
 void launch_bs23_accept_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st) {
     if (a.n > 0) bs23_accept_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl);
+}
+
+void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, cudaStream_t st) {
+    if (a.n > 0) ode23_pkt_begin_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr);
+}
+void launch_bs23_stage_pkt(const Bs23Args& a, const Ode23Pkt& s, int stage, cudaStream_t st) {
+    if (a.n > 0) bs23_stage_pkt_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, s, stage);
+}
+void launch_rhs_pkt(const Ode23Pkt& s, int stage, long long n, const double* k, const double* l, const double* const* e6,
+                    const double* const* e1, double f, double gH, double cgfac, double* const fj[4], cudaStream_t st) {
+    E6 e, e2;
+    for (int i = 0; i < 6; i++) { e.p[i] = e6[i]; e2.p[i] = e1 ? e1[i] : nullptr; }
+    if (n > 0) rhs_pkt_kernel<<<nblk(n, 256), 256, 0, st>>>(s, stage, n, k, l, e, e2, e1 != nullptr, f, gH, cgfac, fj[0], fj[1], fj[2], fj[3]);
+}
+void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, cudaStream_t st) {
+    if (a.n > 0) ode23_pkt_decide_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, round);
 }
 
 void launch_fill(double* p, double v, long long n, cudaStream_t st) {

@@ -79,9 +79,12 @@ __device__ __forceinline__ Node4 ldg_node4(const Node4* p) {        // SASS LDG.
     return r;
 }
 
-template <bool WITH_H, bool WITH_GRAD = true>
+// MIX (swrt_ode23_packets): with mix set, every node is (1 - al) * grid + al * grid1 formed as axpby_dev_kernel forms the
+// blended fine grid, so the sums equal those over that grid; without it the quad reads `grid` alone
+template <bool WITH_H, bool WITH_GRAD = true, bool MIX = false>
 __device__ __forceinline__ void nufft_eval6(const double2* __restrict__ grid, const double* __restrict__ uvh, int nf,
-                                            double beta, double dscale, double xl, double yl, int q, int quad_base, double* F) {
+                                            double beta, double dscale, double xl, double yl, int q, int quad_base, double* F,
+                                            const double2* __restrict__ grid1 = nullptr, double al = 0.0, bool mix = false) {
     int ib, jb; double tx, ty;
     stencil_origin(xl, nf, ib, tx);
     stencil_origin(yl, nf, jb, ty);
@@ -118,6 +121,11 @@ __device__ __forceinline__ void nufft_eval6(const double2* __restrict__ grid, co
                     const Node4 nd = ldg_node4(reinterpret_cast<const Node4*>(uvh) + (size_t)iy * nf + ixr[r]);
                     g.x = nd.u; g.y = nd.v;
                     sh0 = fma(wx0[r], nd.h, sh0);
+                } else if (MIX && mix) {
+                    const double2 g0 = __ldg(grid + (size_t)iy * nf + ixr[r]), g1 = __ldg(grid1 + (size_t)iy * nf + ixr[r]);
+                    const double wa = __dsub_rn(1.0, al);
+                    g.x = fma(wa, g0.x, __dmul_rn(al, g1.x));
+                    g.y = fma(wa, g0.y, __dmul_rn(al, g1.y));
                 } else {
                     g = __ldg(grid + (size_t)iy * nf + ixr[r]);
                 }
@@ -176,6 +184,26 @@ __global__ void __launch_bounds__(kBlock) nufft_eval_dev_kernel(const NufftArgs 
     nufft_eval6<false>(grid, nullptr, a.nf, a.beta, a.dscale, reduced_coord(a.xin[pc], a.dx, a.nxd),
                        reduced_coord(a.yin[pc], a.dx, a.nxd), q, qb, F);
     if (p < a.n && q == 0) {
+#pragma unroll
+        for (int c = 0; c < 6; c++)
+            if (a.out[c]) a.out[c][p] = F[c];
+    }
+}
+
+// swrt_ode23_packets' evaluation of the six planes at each packet's own alpha: frame 0, frame 1, or both blended node by
+// node.  The choice is per quad; every quad takes part in the shuffles, finished packets store nothing.
+__global__ void __launch_bounds__(kBlock) nufft_eval_pkt_kernel(const NufftArgs a, const double2* __restrict__ grid1,
+                                                                const Ode23Pkt s, int stage) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long p = t >> LPP_SHIFT;
+    const int lane = threadIdx.x & 31, q = lane & (LPP - 1), qb = lane & ~(LPP - 1);
+    const long long pc = p < a.n ? p : a.n - 1;
+    const double al = grid1 ? ode23_pkt_alpha(s, stage)[pc] : 0.0;
+    const double2* grid = al == 1.0 ? grid1 : a.grid;
+    double F[7];
+    nufft_eval6<false, true, true>(grid, nullptr, a.nf, a.beta, a.dscale, reduced_coord(a.xin[pc], a.dx, a.nxd),
+                                   reduced_coord(a.yin[pc], a.dx, a.nxd), q, qb, F, grid1, al, al != 0.0 && al != 1.0);
+    if (p < a.n && q == 0 && !ode23_pkt_idle(s, p)) {
 #pragma unroll
         for (int c = 0; c < 6; c++)
             if (a.out[c]) a.out[c][p] = F[c];
@@ -341,6 +369,11 @@ cudaError_t launch_nufft_eval(const NufftArgs& a, cudaStream_t st) {
 cudaError_t launch_nufft_eval_dev(const NufftArgs& a, const Ode23Sel& sel, cudaStream_t st) {
     if (a.n <= 0) return cudaSuccess;
     nufft_eval_dev_kernel<<<(unsigned)(((long long)LPP * a.n + kBlock - 1) / kBlock), kBlock, 0, st>>>(a, sel);
+    return cudaGetLastError();
+}
+cudaError_t launch_nufft_eval_pkt(const NufftArgs& a, const double2* grid1, const Ode23Pkt& s, int stage, cudaStream_t st) {
+    if (a.n <= 0) return cudaSuccess;
+    nufft_eval_pkt_kernel<<<(unsigned)(((long long)LPP * a.n + kBlock - 1) / kBlock), kBlock, 0, st>>>(a, grid1, s, stage);
     return cudaGetLastError();
 }
 cudaError_t launch_nufft_leapfrog(const NufftArgs& a, cudaStream_t st) {

@@ -87,6 +87,11 @@ struct swrt_handle {
     Ode23Ctl* ode_ctl = nullptr;          // swrt_ode23: the controller state on the device ...
     Ode23Ctl* ode_host = nullptr;         // ... and its pinned host image (set-up and read-back)
     cudaEvent_t ode_ev = nullptr;
+    // swrt_ode23_packets: the per-packet controller state (Ode23Pkt: 10 double and 5 int arrays of pkt_cap entries, then the
+    // report words), its pinned report image, and the alpha-1 planes of a two-frame SPECTRAL solve
+    double* pkt_d = nullptr; int* pkt_i = nullptr; int64_t pkt_cap = 0;
+    int* pkt_rep_host = nullptr;
+    double* pkt_e1 = nullptr;
     double* edges_dev = nullptr; int edges_cap = 0;
     std::vector<double> edges_host;       // what edges_dev currently holds
     unsigned long long* counts_dev = nullptr; int counts_cap = 0;
@@ -703,6 +708,8 @@ int swrt_destroy(swrt_handle* h) {
     for (auto& row : h->bs_f) for (auto& p : row) dfree(p);
     dfree(h->ode_ctl);
     if (h->ode_host) cudaFreeHost(h->ode_host);
+    dfree(h->pkt_d); dfree(h->pkt_i); dfree(h->pkt_e1);
+    if (h->pkt_rep_host) cudaFreeHost(h->pkt_rep_host);
     if (h->ode_ev) cudaEventDestroy(h->ode_ev);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
@@ -1917,3 +1924,4 @@ int swrt_spectral_geometry(int nx, int nplanes, int mtiles, int64_t out[10]) {
 
 #include "swrt_group.inc"     // multi-device handles: sharding + in-library NCCL
 #include "swrt_ode23.inc"     // swrt_ode23: a whole ode23 solve with the controller on the device
+#include "swrt_ode23_packets.inc"   // swrt_ode23_packets: the same solve with one controller per packet

@@ -77,6 +77,32 @@ struct Ode23Sel {
     const void* blend;
 };
 __device__ __forceinline__ bool ode23_idle(const Ode23Ctl* c) { return c->done || c->status; }
+// attempts to queue before the host looks at the state again: the steps left if every step grew five-fold up to hmax
+// (the most the controller allows, so a lower bound) plus a margin for rejections and slower growth
+__host__ __device__ inline int ode23_batch_estimate(double tfinal, double t, double absh, double hmax) {
+    double left = fabs(tfinal - t), hh = absh;
+    int est = 0;
+    while (left > 0.0 && est < 1024) { left -= hh < hmax ? hh : hmax; hh *= 5.0; est++; }
+    const int b = est + 2 + est / 4;
+    return b < 256 ? b : 256;
+}
+
+// swrt_ode23_packets: every packet under its own controller.  The state of Ode23Ctl's controller section, one entry per
+// packet (SoA, n each); a kernel loads a packet's entries into a local Ode23Ctl that also carries the per-solve
+// constants, applies swrt_ode23's rules to it and stores it back.
+constexpr int kPktLast = 1, kPktNofailed = 2, kPktDone = 4, kPktStopped = 8;
+struct Ode23Pkt {
+    double *t, *absh, *h, *hmin, *tnew, *al[3], *t_acc, *h_acc;
+    int* flags;                    // kPkt* bits
+    int* cnt;                      // 3 x n: accepted steps, rejected steps, status (1 = stopped: step size below hmin)
+    int* nxt;                      // next dense row to write
+    int* report;                   // 2 x {unfinished packets, attempts to queue}: decide kernel of round r writes pair r & 1
+};
+__device__ __forceinline__ bool ode23_pkt_idle(const Ode23Pkt& s, long long i) { return s.flags[i] & (kPktDone | kPktStopped); }
+// the alphas of `stage` (selected, not indexed: a run-time index would move the kernel argument to local memory)
+__device__ __forceinline__ const double* ode23_pkt_alpha(const Ode23Pkt& s, int stage) {
+    return stage == 0 ? s.al[0] : stage == 1 ? s.al[1] : s.al[2];
+}
 
 PackGeom make_geom(int nx, int npl, const int* plane_ids, int mtiles, int twiddle_pref = 0);
 
@@ -275,6 +301,16 @@ void launch_axpby_dev(double* out, const double* a, const double* b, const Ode23
 cudaError_t launch_spectral_eval_dev(const SpecArgs& a, int num_sms, cudaStream_t st);     // a.sel set
 cudaError_t launch_nufft_eval_dev(const NufftArgs& a, const Ode23Sel& sel, cudaStream_t st);
 cudaError_t launch_lagrange_eval_dev(const LagArgs& a, const Ode23Ctl* ctl, int stage, cudaStream_t st);
+// swrt_ode23_packets: `k` holds the per-solve constants (controller section zero, t = t0).  begin: the rh norm and the
+// initial step of every packet from f1; stage / RHS / decide as their swrt_ode23 counterparts with each packet's own h and
+// alphas.  With e1 set (SPECTRAL, two frames) the RHS blends e (alpha 0) and e1 (alpha 1) at the packet's alpha.
+void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, cudaStream_t st);
+void launch_bs23_stage_pkt(const Bs23Args& a, const Ode23Pkt& s, int stage, cudaStream_t st);
+void launch_rhs_pkt(const Ode23Pkt& s, int stage, long long n, const double* k, const double* l, const double* const* e6,
+                    const double* const* e1, double f, double gH, double cgfac, double* const fj[4], cudaStream_t st);
+void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, cudaStream_t st);
+cudaError_t launch_nufft_eval_pkt(const NufftArgs& a, const double2* grid1, const Ode23Pkt& s, int stage, cudaStream_t st);
+cudaError_t launch_lagrange_eval_pkt(const LagArgs& a, const Ode23Pkt& s, int stage, cudaStream_t st);
 // (rtol/err)^(1/3) as glibc's correctly rounded-in-practice pow gives it (host and device, misc_kernels.cu)
 __host__ __device__ double pow_third(double x);
 

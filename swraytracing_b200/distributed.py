@@ -108,10 +108,14 @@ class ShardedEnsemble:
     def step(self, scheme, dt, nsteps, alpha0=0.0, dalpha=0.0):
         self.engine.step(scheme, dt, nsteps, alpha0, dalpha)
 
-    def ode23(self, tspan, tmax, rtol=1e-3, atol=1e-6):
+    def ode23(self, tspan, tmax, rtol=1e-3, atol=1e-6, per_packet=False):
         """the reference's per-flow-step ode23 solve over ALL shards: the error norm is MAX-all-reduced so
-        that every rank accepts/rejects the same steps (the reference's norm couples all packets)."""
+        that every rank accepts/rejects the same steps (the reference's norm couples all packets).
+        ``per_packet=True``: every packet under its own controller (``Engine.ode23_packets``) on the local shard, with no
+        collective; the returned counts are this rank's."""
         from .reference_api import ode23
+        if per_packet:
+            return ode23(self.engine, tspan, tmax, rtol, atol, per_packet=True)
         return ode23(self.engine, tspan, tmax, rtol, atol, reduce_max=self._allreduce_max)
 
     def _allreduce_max(self, v):

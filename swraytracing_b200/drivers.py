@@ -51,8 +51,9 @@ def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_da
                   integrator="ode23", mode=MODE_SPECTRAL, r_drag=0.1, beta=0.0, force_strength=0.1, max_steps=None,
                   seed=146, device=0, log=print, leapfrog_substeps=4):
     """qgsw_raytrace.m:1-180 on the device.  ``integrator``: 'ode23' (the reference), 'ode23_device' (the same solve
-    with the controller on the device, swrt_ode23) or 'leapfrog' (the fused symplectic stepper with time-centred frame
-    blending).  ``max_steps`` truncates the run (tests)."""
+    with the controller on the device, swrt_ode23), 'ode23_packets' (ode23 once per packet, each under its own controller,
+    swrt_ode23_packets: a packet that blows up stops alone, counted in ``ode23_stopped_packets``) or 'leapfrog' (the fused
+    symplectic stepper with time-centred frame blending).  ``max_steps`` truncates the run (tests)."""
     L = 2 * np.pi
     dx = L / nx
     xg = matlab_linspace(-L / 2, L / 2, nx)
@@ -105,6 +106,8 @@ def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_da
     t = 0.0
     tic = time.time()
     stats = {"packet_steps": 0, "ode23_steps": 0, "ode23_failed": 0}
+    if integrator == "ode23_packets":
+        stats["ode23_stopped_packets"] = 0
     for step in range(1, Nsteps + 1):
         if Npackets > 0 and t + dt > packet_delay:
             qg.to_flow(eng, 0)                                         # background_flow1 = grid_U(prev_qk), :141
@@ -112,9 +115,12 @@ def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_da
         t += dt
         if Npackets > 0 and t > packet_delay:
             qg.to_flow(eng, 1)                                         # background_flow2 = grid_U(qk), :142
-            if integrator in ("ode23", "ode23_device"):
-                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device")      # :143-150
+            if integrator in ("ode23", "ode23_device", "ode23_packets"):
+                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device",
+                           per_packet=integrator == "ode23_packets")                          # :143-150
                 stats["ode23_steps"] += st["nsteps"]; stats["ode23_failed"] += st["nfailed"]
+                if integrator == "ode23_packets":
+                    stats["ode23_stopped_packets"] += st["stopped"]
             else:
                 m = leapfrog_substeps
                 eng.step(SCHEME_LEAPFROG, dt / m, m, 0.5 / m, 1.0 / m)
@@ -221,7 +227,8 @@ def SW_zero_background_raytracing(q=None, *, nx=None, f=None, Cg=None, run_log_f
     """SW_zero_background_raytracing.m:1-132 (BASELINE config 1): the same frozen frame and packet ring, integrated
     by ``ode23`` with RelTol 1e-6 / AbsTol 1e-7 and output requested at ``t_hist = dt*(0:Nsteps)`` (:70-78), RHS
     ``dx/dt = U + gH k/omega`` (:134-145,182-184).  ``q = zeros`` is the "zero background" of the file name
-    (the hint on :28-29).  ``integrator='ode23_device'`` runs the solve with the controller on the device (swrt_ode23).
+    (the hint on :28-29).  ``integrator='ode23_device'`` runs the solve with the controller on the device (swrt_ode23),
+    ``integrator='ode23_packets'`` solves every packet under its own controller (swrt_ode23_packets).
     Returns dict(t_hist, solver_x, solver_k, solver_error, w, Omega_0, U0, Fr, dt, stats)."""
     from .engine import FLAG_RHS_GH
     from .reference_api import ode23
@@ -244,7 +251,8 @@ def SW_zero_background_raytracing(q=None, *, nx=None, f=None, Cg=None, run_log_f
     eng = Engine(nx, L, f, gH, mode, device, flags=FLAG_RHS_GH)
     eng.set_flow_spectral(scheme.psik)
     eng.set_packets(x[0, 0], x[0, 1], k[0, 0], k[0, 1])
-    stats = ode23(eng, t_hist, None, rtol=rtol, atol=atol, on_device=integrator == "ode23_device")   # steady flow: slot 0
+    stats = ode23(eng, t_hist, None, rtol=rtol, atol=atol, on_device=integrator == "ode23_device",
+                  per_packet=integrator == "ode23_packets")                                         # steady flow: slot 0
     Y = stats.pop("Y")
     eng.close()
     solver_x, solver_k = Y[:, 0:2, :], Y[:, 2:4, :]
@@ -385,7 +393,8 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
                         leapfrog_substeps=4):
     """qg_flow_ray_trace/qg2layersw_raytrace.m:1-247 (BASELINE config 4) on the device: two-layer QG with mean shear on
     L = 20, adaptive dt (:156-165), AB3 + integrating factor, packets advected through the TOP layer's
-    ``grid_U`` frames (:187-196) by ode23 over [0, dt] ('ode23_device': controller on the device), packet frames every
+    ``grid_U`` frames (:187-196) by ode23 over [0, dt] ('ode23_device': controller on the device; 'ode23_packets': one
+    controller per packet, stopped packets counted in ``ode23_stopped_packets``), packet frames every
     25 steps.  ``k_max`` (30 in the reference)
     and ``max_steps`` exist for tests."""
     L = 20.0
@@ -440,6 +449,8 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
     step = 0
     tic = time.time()
     stats = {"packet_steps": 0, "ode23_steps": 0, "ode23_failed": 0, "dt_changes": 0}
+    if integrator == "ode23_packets":
+        stats["ode23_stopped_packets"] = 0
     while t <= T and (max_steps is None or step < max_steps):
         step += 1
         U0 = qg.max_speed()
@@ -455,9 +466,11 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
         t = t + dt
         if advect:
             qg.to_flow(eng, 1)                                         # background_flow2 = grid_U(qk(:,:,:,1)), :188
-            if integrator in ("ode23", "ode23_device"):
-                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device")
+            if integrator in ("ode23", "ode23_device", "ode23_packets"):
+                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device", per_packet=integrator == "ode23_packets")
                 stats["ode23_steps"] += st["nsteps"]; stats["ode23_failed"] += st["nfailed"]
+                if integrator == "ode23_packets":
+                    stats["ode23_stopped_packets"] += st["stopped"]
             else:
                 m = leapfrog_substeps
                 eng.step(SCHEME_LEAPFROG, dt / m, m, 0.5 / m, 1.0 / m)

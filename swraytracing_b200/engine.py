@@ -64,6 +64,8 @@ SIGNATURES = {
     "swrt_bs23_accept": (C.c_int, [C.c_void_p]),
     "swrt_bs23_interp": (C.c_int, [C.c_void_p, C.c_double, C.c_double] + [_dp] * 4),
     "swrt_ode23": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int64), _dp, C.c_int]),
+    "swrt_ode23_packets": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int32), _dp,
+                                     C.POINTER(C.c_int64)]),
     "swrt_hist_omega_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_launch": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_wait": (C.c_int, [C.c_void_p]),
@@ -349,6 +351,29 @@ class Engine:
             out["Y"] = Y
         if trace > 0:
             out["h"] = hs[:min(st[0], hs.size)].copy()
+        return out
+
+    def ode23_packets(self, tspan, tmax, rtol=1e-3, atol=1e-6):
+        """``ode23`` once per packet (swrt_ode23_packets): every packet under its own step-size controller, exactly as
+        ``ode23`` advances an ensemble holding that packet alone, so a packet's result does not depend on the others.
+        Returns ``ode23``'s dict with ``nsteps``, ``nfailed`` and ``nfevals`` summed over packets, plus ``stopped``
+        (packets whose step size fell below hmin: they keep their last accepted state, the others carry on),
+        ``host_waits``, and the per-packet arrays ``steps``, ``rejected``, ``status`` (0 reached tfinal, 1 stopped) and
+        ``t_end`` (where each packet stopped).  ``Y`` when ``tspan`` has more than two entries (NaN in the rows a stopped
+        packet did not reach)."""
+        ts = _f64(tspan)
+        dense = ts.size > 2
+        Y = np.empty((ts.size, 4, self.n)) if dense else None
+        pstat = np.empty((3, self.n), dtype=np.int32)          # the C side's n x 3 column-major block
+        t_end = np.empty(self.n)
+        st = (C.c_int64 * 5)()
+        self._check(self.lib.swrt_ode23_packets(self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol),
+                                                _ptr(Y) if dense else None, pstat.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                _ptr(t_end), st))
+        out = {"nsteps": st[0], "nfailed": st[1], "nfevals": st[2], "t": float(ts[-1]), "stopped": st[3], "host_waits": st[4],
+               "steps": pstat[0].copy(), "rejected": pstat[1].copy(), "status": pstat[2].copy(), "t_end": t_end}
+        if dense:
+            out["Y"] = Y
         return out
 
     # -- diagnostics --

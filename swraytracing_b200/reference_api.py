@@ -297,7 +297,7 @@ def omega(k, f, gH):
 # ode23 -- the production drivers' integrator (qgsw_raytrace.m:149, qg2layersw_raytrace.m:195)
 # ------------------------------------------------------------------------------------------------
 
-def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=False):
+def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=False, per_packet=False):
     """``[~, Y] = ode23(ray_ode, [0 dt], y0)`` for the packets resident in ``target`` (an Engine):
     MATLAB's ode23 = Bogacki-Shampine 3(2) pair with first-same-as-last, restated from its published
     description (Shampine & Reichelt, "The MATLAB ODE Suite", SIAM J. Sci. Comput. 18, 1997; MATLAB
@@ -318,7 +318,15 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=
     raises; MATLAB's ``if err > rtol`` is false for NaN, so it would accept the step and carry NaNs on silently.
 
     ``on_device=True`` (single-process callers, no ``reduce_max``) runs the same solve as one ``Engine.ode23`` call, the
-    controller in device memory (swrt_ode23); the returned dict then also holds ``host_waits``."""
+    controller in device memory (swrt_ode23); the returned dict then also holds ``host_waits``.
+
+    ``per_packet=True`` solves every packet under its own controller instead (``Engine.ode23_packets``,
+    swrt_ode23_packets): what MATLAB gives when ``ode23`` is called once per packet.  Nothing couples the packets, so
+    ``reduce_max`` is refused with it; a packet whose step size falls below hmin stops alone (``stopped``, ``status``)."""
+    if per_packet:
+        if reduce_max is not None:
+            raise ValueError("ode23: per_packet=True needs no reduce_max (the packets are not coupled)")
+        return target.ode23_packets(tspan, tmax, rtol, atol)
     if on_device and reduce_max is None:
         return target.ode23(tspan, tmax, rtol, atol)
     red = reduce_max if reduce_max is not None else (lambda v: v)
