@@ -182,6 +182,40 @@ int swrt_ode23(swrt_handle* h, const double* tspan, int ntspan, double tmax, dou
 int swrt_ode23_packets(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol, double* Y,
                        int32_t* pstat, double* t_end, int64_t stats[5]);
 
+/* [t, Y, te, ye, ie] = ode23(odefun_i, tspan, y_i, odeset('Events', ...)) for every packet i on its own: event j is a level
+ * crossing of g_j(x, y, k, l), a function of the packet state alone.  omega is swrt_hist_omega's intrinsic frequency
+ * sqrt(f^2 + gH (k^2 + l^2)) (analysis/load_data.m:33); every operation is rounded on its own.                       */
+#define SWRT_EVENT_X      0   /* g = x - level (unwrapped) */
+#define SWRT_EVENT_Y      1   /* g = y - level             */
+#define SWRT_EVENT_K      2   /* g = k - level             */
+#define SWRT_EVENT_L      3   /* g = l - level             */
+#define SWRT_EVENT_KMAG   4   /* g = sqrt(k^2 + l^2) - level */
+#define SWRT_EVENT_OMEGA  5   /* g = omega - level         */
+#define SWRT_MAX_EVENTS   8
+typedef struct swrt_event {
+    int32_t kind;        /* SWRT_EVENT_* */
+    int32_t direction;   /* 0 any crossing, +1 rising only (g: < 0 to >= 0), -1 falling only (g: > 0 to <= 0) */
+    int32_t terminal;    /* 1: the packet stops at the event */
+    int32_t reserved;    /* 0 */
+    double level;        /* finite */
+} swrt_event;
+/* The solve of swrt_ode23_packets; tspan must be strictly increasing.  After every accepted step from t to tnew, event j
+ * fires when g_j at the previous accepted state (y0 at the start) is non-zero, neither value is NaN, the sign changes and
+ * the direction allows it; a zero at the left end is never an event (none at t0).  It is located on the step's ntrp23
+ * cubic by Illinois regula falsi (DESIGN.md section 11): te is the first point found with g_j = 0 or of the post-crossing
+ * sign, ye the cubic there.  Events never change a step decision.
+ * Records per packet, in ascending (te, ie) order over the solve: te[r*n+i], ye[(r*4+c)*n+i] (c = x, y, k, l) and ie[r*n+i]
+ * (1-based event index) for r < ev_cap, NaN / 0 when unused; ne[i] counts every event found (> ev_cap: records were
+ * dropped).  Any of te, ye, ie, ne may be NULL.  A terminal event stops its packet at the earliest terminal te* of the
+ * step: records after te* are not kept, the packet's state becomes that record's ye, t_end = te*, status = 2, and the
+ * dense rows after te* stay NaN.  Y, pstat (status 2 = terminal event), t_end and stats[0..4] as in
+ * swrt_ode23_packets; stats[5] = events found, stats[6] = packets stopped by a terminal event.
+ * SWRT_ERR_ARG: nev outside 1..SWRT_MAX_EVENTS, ev_cap < 0, an unknown kind, a direction outside {-1, 0, 1}, a terminal
+ * flag outside {0, 1}, reserved != 0, a non-finite level, a tspan not strictly increasing.                          */
+int swrt_ode23_packets_events(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol,
+                              const swrt_event* ev, int nev, int ev_cap, double* Y, int32_t* pstat, double* t_end,
+                              double* te, double* ye, int32_t* ie, int32_t* ne, int64_t stats[7]);
+
 /* ---- diagnostics -------------------------------------------------------------------------- */
 /* histcounts(omega, edges) (analysis/load_data.m:39-47): counts[nedges-1], bin i = [e_i,e_i+1),
  * last bin closed; accumulate != 0 adds to counts instead of overwriting.                      */

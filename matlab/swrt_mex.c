@@ -324,6 +324,53 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
             for (size_t i = 0; i < 3 * n; i++) mxGetPr(plhs[2])[i] = (double)ps[i];
             mxFree(ps);
         }
+    } else if (!strcmp(cmd, "ode23_events")) {        /* [stats, Y, pstat, t_end, te, ye, ie, ne] = (h, tspan, tmax, rtol, atol, ev, ev_cap) */
+        need(nrhs, 8, "'ode23_events', h, tspan, tmax, rtol, atol, ev, ev_cap");
+        int nt = (int)mxGetNumberOfElements(prhs[2]);
+        /* ev: nev x 4, columns [kind level direction terminal] */
+        int nev = (int)mxGetM(prhs[6]), cap = (int)mxGetScalar(prhs[7]);
+        if (mxGetN(prhs[6]) != 4) mexErrMsgIdAndTxt("swrt:usage", "ode23_events: ev must be nev x 4 = [kind level direction terminal]");
+        if (nev < 1 || nev > SWRT_MAX_EVENTS) mexErrMsgIdAndTxt("swrt:usage", "ode23_events: 1 to %d events", SWRT_MAX_EVENTS);
+        const double* e = mxGetPr(prhs[6]);
+        swrt_event ev[SWRT_MAX_EVENTS];
+        for (int j = 0; j < nev; j++) {
+            ev[j].kind = (int32_t)e[j]; ev[j].level = e[nev + j]; ev[j].direction = (int32_t)e[2 * nev + j];
+            ev[j].terminal = (int32_t)e[3 * nev + j]; ev[j].reserved = 0;
+        }
+        size_t nc = cap > 0 ? (size_t)cap : 0;
+        int64_t st[7];
+        double *Y = NULL, *t_end = NULL;
+        if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix((size_t)n, nt > 2 ? (size_t)4 * nt : 0, mxREAL); if (nt > 2) Y = mxGetPr(plhs[1]); }
+        int32_t* ps = nlhs > 2 ? (int32_t*)mxCalloc((size_t)3 * (n > 0 ? n : 1), sizeof(int32_t)) : NULL;
+        if (nlhs > 3) t_end = outv(plhs, 3, n);
+        /* te, ie: n x ev_cap (record r of packet i in row i, column r); ye: n x 4*ev_cap (reshape(ye, n, 4, []) gives
+           [x y k l] of every record); ne: n x 1 */
+        double *te = NULL, *ye = NULL;
+        int32_t *ie = NULL, *ne = NULL;
+        if (nlhs > 4) { plhs[4] = mxCreateDoubleMatrix((size_t)n, nc, mxREAL); te = mxGetPr(plhs[4]); }
+        if (nlhs > 5) { plhs[5] = mxCreateDoubleMatrix((size_t)n, 4 * nc, mxREAL); ye = mxGetPr(plhs[5]); }
+        if (nlhs > 6) ie = (int32_t*)mxCalloc(n * nc > 0 ? n * nc : 1, sizeof(int32_t));
+        if (nlhs > 7) ne = (int32_t*)mxCalloc(n > 0 ? n : 1, sizeof(int32_t));
+        if (swrt_ode23_packets_events(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), ev, nev,
+                                      cap, Y, ps, t_end, te, ye, ie, ne, st))
+            fail(h, cmd);
+        plhs[0] = mxCreateDoubleMatrix(1, 7, mxREAL);
+        for (int i = 0; i < 7; i++) mxGetPr(plhs[0])[i] = (double)st[i];
+        if (ps) {
+            plhs[2] = mxCreateDoubleMatrix((size_t)n, 3, mxREAL);
+            for (size_t i = 0; i < 3 * n; i++) mxGetPr(plhs[2])[i] = (double)ps[i];
+            mxFree(ps);
+        }
+        if (ie) {
+            plhs[6] = mxCreateDoubleMatrix((size_t)n, nc, mxREAL);
+            for (size_t i = 0; i < n * nc; i++) mxGetPr(plhs[6])[i] = (double)ie[i];
+            mxFree(ie);
+        }
+        if (ne) {
+            plhs[7] = mxCreateDoubleMatrix((size_t)n, 1, mxREAL);
+            for (size_t i = 0; i < n; i++) mxGetPr(plhs[7])[i] = (double)ne[i];
+            mxFree(ne);
+        }
     } else if (!strcmp(cmd, "hist_omega")) {          /* counts = (h, kind, alpha, edges) */
         need(nrhs, 5, "'hist_omega', h, kind, alpha, edges");
         int ne = (int)mxGetNumberOfElements(prhs[4]);

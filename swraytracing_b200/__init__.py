@@ -1,8 +1,10 @@
 """swraytracing_b200 -- B200-native engine for SWRaytracing's packet hot path (see DESIGN.md)."""
 from .engine import (Engine, QGFlow, QG2Flow, SwrtError, load_library, interpolate_dev, g2k_dev, k2g_dev,
                      MODE_SPECTRAL, MODE_LAGRANGE6, MODE_NUFFT, SCHEME_LEAPFROG, SCHEME_RK4_PACKET, SCHEME_RK4_XKA,
-                     HIST_INTRINSIC, HIST_ABSOLUTE, FLAG_RHS_GH)
+                     HIST_INTRINSIC, HIST_ABSOLUTE, FLAG_RHS_GH, EVENT_X, EVENT_Y, EVENT_K, EVENT_L, EVENT_KMAG,
+                     EVENT_OMEGA, MAX_EVENTS)
 
 __all__ = ["Engine", "QGFlow", "QG2Flow", "SwrtError", "load_library", "interpolate_dev", "g2k_dev", "k2g_dev",
            "MODE_SPECTRAL", "MODE_LAGRANGE6", "MODE_NUFFT", "SCHEME_LEAPFROG", "SCHEME_RK4_PACKET", "SCHEME_RK4_XKA",
-           "HIST_INTRINSIC", "HIST_ABSOLUTE", "FLAG_RHS_GH"]
+           "HIST_INTRINSIC", "HIST_ABSOLUTE", "FLAG_RHS_GH", "EVENT_X", "EVENT_Y", "EVENT_K", "EVENT_L", "EVENT_KMAG",
+           "EVENT_OMEGA", "MAX_EVENTS"]

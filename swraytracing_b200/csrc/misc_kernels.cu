@@ -2,6 +2,7 @@
 // qgsw_raytrace.m:259-265, the point-wise RK4 glue used by the SPECTRAL mode of step_packet /
 // step_packet_xka, omega / Omega (symplectic_full_fourier.m:41,54-56), histcounts
 // (analysis/load_data.m:39-47) and the reduction diagnostics.
+#include "../../include/swrt.h"
 #include "swrt_internal.h"
 
 namespace swrt {
@@ -400,8 +401,15 @@ __device__ __forceinline__ double take_norm(unsigned long long* norm) {
 // after f1 and the scale norm of swrt_bs23_begin
 __global__ void ode23_init_kernel(Ode23Ctl* c, unsigned long long* norm) { ode23_init(*c, take_norm(norm)); }
 __global__ void ode23_control_kernel(Ode23Ctl* c, unsigned long long* norm) { ode23_control(*c, take_norm(norm)); }
-// ntrp23 rows [c.nxt, c.nxt_end) of packet i after the accepted step: s == 1 gives ynew itself, the weights are formed as
-// swrt_bs23_interp forms them
+// the ntrp23 weights at s of a step of size h, as swrt_bs23_interp forms them
+__device__ __forceinline__ void ntrp23_weights(double s, double h, double w[4]) {
+    const double s2 = __dmul_rn(s, s), s3 = __dmul_rn(s2, s);
+    w[0] = __dmul_rn(h, __dadd_rn(__dsub_rn(s, __dmul_rn(4.0 / 3.0, s2)), __dmul_rn(5.0 / 9.0, s3)));
+    w[1] = __dmul_rn(h, __dsub_rn(s2, __dmul_rn(2.0 / 3.0, s3)));
+    w[2] = __dmul_rn(h, __dsub_rn(__dmul_rn(4.0 / 3.0, s2), __dmul_rn(8.0 / 9.0, s3)));
+    w[3] = __dmul_rn(h, __dadd_rn(-s2, s3));
+}
+// ntrp23 rows [c.nxt, c.nxt_end) of packet i after the accepted step: s == 1 gives ynew itself
 __device__ __forceinline__ void bs23_rows_at(const Bs23Args& a, long long i, const Ode23Ctl& c) {
     const double t0 = c.t_acc, h = c.h_acc, tnew = c.t;
     for (int j = c.nxt; j < c.nxt_end; j++) {
@@ -413,15 +421,12 @@ __device__ __forceinline__ void bs23_rows_at(const Bs23Args& a, long long i, con
             for (int c = 0; c < 4; c++) row[(size_t)c * a.n + i] = a.yt[c][i];
             continue;
         }
-        const double s2 = __dmul_rn(s, s), s3 = __dmul_rn(s2, s);
-        const double w0 = __dmul_rn(h, __dadd_rn(__dsub_rn(s, __dmul_rn(4.0 / 3.0, s2)), __dmul_rn(5.0 / 9.0, s3)));
-        const double w1 = __dmul_rn(h, __dsub_rn(s2, __dmul_rn(2.0 / 3.0, s3)));
-        const double w2 = __dmul_rn(h, __dsub_rn(__dmul_rn(4.0 / 3.0, s2), __dmul_rn(8.0 / 9.0, s3)));
-        const double w3 = __dmul_rn(h, __dadd_rn(-s2, s3));
+        double w[4];
+        ntrp23_weights(s, h, w);
 #pragma unroll
         for (int c = 0; c < 4; c++)
-            row[(size_t)c * a.n + i] = __dadd_rn(a.y[c][i], __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(a.f[0][c][i], w0), __dmul_rn(a.f[1][c][i], w1)),
-                                                                             __dmul_rn(a.f[2][c][i], w2)), __dmul_rn(a.f[3][c][i], w3)));
+            row[(size_t)c * a.n + i] = __dadd_rn(a.y[c][i], __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(a.f[0][c][i], w[0]), __dmul_rn(a.f[1][c][i], w[1])),
+                                                                             __dmul_rn(a.f[2][c][i], w[2])), __dmul_rn(a.f[3][c][i], w[3])));
     }
 }
 __global__ void bs23_interp_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
@@ -466,11 +471,138 @@ __device__ __forceinline__ double pkt_norm(const Bs23Args& a, long long i, int m
     const double m = bs23_norm_packet(a, i, mode, thr, 0.0);
     return m != m ? __longlong_as_double(0x7ff0000000000000LL) : m;
 }
-__global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr) {
+// ---- events (swrt_ode23_packets_events): every operation rounded on its own (this file is compiled with FMA contraction) --
+// g_j(x, y, k, l); OMEGA is omega_kernel's expression, so an event level and a histogram edge agree on a state's side
+__device__ __forceinline__ double ev_g(int kind, double level, double f, double gH, const double v[4]) {
+    const double kl = __dadd_rn(__dmul_rn(v[2], v[2]), __dmul_rn(v[3], v[3]));
+    const double g = kind == SWRT_EVENT_X ? v[0] : kind == SWRT_EVENT_Y ? v[1] : kind == SWRT_EVENT_K ? v[2]
+                   : kind == SWRT_EVENT_L ? v[3] : kind == SWRT_EVENT_KMAG ? __dsqrt_rn(kl)
+                   : __dsqrt_rn(__dadd_rn(__dmul_rn(f, f), __dmul_rn(gH, kl)));
+    return __dsub_rn(g, level);
+}
+// one accepted step of a packet: y, f1..f4 and ynew, from t0 with step h to tnew
+struct EvStep { double y[4], f[4][4], yn[4]; double t0, h, tnew; };
+// the step's ntrp23 interpolant at tau, exactly as bs23_rows_at writes a dense row (p(tnew) = ynew)
+__device__ __forceinline__ void ev_point(const EvStep& q, double tau, double out[4]) {
+    const double s = tau == q.tnew ? 1.0 : __ddiv_rn(__dsub_rn(tau, q.t0), q.h);
+    if (s == 1.0) {
+#pragma unroll
+        for (int c = 0; c < 4; c++) out[c] = q.yn[c];
+        return;
+    }
+    double w[4];
+    ntrp23_weights(s, q.h, w);
+#pragma unroll
+    for (int c = 0; c < 4; c++)
+        out[c] = __dadd_rn(q.y[c], __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(q.f[0][c], w[0]), __dmul_rn(q.f[1][c], w[1])),
+                                                       __dmul_rn(q.f[2][c], w[2])), __dmul_rn(q.f[3][c], w[3])));
+}
+__device__ __forceinline__ double spacing(double t) {          // np.spacing(abs(t))
+    t = fabs(t);
+    return __dsub_rn(nextafter(t, __longlong_as_double(0x7ff0000000000000LL)), t);
+}
+// the crossing of event j inside the step, g(t0) = vL and g(tnew) = vR of opposite signs: Illinois regula falsi on the
+// interpolant (DESIGN.md section 11).  Returns te; g at p(te) is 0 or has vR's sign.
+__device__ double ev_locate(const EvStep& q, int kind, double level, double f, double gH, double vL, double vR) {
+    if (vR == 0.0) return q.tnew;
+    double tL = q.t0, tR = q.tnew, gL = vL, gR = vR;
+    const double tol = __dmul_rn(128.0, fmax(spacing(tL), spacing(tR))), half = __dmul_rn(0.5, tol);
+    int moved = 0;                                               // the end that moved last: -1 left, +1 right
+    for (int it = 0; it < 64 && __dsub_rn(tR, tL) > tol; it++) {
+        double tm = __dsub_rn(tR, __dmul_rn(gR, __ddiv_rn(__dsub_rn(tR, tL), __dsub_rn(gR, gL))));
+        tm = py_min(py_max(tm, __dadd_rn(tL, half)), __dsub_rn(tR, half));
+        double v[4];
+        ev_point(q, tm, v);
+        const double gm = ev_g(kind, level, f, gH, v);
+        if (gm == 0.0) { tR = tm; break; }
+        if ((gm < 0.0) == (gL < 0.0)) {                          // the sign changes across [tm, tR]
+            tL = tm; gL = gm;
+            if (moved < 0) gR = __dmul_rn(0.5, gR);
+            moved = -1;
+        } else {                                                 // across [tL, tm]
+            tR = tm; gR = gm;
+            if (moved > 0) gL = __dmul_rn(0.5, gL);
+            moved = 1;
+        }
+    }
+    return tR;
+}
+// after packet i's accepted step (c.t = tnew): detect, locate and record its events in (te, ie) order.  Returns true on a
+// terminal stop, with its time and state in tstop / ystop; records after tstop are not kept.
+__device__ __forceinline__ bool pkt_events(const Bs23Args& a, long long i, const Ode23Ctl& c, const Ode23Ev& ev, double& tstop,
+                                           double ystop[4]) {
+    const long long n = a.n;
+    EvStep q;
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        q.y[k] = a.y[k][i]; q.yn[k] = a.yt[k][i];
+#pragma unroll
+        for (int j = 0; j < 4; j++) q.f[j][k] = a.f[j][k][i];
+    }
+    q.t0 = c.t_acc; q.h = c.h_acc; q.tnew = c.t;
+    double te[kMaxEvents];
+    unsigned fired = 0;
+    bool stop = false;
+#pragma unroll
+    for (int j = 0; j < kMaxEvents; j++) {
+        te[j] = 0.0;
+        if (j >= ev.nev) continue;
+        const double vL = ev.vl[j * n + i], vR = ev_g(ev.kind[j], ev.level[j], ev.f, ev.gH, q.yn);
+        ev.vl[j * n + i] = vR;
+        // vL != 0, no NaN, a sign change the direction allows (a zero at the left end is never an event)
+        if ((vL < 0.0 && vR >= 0.0 && ev.dir[j] >= 0) || (vL > 0.0 && vR <= 0.0 && ev.dir[j] <= 0)) {
+            te[j] = ev_locate(q, ev.kind[j], ev.level[j], ev.f, ev.gH, vL, vR);
+            fired |= 1u << j;
+            if (ev.term[j] && (!stop || te[j] < tstop)) { tstop = te[j]; stop = true; }
+        }
+    }
+    if (!fired) return false;
+#pragma unroll
+    for (int j = 0; j < kMaxEvents; j++)
+        if (stop && te[j] > tstop) fired &= ~(1u << j);
+    int cnt = ev.ne[i];
+    while (fired) {                                              // the earliest (te, j) first
+        int jm = -1;
+        double tm = 0.0;
+#pragma unroll
+        for (int j = 0; j < kMaxEvents; j++)
+            if (((fired >> j) & 1u) && (jm < 0 || te[j] < tm)) { jm = j; tm = te[j]; }
+        fired &= ~(1u << jm);
+        if (cnt < ev.cap) {
+            double v[4];
+            ev_point(q, tm, v);
+            const long long r = (long long)cnt * n + i;
+            ev.te[r] = tm; ev.ie[r] = jm + 1;
+#pragma unroll
+            for (int k = 0; k < 4; k++) ev.ye[((long long)cnt * 4 + k) * n + i] = v[k];
+        }
+        cnt++;
+    }
+    ev.ne[i] = cnt;
+    if (stop) ev_point(q, tstop, ystop);
+    return stop;
+}
+
+template <bool EV>
+__global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, Ode23Ev ev) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n) return;
     ode23_init(c, pkt_norm(a, i, 1, thr));
     pkt_store(s, i, a.n, c);
+    if constexpr (EV) {                                         // g_j(y0), and no records yet
+        const long long n = a.n;
+        const double v[4] = {a.y[0][i], a.y[1][i], a.y[2][i], a.y[3][i]};
+#pragma unroll
+        for (int j = 0; j < kMaxEvents; j++)
+            if (j < ev.nev) ev.vl[j * n + i] = ev_g(ev.kind[j], ev.level[j], ev.f, ev.gH, v);
+        const double nan = __longlong_as_double(0xffffffffffffffffLL);
+        for (int r = 0; r < ev.cap; r++) {
+            ev.te[(long long)r * n + i] = nan; ev.ie[(long long)r * n + i] = 0;
+#pragma unroll
+            for (int k = 0; k < 4; k++) ev.ye[((long long)r * 4 + k) * n + i] = nan;
+        }
+        ev.ne[i] = 0;
+    }
 }
 __global__ void bs23_stage_pkt_kernel(Bs23Args a, Ode23Pkt s, int stage) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -496,16 +628,31 @@ __global__ void rhs_pkt_kernel(Ode23Pkt s, int stage, long long n, const double*
 }
 // after a round's three stages: each unfinished packet's norm, its controller, its dense rows and its predicated accept.
 // Block-reduced into the report pair of this round: the packets still unfinished and the attempts the slowest of them
-// needs; the other pair is cleared for the next round.
-__global__ void __launch_bounds__(256) ode23_pkt_decide_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, int round) {
+// needs; the other pair is cleared for the next round.  EV: the accepted step's events; a terminal one stops the packet
+// at its te (status 2) with that record's state, and only the dense rows up to te are written.
+template <bool EV>
+__global__ void __launch_bounds__(256) ode23_pkt_decide_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, int round, Ode23Ev ev) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     int open = 0, batch = 0;
     if (i < a.n && !ode23_pkt_idle(s, i)) {
         pkt_load(s, i, a.n, c);
         ode23_control(c, pkt_norm(a, i, 0, thr));
         if (c.accepted) {
+            bool stop = false;
+            double tstop = 0.0, ystop[4];
+            if constexpr (EV) {
+                stop = pkt_events(a, i, c, ev, tstop, ystop);
+                if (stop && c.ntspan > 2)
+                    while (c.nxt_end > c.nxt && c.tspan[c.nxt_end - 1] > tstop) c.nxt_end--;
+            }
             if (c.ntspan > 2) bs23_rows_at(a, i, c);
             bs23_accept_at(a, i);
+            if (stop) {
+#pragma unroll
+                for (int k = 0; k < 4; k++) a.y[k][i] = ystop[k];
+                c.t = tstop;
+                c.status = 2;
+            }
         }
         pkt_store(s, i, a.n, c);
         if (!c.done && !c.status) { open = 1; batch = ode23_batch_estimate(c.tfinal, c.t, c.absh, c.hmax); }
@@ -586,8 +733,11 @@ void launch_bs23_accept_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t
     if (a.n > 0) bs23_accept_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl);
 }
 
-void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, cudaStream_t st) {
-    if (a.n > 0) ode23_pkt_begin_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr);
+void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, const Ode23Ev* ev,
+                            cudaStream_t st) {
+    if (a.n <= 0) return;
+    if (ev) ode23_pkt_begin_kernel<true><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, *ev);
+    else ode23_pkt_begin_kernel<false><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, Ode23Ev{});
 }
 void launch_bs23_stage_pkt(const Bs23Args& a, const Ode23Pkt& s, int stage, cudaStream_t st) {
     if (a.n > 0) bs23_stage_pkt_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, s, stage);
@@ -598,8 +748,11 @@ void launch_rhs_pkt(const Ode23Pkt& s, int stage, long long n, const double* k, 
     for (int i = 0; i < 6; i++) { e.p[i] = e6[i]; e2.p[i] = e1 ? e1[i] : nullptr; }
     if (n > 0) rhs_pkt_kernel<<<nblk(n, 256), 256, 0, st>>>(s, stage, n, k, l, e, e2, e1 != nullptr, f, gH, cgfac, fj[0], fj[1], fj[2], fj[3]);
 }
-void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, cudaStream_t st) {
-    if (a.n > 0) ode23_pkt_decide_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, round);
+void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, const Ode23Ev* ev,
+                             cudaStream_t st) {
+    if (a.n <= 0) return;
+    if (ev) ode23_pkt_decide_kernel<true><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, round, *ev);
+    else ode23_pkt_decide_kernel<false><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, round, Ode23Ev{});
 }
 
 void launch_fill(double* p, double v, long long n, cudaStream_t st) {

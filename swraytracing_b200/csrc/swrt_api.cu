@@ -92,6 +92,9 @@ struct swrt_handle {
     double* pkt_d = nullptr; int* pkt_i = nullptr; int64_t pkt_cap = 0;
     int* pkt_rep_host = nullptr;
     double* pkt_e1 = nullptr;
+    // swrt_ode23_packets_events: the event values and records of the packets (Ode23Ev's arrays)
+    double* ev_d = nullptr; size_t ev_dcap = 0;
+    int* ev_i = nullptr; size_t ev_icap = 0;
     double* edges_dev = nullptr; int edges_cap = 0;
     std::vector<double> edges_host;       // what edges_dev currently holds
     unsigned long long* counts_dev = nullptr; int counts_cap = 0;
@@ -708,7 +711,7 @@ int swrt_destroy(swrt_handle* h) {
     for (auto& row : h->bs_f) for (auto& p : row) dfree(p);
     dfree(h->ode_ctl);
     if (h->ode_host) cudaFreeHost(h->ode_host);
-    dfree(h->pkt_d); dfree(h->pkt_i); dfree(h->pkt_e1);
+    dfree(h->pkt_d); dfree(h->pkt_i); dfree(h->pkt_e1); dfree(h->ev_d); dfree(h->ev_i);
     if (h->pkt_rep_host) cudaFreeHost(h->pkt_rep_host);
     if (h->ode_ev) cudaEventDestroy(h->ode_ev);
     if (h->ev0) cudaEventDestroy(h->ev0);

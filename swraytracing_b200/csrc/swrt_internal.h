@@ -99,6 +99,21 @@ struct Ode23Pkt {
     int* report;                   // 2 x {unfinished packets, attempts to queue}: decide kernel of round r writes pair r & 1
 };
 __device__ __forceinline__ bool ode23_pkt_idle(const Ode23Pkt& s, long long i) { return s.flags[i] & (kPktDone | kPktStopped); }
+// swrt_ode23_packets_events: up to kMaxEvents level crossings of a function of the packet state, located on each accepted
+// step's ntrp23 cubic by the decide kernel (DESIGN.md section 11).  Passed by value; the arrays are per-packet SoA buffers
+// of the handle (n entries per row).
+constexpr int kMaxEvents = 8;
+struct Ode23Ev {
+    int nev, cap;                                        // events, records kept per packet
+    int kind[kMaxEvents], dir[kMaxEvents], term[kMaxEvents];
+    double level[kMaxEvents];
+    double f, gH;                                        // SWRT_EVENT_OMEGA: omega = sqrt(f^2 + gH (k^2 + l^2))
+    double* vl;                                          // nev x n: g_j at the last accepted state
+    double* te;                                          // cap x n (NaN when unused)
+    double* ye;                                          // cap x 4 x n (NaN when unused)
+    int* ie;                                             // cap x n: 1-based event index (0 when unused)
+    int* ne;                                             // n: events found (may exceed cap)
+};
 // the alphas of `stage` (selected, not indexed: a run-time index would move the kernel argument to local memory)
 __device__ __forceinline__ const double* ode23_pkt_alpha(const Ode23Pkt& s, int stage) {
     return stage == 0 ? s.al[0] : stage == 1 ? s.al[1] : s.al[2];
@@ -304,11 +319,15 @@ cudaError_t launch_lagrange_eval_dev(const LagArgs& a, const Ode23Ctl* ctl, int 
 // swrt_ode23_packets: `k` holds the per-solve constants (controller section zero, t = t0).  begin: the rh norm and the
 // initial step of every packet from f1; stage / RHS / decide as their swrt_ode23 counterparts with each packet's own h and
 // alphas.  With e1 set (SPECTRAL, two frames) the RHS blends e (alpha 0) and e1 (alpha 1) at the packet's alpha.
-void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, cudaStream_t st);
+// With ev set, begin also seeds the event values and clears the records, and decide locates and records the events of
+// every accepted step and applies a terminal stop.
+void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, const Ode23Ev* ev,
+                            cudaStream_t st);
 void launch_bs23_stage_pkt(const Bs23Args& a, const Ode23Pkt& s, int stage, cudaStream_t st);
 void launch_rhs_pkt(const Ode23Pkt& s, int stage, long long n, const double* k, const double* l, const double* const* e6,
                     const double* const* e1, double f, double gH, double cgfac, double* const fj[4], cudaStream_t st);
-void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, cudaStream_t st);
+void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, const Ode23Ev* ev,
+                             cudaStream_t st);
 cudaError_t launch_nufft_eval_pkt(const NufftArgs& a, const double2* grid1, const Ode23Pkt& s, int stage, cudaStream_t st);
 cudaError_t launch_lagrange_eval_pkt(const LagArgs& a, const Ode23Pkt& s, int stage, cudaStream_t st);
 // (rtol/err)^(1/3) as glibc's correctly rounded-in-practice pow gives it (host and device, misc_kernels.cu)

@@ -108,14 +108,16 @@ class ShardedEnsemble:
     def step(self, scheme, dt, nsteps, alpha0=0.0, dalpha=0.0):
         self.engine.step(scheme, dt, nsteps, alpha0, dalpha)
 
-    def ode23(self, tspan, tmax, rtol=1e-3, atol=1e-6, per_packet=False):
+    def ode23(self, tspan, tmax, rtol=1e-3, atol=1e-6, per_packet=False, events=None, ev_cap=4):
         """the reference's per-flow-step ode23 solve over ALL shards: the error norm is MAX-all-reduced so
         that every rank accepts/rejects the same steps (the reference's norm couples all packets).
         ``per_packet=True``: every packet under its own controller (``Engine.ode23_packets``) on the local shard, with no
-        collective; the returned counts are this rank's."""
+        collective; the returned counts are this rank's, and so are the event records with ``events`` (per-packet only)."""
         from .reference_api import ode23
+        if events is not None and not per_packet:
+            raise ValueError("ode23: events need per_packet=True (the coupled solve has no events)")
         if per_packet:
-            return ode23(self.engine, tspan, tmax, rtol, atol, per_packet=True)
+            return ode23(self.engine, tspan, tmax, rtol, atol, per_packet=True, events=events, ev_cap=ev_cap)
         return ode23(self.engine, tspan, tmax, rtol, atol, reduce_max=self._allreduce_max)
 
     def _allreduce_max(self, v):

@@ -18,8 +18,15 @@ MODE_SPECTRAL, MODE_LAGRANGE6, MODE_NUFFT = 0, 1, 2
 SCHEME_LEAPFROG, SCHEME_RK4_PACKET, SCHEME_RK4_XKA = 0, 1, 2
 HIST_INTRINSIC, HIST_ABSOLUTE = 0, 1
 FLAG_RHS_GH = 1
+EVENT_X, EVENT_Y, EVENT_K, EVENT_L, EVENT_KMAG, EVENT_OMEGA = 0, 1, 2, 3, 4, 5
+MAX_EVENTS = 8
 
 _dp = C.POINTER(C.c_double)
+
+
+class _Event(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("direction", C.c_int32), ("terminal", C.c_int32), ("reserved", C.c_int32),
+                ("level", C.c_double)]
 
 
 class SwrtError(RuntimeError):
@@ -66,6 +73,9 @@ SIGNATURES = {
     "swrt_ode23": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int64), _dp, C.c_int]),
     "swrt_ode23_packets": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int32), _dp,
                                      C.POINTER(C.c_int64)]),
+    "swrt_ode23_packets_events": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, C.POINTER(_Event), C.c_int,
+                                            C.c_int, _dp, C.POINTER(C.c_int32), _dp, _dp, _dp, C.POINTER(C.c_int32),
+                                            C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
     "swrt_hist_omega_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_launch": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_wait": (C.c_int, [C.c_void_p]),
@@ -353,27 +363,49 @@ class Engine:
             out["h"] = hs[:min(st[0], hs.size)].copy()
         return out
 
-    def ode23_packets(self, tspan, tmax, rtol=1e-3, atol=1e-6):
+    def ode23_packets(self, tspan, tmax, rtol=1e-3, atol=1e-6, events=None, ev_cap=4):
         """``ode23`` once per packet (swrt_ode23_packets): every packet under its own step-size controller, exactly as
         ``ode23`` advances an ensemble holding that packet alone, so a packet's result does not depend on the others.
         Returns ``ode23``'s dict with ``nsteps``, ``nfailed`` and ``nfevals`` summed over packets, plus ``stopped``
         (packets whose step size fell below hmin: they keep their last accepted state, the others carry on),
         ``host_waits``, and the per-packet arrays ``steps``, ``rejected``, ``status`` (0 reached tfinal, 1 stopped) and
         ``t_end`` (where each packet stopped).  ``Y`` when ``tspan`` has more than two entries (NaN in the rows a stopped
-        packet did not reach)."""
+        packet did not reach).
+
+        ``events``: MATLAB's ``odeset('Events', ...)`` per packet (swrt_ode23_packets_events), a list of
+        ``(kind, level, direction=0, terminal=False)`` with ``kind`` one of ``EVENT_X``, ``EVENT_Y``, ``EVENT_K``,
+        ``EVENT_L``, ``EVENT_KMAG`` (|k|) and ``EVENT_OMEGA`` (omega as ``omega()`` computes it); tspan must be strictly
+        increasing.  The result then also holds ``te`` (ev_cap, n), ``ye`` (ev_cap, 4, n) and ``ie`` (ev_cap, n, 1-based
+        event index): each packet's first ``ev_cap`` records in ascending (te, ie) order, NaN / 0 where unused; ``ne``
+        (events found per packet, may exceed ev_cap); ``events`` (their total) and ``terminated`` (packets stopped by a
+        terminal event: status 2, state and ``t_end`` those of the event)."""
         ts = _f64(tspan)
         dense = ts.size > 2
         Y = np.empty((ts.size, 4, self.n)) if dense else None
         pstat = np.empty((3, self.n), dtype=np.int32)          # the C side's n x 3 column-major block
         t_end = np.empty(self.n)
-        st = (C.c_int64 * 5)()
-        self._check(self.lib.swrt_ode23_packets(self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol),
-                                                _ptr(Y) if dense else None, pstat.ctypes.data_as(C.POINTER(C.c_int32)),
-                                                _ptr(t_end), st))
+        i32 = C.POINTER(C.c_int32)
+        if events is None:
+            st = (C.c_int64 * 5)()
+            self._check(self.lib.swrt_ode23_packets(self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol),
+                                                    _ptr(Y) if dense else None, pstat.ctypes.data_as(i32), _ptr(t_end), st))
+        else:
+            evs = [tuple(e) + (0, False)[len(e) - 2:] for e in events]      # direction 0, not terminal by default
+            arr = (_Event * max(len(evs), 1))(*[_Event(int(kind), int(d), int(term), 0, float(level)) for kind, level, d, term in evs])
+            cap = max(int(ev_cap), 0)
+            te, ye, ie = np.empty((cap, self.n)), np.empty((cap, 4, self.n)), np.empty((cap, self.n), dtype=np.int32)
+            ne = np.empty(self.n, dtype=np.int32)
+            st = (C.c_int64 * 7)()
+            self._check(self.lib.swrt_ode23_packets_events(
+                self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol), arr, len(evs), int(ev_cap),
+                _ptr(Y) if dense else None, pstat.ctypes.data_as(i32), _ptr(t_end), _ptr(te), _ptr(ye), ie.ctypes.data_as(i32),
+                ne.ctypes.data_as(i32), st))
         out = {"nsteps": st[0], "nfailed": st[1], "nfevals": st[2], "t": float(ts[-1]), "stopped": st[3], "host_waits": st[4],
                "steps": pstat[0].copy(), "rejected": pstat[1].copy(), "status": pstat[2].copy(), "t_end": t_end}
         if dense:
             out["Y"] = Y
+        if events is not None:
+            out.update(te=te, ye=ye, ie=ie, ne=ne, events=st[5], terminated=st[6])
         return out
 
     # -- diagnostics --

@@ -297,7 +297,7 @@ def omega(k, f, gH):
 # ode23 -- the production drivers' integrator (qgsw_raytrace.m:149, qg2layersw_raytrace.m:195)
 # ------------------------------------------------------------------------------------------------
 
-def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=False, per_packet=False):
+def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=False, per_packet=False, events=None, ev_cap=4):
     """``[~, Y] = ode23(ray_ode, [0 dt], y0)`` for the packets resident in ``target`` (an Engine):
     MATLAB's ode23 = Bogacki-Shampine 3(2) pair with first-same-as-last, restated from its published
     description (Shampine & Reichelt, "The MATLAB ODE Suite", SIAM J. Sci. Comput. 18, 1997; MATLAB
@@ -322,11 +322,17 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=
 
     ``per_packet=True`` solves every packet under its own controller instead (``Engine.ode23_packets``,
     swrt_ode23_packets): what MATLAB gives when ``ode23`` is called once per packet.  Nothing couples the packets, so
-    ``reduce_max`` is refused with it; a packet whose step size falls below hmin stops alone (``stopped``, ``status``)."""
+    ``reduce_max`` is refused with it; a packet whose step size falls below hmin stops alone (``stopped``, ``status``).
+    ``events`` / ``ev_cap`` (per-packet solve only: the coupled solve has no events) locate level crossings of each
+    packet's state as MATLAB's ``odeset('Events', ...)`` would, see ``Engine.ode23_packets``."""
+    if events is not None and not per_packet:
+        raise ValueError("ode23: events need per_packet=True (the coupled solve has no events)")
     if per_packet:
         if reduce_max is not None:
             raise ValueError("ode23: per_packet=True needs no reduce_max (the packets are not coupled)")
-        return target.ode23_packets(tspan, tmax, rtol, atol)
+        if events is None:
+            return target.ode23_packets(tspan, tmax, rtol, atol)
+        return target.ode23_packets(tspan, tmax, rtol, atol, events=events, ev_cap=ev_cap)
     if on_device and reduce_max is None:
         return target.ode23(tspan, tmax, rtol, atol)
     red = reduce_max if reduce_max is not None else (lambda v: v)
