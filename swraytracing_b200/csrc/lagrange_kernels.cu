@@ -233,46 +233,20 @@ __global__ void __launch_bounds__(128, TWO ? SWRT_LAG_TWO_MINB : SWRT_LAG_MINB) 
     }
 }
 
-// swrt_ode23's evaluation: the frames lag_frames picks for the controller's alpha (one grid at alpha 0 or 1, else both
-// blended as above); nothing to do once the solve is done
-template <int NPL>
-__global__ void __launch_bounds__(128, SWRT_LAG_TWO_MINB) lagrange_eval_dev_kernel(const LagArgs a, const Ode23Ctl* ctl, int stage) {
-    if (ode23_idle(ctl)) return;
-    const double al = a.grid2 ? ctl->al[stage] : 0.0;
+// swrt_ode23 / swrt_ode23_packets' evaluation at the view's alpha of `stage`: the frames lag_frames picks for that alpha
+// (one grid at alpha 0 or 1, else both blended as above), per packet.  gather_pair / gather_pair2 do no shuffles, so the
+// quads of a warp may take different branches; idle packets join make_stencil_quad and store nothing.
+template <int NPL, class View>
+__global__ void __launch_bounds__(128, SWRT_LAG_TWO_MINB) lagrange_eval_ode23_kernel(const LagArgs a, const View v, int stage) {
+    if (v.done()) return;
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long p = t >> 2;
     const int lane = threadIdx.x & 31, q = lane & 3, qb = lane & ~3;
     const long long pc = p < a.n ? p : a.n - 1;
-    Stencil s;
-    make_stencil_quad(a.xin[pc], a.yin[pc], a.dx, a.nx, a.bump, q, qb, s);
-    double F0, F1;
-    if (al == 0.0 || al == 1.0) {
-        gather_pair<NPL>(al == 0.0 ? a.grid : a.grid2, a.nx, s, q, F0, F1);
-    } else {
-        double G0, G1;
-        gather_pair2<NPL>(a.grid, a.grid2, a.nx, s, q, F0, F1, G0, G1);
-        F0 = (1.0 - al) * F0 + al * G0;
-        F1 = (1.0 - al) * F1 + al * G1;
-    }
-    if (p < a.n) {
-        if (2 * q < NPL && a.out[2 * q]) a.out[2 * q][p] = F0;
-        if (2 * q + 1 < NPL && a.out[2 * q + 1]) a.out[2 * q + 1][p] = F1;
-    }
-}
-
-// swrt_ode23_packets' evaluation: the same choice per packet from its own alpha.  gather_pair / gather_pair2 do no
-// shuffles, so the quads of a warp may take different branches; finished packets join make_stencil_quad and store nothing.
-template <int NPL>
-__global__ void __launch_bounds__(128, SWRT_LAG_TWO_MINB) lagrange_eval_pkt_kernel(const LagArgs a, const Ode23Pkt s, int stage) {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long p = t >> 2;
-    const int lane = threadIdx.x & 31, q = lane & 3, qb = lane & ~3;
-    const long long pc = p < a.n ? p : a.n - 1;
-    const bool store = p < a.n && !ode23_pkt_idle(s, pc);
-    const double al = a.grid2 ? ode23_pkt_alpha(s, stage)[pc] : 0.0;
+    const double al = a.grid2 ? v.alpha(stage, pc) : 0.0;
     Stencil st;
     make_stencil_quad(a.xin[pc], a.yin[pc], a.dx, a.nx, a.bump, q, qb, st);
-    if (!store) return;
+    if (v.idle(pc)) return;
     double F0, F1;
     if (al == 0.0 || al == 1.0) {
         gather_pair<NPL>(al == 0.0 ? a.grid : a.grid2, a.nx, st, q, F0, F1);
@@ -282,8 +256,10 @@ __global__ void __launch_bounds__(128, SWRT_LAG_TWO_MINB) lagrange_eval_pkt_kern
         F0 = (1.0 - al) * F0 + al * G0;
         F1 = (1.0 - al) * F1 + al * G1;
     }
-    if (2 * q < NPL && a.out[2 * q]) a.out[2 * q][p] = F0;
-    if (2 * q + 1 < NPL && a.out[2 * q + 1]) a.out[2 * q + 1][p] = F1;
+    if (p < a.n) {
+        if (2 * q < NPL && a.out[2 * q]) a.out[2 * q][p] = F0;
+        if (2 * q + 1 < NPL && a.out[2 * q + 1]) a.out[2 * q + 1][p] = F1;
+    }
 }
 
 // ode_symplectic.m:13-21,33-37 with scheme.U / grad_U = six Lagrange interpolations at x1
@@ -496,23 +472,16 @@ cudaError_t launch_lagrange_eval(const LagArgs& a, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_lagrange_eval_dev(const LagArgs& a, const Ode23Ctl* ctl, int stage, cudaStream_t st) {
+template <class View> cudaError_t launch_lagrange_eval_ode23(const LagArgs& a, const View& v, int stage, cudaStream_t st) {
     if (a.n <= 0) return cudaSuccess;
     const unsigned nb = blocks_for(4 * a.n, 128);
-    if (a.npl == 6) lagrange_eval_dev_kernel<6><<<nb, 128, 0, st>>>(a, ctl, stage);
-    else if (a.npl == 7) lagrange_eval_dev_kernel<7><<<nb, 128, 0, st>>>(a, ctl, stage);
+    if (a.npl == 6) lagrange_eval_ode23_kernel<6><<<nb, 128, 0, st>>>(a, v, stage);
+    else if (a.npl == 7) lagrange_eval_ode23_kernel<7><<<nb, 128, 0, st>>>(a, v, stage);
     else return cudaErrorInvalidValue;
     return cudaGetLastError();
 }
-
-cudaError_t launch_lagrange_eval_pkt(const LagArgs& a, const Ode23Pkt& s, int stage, cudaStream_t st) {
-    if (a.n <= 0) return cudaSuccess;
-    const unsigned nb = blocks_for(4 * a.n, 128);
-    if (a.npl == 6) lagrange_eval_pkt_kernel<6><<<nb, 128, 0, st>>>(a, s, stage);
-    else if (a.npl == 7) lagrange_eval_pkt_kernel<7><<<nb, 128, 0, st>>>(a, s, stage);
-    else return cudaErrorInvalidValue;
-    return cudaGetLastError();
-}
+template cudaError_t launch_lagrange_eval_ode23(const LagArgs&, const Ode23CtlView&, int, cudaStream_t);
+template cudaError_t launch_lagrange_eval_ode23(const LagArgs&, const Ode23PktView&, int, cudaStream_t);
 
 cudaError_t launch_lagrange_leapfrog(const LagArgs& a, cudaStream_t st) {
     if (a.n <= 0) return cudaSuccess;

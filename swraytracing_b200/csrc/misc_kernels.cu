@@ -29,17 +29,23 @@ __device__ __forceinline__ void rhs_at(long long i, const double* __restrict__ k
     if (dkdt) dkdt[i] = -__dadd_rn(__dmul_rn(e.p[2][i], kk), __dmul_rn(e.p[4][i], ll));
     if (dldt) dldt[i] = -__dadd_rn(__dmul_rn(e.p[3][i], kk), __dmul_rn(e.p[5][i], ll));
 }
-__global__ void rhs_kernel(long long n, const double* __restrict__ k, const double* __restrict__ l, E6 e, double f,
-                           double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt) {
+// the view's idle packets write nothing.  two: the planes come from two evaluations, e at alpha 0 and e1 at alpha 1;
+// between the frames they are blended at the packet's alpha, in place in e (packet i's entries are this thread's own scratch)
+template <class View>
+__global__ void rhs_kernel(View v, int stage, long long n, const double* __restrict__ k, const double* __restrict__ l, E6 e,
+                           E6 e1, bool two, double f, double gH, double cgfac, double* dxdt, double* dydt, double* dkdt,
+                           double* dldt) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    rhs_at(i, k, l, e, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
-}
-__global__ void rhs_dev_kernel(const Ode23Ctl* ctl, long long n, const double* __restrict__ k, const double* __restrict__ l, E6 e,
-                               double f, double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || ode23_idle(ctl)) return;
-    rhs_at(i, k, l, e, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
+    if (i >= n || v.done() || v.idle(i)) return;
+    const double al = two ? v.alpha(stage, i) : 0.0;
+    E6 src;
+#pragma unroll
+    for (int c = 0; c < 6; c++) {
+        src.p[c] = al == 1.0 ? e1.p[c] : e.p[c];
+        if (al != 0.0 && al != 1.0)
+            const_cast<double*>(e.p[c])[i] = __dadd_rn(__dmul_rn(__dsub_rn(1.0, al), e.p[c][i]), __dmul_rn(al, e1.p[c][i]));
+    }
+    rhs_at(i, k, l, src, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
 }
 
 __global__ void omega_kernel(long long n, const double* __restrict__ k, const double* __restrict__ l,
@@ -232,21 +238,17 @@ __device__ __forceinline__ void bs23_stage_at(const Bs23Args& a, long long i, do
         a.yt[c][i] = __dadd_rn(a.y[c][i], acc);
     }
 }
-__global__ void bs23_stage_kernel(Bs23Args a, double hb1, double hb2, double hb3) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n) return;
-    bs23_stage_at(a, i, hb1, hb2, hb3);
-}
-// the same stages with h from the controller: hB(:,stage) as swrt_bs23_attempt forms it on the host
+// hB(:,stage) with each product h*B rounded on its own: A = [1/2 3/4 1], B = [1/2 0 2/9; 0 3/4 1/3; 0 0 4/9; 0 0 0]
 __device__ __forceinline__ void bs23_stage_h(const Bs23Args& a, long long i, int stage, double h) {
     if (stage == 0) bs23_stage_at(a, i, __dmul_rn(h, 0.5), 0.0, 0.0);
     else if (stage == 1) bs23_stage_at(a, i, 0.0, __dmul_rn(h, 0.75), 0.0);
     else bs23_stage_at(a, i, __dmul_rn(h, 2.0 / 9.0), __dmul_rn(h, 1.0 / 3.0), __dmul_rn(h, 4.0 / 9.0));
 }
-__global__ void bs23_stage_dev_kernel(Bs23Args a, const Ode23Ctl* ctl, int stage) {
+template <class View>
+__global__ void bs23_stage_kernel(Bs23Args a, View v, int stage) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n || ode23_idle(ctl)) return;
-    bs23_stage_h(a, i, stage, ctl->h);
+    if (i >= a.n || v.done() || v.idle(i)) return;
+    bs23_stage_h(a, i, stage, v.h(i));
 }
 // err = max_i |(f*E)_i| / max(max(|y_i|,|ynew_i|), threshold)   (without the absh factor);
 // mode 1: rh = max_i |f1_i| / max(|y_i|, threshold) for the initial step size
@@ -284,18 +286,23 @@ __device__ __forceinline__ void bs23_norm_body(const Bs23Args& a, int mode, doub
         atomicMax(out, (unsigned long long)__double_as_longlong(v));     // non-negative doubles order like their bit patterns
     }
 }
-__global__ void __launch_bounds__(256) bs23_norm_kernel(Bs23Args a, int mode, double thr, unsigned long long* out) {
-    bs23_norm_body(a, mode, thr, out);
+// MODE a constant: a run-time mode keeps both ratios' registers live (54 instead of 32)
+template <int MODE, class View>
+__global__ void __launch_bounds__(256) bs23_norm_kernel(Bs23Args a, View v, double thr, unsigned long long* out) {
+    if (v.done()) return;
+    bs23_norm_body(a, MODE, thr, out);
 }
-__global__ void __launch_bounds__(256) bs23_norm_dev_kernel(Bs23Args a, const Ode23Ctl* ctl, double thr, unsigned long long* out) {
-    if (ode23_idle(ctl)) return;
-    bs23_norm_body(a, 0, thr, out);
-}
-__global__ void bs23_accept_kernel(Bs23Args a) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n) return;
+// y <- ynew, f1 <- f4 (first same as last)
+__device__ __forceinline__ void bs23_accept_at(const Bs23Args& a, long long i) {
 #pragma unroll
     for (int c = 0; c < 4; c++) { a.y[c][i] = a.yt[c][i]; a.f[0][c][i] = a.f[3][c][i]; }
+}
+// predicated on the controller's decision
+template <class View>
+__global__ void bs23_accept_kernel(Bs23Args a, View v) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n || !v.accepted()) return;
+    bs23_accept_at(a, i);
 }
 // ntrp23: out = y + (f1 w1 + f2 w2 + f3 w3 + f4 w4), w_j = hstep * (BI_j . [s s^2 s^3])
 struct Bs23Interp { double w[4]; double* out[4]; };
@@ -434,17 +441,6 @@ __global__ void bs23_interp_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
     if (i >= a.n || !ctl->accepted) return;
     bs23_rows_at(a, i, *ctl);
 }
-// y <- ynew, f1 <- f4 (first same as last), predicated on the controller's decision
-__device__ __forceinline__ void bs23_accept_at(const Bs23Args& a, long long i) {
-#pragma unroll
-    for (int c = 0; c < 4; c++) { a.y[c][i] = a.yt[c][i]; a.f[0][c][i] = a.f[3][c][i]; }
-}
-__global__ void bs23_accept_dev_kernel(Bs23Args a, const Ode23Ctl* ctl) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n || !ctl->accepted) return;
-    bs23_accept_at(a, i);
-}
-
 // ---- swrt_ode23_packets: the same rules, one controller per packet ---------------------------------------------------
 __device__ __forceinline__ void pkt_load(const Ode23Pkt& s, long long i, long long n, Ode23Ctl& c) {
     c.t = s.t[i]; c.absh = s.absh[i]; c.h = s.h[i]; c.hmin = s.hmin[i]; c.tnew = s.tnew[i];
@@ -604,28 +600,6 @@ __global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, doubl
         ev.ne[i] = 0;
     }
 }
-__global__ void bs23_stage_pkt_kernel(Bs23Args a, Ode23Pkt s, int stage) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n || ode23_pkt_idle(s, i)) return;
-    bs23_stage_h(a, i, stage, s.h[i]);
-}
-// two: the planes come from two evaluations, e at alpha 0 and e1 at alpha 1; between the frames they are blended at the
-// packet's alpha, in place in e (packet i's entries are this thread's own scratch)
-__global__ void rhs_pkt_kernel(Ode23Pkt s, int stage, long long n, const double* __restrict__ k, const double* __restrict__ l,
-                               E6 e, E6 e1, bool two, double f, double gH, double cgfac, double* dxdt, double* dydt,
-                               double* dkdt, double* dldt) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || ode23_pkt_idle(s, i)) return;
-    const double al = two ? ode23_pkt_alpha(s, stage)[i] : 0.0;
-    E6 src;
-#pragma unroll
-    for (int c = 0; c < 6; c++) {
-        src.p[c] = al == 1.0 ? e1.p[c] : e.p[c];
-        if (al != 0.0 && al != 1.0)
-            const_cast<double*>(e.p[c])[i] = __dadd_rn(__dmul_rn(__dsub_rn(1.0, al), e.p[c][i]), __dmul_rn(al, e1.p[c][i]));
-    }
-    rhs_at(i, k, l, src, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
-}
 // after a round's three stages: each unfinished packet's norm, its controller, its dense rows and its predicated accept.
 // Block-reduced into the report pair of this round: the packets still unfinished and the attempts the slowest of them
 // needs; the other pair is cleared for the next round.  EV: the accepted step's events; a terminal one stops the packet
@@ -696,41 +670,44 @@ void launch_bs23_interp(const Bs23Args& a, const double w[4], double* const out[
     for (int j = 0; j < 4; j++) { q.w[j] = w[j]; q.out[j] = out[j]; }
     if (a.n > 0) bs23_interp_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, q);
 }
-void launch_bs23_stage(const Bs23Args& a, double hb1, double hb2, double hb3, cudaStream_t st) {
-    if (a.n > 0) bs23_stage_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, hb1, hb2, hb3);
+template <class View> void launch_bs23_stage(const Bs23Args& a, const View& v, int stage, cudaStream_t st) {
+    if (a.n > 0) bs23_stage_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, v, stage);
 }
-void launch_bs23_norm(const Bs23Args& a, int mode, double thr, unsigned long long* out, cudaStream_t st) {
-    cudaMemsetAsync(out, 0, sizeof(unsigned long long), st);
+template <int MODE, class View>
+void launch_bs23_norm(const Bs23Args& a, const View& v, double thr, unsigned long long* out, cudaStream_t st) {
     if (a.n <= 0) return;
     unsigned nb = nblk(a.n, 256 * 4);
     if (nb > 148 * 8) nb = 148 * 8;
-    bs23_norm_kernel<<<nb, 256, 0, st>>>(a, mode, thr, out);
+    bs23_norm_kernel<MODE><<<nb, 256, 0, st>>>(a, v, thr, out);
 }
-void launch_bs23_accept(const Bs23Args& a, cudaStream_t st) {
-    if (a.n > 0) bs23_accept_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a);
+template <class View> void launch_bs23_accept(const Bs23Args& a, const View& v, cudaStream_t st) {
+    if (a.n > 0) bs23_accept_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, v);
 }
-void launch_bs23_stage_dev(const Bs23Args& a, const Ode23Ctl* ctl, int stage, cudaStream_t st) {
-    if (a.n > 0) bs23_stage_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl, stage);
+template <class View>
+void launch_rhs(const View& v, int stage, long long n, const double* k, const double* l, const double* const* e6,
+                const double* const* e1, double f, double gH, double cgfac, double* const fj[4], cudaStream_t st) {
+    E6 e, e2;
+    for (int i = 0; i < 6; i++) { e.p[i] = e6[i]; e2.p[i] = e1 ? e1[i] : nullptr; }
+    if (n > 0) rhs_kernel<<<nblk(n, 256), 256, 0, st>>>(v, stage, n, k, l, e, e2, e1 != nullptr, f, gH, cgfac, fj[0], fj[1], fj[2], fj[3]);
 }
-void launch_rhs_dev(const Ode23Ctl* ctl, long long n, const double* k, const double* l, const double* const* e6, double f,
-                    double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt, cudaStream_t st) {
-    E6 e; for (int i = 0; i < 6; i++) e.p[i] = e6[i];
-    if (n > 0) rhs_dev_kernel<<<nblk(n, 256), 256, 0, st>>>(ctl, n, k, l, e, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
-}
-// the norm word is zeroed by the controller kernel that consumes it (and by swrt_bs23_begin's launch before the solve)
-void launch_bs23_norm_dev(const Bs23Args& a, const Ode23Ctl* ctl, double thr, unsigned long long* out, cudaStream_t st) {
-    if (a.n <= 0) return;
-    unsigned nb = nblk(a.n, 256 * 4);
-    if (nb > 148 * 8) nb = 148 * 8;
-    bs23_norm_dev_kernel<<<nb, 256, 0, st>>>(a, ctl, thr, out);
-}
+template void launch_bs23_stage(const Bs23Args&, const Ode23ValView&, int, cudaStream_t);
+template void launch_bs23_stage(const Bs23Args&, const Ode23CtlView&, int, cudaStream_t);
+template void launch_bs23_stage(const Bs23Args&, const Ode23PktView&, int, cudaStream_t);
+template void launch_bs23_norm<0>(const Bs23Args&, const Ode23ValView&, double, unsigned long long*, cudaStream_t);
+template void launch_bs23_norm<1>(const Bs23Args&, const Ode23ValView&, double, unsigned long long*, cudaStream_t);
+template void launch_bs23_norm<0>(const Bs23Args&, const Ode23CtlView&, double, unsigned long long*, cudaStream_t);
+template void launch_bs23_accept(const Bs23Args&, const Ode23ValView&, cudaStream_t);
+template void launch_bs23_accept(const Bs23Args&, const Ode23CtlView&, cudaStream_t);
+template void launch_rhs(const Ode23ValView&, int, long long, const double*, const double*, const double* const*, const double* const*,
+                         double, double, double, double* const[4], cudaStream_t);
+template void launch_rhs(const Ode23CtlView&, int, long long, const double*, const double*, const double* const*, const double* const*,
+                         double, double, double, double* const[4], cudaStream_t);
+template void launch_rhs(const Ode23PktView&, int, long long, const double*, const double*, const double* const*, const double* const*,
+                         double, double, double, double* const[4], cudaStream_t);
 void launch_ode23_init(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st) { ode23_init_kernel<<<1, 1, 0, st>>>(ctl, norm); }
 void launch_ode23_control(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st) { ode23_control_kernel<<<1, 1, 0, st>>>(ctl, norm); }
 void launch_bs23_interp_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st) {
     if (a.n > 0) bs23_interp_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl);
-}
-void launch_bs23_accept_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st) {
-    if (a.n > 0) bs23_accept_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl);
 }
 
 void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, const Ode23Ev* ev,
@@ -738,15 +715,6 @@ void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl
     if (a.n <= 0) return;
     if (ev) ode23_pkt_begin_kernel<true><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, *ev);
     else ode23_pkt_begin_kernel<false><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, Ode23Ev{});
-}
-void launch_bs23_stage_pkt(const Bs23Args& a, const Ode23Pkt& s, int stage, cudaStream_t st) {
-    if (a.n > 0) bs23_stage_pkt_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, s, stage);
-}
-void launch_rhs_pkt(const Ode23Pkt& s, int stage, long long n, const double* k, const double* l, const double* const* e6,
-                    const double* const* e1, double f, double gH, double cgfac, double* const fj[4], cudaStream_t st) {
-    E6 e, e2;
-    for (int i = 0; i < 6; i++) { e.p[i] = e6[i]; e2.p[i] = e1 ? e1[i] : nullptr; }
-    if (n > 0) rhs_pkt_kernel<<<nblk(n, 256), 256, 0, st>>>(s, stage, n, k, l, e, e2, e1 != nullptr, f, gH, cgfac, fj[0], fj[1], fj[2], fj[3]);
 }
 void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, const Ode23Ev* ev,
                              cudaStream_t st) {
@@ -757,11 +725,6 @@ void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ct
 
 void launch_fill(double* p, double v, long long n, cudaStream_t st) {
     if (n > 0) fill_kernel<<<nblk(n, 256), 256, 0, st>>>(p, v, n);
-}
-void launch_rhs(long long n, const double* k, const double* l, const double* const* e6, double f, double gH, double cgfac,
-                double* dxdt, double* dydt, double* dkdt, double* dldt, cudaStream_t st) {
-    E6 e; for (int i = 0; i < 6; i++) e.p[i] = e6[i];
-    if (n > 0) rhs_kernel<<<nblk(n, 256), 256, 0, st>>>(n, k, l, e, f, gH, cgfac, dxdt, dydt, dkdt, dldt);
 }
 void launch_omega(long long n, const double* k, const double* l, const double* u, const double* v, double f, double gH,
                   double* omega, double* Omega_abs, cudaStream_t st) {

@@ -330,6 +330,20 @@ void fill_psi_args(const swrt_handle* h, double alpha, SpecArgs& a) {
 
 int active_nufft_grid(swrt_handle* h, double alpha, const double** out, const double** hout);
 void fill_nufft_args(const swrt_handle* h, const double* grid, NufftArgs& a);
+// SpecArgs / SpecRk4Args: grid spacing, nx, and 1/nx when nx is a power of two (exact), else 0
+template <class A> void fill_spec_geom(const swrt_handle* h, A& a) {
+    a.dx = h->p.L / h->p.nx; a.nxd = (double)h->p.nx;
+    a.inv_nx = (h->p.nx & (h->p.nx - 1)) == 0 ? 1.0 / h->p.nx : 0.0;
+}
+// LagArgs: the grid geometry (the grids themselves are the caller's)
+void fill_lag_args(const swrt_handle* h, LagArgs& a) {
+    a.nx = h->p.nx; a.npl = h->grid_npl; a.dx = h->p.L / h->p.nx; a.bump = h->p.bump;
+}
+// LagArgs / NufftArgs of an evaluation: n device positions (xd, yd); out[c] receives the c-th plane of subset `sub`
+template <class A> void fill_eval_io(A& a, int sub, int64_t n, const double* xd, const double* yd, double* const* out) {
+    a.n = n; a.xin = xd; a.yin = yd;
+    for (int c = 0; c < kSubsetN[sub]; c++) a.out[kSubsetIds[sub][c]] = out[c];
+}
 
 // evaluate subset planes at device positions into device outputs out[c] (c indexes subset planes)
 int eval_dev(swrt_handle* h, int sub, double alpha, int64_t n, const double* xd, const double* yd,
@@ -344,8 +358,7 @@ int eval_dev(swrt_handle* h, int sub, double alpha, int64_t n, const double* xd,
         if (psi) fill_psi_args(h, alpha, a);
         a.n = n; a.xin = xd; a.yin = yd;
         for (int c = 0; c < kSubsetN[sub]; c++) a.out[c] = out[c];
-        a.dx = h->p.L / h->p.nx; a.nxd = (double)h->p.nx;
-        a.inv_nx = (h->p.nx & (h->p.nx - 1)) == 0 ? 1.0 / h->p.nx : 0.0;
+        fill_spec_geom(h, a);
         if ((rc = ensure_twid(h, a.g, &a.twid))) return rc;
         CU(h, launch_spectral(a, SPEC_EVAL, mt, h->num_sms, h->stream));
         h->launches++;
@@ -361,8 +374,7 @@ int eval_dev(swrt_handle* h, int sub, double alpha, int64_t n, const double* xd,
         NufftArgs a{};
         fill_nufft_args(h, g, a);
         a.hgrid = gh;
-        a.n = n; a.xin = xd; a.yin = yd;
-        for (int c = 0; c < kSubsetN[sub]; c++) a.out[kSubsetIds[sub][c]] = out[c];
+        fill_eval_io(a, sub, n, xd, yd, out);
         CU(h, launch_nufft_eval(a, h->stream));
         h->launches++;
         return SWRT_OK;
@@ -371,9 +383,8 @@ int eval_dev(swrt_handle* h, int sub, double alpha, int64_t n, const double* xd,
     int rc = lag_frames(h, alpha, true, a);
     if (rc) return rc;
     REQUIRE(h, !(sub == SUB_SEVEN || sub == SUB_UVH) || h->grid_npl == 7, SWRT_ERR_STATE, "no H grid was set");
-    a.nx = h->p.nx; a.npl = h->grid_npl; a.n = n; a.xin = xd; a.yin = yd;
-    for (int c = 0; c < kSubsetN[sub]; c++) a.out[kSubsetIds[sub][c]] = out[c];
-    a.dx = h->p.L / h->p.nx; a.bump = h->p.bump;
+    fill_lag_args(h, a);
+    fill_eval_io(a, sub, n, xd, yd, out);
     CU(h, launch_lagrange_eval(a, h->stream));
     h->launches++;
     return SWRT_OK;
@@ -946,7 +957,8 @@ int swrt_rhs(swrt_handle* h, double alpha, double* dxdt, double* dydt, double* d
     int rc = ensure_scratch(h, h->n);
     if (rc) return rc;
     if ((rc = eval_dev(h, SUB_SIX, alpha, h->n, h->x, h->y, h->e))) return rc;
-    launch_rhs(h->n, h->k, h->l, h->e, h->p.f, h->p.gH, rhs_cgfac(h), h->xs, h->ys, h->ax, h->ay, h->stream);
+    double* const fj[4] = {h->xs, h->ys, h->ax, h->ay};
+    launch_rhs(Ode23ValView{}, 0, h->n, h->k, h->l, h->e, nullptr, h->p.f, h->p.gH, rhs_cgfac(h), fj, h->stream);
     h->launches++;
     if ((rc = d2h(h, dxdt, h->xs, h->n)) || (rc = d2h(h, dydt, h->ys, h->n)) || (rc = d2h(h, dkdt, h->ax, h->n)) ||
         (rc = d2h(h, dldt, h->ay, h->n)))
@@ -1071,8 +1083,7 @@ static int prepare_run(swrt_handle* h, int scheme, double dt, double alpha0, dou
         if (psi) { a.psi = true; a.kappa = 2.0 * M_PI / h->p.L; a.u_mean0 = h->u_mean[0]; a.u_mean1 = h->slot_set[1] ? h->u_mean[1] : 0.0; }
         a.alpha0 = alpha0; a.dalpha = dalpha; a.j0 = j0;
         a.x = h->x; a.y = h->y; a.k = h->k; a.l = h->l;
-        a.dx = h->p.L / h->p.nx; a.nxd = (double)h->p.nx;
-        a.inv_nx = (h->p.nx & (h->p.nx - 1)) == 0 ? 1.0 / h->p.nx : 0.0;
+        fill_spec_geom(h, a);
         a.f2 = h->p.f * h->p.f; a.gH = h->p.gH; a.dt = dt; a.nsteps = m;
         if (r.anchored) {       // odd expansion orders contract the S/D-swapped stacks (one per step of a time-dependent run)
             const size_t nd = (size_t)(a.nstack > 1 ? a.nstack : 1) * a.g.total_doubles;
@@ -1128,9 +1139,9 @@ static int prepare_run(swrt_handle* h, int scheme, double dt, double alpha0, dou
             h->launches++;
             a.grid = h->arena; a.grid2 = nullptr; a.gstride = nd;
         }
-        a.nx = h->p.nx; a.npl = h->grid_npl;
+        fill_lag_args(h, a);
         a.x = h->x; a.y = h->y; a.k = h->k; a.l = h->l; a.a = h->a;
-        a.dx = h->p.L / h->p.nx; a.bump = h->p.bump; a.f = h->p.f; a.gH = h->p.gH; a.C0 = C0; a.dt = dt; a.nsteps = m;
+        a.f = h->p.f; a.gH = h->p.gH; a.C0 = C0; a.dt = dt; a.nsteps = m;
         return SWRT_OK;
     }
     if (mode == SWRT_MODE_SPECTRAL && !h->unfused_rk4) {
@@ -1160,8 +1171,7 @@ static int prepare_run(swrt_handle* h, int scheme, double dt, double alpha0, dou
         a.kappa = 2.0 * M_PI / h->p.L; a.u_mean0 = h->u_mean[0]; a.u_mean1 = h->slot_set[1] ? h->u_mean[1] : 0.0;
         a.alpha0 = alpha0; a.dalpha = dalpha; a.j0 = j0;
         a.x = h->x; a.y = h->y; a.k = h->k; a.l = h->l; a.a = h->a;
-        a.dx = h->p.L / h->p.nx; a.nxd = (double)h->p.nx;
-        a.inv_nx = (h->p.nx & (h->p.nx - 1)) == 0 ? 1.0 / h->p.nx : 0.0;
+        fill_spec_geom(h, a);
         a.f = h->p.f; a.C0 = C0; a.dt = dt; a.nsteps = m;
         return SWRT_OK;
     }
@@ -1628,7 +1638,7 @@ static int bs23_setup(swrt_handle* h, Bs23Args& a) {
 static int bs23_rhs(swrt_handle* h, double alpha, double* const st[4], double* const fj[4]) {
     int rc = eval_dev(h, SUB_SIX, alpha, h->n, st[0], st[1], h->e);
     if (rc) return rc;
-    launch_rhs(h->n, st[2], st[3], h->e, h->p.f, h->p.gH, rhs_cgfac(h), fj[0], fj[1], fj[2], fj[3], h->stream);
+    launch_rhs(Ode23ValView{}, 0, h->n, st[2], st[3], h->e, nullptr, h->p.f, h->p.gH, rhs_cgfac(h), fj, h->stream);
     h->launches++;
     return SWRT_OK;
 }
@@ -1649,7 +1659,8 @@ static int bs23_begin_launch(swrt_handle* h, double alpha, double threshold) {
     if (rc) return rc;
     double* f1[4] = {a.f[0][0], a.f[0][1], a.f[0][2], a.f[0][3]};
     if ((rc = bs23_rhs(h, alpha, a.y, f1))) return rc;
-    launch_bs23_norm(a, 1, threshold, h->bs_norm_dev, h->stream);
+    CU(h, cudaMemsetAsync(h->bs_norm_dev, 0, sizeof(unsigned long long), h->stream));
+    launch_bs23_norm<1>(a, Ode23ValView{}, threshold, h->bs_norm_dev, h->stream);
     h->launches++;
     h->bs_ready = true;
     return SWRT_OK;
@@ -1672,14 +1683,15 @@ static int bs23_attempt_launch(swrt_handle* h, double hstep, const double alpha[
     double* f2[4] = {a.f[1][0], a.f[1][1], a.f[1][2], a.f[1][3]};
     double* f3[4] = {a.f[2][0], a.f[2][1], a.f[2][2], a.f[2][3]};
     double* f4[4] = {a.f[3][0], a.f[3][1], a.f[3][2], a.f[3][3]};
-    // A = [1/2 3/4 1], B = [1/2 0 2/9; 0 3/4 1/3; 0 0 4/9; 0 0 0]
-    launch_bs23_stage(a, hstep * 0.5, 0.0, 0.0, h->stream);
+    const Ode23ValView v{hstep, {alpha[0], alpha[1], alpha[2]}};
+    launch_bs23_stage(a, v, 0, h->stream);
     if ((rc = bs23_rhs(h, alpha[0], a.yt, f2))) return rc;
-    launch_bs23_stage(a, 0.0, hstep * 0.75, 0.0, h->stream);
+    launch_bs23_stage(a, v, 1, h->stream);
     if ((rc = bs23_rhs(h, alpha[1], a.yt, f3))) return rc;
-    launch_bs23_stage(a, hstep * (2.0 / 9.0), hstep * (1.0 / 3.0), hstep * (4.0 / 9.0), h->stream);   // ynew
+    launch_bs23_stage(a, v, 2, h->stream);   // ynew
     if ((rc = bs23_rhs(h, alpha[2], a.yt, f4))) return rc;
-    launch_bs23_norm(a, 0, threshold, h->bs_norm_dev, h->stream);
+    CU(h, cudaMemsetAsync(h->bs_norm_dev, 0, sizeof(unsigned long long), h->stream));
+    launch_bs23_norm<0>(a, v, threshold, h->bs_norm_dev, h->stream);
     h->launches += 4;
     return SWRT_OK;
 }
@@ -1704,7 +1716,7 @@ int swrt_bs23_accept(swrt_handle* h) {
     Bs23Args a{};
     int rc = bs23_setup(h, a);
     if (rc) return rc;
-    launch_bs23_accept(a, h->stream);
+    launch_bs23_accept(a, Ode23ValView{}, h->stream);
     h->launches++;
     CU(h, cudaStreamSynchronize(h->stream));
     return SWRT_OK;

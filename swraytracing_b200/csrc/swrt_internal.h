@@ -119,6 +119,39 @@ __device__ __forceinline__ const double* ode23_pkt_alpha(const Ode23Pkt& s, int 
     return stage == 0 ? s.al[0] : stage == 1 ? s.al[1] : s.al[2];
 }
 
+// The controller an attempt kernel (stage, RHS, norm, accept, LAGRANGE6 evaluation) reads, one view per solve:
+//   done()           nothing is left in this launch (uniform: the kernel returns at its top)
+//   idle(i)          packet i is finished and writes nothing
+//   h(i)             packet i's step size
+//   alpha(stage, i)  packet i's flow alpha of the RHS evaluation of `stage`
+//   accepted()       the accept kernel's predicate
+// The host controller (swrt_bs23_*, swrt_rhs): h and the alphas as values, never idle.
+struct Ode23ValView {
+    double hv, al[3];
+    __device__ bool done() const { return false; }
+    __device__ bool idle(long long) const { return false; }
+    __device__ double h(long long) const { return hv; }
+    __device__ double alpha(int stage, long long) const { return stage == 0 ? al[0] : stage == 1 ? al[1] : al[2]; }
+    __device__ bool accepted() const { return true; }
+};
+// swrt_ode23: one controller in device memory for the whole launch
+struct Ode23CtlView {
+    const Ode23Ctl* ctl;
+    __device__ bool done() const { return ode23_idle(ctl); }
+    __device__ bool idle(long long) const { return false; }
+    __device__ double h(long long) const { return ctl->h; }
+    __device__ double alpha(int stage, long long) const { return ctl->al[stage]; }
+    __device__ bool accepted() const { return ctl->accepted; }
+};
+// swrt_ode23_packets: one controller per packet (its norm and accept are part of the decide kernel)
+struct Ode23PktView {
+    Ode23Pkt s;
+    __device__ bool done() const { return false; }
+    __device__ bool idle(long long i) const { return ode23_pkt_idle(s, i); }
+    __device__ double h(long long i) const { return s.h[i]; }
+    __device__ double alpha(int stage, long long i) const { return ode23_pkt_alpha(s, stage)[i]; }
+};
+
 PackGeom make_geom(int nx, int npl, const int* plane_ids, int mtiles, int twiddle_pref = 0);
 
 // one source slot: complex planes on the device, [plane][ky][kx+kmax] as double2 (kx fastest)
@@ -251,8 +284,12 @@ struct Rk4Args {   // spectral-mode RK4 glue (point-wise composition), all devic
 };
 void launch_rk4_stage(const Rk4Args& a, cudaStream_t st);
 void launch_rk4_final(const Rk4Args& a, cudaStream_t st);
-void launch_rhs(long long n, const double* k, const double* l, const double* const* e6, double f, double gH, double cgfac,
-                double* dxdt, double* dydt, double* dkdt, double* dldt, cudaStream_t st);
+// RHS of the planes e6 at (k, l) into fj[0..3], skipped for the view's idle packets.  With e1 set (swrt_ode23_packets,
+// SPECTRAL, two frames) e6 holds the planes at alpha 0 and e1 at alpha 1, and each packet blends them at its alpha of
+// `stage`, in place in e6.
+template <class View>
+void launch_rhs(const View& v, int stage, long long n, const double* k, const double* l, const double* const* e6,
+                const double* const* e1, double f, double gH, double cgfac, double* const fj[4], cudaStream_t st);
 void launch_omega(long long n, const double* k, const double* l, const double* u, const double* v,
                   double f, double gH, double* omega, double* Omega_abs, cudaStream_t st);
 void launch_hist(long long n, const double* w, const double* edges_dev, int nedges,
@@ -297,39 +334,32 @@ struct Bs23Args {          // ode23 work arrays, component order x,y,k,l
     double* yt[4];         // stage state / ynew
     double* f[4][4];       // f1..f4
 };
-void launch_bs23_stage(const Bs23Args& a, double hb1, double hb2, double hb3, cudaStream_t st);
-void launch_bs23_norm(const Bs23Args& a, int mode, double thr, unsigned long long* out, cudaStream_t st);
-void launch_bs23_accept(const Bs23Args& a, cudaStream_t st);
+// the attempt kernels for the views of the host controller (Ode23ValView), swrt_ode23 (Ode23CtlView) and, for the stage,
+// RHS and LAGRANGE6 evaluation, swrt_ode23_packets (Ode23PktView)
+template <class View> void launch_bs23_stage(const Bs23Args& a, const View& v, int stage, cudaStream_t st);
+// atomicMax of the error norm into `out`, which the caller has zeroed; MODE 1: the scale norm of the initial step
+template <int MODE, class View>
+void launch_bs23_norm(const Bs23Args& a, const View& v, double thr, unsigned long long* out, cudaStream_t st);
+template <class View> void launch_bs23_accept(const Bs23Args& a, const View& v, cudaStream_t st);
+template <class View> cudaError_t launch_lagrange_eval_ode23(const LagArgs& a, const View& v, int stage, cudaStream_t st);
 void launch_bs23_interp(const Bs23Args& a, const double w[4], double* const out[4], cudaStream_t st);
 
-
-void launch_bs23_stage_dev(const Bs23Args& a, const Ode23Ctl* ctl, int stage, cudaStream_t st);
-void launch_rhs_dev(const Ode23Ctl* ctl, long long n, const double* k, const double* l, const double* const* e6, double f,
-                    double gH, double cgfac, double* dxdt, double* dydt, double* dkdt, double* dldt, cudaStream_t st);
-void launch_bs23_norm_dev(const Bs23Args& a, const Ode23Ctl* ctl, double thr, unsigned long long* out, cudaStream_t st);
 void launch_ode23_init(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st);
 void launch_ode23_control(Ode23Ctl* ctl, unsigned long long* norm, cudaStream_t st);
 void launch_bs23_interp_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st);
-void launch_bs23_accept_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t st);
 // out = (1 - al)*a + al*b with al = ctl->al[stage], skipped when al is 0 or 1 (the evaluation then reads a frame itself)
 void launch_axpby_dev(double* out, const double* a, const double* b, const Ode23Ctl* ctl, int stage, size_t n, cudaStream_t st);
 cudaError_t launch_spectral_eval_dev(const SpecArgs& a, int num_sms, cudaStream_t st);     // a.sel set
 cudaError_t launch_nufft_eval_dev(const NufftArgs& a, const Ode23Sel& sel, cudaStream_t st);
-cudaError_t launch_lagrange_eval_dev(const LagArgs& a, const Ode23Ctl* ctl, int stage, cudaStream_t st);
 // swrt_ode23_packets: `k` holds the per-solve constants (controller section zero, t = t0).  begin: the rh norm and the
-// initial step of every packet from f1; stage / RHS / decide as their swrt_ode23 counterparts with each packet's own h and
-// alphas.  With e1 set (SPECTRAL, two frames) the RHS blends e (alpha 0) and e1 (alpha 1) at the packet's alpha.
-// With ev set, begin also seeds the event values and clears the records, and decide locates and records the events of
-// every accepted step and applies a terminal stop.
+// initial step of every packet from f1; decide: each packet's norm, controller, dense rows and accept, as swrt_ode23's
+// kernels with the packet's own state.  With ev set, begin also seeds the event values and clears the records, and decide
+// locates and records the events of every accepted step and applies a terminal stop.
 void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, const Ode23Ev* ev,
                             cudaStream_t st);
-void launch_bs23_stage_pkt(const Bs23Args& a, const Ode23Pkt& s, int stage, cudaStream_t st);
-void launch_rhs_pkt(const Ode23Pkt& s, int stage, long long n, const double* k, const double* l, const double* const* e6,
-                    const double* const* e1, double f, double gH, double cgfac, double* const fj[4], cudaStream_t st);
 void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, const Ode23Ev* ev,
                              cudaStream_t st);
 cudaError_t launch_nufft_eval_pkt(const NufftArgs& a, const double2* grid1, const Ode23Pkt& s, int stage, cudaStream_t st);
-cudaError_t launch_lagrange_eval_pkt(const LagArgs& a, const Ode23Pkt& s, int stage, cudaStream_t st);
 // (rtol/err)^(1/3) as glibc's correctly rounded-in-practice pow gives it (host and device, misc_kernels.cu)
 __host__ __device__ double pow_third(double x);
 

@@ -22,6 +22,31 @@ from .engine import (Engine, QGFlow, QG2Flow, MODE_SPECTRAL, SCHEME_LEAPFROG, SC
 from .reference_api import ode23, matlab_linspace
 
 
+class _Integrator:
+    """A driver's ``integrator=`` name: 'ode23' (reference_api.ode23, the host controller), 'ode23_device' (the controller
+    on the device, swrt_ode23), 'ode23_packets' (one controller per packet, swrt_ode23_packets) or, where the driver has
+    it, 'leapfrog'.  Any other name raises ValueError."""
+
+    def __init__(self, name, driver, leapfrog=True):
+        names = ("ode23", "ode23_device", "ode23_packets") + (("leapfrog",) if leapfrog else ())
+        if name not in names:
+            raise ValueError(f"{driver}: unknown integrator {name!r} (expected one of {', '.join(names)})")
+        self.ode23 = name != "leapfrog"
+        self.per_packet = name == "ode23_packets"
+        self.opts = {"on_device": name == "ode23_device", "per_packet": self.per_packet}
+
+    def counters(self):
+        """the stats entries only the per-packet solve reports"""
+        return {"ode23_stopped_packets": 0} if self.per_packet else {}
+
+    def step(self, eng, dt, stats):
+        """ode23 over [0, dt] between flow slots 0 and 1, counted into ``stats``"""
+        st = ode23(eng, [0.0, dt], dt, **self.opts)
+        stats["ode23_steps"] += st["nsteps"]; stats["ode23_failed"] += st["nfailed"]
+        if self.per_packet:
+            stats["ode23_stopped_packets"] += st["stopped"]
+
+
 def wavenumber_grids(nx):
     """[kx_,ky_] = ndgrid(-kmax:kmax, 0:kmax) (qgsw_raytrace.m:18-20)"""
     kmax = nx // 2 - 1
@@ -54,6 +79,7 @@ def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_da
     with the controller on the device, swrt_ode23), 'ode23_packets' (ode23 once per packet, each under its own controller,
     swrt_ode23_packets: a packet that blows up stops alone, counted in ``ode23_stopped_packets``) or 'leapfrog' (the fused
     symplectic stepper with time-centred frame blending).  ``max_steps`` truncates the run (tests)."""
+    integ = _Integrator(integrator, "qgsw_raytrace")
     L = 2 * np.pi
     dx = L / nx
     xg = matlab_linspace(-L / 2, L / 2, nx)
@@ -105,9 +131,7 @@ def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_da
     eng.set_packets(px, py, pk, pl)
     t = 0.0
     tic = time.time()
-    stats = {"packet_steps": 0, "ode23_steps": 0, "ode23_failed": 0}
-    if integrator == "ode23_packets":
-        stats["ode23_stopped_packets"] = 0
+    stats = {"packet_steps": 0, "ode23_steps": 0, "ode23_failed": 0, **integ.counters()}
     for step in range(1, Nsteps + 1):
         if Npackets > 0 and t + dt > packet_delay:
             qg.to_flow(eng, 0)                                         # background_flow1 = grid_U(prev_qk), :141
@@ -115,12 +139,8 @@ def qgsw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_delay_da
         t += dt
         if Npackets > 0 and t > packet_delay:
             qg.to_flow(eng, 1)                                         # background_flow2 = grid_U(qk), :142
-            if integrator in ("ode23", "ode23_device", "ode23_packets"):
-                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device",
-                           per_packet=integrator == "ode23_packets")                          # :143-150
-                stats["ode23_steps"] += st["nsteps"]; stats["ode23_failed"] += st["nfailed"]
-                if integrator == "ode23_packets":
-                    stats["ode23_stopped_packets"] += st["stopped"]
+            if integ.ode23:
+                integ.step(eng, dt, stats)                                     # :143-150
             else:
                 m = leapfrog_substeps
                 eng.step(SCHEME_LEAPFROG, dt / m, m, 0.5 / m, 1.0 / m)
@@ -231,7 +251,7 @@ def SW_zero_background_raytracing(q=None, *, nx=None, f=None, Cg=None, run_log_f
     ``integrator='ode23_packets'`` solves every packet under its own controller (swrt_ode23_packets).
     Returns dict(t_hist, solver_x, solver_k, solver_error, w, Omega_0, U0, Fr, dt, stats)."""
     from .engine import FLAG_RHS_GH
-    from .reference_api import ode23
+    integ = _Integrator(integrator, "SW_zero_background_raytracing", leapfrog=False)
     if run_log_file is not None:
         lnx, _, lf, lCg, _ = parse_data(run_log_file)
         nx, f, Cg = nx or lnx, f if f is not None else lf, Cg if Cg is not None else lCg
@@ -251,8 +271,7 @@ def SW_zero_background_raytracing(q=None, *, nx=None, f=None, Cg=None, run_log_f
     eng = Engine(nx, L, f, gH, mode, device, flags=FLAG_RHS_GH)
     eng.set_flow_spectral(scheme.psik)
     eng.set_packets(x[0, 0], x[0, 1], k[0, 0], k[0, 1])
-    stats = ode23(eng, t_hist, None, rtol=rtol, atol=atol, on_device=integrator == "ode23_device",
-                  per_packet=integrator == "ode23_packets")                                         # steady flow: slot 0
+    stats = ode23(eng, t_hist, None, rtol=rtol, atol=atol, **integ.opts)                          # steady flow: slot 0
     Y = stats.pop("Y")
     eng.close()
     solver_x, solver_k = Y[:, 0:2, :], Y[:, 2:4, :]
@@ -397,6 +416,7 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
     controller per packet, stopped packets counted in ``ode23_stopped_packets``), packet frames every
     25 steps.  ``k_max`` (30 in the reference)
     and ``max_steps`` exist for tests."""
+    integ = _Integrator(integrator, "qg2layersw_raytrace")
     L = 20.0
     dx = L / nx
     xg = matlab_linspace(-L / 2, L / 2, nx)
@@ -448,9 +468,7 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
     t = 0.0
     step = 0
     tic = time.time()
-    stats = {"packet_steps": 0, "ode23_steps": 0, "ode23_failed": 0, "dt_changes": 0}
-    if integrator == "ode23_packets":
-        stats["ode23_stopped_packets"] = 0
+    stats = {"packet_steps": 0, "ode23_steps": 0, "ode23_failed": 0, "dt_changes": 0, **integ.counters()}
     while t <= T and (max_steps is None or step < max_steps):
         step += 1
         U0 = qg.max_speed()
@@ -466,11 +484,8 @@ def qg2layersw_raytrace(nx, Npackets, near_inertial_factor, T_Fr_days, packet_de
         t = t + dt
         if advect:
             qg.to_flow(eng, 1)                                         # background_flow2 = grid_U(qk(:,:,:,1)), :188
-            if integrator in ("ode23", "ode23_device", "ode23_packets"):
-                st = ode23(eng, [0.0, dt], dt, on_device=integrator == "ode23_device", per_packet=integrator == "ode23_packets")
-                stats["ode23_steps"] += st["nsteps"]; stats["ode23_failed"] += st["nfailed"]
-                if integrator == "ode23_packets":
-                    stats["ode23_stopped_packets"] += st["stopped"]
+            if integ.ode23:
+                integ.step(eng, dt, stats)
             else:
                 m = leapfrog_substeps
                 eng.step(SCHEME_LEAPFROG, dt / m, m, 0.5 / m, 1.0 / m)
