@@ -166,15 +166,18 @@ int swrt_bs23_interp(swrt_handle* h, double hstep, double s, double* x, double* 
  * SW_zero_background_raytracing.m:73-78) in one call, the step-size controller on the device: the decisions of
  * reference_api.ode23 (MATLAB's ode23 with MaxStep 0.1*|tf - t0|).  alpha = t/tmax (tmax = 0: steady flow, slot 0).
  * ntspan >= 2; when ntspan > 2, Y (ntspan x 4 x n, host, may be NULL) receives the state at every tspan entry (ntrp23
- * dense output).  stats[0..3] = accepted steps, rejected steps, RHS evaluations, host waits.  h_trace (may be NULL)
- * receives up to h_cap accepted step sizes.  SWRT_ERR_STATE when the step size falls below 16*eps(t) (a packet blew
+ * dense output).  A decreasing tspan (tspan[end] < tspan[0]) integrates backward in time, as MATLAB's ode23 does: every
+ * step is h = -absh; an entry that steps against the direction from tspan[0] to tspan[end] is SWRT_ERR_ARG (equal
+ * neighbours are allowed).  stats[0..3] = accepted steps, rejected steps, RHS evaluations, host waits.  h_trace (may be
+ * NULL) receives up to h_cap accepted step sizes, signed (negative when integrating backward).  SWRT_ERR_STATE when the step size falls below 16*eps(t) (a packet blew
  * up; the message names t); the packets are then those of the last accepted step.                               */
 int swrt_ode23(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol, double* Y,
                int64_t stats[4], double* h_trace, int h_cap);
 /* [~, Y] = ode23(odefun_i, tspan, y_i) for every packet i on its own: packet i advances exactly as swrt_ode23 advances an
  * ensemble holding packet i alone (its own error norm, initial step, rejections and dense output), so a packet's result
- * does not depend on the other packets, their number or the sharding.  Y as in swrt_ode23 (ntspan x 4 x n, may be NULL;
- * the rows after a stopped packet's t_end are NaN).
+ * does not depend on the other packets, their number or the sharding.  tspan as in swrt_ode23 (a decreasing tspan
+ * integrates backward in time).  Y as in swrt_ode23 (ntspan x 4 x n, may be NULL; the rows after a stopped packet's
+ * t_end are NaN).
  * pstat (may be NULL): n x 3 int32, column-major = accepted steps, rejected steps, status (0 reached tfinal, 1 step size
  * fell below 16*eps(t)); t_end (may be NULL): tfinal, or the t at which the packet stopped (it keeps its last accepted
  * state).  stats[0..4] = accepted steps, rejected steps and RHS evaluations summed over packets, packets that stopped,

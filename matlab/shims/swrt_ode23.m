@@ -9,6 +9,11 @@ function stats = swrt_ode23(eng, tspan, tmax, rtol, atol)
 if nargin < 4, rtol = 1e-3; end
 if nargin < 5, atol = 1e-6; end
 t0 = tspan(1); tfinal = tspan(end);
+% MATLAB's tdir: a decreasing tspan ([T 0]) integrates backward; every step is h = tdir*absh
+if tfinal >= t0, tdir = 1; else, tdir = -1; end
+if any(tdir * diff(tspan) < 0)
+    error('swrt:ode23', 'tspan must be monotonic (an entry goes against the direction from tspan(1) to tspan(end))');
+end
 pw = 1/3; threshold = atol / rtol;
 hmax = min(abs(tfinal - t0), abs(0.1 * (tfinal - t0)));
 t = t0;
@@ -20,7 +25,7 @@ nsteps = 0; nfailed = 0; done = false;
 while ~done
     hmin = 16 * eps(t);
     absh = min(hmax, max(hmin, absh));
-    h = absh;
+    h = tdir * absh;
     if 1.1 * absh >= abs(tfinal - t)
         h = tfinal - t; absh = abs(h); done = true;
     end
@@ -37,7 +42,7 @@ while ~done
             else
                 absh = max(hmin, 0.5 * absh);
             end
-            h = absh; done = false;
+            h = tdir * absh; done = false;
         else
             break
         end

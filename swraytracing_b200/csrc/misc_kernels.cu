@@ -334,11 +334,12 @@ __device__ __forceinline__ void ode23_set_attempt(Ode23Ctl& c) {
     c.al[1] = ode23_alpha(c, __dadd_rn(c.t, __dmul_rn(0.75, c.h)));
     c.al[2] = ode23_alpha(c, c.tnew);
 }
-// head of the host controller's outer loop: hmin, the MaxStep clamp and the 1.1 stretch onto tfinal
+// head of the host controller's outer loop: hmin, the MaxStep clamp and the 1.1 stretch onto tfinal.  Every step is
+// h = tdir * absh (exact: tdir is +1 or -1).
 __device__ __forceinline__ void ode23_new_step(Ode23Ctl& c) {
     c.hmin = eps16(c.t);
     c.absh = py_min(c.hmax, py_max(c.hmin, c.absh));
-    c.h = c.absh;
+    c.h = __dmul_rn(c.tdir, c.absh);
     c.last = 0;
     if (__dmul_rn(1.1, c.absh) >= fabs(__dsub_rn(c.tfinal, c.t))) {
         c.h = __dsub_rn(c.tfinal, c.t);
@@ -378,7 +379,7 @@ __device__ __forceinline__ void ode23_control(Ode23Ctl& c, double nrm) {
         } else {
             c.absh = py_max(c.hmin, __dmul_rn(0.5, c.absh));
         }
-        c.h = c.absh;
+        c.h = __dmul_rn(c.tdir, c.absh);
         c.last = 0;
         ode23_set_attempt(c);
         return;
@@ -389,7 +390,7 @@ __device__ __forceinline__ void ode23_control(Ode23Ctl& c, double nrm) {
     c.t_acc = c.t; c.h_acc = c.h;
     if (c.ntspan > 2) {
         int j = c.nxt;
-        while (j < c.ntspan && __dsub_rn(c.tnew, c.tspan[j]) >= 0.0) j++;
+        while (j < c.ntspan && __dmul_rn(c.tdir, __dsub_rn(c.tnew, c.tspan[j])) >= 0.0) j++;
         c.nxt_end = j;
     }
     if (c.nofailed) {

@@ -67,6 +67,8 @@ struct Ode23Ctl {
     int status;                                        // 0, or 1 = step size below hmin (t holds where)
     int nxt, nxt_end;                                  // dense rows [nxt, nxt_end) are written after this attempt
     long long nsteps, nfailed, nfevals;
+    // per solve, appended so that the fields above keep their offsets
+    double tdir;                                       // +1 (tfinal >= t0) or -1 (a decreasing tspan: backward in time)
 };
 // a pointer-argument evaluation: the frame is chosen on the device from ctl->al[stage] as the host picks it for a value
 // alpha (alpha == 0: frame 0, alpha == 1: frame 1, else the blend); frame1 / blend may be null for a steady flow

@@ -347,8 +347,10 @@ class Engine:
         """a whole ``[~, Y] = ode23(ray_ode, tspan, y0)`` solve in one call (swrt_ode23): the decisions of
         ``reference_api.ode23`` made by a controller in device memory, the host waiting a few times per solve instead of
         twice per attempt.  ``tmax`` None / 0 = steady flow.  Returns the same dict as ``reference_api.ode23`` (``Y`` when
-        ``tspan`` has more than two entries) plus ``host_waits``, and ``h`` (the first ``trace`` accepted step sizes)
-        when ``trace`` > 0.  A step size below hmin raises SwrtError (SWRT_ERR_STATE) naming t."""
+        ``tspan`` has more than two entries) plus ``host_waits``, and ``h`` (the first ``trace`` accepted step sizes, signed)
+        when ``trace`` > 0.  A decreasing ``tspan`` (``[T 0]``) integrates backward in time, as MATLAB's ode23 does; an
+        entry that steps against the direction from ``tspan[0]`` to ``tspan[-1]`` raises SwrtError (SWRT_ERR_ARG).  A step
+        size below hmin raises SwrtError (SWRT_ERR_STATE) naming t."""
         ts = _f64(tspan)
         dense = ts.size > 2
         Y = np.empty((ts.size, 4, self.n)) if dense else None
@@ -370,7 +372,7 @@ class Engine:
         (packets whose step size fell below hmin: they keep their last accepted state, the others carry on),
         ``host_waits``, and the per-packet arrays ``steps``, ``rejected``, ``status`` (0 reached tfinal, 1 stopped) and
         ``t_end`` (where each packet stopped).  ``Y`` when ``tspan`` has more than two entries (NaN in the rows a stopped
-        packet did not reach).
+        packet did not reach).  A decreasing ``tspan`` integrates backward in time, as in ``ode23``.
 
         ``events``: MATLAB's ``odeset('Events', ...)`` per packet (swrt_ode23_packets_events), a list of
         ``(kind, level, direction=0, terminal=False)`` with ``kind`` one of ``EVENT_X``, ``EVENT_Y``, ``EVENT_K``,

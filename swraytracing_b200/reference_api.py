@@ -314,6 +314,11 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=
     (MATLAB ``ntrp23``, swrt_bs23_interp).  The step sequence follows MATLAB's controller, including the initial step
     ``min(hmax, |tspan(2)-tspan(1)|, 1/rh)``, which for a dense ``tspan`` is bounded by the first output interval.
 
+    A decreasing ``tspan`` (``[T 0]``) integrates backward in time, as MATLAB's ode23 does: ``tdir = -1`` and every step
+    is ``h = tdir*absh``, the step-size rules unchanged (they act on ``absh``); a dense row is written once the step has
+    passed its time in the direction of integration.  A ``tspan`` entry that steps against that direction raises
+    ``ValueError`` (equal neighbours are allowed).  Events stay forward-only.
+
     One deliberate deviation: a non-finite error estimate (a packet that blew up) REJECTS the step here and, at ``hmin``,
     raises; MATLAB's ``if err > rtol`` is false for NaN, so it would accept the step and carry NaNs on silently.
 
@@ -339,6 +344,9 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=
     al = (lambda tt: tt / tmax) if tmax else (lambda tt: 0.0)       # tmax=None: steady flow, slot 0 only
     tspan = np.asarray(tspan, dtype=np.float64)
     t0, tfinal = float(tspan[0]), float(tspan[-1])
+    tdir = 1.0 if tfinal >= t0 else -1.0      # MATLAB's tdir = sign(tfinal - t0): a decreasing tspan integrates backward
+    if np.any(tdir * np.diff(tspan) < 0):
+        raise ValueError("ode23: tspan must be monotonic (an entry goes against the direction from tspan[0] to tspan[-1])")
     dense = tspan.size > 2
     if dense:
         Y = np.zeros((tspan.size, 4, target.n)); Y[0] = np.stack(target.get_packets()); nxt = 1
@@ -360,7 +368,7 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=
     while not done:
         hmin = 16 * np.spacing(abs(t))
         absh = min(hmax, max(hmin, absh))
-        h = absh
+        h = tdir * absh
         if 1.1 * absh >= abs(tfinal - t):
             h = tfinal - t
             absh = abs(h)
@@ -379,13 +387,13 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=
                     absh = max(hmin, absh * max(0.5, 0.8 * (rtol / err) ** pw)) if np.isfinite(err) else max(hmin, 0.5 * absh)
                 else:
                     absh = max(hmin, 0.5 * absh)
-                h = absh
+                h = tdir * absh
                 done = False
             else:
                 break
         nsteps += 1
         if dense:
-            while nxt < tspan.size and tnew - tspan[nxt] >= 0:
+            while nxt < tspan.size and tdir * (tnew - tspan[nxt]) >= 0:
                 Y[nxt] = np.stack(target.bs23_interp(h, 1.0 if tspan[nxt] == tnew else (tspan[nxt] - t) / h))
                 nxt += 1
         target.bs23_accept()
