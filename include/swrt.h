@@ -184,6 +184,18 @@ int swrt_ode23(swrt_handle* h, const double* tspan, int ntspan, double tmax, dou
  * host waits.  A stopped packet is not an error: SWRT_OK is returned.                                               */
 int swrt_ode23_packets(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol, double* Y,
                        int32_t* pstat, double* t_end, int64_t stats[5]);
+/* for i = 1:n, [~, Y] = ode23(odefun_i, tspan(:, i), y_i); end -- swrt_ode23_packets with a tspan of its own for every
+ * packet: staggered observation or release times, and forward and backward packets in one call.  tspan is n x ntspan,
+ * column-major: entry j of packet i is tspan[j*n + i] (ntspan >= 2, shared).  Packet i advances exactly as swrt_ode23
+ * advances a handle holding packet i alone with the tspan of its row: its own direction (+1 when its last entry is >= its
+ * first, else -1), initial step, MaxStep, stop and dense rows.  A row whose entries are all equal takes one step of size 0
+ * and keeps its state.  tmax is shared (alpha = t/tmax for every packet).  Y (ntspan x 4 x n, may be NULL) row j of
+ * packet i is the state at tspan[j*n + i]; Y, pstat, t_end and stats[0..4] as in swrt_ode23_packets.  SWRT_ERR_ARG, with
+ * the packets untouched, when an entry is not finite or steps against its own row's direction (the message names the
+ * packet and the entry; equal neighbours are allowed).                                                               */
+int swrt_ode23_packets_tspans(swrt_handle* h, const double* tspan /* n x ntspan, column-major */, int ntspan,
+                              double tmax, double rtol, double atol, double* Y, int32_t* pstat, double* t_end,
+                              int64_t stats[5]);
 
 /* [t, Y, te, ye, ie] = ode23(odefun_i, tspan, y_i, odeset('Events', ...)) for every packet i on its own: event j is a level
  * crossing of g_j(x, y, k, l), a function of the packet state alone.  omega is swrt_hist_omega's intrinsic frequency

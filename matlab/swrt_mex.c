@@ -306,16 +306,22 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (swrt_ode23(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), Y, st, NULL, 0)) fail(h, cmd);
         plhs[0] = mxCreateDoubleMatrix(1, 4, mxREAL);
         for (int i = 0; i < 4; i++) mxGetPr(plhs[0])[i] = (double)st[i];
-    } else if (!strcmp(cmd, "ode23_packets")) {       /* [stats, Y, pstat, t_end] = (h, tspan, tmax, rtol, atol)  -- one controller per packet */
+    } else if (!strcmp(cmd, "ode23_packets")) {       /* [stats, Y, pstat, t_end] = (h, tspan, tmax, rtol, atol)  -- one controller per packet, tspan shared or one row each */
         need(nrhs, 6, "'ode23_packets', h, tspan, tmax, rtol, atol");
-        int nt = (int)mxGetNumberOfElements(prhs[2]);
+        /* tspan a vector: shared by every packet; an n x m matrix (m >= 2): row i is packet i's own tspan */
+        size_t tm = mxGetM(prhs[2]), tn = mxGetN(prhs[2]);
+        int per_row = tm > 1 && tn > 1;
+        if (per_row && tm != (size_t)n)
+            mexErrMsgIdAndTxt("swrt:usage", "ode23_packets: a tspan matrix must be n x m (one row per packet), got %d x %d", (int)tm, (int)tn);
+        int nt = per_row ? (int)tn : (int)mxGetNumberOfElements(prhs[2]);
         int64_t st[5];
         double *Y = NULL, *t_end = NULL;
         if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix((size_t)n, nt > 2 ? (size_t)4 * nt : 0, mxREAL); if (nt > 2) Y = mxGetPr(plhs[1]); }
         /* pstat: n x 3 = accepted steps, rejected steps, status (0 reached tfinal, 1 stopped); t_end: n x 1 */
         int32_t* ps = nlhs > 2 ? (int32_t*)mxCalloc((size_t)3 * (n > 0 ? n : 1), sizeof(int32_t)) : NULL;
         if (nlhs > 3) t_end = outv(plhs, 3, n);
-        if (swrt_ode23_packets(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), Y, ps, t_end, st))
+        if ((per_row ? swrt_ode23_packets_tspans : swrt_ode23_packets)(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]),
+                                                                      mxGetScalar(prhs[5]), Y, ps, t_end, st))
             fail(h, cmd);
         plhs[0] = mxCreateDoubleMatrix(1, 5, mxREAL);
         for (int i = 0; i < 5; i++) mxGetPr(plhs[0])[i] = (double)st[i];

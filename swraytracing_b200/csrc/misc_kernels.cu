@@ -580,10 +580,36 @@ __device__ __forceinline__ bool pkt_events(const Bs23Args& a, long long i, const
     return stop;
 }
 
-template <bool EV>
-__global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, Ode23Ev ev) {
+// swrt_ode23_packets_tspans: packet i's per-solve constants from its own tspan row, in ode23_consts' operation order (so
+// bit for bit what the host forms for that row), kept in sp's arrays for the decide kernel
+__device__ __forceinline__ void pkt_span_consts(const Ode23Spans& sp, long long i, Ode23Ctl& c) {
+    const double* row = sp.tsp + i * sp.ntspan;
+    const double t0 = row[0], tfinal = row[sp.ntspan - 1];
+    c.tfinal = tfinal;
+    c.tdir = tfinal >= t0 ? 1.0 : -1.0;
+    const double span = fabs(__dsub_rn(tfinal, t0)), span10 = fabs(__dmul_rn(0.1, __dsub_rn(tfinal, t0)));
+    c.hmax = span10 < span ? span10 : span;
+    c.htspan = fabs(__dsub_rn(row[1], row[0]));
+    c.t = t0;
+    sp.tfinal[i] = c.tfinal; sp.hmax[i] = c.hmax; sp.tdir[i] = c.tdir;
+}
+
+// swrt_ode23_packets_tspans, before f1: the shard's tspan columns (col[j*n + i], as uploaded) laid out packet-contiguous in
+// rows, every packet's alpha of its t0 into s.al[0] for the per-packet evaluation of f1, and no packet idle
+__global__ void ode23_pkt_rows_kernel(long long n, int ntspan, const double* __restrict__ col, double* __restrict__ rows,
+                                      Ode23Pkt s, double tmax) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    for (int j = 0; j < ntspan; j++) rows[i * ntspan + j] = col[j * n + i];
+    s.al[0][i] = tmax != 0.0 ? __ddiv_rn(col[i], tmax) : 0.0;
+    s.flags[i] = 0;
+}
+
+template <bool EV, bool SPANS>
+__global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, Ode23Ev ev, Ode23Spans sp) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n) return;
+    if constexpr (SPANS) pkt_span_consts(sp, i, c);
     ode23_init(c, pkt_norm(a, i, 1, thr));
     pkt_store(s, i, a.n, c);
     if constexpr (EV) {                                         // g_j(y0), and no records yet
@@ -604,13 +630,19 @@ __global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, doubl
 // after a round's three stages: each unfinished packet's norm, its controller, its dense rows and its predicated accept.
 // Block-reduced into the report pair of this round: the packets still unfinished and the attempts the slowest of them
 // needs; the other pair is cleared for the next round.  EV: the accepted step's events; a terminal one stops the packet
-// at its te (status 2) with that record's state, and only the dense rows up to te are written.
-template <bool EV>
-__global__ void __launch_bounds__(256) ode23_pkt_decide_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, int round, Ode23Ev ev) {
+// at its te (status 2) with that record's state, and only the dense rows up to te are written.  SPANS: the packet's own
+// tfinal, hmax, tdir and tspan row.
+template <bool EV, bool SPANS>
+__global__ void __launch_bounds__(256) ode23_pkt_decide_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, int round, Ode23Ev ev,
+                                                               Ode23Spans sp) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     int open = 0, batch = 0;
     if (i < a.n && !ode23_pkt_idle(s, i)) {
         pkt_load(s, i, a.n, c);
+        if constexpr (SPANS) {
+            c.tfinal = sp.tfinal[i]; c.hmax = sp.hmax[i]; c.tdir = sp.tdir[i];
+            c.tspan = sp.tsp + i * sp.ntspan;
+        }
         ode23_control(c, pkt_norm(a, i, 0, thr));
         if (c.accepted) {
             bool stop = false;
@@ -711,17 +743,25 @@ void launch_bs23_interp_dev(const Bs23Args& a, const Ode23Ctl* ctl, cudaStream_t
     if (a.n > 0) bs23_interp_dev_kernel<<<nblk(a.n, 256), 256, 0, st>>>(a, ctl);
 }
 
+void launch_ode23_pkt_rows(long long n, int ntspan, const double* col, double* rows, const Ode23Pkt& s, double tmax,
+                           cudaStream_t st) {
+    if (n > 0) ode23_pkt_rows_kernel<<<nblk(n, 256), 256, 0, st>>>(n, ntspan, col, rows, s, tmax);
+}
 void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, const Ode23Ev* ev,
-                            cudaStream_t st) {
+                            const Ode23Spans* sp, cudaStream_t st) {
     if (a.n <= 0) return;
-    if (ev) ode23_pkt_begin_kernel<true><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, *ev);
-    else ode23_pkt_begin_kernel<false><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, Ode23Ev{});
+    const unsigned nb = nblk(a.n, 256);
+    if (ev) ode23_pkt_begin_kernel<true, false><<<nb, 256, 0, st>>>(a, s, k, thr, *ev, Ode23Spans{});
+    else if (sp) ode23_pkt_begin_kernel<false, true><<<nb, 256, 0, st>>>(a, s, k, thr, Ode23Ev{}, *sp);
+    else ode23_pkt_begin_kernel<false, false><<<nb, 256, 0, st>>>(a, s, k, thr, Ode23Ev{}, Ode23Spans{});
 }
 void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, const Ode23Ev* ev,
-                             cudaStream_t st) {
+                             const Ode23Spans* sp, cudaStream_t st) {
     if (a.n <= 0) return;
-    if (ev) ode23_pkt_decide_kernel<true><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, round, *ev);
-    else ode23_pkt_decide_kernel<false><<<nblk(a.n, 256), 256, 0, st>>>(a, s, k, thr, round, Ode23Ev{});
+    const unsigned nb = nblk(a.n, 256);
+    if (ev) ode23_pkt_decide_kernel<true, false><<<nb, 256, 0, st>>>(a, s, k, thr, round, *ev, Ode23Spans{});
+    else if (sp) ode23_pkt_decide_kernel<false, true><<<nb, 256, 0, st>>>(a, s, k, thr, round, Ode23Ev{}, *sp);
+    else ode23_pkt_decide_kernel<false, false><<<nb, 256, 0, st>>>(a, s, k, thr, round, Ode23Ev{}, Ode23Spans{});
 }
 
 void launch_fill(double* p, double v, long long n, cudaStream_t st) {

@@ -116,6 +116,13 @@ struct Ode23Ev {
     int* ie;                                             // cap x n: 1-based event index (0 when unused)
     int* ne;                                             // n: events found (may exceed cap)
 };
+// swrt_ode23_packets_tspans: every packet's own tspan row, packet-contiguous (row i at tsp + i*ntspan), and the per-solve
+// constants of Ode23Ctl that then differ per packet (SoA, n each), formed by the begin kernel and loaded by the decide
+// kernel.  Passed by value; all null when the packets share one tspan.
+struct Ode23Spans {
+    const double* tsp; int ntspan;
+    double *tfinal, *hmax, *tdir;
+};
 // the alphas of `stage` (selected, not indexed: a run-time index would move the kernel argument to local memory)
 __device__ __forceinline__ const double* ode23_pkt_alpha(const Ode23Pkt& s, int stage) {
     return stage == 0 ? s.al[0] : stage == 1 ? s.al[1] : s.al[2];
@@ -356,11 +363,15 @@ cudaError_t launch_nufft_eval_dev(const NufftArgs& a, const Ode23Sel& sel, cudaS
 // swrt_ode23_packets: `k` holds the per-solve constants (controller section zero, t = t0).  begin: the rh norm and the
 // initial step of every packet from f1; decide: each packet's norm, controller, dense rows and accept, as swrt_ode23's
 // kernels with the packet's own state.  With ev set, begin also seeds the event values and clears the records, and decide
-// locates and records the events of every accepted step and applies a terminal stop.
+// locates and records the events of every accepted step and applies a terminal stop.  With sp set (no events), every
+// packet's tfinal, tdir, hmax, htspan, t0 and tspan come from its own row of sp.tsp instead of k.
+// swrt_ode23_packets_tspans: col (n x ntspan column-major) to packet-contiguous rows, s.al[0] = t0/tmax, flags cleared
+void launch_ode23_pkt_rows(long long n, int ntspan, const double* col, double* rows, const Ode23Pkt& s, double tmax,
+                           cudaStream_t st);
 void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, const Ode23Ev* ev,
-                            cudaStream_t st);
+                            const Ode23Spans* sp, cudaStream_t st);
 void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl& k, double thr, int round, const Ode23Ev* ev,
-                             cudaStream_t st);
+                             const Ode23Spans* sp, cudaStream_t st);
 cudaError_t launch_nufft_eval_pkt(const NufftArgs& a, const double2* grid1, const Ode23Pkt& s, int stage, cudaStream_t st);
 // (rtol/err)^(1/3) as glibc's correctly rounded-in-practice pow gives it (host and device, misc_kernels.cu)
 __host__ __device__ double pow_third(double x);

@@ -112,10 +112,16 @@ class ShardedEnsemble:
         """the reference's per-flow-step ode23 solve over ALL shards: the error norm is MAX-all-reduced so
         that every rank accepts/rejects the same steps (the reference's norm couples all packets).
         ``per_packet=True``: every packet under its own controller (``Engine.ode23_packets``) on the local shard, with no
-        collective; the returned counts are this rank's, and so are the event records with ``events`` (per-packet only)."""
+        collective; the returned counts are this rank's, and so are the event records with ``events`` (per-packet only).
+        A 2-D ``tspan`` (per-packet only) is the global ``(ntspan, n_total)`` matrix: this rank solves its columns [lo, hi)."""
         from .reference_api import ode23
         if events is not None and not per_packet:
             raise ValueError("ode23: events need per_packet=True (the coupled solve has no events)")
+        if per_packet and np.ndim(tspan) == 2:
+            tspan = np.asarray(tspan, dtype=np.float64)
+            if tspan.shape[1] != self.n_total:
+                raise ValueError(f"ode23: a per-packet tspan must have n_total = {self.n_total} columns, got {tspan.shape}")
+            tspan = tspan[:, self.lo:self.hi]
         if per_packet:
             return ode23(self.engine, tspan, tmax, rtol, atol, per_packet=True, events=events, ev_cap=ev_cap)
         return ode23(self.engine, tspan, tmax, rtol, atol, reduce_max=self._allreduce_max)

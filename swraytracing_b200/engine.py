@@ -73,6 +73,8 @@ SIGNATURES = {
     "swrt_ode23": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int64), _dp, C.c_int]),
     "swrt_ode23_packets": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int32), _dp,
                                      C.POINTER(C.c_int64)]),
+    "swrt_ode23_packets_tspans": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, _dp, C.POINTER(C.c_int32),
+                                            _dp, C.POINTER(C.c_int64)]),
     "swrt_ode23_packets_events": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, C.POINTER(_Event), C.c_int,
                                             C.c_int, _dp, C.POINTER(C.c_int32), _dp, _dp, _dp, C.POINTER(C.c_int32),
                                             C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
@@ -380,14 +382,32 @@ class Engine:
         increasing.  The result then also holds ``te`` (ev_cap, n), ``ye`` (ev_cap, 4, n) and ``ie`` (ev_cap, n, 1-based
         event index): each packet's first ``ev_cap`` records in ascending (te, ie) order, NaN / 0 where unused; ``ne``
         (events found per packet, may exceed ev_cap); ``events`` (their total) and ``terminated`` (packets stopped by a
-        terminal event: status 2, state and ``t_end`` those of the event)."""
+        terminal event: status 2, state and ``t_end`` those of the event).
+
+        A 2-D ``tspan`` of shape ``(ntspan, n)`` gives every packet its own (swrt_ode23_packets_tspans): column ``i`` is
+        packet ``i``'s tspan, so ``Y[j, :, i]`` is its state at ``tspan[j, i]``, as ``ode23(odefun, tspan(:, i), y0(:, i))``
+        gives it.  Each column has its own direction (backward when it decreases); a constant column keeps its packet
+        where it is.  ``t`` is then the per-packet array ``tspan[-1]``.  Events need a 1-D ``tspan``."""
         ts = _f64(tspan)
-        dense = ts.size > 2
-        Y = np.empty((ts.size, 4, self.n)) if dense else None
+        if ts.ndim == 2:
+            if events is not None:
+                raise ValueError("ode23_packets: events need one shared (1-D) tspan")
+            if ts.shape[0] < 2 or ts.shape[1] != self.n:
+                raise ValueError(f"ode23_packets: a per-packet tspan must be (ntspan >= 2, n = {self.n}), got {ts.shape}")
+        elif ts.ndim != 1:
+            raise ValueError(f"ode23_packets: tspan must be 1-D (shared) or 2-D (ntspan, n), got shape {ts.shape}")
+        nt = ts.shape[0]
+        dense = nt > 2
+        Y = np.empty((nt, 4, self.n)) if dense else None
         pstat = np.empty((3, self.n), dtype=np.int32)          # the C side's n x 3 column-major block
         t_end = np.empty(self.n)
         i32 = C.POINTER(C.c_int32)
-        if events is None:
+        if ts.ndim == 2:                                        # C order (ntspan, n) = the C side's n x ntspan column-major
+            st = (C.c_int64 * 5)()
+            self._check(self.lib.swrt_ode23_packets_tspans(self._h, _ptr(ts), int(nt), float(tmax or 0.0), float(rtol),
+                                                           float(atol), _ptr(Y) if dense else None, pstat.ctypes.data_as(i32),
+                                                           _ptr(t_end), st))
+        elif events is None:
             st = (C.c_int64 * 5)()
             self._check(self.lib.swrt_ode23_packets(self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol),
                                                     _ptr(Y) if dense else None, pstat.ctypes.data_as(i32), _ptr(t_end), st))
@@ -402,7 +422,8 @@ class Engine:
                 self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol), arr, len(evs), int(ev_cap),
                 _ptr(Y) if dense else None, pstat.ctypes.data_as(i32), _ptr(t_end), _ptr(te), _ptr(ye), ie.ctypes.data_as(i32),
                 ne.ctypes.data_as(i32), st))
-        out = {"nsteps": st[0], "nfailed": st[1], "nfevals": st[2], "t": float(ts[-1]), "stopped": st[3], "host_waits": st[4],
+        out = {"nsteps": st[0], "nfailed": st[1], "nfevals": st[2], "t": ts[-1].copy() if ts.ndim == 2 else float(ts[-1]),
+               "stopped": st[3], "host_waits": st[4],
                "steps": pstat[0].copy(), "rejected": pstat[1].copy(), "status": pstat[2].copy(), "t_end": t_end}
         if dense:
             out["Y"] = Y

@@ -329,9 +329,12 @@ def ode23(target, tspan, tmax, rtol=1e-3, atol=1e-6, reduce_max=None, on_device=
     swrt_ode23_packets): what MATLAB gives when ``ode23`` is called once per packet.  Nothing couples the packets, so
     ``reduce_max`` is refused with it; a packet whose step size falls below hmin stops alone (``stopped``, ``status``).
     ``events`` / ``ev_cap`` (per-packet solve only: the coupled solve has no events) locate level crossings of each
-    packet's state as MATLAB's ``odeset('Events', ...)`` would, see ``Engine.ode23_packets``."""
+    packet's state as MATLAB's ``odeset('Events', ...)`` would, see ``Engine.ode23_packets``.  A 2-D ``tspan`` of shape
+    ``(ntspan, Np)`` (per-packet solve only: the coupled solve has one t) gives packet ``i`` the tspan ``tspan[:, i]``."""
     if events is not None and not per_packet:
         raise ValueError("ode23: events need per_packet=True (the coupled solve has no events)")
+    if not per_packet and np.ndim(tspan) != 1:
+        raise ValueError("ode23: a per-packet (2-D) tspan needs per_packet=True (the coupled solve has one t)")
     if per_packet:
         if reduce_max is not None:
             raise ValueError("ode23: per_packet=True needs no reduce_max (the packets are not coupled)")
