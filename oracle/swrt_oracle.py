@@ -584,7 +584,7 @@ def step_packet_xka(P, U, GradU, H, C0, f, dx, dy, dt):
     return out
 
 
-def rk4_step_batch(x, y, k, l, a, dt, C0, f, fields, dx, xka, mode="lagrange", planes_k=None, nx=None):
+def rk4_step_batch(x, y, k, l, a, dt, C0, f, fields, dx, xka, mode="lagrange", planes_k=None, nx=None, eval_planes=None):
     """Vectorised-over-packets restatement of step_packet / step_packet_xka.
 
     mode='lagrange': identical arithmetic to the reference, but the per-packet scalar that the
@@ -594,7 +594,9 @@ def rk4_step_batch(x, y, k, l, a, dt, C0, f, fields, dx, xka, mode="lagrange", p
     mode='spectral': the continuous ray equations -- U,V,H and gradients evaluated by exact trig sum
     at the point and composed pointwise (SURVEY.md 7.2 'step_packet_xka composes fields ...').
     fields: dict u,v,u_x,u_y,v_x,v_y[,H] of grids (lagrange) ; planes_k: list of 6 or 7 coefficient
-    planes (spectral; H plane is eta_g, H = 1 + eta_g is applied by putting 1 in its (0,0) mode)."""
+    planes (spectral; H plane is eta_g, H = 1 + eta_g is applied by putting 1 in its (0,0) mode).
+    eval_planes: optional ``(x, y, planes) -> (len(planes), n)`` evaluator of the spectral mode, e.g. the C oracle's
+    long-double sums (c_oracle.spectral_eval), which are fast enough for grids above 128^2; default spectral_eval here."""
     n = x.size
     K2 = k * k + l * l
     if mode == "lagrange":
@@ -637,6 +639,8 @@ def rk4_step_batch(x, y, k, l, a, dt, C0, f, fields, dx, xka, mode="lagrange", p
     else:
         npl = len(planes_k)
         def e_all(xx, yy, idx):
+            if eval_planes is not None:
+                return list(eval_planes(xx, yy, [planes_k[i] for i in idx]))
             return [spectral_eval(xx, yy, planes_k[i], dx, nx).astype(np.float64) for i in idx]
         def vel(xx, yy):
             if not xka:

@@ -98,12 +98,12 @@ def test_mex_gateway_compiles():
 
 
 def test_spectral_geometry_fits_shared_memory_for_every_size():
-    """host-only: for every even grid size up to 512 and every plane count / m-tile choice the dense kernel's dynamic
+    """host-only: for every even grid size up to 130, a selection up to 1024, and every plane count / m-tile choice the dense kernel's dynamic
     shared memory (chunk ring + barriers + twiddle table) stays inside the 227 KB a CTA may opt into, the ring has at
     least three chunks, chunks tile a pass, and the twiddle table (when on) has one double per lane per k-step per warp"""
     from swraytracing_b200.engine import spectral_geometry
     seen_on = seen_off = 0
-    for nx in list(range(4, 132, 2)) + [160, 192, 200, 250, 256, 258, 320, 384, 500, 512]:
+    for nx in list(range(4, 132, 2)) + [160, 192, 200, 250, 256, 258, 320, 384, 500, 512, 640, 768, 1000, 1024]:
         for npl in range(1, 8):
             for mt in (1, 2):
                 g = spectral_geometry(nx, npl, mt)

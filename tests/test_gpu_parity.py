@@ -14,6 +14,7 @@ from swraytracing_b200 import reference_api as R
 from swraytracing_b200 import workloads as W
 from oracle import swrt_oracle as O
 from oracle import c_oracle as CO
+from test_spectral_large_grids import EVAL_SIZES
 
 pytestmark = pytest.mark.gpu
 
@@ -47,7 +48,7 @@ def make_packets(n, L, seed=5):
 # ------------------------------------------------------------------------------------------------
 # P2: SPECTRAL kernel vs exact-sum oracle
 # ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("nx", [16, 32, 36, 48, 64, 128])
+@pytest.mark.parametrize("nx", EVAL_SIZES)
 @pytest.mark.parametrize("mt", [1, 2])
 @pytest.mark.parametrize("psi", [True, False])
 def test_spectral_eval_vs_exact_sum(nx, mt, psi):
@@ -55,7 +56,7 @@ def test_spectral_eval_vs_exact_sum(nx, mt, psi):
     # psi=False: the six planes contracted directly.  Same oracle, same tolerance.
     L = 2 * np.pi; dx = L / nx
     psik, planes = make_flow(nx)
-    n = 517 if nx <= 64 else 300
+    n = 517 if nx <= 64 else (300 if nx <= 128 else 120)
     x, y, k, l = make_packets(n, L)
     ref = CO.spectral_eval(x, y, planes, dx, nx, precise=True)
     with S.Engine(nx, L, F0, GH0, S.MODE_SPECTRAL) as e:
@@ -875,7 +876,7 @@ def test_scheme_diagnostics_and_difference_scheme_cross_check():
 # NUFFT mode: the same exact Fourier series as SPECTRAL (P2 contract), evaluated by a type-2 non-uniform FFT
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
-@pytest.mark.parametrize("nx", [16, 32, 36, 48, 64, 128, 256])
+@pytest.mark.parametrize("nx", [16, 32, 36, 48, 64, 128, 256, 384, 512, 1024])
 def test_nufft_eval_vs_exact_sum(nx):
     L = 2 * np.pi; dx = L / nx
     psik, planes = make_flow(nx)

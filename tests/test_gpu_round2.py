@@ -246,7 +246,7 @@ def test_multi_device_handle_qg_frame_producer():
 # ------------------------------------------------------------------------------------------------
 # fused SPECTRAL RK4 steppers (one launch per run of steps) against the composed route
 # ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("nx", [32, 64, 128])
+@pytest.mark.parametrize("nx", [32, 64, 128, 130, 256, 512])
 @pytest.mark.parametrize("scheme", ["rk4_packet", "rk4_xka"])
 @pytest.mark.parametrize("flow", ["psi", "planes", "two-frame"])
 def test_spectral_fused_rk4_equals_the_composed_launches(nx, scheme, flow):
@@ -284,12 +284,13 @@ def test_spectral_fused_rk4_equals_the_composed_launches(nx, scheme, flow):
 # ------------------------------------------------------------------------------------------------
 # where the x twiddles live: rotation in registers / shared-memory table / global (L2) table
 # ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("nx", [64, 128, 256])
+@pytest.mark.parametrize("nx", [64, 128, 256, 512])
 def test_twiddle_homes_agree_and_match_the_exact_sum(nx):
     """swrt_set_tuning bits 3-4 pick where the dense kernel keeps a step's x twiddles.  The three homes run the SAME
     recurrences (the table forms tabulate them), so the evaluations agree to the last bits (<= 1e-14 of max|plane|), and each
-    is within 1e-12 of the long-double exact-sum oracle; 20 leapfrog steps agree to 1e-12.  256^2 exercises the L2 table
-    that is now the default above 128^2."""
+    is within 1e-12 of the long-double exact-sum oracle; 20 leapfrog steps agree to 1e-12.  256^2 and 512^2 exercise the L2
+    table that is the default above 128^2.  The leapfrog contracts the six planes: a psi-hat leapfrog at 256^2 and 512^2
+    runs anchored, which has no twiddle home."""
     from oracle import c_oracle as CO
     w = W.make_workload("C3", n_packets=389, nx=nx)
     planes = W.planes_from_psik(w.psik, w.L, w.u_mean)
@@ -303,6 +304,7 @@ def test_twiddle_homes_agree_and_match_the_exact_sum(nx):
         eng.set_packets(w.x, w.y, w.k, w.l)
         ev = eng.eval()
         assert (np.abs(ev - ref) / scale).max() < 1e-12, (nx, tw)
+        eng.set_tuning(twiddles=tw, use_psi_moments=False)
         eng.step(S.SCHEME_LEAPFROG, w.dt, 20)
         evs.append(ev); trajs.append(np.stack(eng.get_packets()))
         eng.close()
