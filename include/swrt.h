@@ -258,6 +258,28 @@ int swrt_ideal_omega_hist(swrt_handle* h, double alpha, int64_t npts, const doub
 int swrt_diag(swrt_handle* h, double alpha, double out[8]);
 /* per-packet intrinsic and absolute frequency (symplectic_full_fourier.m:41,54-56)             */
 int swrt_omega(swrt_handle* h, double alpha, double* omega, double* Omega_abs);
+/* per-packet quantities for swrt_packet_quantity / swrt_hist2; every operation rounded on its own */
+#define SWRT_Q_XMOD       0  /* x periodic in [0, L): r = x - L*floor(x/L); r < 0 -> r + L; then r >= L -> 0 */
+#define SWRT_Q_YMOD       1  /* the same for y */
+#define SWRT_Q_K          2
+#define SWRT_Q_L          3
+#define SWRT_Q_KMAG       4  /* sqrt(k*k + l*l), SWRT_EVENT_KMAG's expression */
+#define SWRT_Q_THETA      5  /* atan2(l, k) in [-pi, pi] (CUDA atan2) */
+#define SWRT_Q_OMEGA      6  /* omega_kernel's omega, bit-identical to swrt_omega */
+#define SWRT_Q_OMEGA_ABS  7  /* Omega = omega + U.k at alpha, bit-identical to swrt_omega's Omega_abs; needs a flow */
+/* out[n]: quantity q of every packet (alpha is used by the two frequencies only).  A multi-device handle fills each
+ * shard's rows.  SWRT_ERR_ARG: an unknown q or a null out; SWRT_ERR_STATE: OMEGA_ABS without flow slot 0, or a
+ * two-frame alpha without slot 1.                                                                                  */
+int swrt_packet_quantity(swrt_handle* h, int q, double alpha, double* out /* n */);
+/* N = histcounts2(Qx, Qy, xedges, yedges) of the packets' quantities qx, qy, each value exactly what
+ * swrt_packet_quantity returns: counts (nxe-1) x (nye-1) column-major, counts[i + j*(nxe-1)] = N(i,j); bin
+ * [e_i, e_i+1) on each axis, last bin closed; NaN or out of range in either coordinate is not counted; accumulate
+ * != 0 adds to counts.  alpha is used by SWRT_Q_OMEGA / SWRT_Q_OMEGA_ABS only.  A multi-device handle SUM-all-reduces
+ * the u64 counts of its shards (bit-exact under any sharding).  SWRT_ERR_ARG, with the handle usable: an unknown
+ * quantity, nxe or nye outside 2..4096, edges not finite or decreasing, a null pointer; SWRT_ERR_STATE as in
+ * swrt_packet_quantity.                                                                                            */
+int swrt_hist2(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
+               double alpha, uint64_t* counts, int accumulate);
 
 /* ---- spectral <-> grid kit on the device (setup, not hot path) ----------------------------- */
 /* fk = g2k(fg) (g2k.m:5-9) and fg = k2g(fk) (k2g.m:5-6, fulspec.m:10-19), column-major.         */

@@ -391,6 +391,20 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (swrt_ideal_omega_hist(h, mxGetScalar(prhs[2]), (int64_t)mxGetNumberOfElements(prhs[3]), mxGetPr(prhs[3]), mxGetPr(prhs[4]), mxGetPr(prhs[5]),
                                   mxGetPr(prhs[6]), (int)mxGetNumberOfElements(prhs[5]), mxGetScalar(prhs[7]), mxGetPr(prhs[8]), ne,
                                   (uint64_t*)mxGetData(plhs[0]))) fail(h, cmd);
+    } else if (!strcmp(cmd, "hist2")) {               /* N = (h, qx, xedges, qy, yedges [, alpha])  -- histcounts2, N double */
+        need(nrhs, 6, "'hist2', h, qx, xedges, qy, yedges [, alpha]");
+        int nxe = (int)mxGetNumberOfElements(prhs[3]), nye = (int)mxGetNumberOfElements(prhs[5]);
+        if (nxe < 2 || nye < 2) mexErrMsgIdAndTxt("swrt:usage", "hist2: at least two edges on each axis");
+        size_t nb = (size_t)(nxe - 1) * (size_t)(nye - 1);
+        uint64_t* c = (uint64_t*)mxCalloc(nb, sizeof(uint64_t));
+        if (swrt_hist2(h, (int)mxGetScalar(prhs[2]), mxGetPr(prhs[3]), nxe, (int)mxGetScalar(prhs[4]), mxGetPr(prhs[5]), nye,
+                       sc(prhs, nrhs, 6, 0.0), c, 0)) fail(h, cmd);
+        plhs[0] = mxCreateDoubleMatrix((size_t)nxe - 1, (size_t)nye - 1, mxREAL);
+        for (size_t i = 0; i < nb; i++) mxGetPr(plhs[0])[i] = (double)c[i];
+        mxFree(c);
+    } else if (!strcmp(cmd, "packet_quantity")) {     /* q = (h, qkind [, alpha]) */
+        need(nrhs, 3, "'packet_quantity', h, qkind [, alpha]");
+        if (swrt_packet_quantity(h, (int)mxGetScalar(prhs[2]), sc(prhs, nrhs, 3, 0.0), vec(&plhs[0], n))) fail(h, cmd);
     } else if (!strcmp(cmd, "diag")) {                /* d = (h, alpha) */
         if (swrt_diag(h, sc(prhs, nrhs, 2, 0.0), vec(&plhs[0], 8))) fail(h, cmd);
     } else if (!strcmp(cmd, "omega")) {               /* [omega, Omega] = (h, alpha) */

@@ -127,6 +127,15 @@ __global__ void rk4_final_kernel(Rk4Args a) {
 
 // histcounts(w, edges): bin i = [e_i, e_{i+1}), last bin closed; NaN / out of range dropped.
 constexpr int kMaxSmemBins = 4096;
+// the bin of v, e[0] <= v <= e[nb]: the last a with e[a] <= v; v == e[nb] lands in a = nb-1 because b never drops below nb
+__device__ __forceinline__ int bin_index(const double* e, int nb, double v) {
+    int a = 0, b = nb;
+    while (b - a > 1) {
+        int m = (a + b) >> 1;
+        if (e[m] <= v) a = m; else b = m;
+    }
+    return a;
+}
 __global__ void hist_kernel(long long n, const double* __restrict__ w, const double* __restrict__ edges, int nedges,
                             unsigned long long* __restrict__ counts) {
     extern __shared__ unsigned char hs[];
@@ -141,12 +150,7 @@ __global__ void hist_kernel(long long n, const double* __restrict__ w, const dou
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const double v = w[i];
         if (!(v >= lo && v <= hi)) continue;   // also drops NaN
-        int a = 0, b = nb;                     // find last a with se[a] <= v
-        while (b - a > 1) {
-            int m = (a + b) >> 1;
-            if (se[m] <= v) a = m; else b = m;
-        }
-        atomicAdd(&sc[a], 1u);                 // v == hi lands in a = nb-1 because b never drops below nb
+        atomicAdd(&sc[bin_index(se, nb, v)], 1u);
     }
     __syncthreads();
     for (int i = threadIdx.x; i < nb; i += blockDim.x)
@@ -175,14 +179,78 @@ __global__ void ideal_hist_kernel(long long npts, const double* __restrict__ u, 
         for (int j = 0; j < nang; j++) {
             const double w = __dadd_rn(omega0, __dadd_rn(__dmul_rn(uu, sk[j]), __dmul_rn(vv, sk[nang + j])));
             if (!(w >= lo && w <= hi)) continue;
-            int a = 0, b = nb;
-            while (b - a > 1) { int m = (a + b) >> 1; if (se[m] <= w) a = m; else b = m; }
-            atomicAdd(&sc[a], 1u);
+            atomicAdd(&sc[bin_index(se, nb, w)], 1u);
         }
     }
     __syncthreads();
     for (int i = threadIdx.x; i < nb; i += blockDim.x)
         if (sc[i]) atomicAdd(&counts[i], (unsigned long long)sc[i]);
+}
+
+// ---- swrt_packet_quantity / swrt_hist2 ------------------------------------------------------------------------------
+// x periodic in [0, L): every operation rounded on its own (this file is compiled with FMA contraction)
+__device__ __forceinline__ double wrap_period(double x, double L) {
+    double r = __dsub_rn(x, __dmul_rn(L, floor(__ddiv_rn(x, L))));
+    if (r < 0.0) r = __dadd_rn(r, L);
+    return r >= L ? 0.0 : r;
+}
+// quantity q of packet i: the one definition both swrt_packet_quantity and the histogram bin, so a binned value is
+// exactly the value the caller reads back.  OMEGA / OMEGA_ABS are omega_kernel's outputs (bit-identical to swrt_omega).
+__device__ __forceinline__ double packet_quantity(int q, const PktQ& p, long long i) {
+    switch (q) {
+        case SWRT_Q_XMOD: return wrap_period(p.x[i], p.L);
+        case SWRT_Q_YMOD: return wrap_period(p.y[i], p.L);
+        case SWRT_Q_K: return p.k[i];
+        case SWRT_Q_L: return p.l[i];
+        case SWRT_Q_KMAG: { const double k = p.k[i], l = p.l[i]; return __dsqrt_rn(__dadd_rn(__dmul_rn(k, k), __dmul_rn(l, l))); }
+        case SWRT_Q_THETA: return atan2(p.l[i], p.k[i]);
+        case SWRT_Q_OMEGA: return p.om[i];
+        default: return p.Om[i];
+    }
+}
+__global__ void packet_quantity_kernel(long long n, int q, PktQ p, double* __restrict__ out) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = packet_quantity(q, p, i);
+}
+// histcounts2: bin (i, j) = [xe_i, xe_i+1) x [ye_j, ye_j+1), last bin closed on each axis, counts[i + j*nbx].  Both edge
+// arrays sit in shared memory; SMEM: so do the CTA's u32 counters, flushed (non-zero bins) with u64 global atomics, else
+// every count goes to the global u64 counters.  The lanes of a warp holding the same bin are counted by one atomic of
+// their number (__match_any_sync), so a histogram whose packets crowd into a few bins -- a wavenumber ring -- does not
+// serialise on those addresses.  The loop is warp-uniform so that every lane takes part in the match.
+template <bool SMEM>
+__global__ void __launch_bounds__(1024) hist2_kernel(long long n, int qx, int qy, PktQ p, const double* __restrict__ edges,
+                                                    int nxe, int nye, unsigned long long* __restrict__ counts) {
+    extern __shared__ unsigned char hs[];
+    double* ex = reinterpret_cast<double*>(hs);
+    double* ey = ex + nxe;
+    unsigned int* sc = reinterpret_cast<unsigned int*>(ey + nye);
+    const int nbx = nxe - 1, nby = nye - 1;
+    for (int i = threadIdx.x; i < nxe + nye; i += blockDim.x) ex[i] = edges[i];
+    if (SMEM)
+        for (int i = threadIdx.x; i < nbx * nby; i += blockDim.x) sc[i] = 0;
+    __syncthreads();
+    const double xlo = ex[0], xhi = ex[nbx], ylo = ey[0], yhi = ey[nby];
+    const int lane = threadIdx.x & 31;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long i0 = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); i0 < n; i0 += stride) {
+        const long long i = i0 + lane;
+        int bin = -1;
+        if (i < n) {
+            const double vx = packet_quantity(qx, p, i), vy = packet_quantity(qy, p, i);
+            if (vx >= xlo && vx <= xhi && vy >= ylo && vy <= yhi)             // also drops NaN
+                bin = bin_index(ex, nbx, vx) + bin_index(ey, nby, vy) * nbx;
+        }
+        const unsigned peers = __match_any_sync(0xffffffffu, bin);
+        if (bin >= 0 && lane == __ffs(peers) - 1) {
+            if (SMEM) atomicAdd(&sc[bin], (unsigned)__popc(peers));
+            else atomicAdd(&counts[bin], (unsigned long long)__popc(peers));
+        }
+    }
+    if (SMEM) {
+        __syncthreads();
+        for (int i = threadIdx.x; i < nbx * nby; i += blockDim.x)
+            if (sc[i]) atomicAdd(&counts[i], (unsigned long long)sc[i]);
+    }
 }
 
 // partial sums per block, then one block reduces the partials in a fixed order (deterministic)
@@ -792,6 +860,33 @@ void launch_ideal_hist(long long npts, const double* u, const double* v, const d
     unsigned nb = nblk(npts, 256);
     if (nb > 148 * 8) nb = 148 * 8;
     ideal_hist_kernel<<<nb, 256, smem, st>>>(npts, u, v, kvx, kvy, nang, omega0, edges_dev, nedges, counts_dev);
+}
+void launch_packet_quantity(long long n, int q, const PktQ& p, double* out, cudaStream_t st) {
+    if (n > 0) packet_quantity_kernel<<<nblk(n, 256), 256, 0, st>>>(n, q, p, out);
+}
+cudaError_t launch_hist2(long long n, int qx, int qy, const PktQ& p, const double* edges_dev, int nxe, int nye,
+                         unsigned long long* counts_dev, cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    int dev = 0, optin = 0, nsm = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return e;
+    // the path is chosen by size alone: private counters when they fit beside the edges
+    const size_t edge_bytes = (size_t)(nxe + nye) * 8;
+    const size_t smem_path = edge_bytes + (size_t)(nxe - 1) * (nye - 1) * 4;
+    const bool smem = smem_path <= (size_t)optin;
+    const size_t bytes = smem ? smem_path : edge_bytes;
+    auto kern = smem ? hist2_kernel<true> : hist2_kernel<false>;
+    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes)) != cudaSuccess) return e;
+    // 1024 threads: the shared-memory path fits one CTA an SM, and the kernel is bound by latency, not bandwidth
+    int per_sm = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 1024, bytes)) != cudaSuccess) return e;
+    // one wave of CTAs: each pays for zeroing and flushing its counters once
+    unsigned nb = (unsigned)(per_sm > 0 ? per_sm : 1) * (unsigned)nsm;
+    if (nb > nblk(n, 1024)) nb = nblk(n, 1024);
+    kern<<<nb, 1024, bytes, st>>>(n, qx, qy, p, edges_dev, nxe, nye, counts_dev);
+    return cudaGetLastError();
 }
 void launch_diag(long long n, const double* x, const double* y, const double* k, const double* l, const double* a,
                  const double* omega, const double* Omega_abs, double* out8_dev, cudaStream_t st) {

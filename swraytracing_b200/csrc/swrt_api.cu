@@ -98,6 +98,10 @@ struct swrt_handle {
     double* edges_dev = nullptr; int edges_cap = 0;
     std::vector<double> edges_host;       // what edges_dev currently holds
     unsigned long long* counts_dev = nullptr; int counts_cap = 0;
+    // swrt_hist2: xedges then yedges on the device (h2_edges_host and h2_nxe: what they hold) and the u64 counts
+    double* h2_edges_dev = nullptr; int h2_edges_cap = 0;
+    std::vector<double> h2_edges_host; int h2_nxe = 0;
+    unsigned long long* h2_counts_dev = nullptr; int64_t h2_counts_cap = 0;
     // instrumentation
     int64_t launches = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, hist_ev = nullptr;
@@ -154,6 +158,8 @@ int grp_bs23_begin(swrt_handle* g, double alpha, double threshold, double* rh_no
 int grp_bs23_attempt(swrt_handle* g, double hstep, const double alpha[3], double threshold, double* err_norm);
 int grp_ideal_omega_hist(swrt_handle* g, double alpha, int64_t npts, const double* x, const double* y, const double* kvx,
                          const double* kvy, int nangles, double omega0, const double* edges, int nedges, uint64_t* counts);
+int grp_hist2(swrt_handle* g, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye, double alpha,
+              uint64_t* counts, int accumulate);
 int up(swrt_handle* g, swrt_handle* c, int rc);
 inline double* at(double* p, int64_t lo) { return p ? p + lo : nullptr; }
 void stager_free(swrt_handle* h);
@@ -718,6 +724,7 @@ int swrt_destroy(swrt_handle* h) {
     for (auto& p : h->e) dfree(p);
     dfree(h->xs); dfree(h->ys); dfree(h->ax); dfree(h->ay); dfree(h->om); dfree(h->Om);
     dfree(h->diag_dev); dfree(h->edges_dev); dfree(h->counts_dev); dfree(h->bs_norm_dev);
+    dfree(h->h2_edges_dev); dfree(h->h2_counts_dev);
     for (auto& p : h->bs_yt) dfree(p);
     for (auto& row : h->bs_f) for (auto& p : row) dfree(p);
     dfree(h->ode_ctl);
@@ -1592,6 +1599,99 @@ int swrt_ideal_omega_hist(swrt_handle* h, double alpha, int64_t npts, const doub
     if (e == cudaSuccess) e = cudaGetLastError();
     cudaFree(dk); cudaFree(de); cudaFree(dc);
     if (e != cudaSuccess) return fail(h, SWRT_ERR_CUDA, "swrt_ideal_omega_hist: %s", cudaGetErrorString(e));
+    return SWRT_OK;
+}
+
+// ---- swrt_packet_quantity / swrt_hist2 ----
+static bool valid_quantity(int q) { return q >= SWRT_Q_XMOD && q <= SWRT_Q_OMEGA_ABS; }
+// the packet arrays of the quantities qa, qb; om / Om computed first when one of them is a frequency
+static int quantity_inputs(swrt_handle* h, int qa, int qb, double alpha, PktQ& p) {
+    const bool need_abs = qa == SWRT_Q_OMEGA_ABS || qb == SWRT_Q_OMEGA_ABS;
+    if (need_abs || qa == SWRT_Q_OMEGA || qb == SWRT_Q_OMEGA) {
+        int rc = compute_omega(h, alpha, need_abs);
+        if (rc) return rc;
+    }
+    p = PktQ{h->x, h->y, h->k, h->l, h->om, h->Om, h->p.L};
+    return SWRT_OK;
+}
+
+int swrt_packet_quantity(swrt_handle* h, int q, double alpha, double* out) {
+    if (!h) return SWRT_ERR_ARG;
+    REQUIRE(h, valid_quantity(q), SWRT_ERR_ARG, "unknown packet quantity %d", q);
+    REQUIRE(h, out, SWRT_ERR_ARG, "null out");
+    GROUP(h, grp_each_slice(h, [&](swrt_handle* c, int64_t lo) { return swrt_packet_quantity(c, q, alpha, out + lo); }));
+    CU(h, cudaSetDevice(h->p.device));
+    int rc = ensure_scratch(h, h->n);
+    if (rc) return rc;
+    PktQ p;
+    if ((rc = quantity_inputs(h, q, q, alpha, p))) return rc;
+    launch_packet_quantity(h->n, q, p, h->xs, h->stream);
+    h->launches++;
+    if ((rc = d2h(h, out, h->xs, h->n))) return rc;
+    CU(h, cudaStreamSynchronize(h->stream));
+    CU(h, cudaGetLastError());
+    return SWRT_OK;
+}
+
+static int hist2_args(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye) {
+    REQUIRE(h, valid_quantity(qx) && valid_quantity(qy), SWRT_ERR_ARG, "unknown packet quantity (%d, %d)", qx, qy);
+    REQUIRE(h, xedges && yedges, SWRT_ERR_ARG, "null edges");
+    REQUIRE(h, nxe >= 2 && nxe <= 4096 && nye >= 2 && nye <= 4096, SWRT_ERR_ARG, "bad edges (2 <= nxe, nye <= 4096): %d, %d", nxe, nye);
+    for (int a = 0; a < 2; a++) {
+        const double* e = a ? yedges : xedges;
+        for (int i = 0, ne = a ? nye : nxe; i < ne; i++) {
+            REQUIRE(h, std::isfinite(e[i]), SWRT_ERR_ARG, "%s edge %d is not finite", a ? "y" : "x", i);
+            REQUIRE(h, i == 0 || e[i] >= e[i - 1], SWRT_ERR_ARG, "%s edges must be non-decreasing (edge %d)", a ? "y" : "x", i);
+        }
+    }
+    return SWRT_OK;
+}
+// the histogram into h2_counts_dev (queued, no host wait); the arguments have been checked
+static int hist2_to_device(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
+                           double alpha) {
+    int rc;
+    PktQ p;
+    if ((rc = quantity_inputs(h, qx, qy, alpha, p))) return rc;
+    const int ne = nxe + nye;
+    const int64_t nb = (int64_t)(nxe - 1) * (nye - 1);
+    if (ne > h->h2_edges_cap) {
+        dfree(h->h2_edges_dev); h->h2_edges_cap = 0; h->h2_edges_host.clear();
+        CU(h, cudaMalloc(&h->h2_edges_dev, (size_t)ne * 8));
+        h->h2_edges_cap = ne;
+    }
+    if (nb > h->h2_counts_cap) {
+        dfree(h->h2_counts_dev); h->h2_counts_cap = 0;
+        CU(h, cudaMalloc(&h->h2_counts_dev, (size_t)nb * 8));
+        h->h2_counts_cap = nb;
+    }
+    if (h->h2_nxe != nxe || (int)h->h2_edges_host.size() != ne || memcmp(h->h2_edges_host.data(), xedges, (size_t)nxe * 8) != 0 ||
+        memcmp(h->h2_edges_host.data() + nxe, yedges, (size_t)nye * 8) != 0) {
+        h->h2_edges_host.assign(xedges, xedges + nxe);            // upload only when the edges changed
+        h->h2_edges_host.insert(h->h2_edges_host.end(), yedges, yedges + nye);
+        h->h2_nxe = nxe;
+        CU(h, cudaMemcpyAsync(h->h2_edges_dev, h->h2_edges_host.data(), (size_t)ne * 8, cudaMemcpyHostToDevice, h->stream));
+    }
+    CU(h, cudaMemsetAsync(h->h2_counts_dev, 0, (size_t)nb * 8, h->stream));
+    CU(h, launch_hist2(h->n, qx, qy, p, h->h2_edges_dev, nxe, nye, h->h2_counts_dev, h->stream));
+    h->launches++;
+    return SWRT_OK;
+}
+
+int swrt_hist2(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye, double alpha,
+               uint64_t* counts, int accumulate) {
+    if (!h) return SWRT_ERR_ARG;
+    REQUIRE(h, counts, SWRT_ERR_ARG, "null counts");
+    int rc = hist2_args(h, qx, xedges, nxe, qy, yedges, nye);
+    if (rc) return rc;
+    GROUP(h, grp_hist2(h, qx, xedges, nxe, qy, yedges, nye, alpha, counts, accumulate));
+    CU(h, cudaSetDevice(h->p.device));
+    if ((rc = hist2_to_device(h, qx, xedges, nxe, qy, yedges, nye, alpha))) return rc;
+    const size_t nb = (size_t)(nxe - 1) * (nye - 1);
+    std::vector<uint64_t> tmp(nb);
+    CU(h, cudaMemcpyAsync(tmp.data(), h->h2_counts_dev, nb * 8, cudaMemcpyDeviceToHost, h->stream));
+    CU(h, cudaStreamSynchronize(h->stream));
+    CU(h, cudaGetLastError());
+    for (size_t i = 0; i < nb; i++) counts[i] = accumulate ? counts[i] + tmp[i] : tmp[i];
     return SWRT_OK;
 }
 

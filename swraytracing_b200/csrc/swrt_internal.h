@@ -305,6 +305,14 @@ void launch_hist(long long n, const double* w, const double* edges_dev, int nedg
                  unsigned long long* counts_dev, cudaStream_t st);
 void launch_ideal_hist(long long npts, const double* u, const double* v, const double* kvx, const double* kvy, int nang,
                        double omega0, const double* edges_dev, int nedges, unsigned long long* counts_dev, cudaStream_t st);
+// swrt_packet_quantity / swrt_hist2: the packet arrays a quantity SWRT_Q_* is computed from (om / Om as compute_omega
+// filled them; only the arrays the requested quantities read need be set)
+struct PktQ { const double *x, *y, *k, *l, *om, *Om; double L; };
+void launch_packet_quantity(long long n, int q, const PktQ& p, double* out, cudaStream_t st);
+// histcounts2 of (qx, qy) into counts_dev ((nxe-1)*(nye-1) u64, column-major, added to); edges_dev = xedges then yedges.
+// Per-CTA shared-memory counters when they fit the opt-in shared memory, else global atomics.  Returns the launch error.
+cudaError_t launch_hist2(long long n, int qx, int qy, const PktQ& p, const double* edges_dev, int nxe, int nye,
+                         unsigned long long* counts_dev, cudaStream_t st);
 void launch_diag(long long n, const double* x, const double* y, const double* k, const double* l, const double* a,
                  const double* omega, const double* Omega_abs, double* out8_dev, cudaStream_t st);
 void launch_fill(double* p, double v, long long n, cudaStream_t st);

@@ -161,6 +161,12 @@ class ShardedEnsemble:
         local = self.engine.hist_omega(edges, kind, alpha)
         return self._allreduce_sum(local.astype(np.int64)).astype(np.uint64)
 
+    def hist2(self, qx, xedges, qy, yedges, alpha=0.0):
+        """global histcounts2 of two packet quantities (``Engine.hist2``) over all shards: each rank's local u64 counts,
+        SUM-all-reduced (bit-exact under any world size)"""
+        local = np.asarray(self.engine.hist2(qx, xedges, qy, yedges, alpha))
+        return self._allreduce_sum(local.astype(np.int64)).astype(np.uint64)
+
     def hist_pipeline(self, edges, kind=0):
         return HistPipeline(self, edges, kind)
 

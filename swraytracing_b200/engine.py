@@ -20,6 +20,7 @@ HIST_INTRINSIC, HIST_ABSOLUTE = 0, 1
 FLAG_RHS_GH = 1
 EVENT_X, EVENT_Y, EVENT_K, EVENT_L, EVENT_KMAG, EVENT_OMEGA = 0, 1, 2, 3, 4, 5
 MAX_EVENTS = 8
+Q_XMOD, Q_YMOD, Q_K, Q_L, Q_KMAG, Q_THETA, Q_OMEGA, Q_OMEGA_ABS = 0, 1, 2, 3, 4, 5, 6, 7
 
 _dp = C.POINTER(C.c_double)
 
@@ -85,6 +86,8 @@ SIGNATURES = {
                                         C.POINTER(C.c_uint64)]),
     "swrt_diag": (C.c_int, [C.c_void_p, C.c_double, _dp]),
     "swrt_omega": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp]),
+    "swrt_packet_quantity": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp]),
+    "swrt_hist2": (C.c_int, [C.c_void_p, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_double, C.POINTER(C.c_uint64), C.c_int]),
     "swrt_g2k": (C.c_int, [C.c_int, _dp, C.c_int, _dp, _dp]),
     "swrt_k2g": (C.c_int, [C.c_int, _dp, _dp, C.c_int, _dp]),
     "swrt_qg_create": (C.c_int, [C.c_int, C.c_int] + [C.c_double] * 8 + [_dp, _dp, C.POINTER(C.c_void_p)]),
@@ -475,6 +478,31 @@ class Engine:
         Om = np.empty(self.n) if absolute else None
         self._check(self.lib.swrt_omega(self._h, float(alpha), _ptr(om), _ptr(Om)))
         return om, Om
+
+    def packet_quantity(self, q, alpha=0.0):
+        """quantity ``q`` (``Q_XMOD``, ``Q_YMOD``, ``Q_K``, ``Q_L``, ``Q_KMAG``, ``Q_THETA``, ``Q_OMEGA``, ``Q_OMEGA_ABS``) of
+        every packet, exactly the values ``hist2`` bins; ``alpha`` is the flow time of the two frequencies"""
+        out = np.empty(self.n)
+        self._check(self.lib.swrt_packet_quantity(self._h, int(q), float(alpha), _ptr(out)))
+        return out
+
+    def hist2(self, qx, xedges, qy, yedges, alpha=0.0, counts=None):
+        """MATLAB's ``histcounts2(Qx, Qy, xedges, yedges)`` of two packet quantities on the device (swrt_hist2): a
+        ``(nxe-1, nye-1)`` uint64 array, ``N[i, j]`` the packets with ``xedges[i] <= Qx < xedges[i+1]`` and
+        ``yedges[j] <= Qy < yedges[j+1]`` (the last bin of each axis closed); NaN or out-of-range packets are not counted.
+        ``counts`` (uint64, that shape) is added to and returned."""
+        xe, ye = _f64(xedges).ravel(), _f64(yedges).ravel()
+        shape = (max(xe.size - 1, 0), max(ye.size - 1, 0))
+        acc = counts is not None
+        if acc and (not isinstance(counts, np.ndarray) or counts.dtype != np.uint64 or counts.shape != shape):
+            raise ValueError(f"hist2: counts must be a uint64 array of shape {shape}")
+        buf = np.zeros(shape, dtype=np.uint64, order="F") if not acc else np.asfortranarray(counts)   # C: counts[i + j*(nxe-1)]
+        self._check(self.lib.swrt_hist2(self._h, int(qx), _ptr(xe), xe.size, int(qy), _ptr(ye), ye.size, float(alpha),
+                                        buf.ctypes.data_as(C.POINTER(C.c_uint64)), int(acc)))
+        if acc and buf is not counts:
+            counts[...] = buf
+            return counts
+        return buf
 
     # -- instrumentation --
     def launch_count(self, reset=False):
