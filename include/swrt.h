@@ -192,7 +192,7 @@ int swrt_ode23_packets(swrt_handle* h, const double* tspan, int ntspan, double t
  * and keeps its state.  tmax is shared (alpha = t/tmax for every packet).  Y (ntspan x 4 x n, may be NULL) row j of
  * packet i is the state at tspan[j*n + i]; Y, pstat, t_end and stats[0..4] as in swrt_ode23_packets.  SWRT_ERR_ARG, with
  * the packets untouched, when an entry is not finite or steps against its own row's direction (the message names the
- * packet and the entry; equal neighbours are allowed).                                                               */
+ * packet and the entry; equal neighbours are allowed).  With events: swrt_ode23_packets_tspans_events.               */
 int swrt_ode23_packets_tspans(swrt_handle* h, const double* tspan /* n x ntspan, column-major */, int ntspan,
                               double tmax, double rtol, double atol, double* Y, int32_t* pstat, double* t_end,
                               int64_t stats[5]);
@@ -226,10 +226,31 @@ typedef struct swrt_event {
  * dense rows after te* stay NaN.  Y, pstat (status 2 = terminal event), t_end and stats[0..4] as in
  * swrt_ode23_packets; stats[5] = events found, stats[6] = packets stopped by a terminal event.
  * SWRT_ERR_ARG: nev outside 1..SWRT_MAX_EVENTS, ev_cap < 0, an unknown kind, a direction outside {-1, 0, 1}, a terminal
- * flag outside {0, 1}, reserved != 0, a non-finite level, a tspan not strictly increasing.                          */
+ * flag outside {0, 1}, reserved != 0, a non-finite level, a tspan not strictly increasing.  Backward solves and a
+ * tspan per packet with events: swrt_ode23_packets_tspans_events.                                                  */
 int swrt_ode23_packets_events(swrt_handle* h, const double* tspan, int ntspan, double tmax, double rtol, double atol,
                               const swrt_event* ev, int nev, int ev_cap, double* Y, int32_t* pstat, double* t_end,
                               double* te, double* ye, int32_t* ie, int32_t* ne, int64_t stats[7]);
+/* for i = 1:n, [t, Y, te, ye, ie] = ode23(odefun_i, tspan(:, i), y_i, odeset('Events', ...)); end -- the events of
+ * swrt_ode23_packets_events on the solve of swrt_ode23_packets_tspans: a tspan row per packet (n x ntspan, column-major,
+ * entry j of packet i at tspan[j*n + i]), each in its own direction tdir (+1 when its last entry is >= its first, else
+ * -1), so back-traced, staggered and mixed-direction packets find their events in one call.  tmax, Y, pstat and t_end
+ * as in swrt_ode23_packets_tspans; ev, ev_cap, te, ye, ie, ne, status 2 and stats[0..6] as in
+ * swrt_ode23_packets_events.  Everything follows the packet's direction of integration:
+ * - detection is unchanged: rising (g: < 0 to >= 0) is rising along the integration, i.e. as t decreases backward;
+ * - te is located on [t, tnew] in integration order by the same Illinois regula falsi, mirrored for tdir = -1 (t -> -t
+ *   gives te bit for bit up to sign);
+ * - records are kept in order of encounter: ascending tdir*te, then ie;
+ * - a terminal event stops its packet at the first terminal te* in integration order: records and dense rows beyond te*
+ *   (tdir*(t - te*) > 0) are not kept / stay NaN.
+ * A row of equal entries takes one step of size 0: it finds no event and keeps its state.  Apart from a terminal stop a
+ * packet's solve is bit for bit that of swrt_ode23_packets_tspans.  SWRT_ERR_ARG, with the packets untouched: a row
+ * entry not finite or stepping against its own row's direction, and every event fault swrt_ode23_packets_events
+ * refuses.                                                                                                         */
+int swrt_ode23_packets_tspans_events(swrt_handle* h, const double* tspan /* n x ntspan, column-major */, int ntspan,
+                                     double tmax, double rtol, double atol, const swrt_event* ev, int nev, int ev_cap,
+                                     double* Y, int32_t* pstat, double* t_end, double* te, double* ye, int32_t* ie,
+                                     int32_t* ne, int64_t stats[7]);
 
 /* ---- diagnostics -------------------------------------------------------------------------- */
 /* histcounts(omega, edges) (analysis/load_data.m:39-47): counts[nedges-1], bin i = [e_i,e_i+1),

@@ -330,13 +330,33 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
             for (size_t i = 0; i < 3 * n; i++) mxGetPr(plhs[2])[i] = (double)ps[i];
             mxFree(ps);
         }
-    } else if (!strcmp(cmd, "ode23_events")) {        /* [stats, Y, pstat, t_end, te, ye, ie, ne] = (h, tspan, tmax, rtol, atol, ev, ev_cap) */
-        need(nrhs, 8, "'ode23_events', h, tspan, tmax, rtol, atol, ev, ev_cap");
+    } else if (!strcmp(cmd, "ode23_events") || !strcmp(cmd, "ode23_tspans_events")) {
+        /* [stats, Y, pstat, t_end, te, ye, ie, ne] = (h, tspan, tmax, rtol, atol, ev, ev_cap).  'ode23_tspans_events': tspan
+           is a vector shared by every packet, in either direction, or an n x m matrix (m >= 2) whose row i is packet i's
+           own; the events then follow each packet's direction of integration */
+        int spans = !strcmp(cmd, "ode23_tspans_events");
+        need(nrhs, 8, spans ? "'ode23_tspans_events', h, tspan, tmax, rtol, atol, ev, ev_cap" : "'ode23_events', h, tspan, tmax, rtol, atol, ev, ev_cap");
         int nt = (int)mxGetNumberOfElements(prhs[2]);
+        const double* tsp = mxGetPr(prhs[2]);
+        double* rows = NULL;
+        if (spans) {
+            size_t tm = mxGetM(prhs[2]), tn = mxGetN(prhs[2]);
+            if (tm > 1 && tn > 1) {
+                if (tm != (size_t)n)
+                    mexErrMsgIdAndTxt("swrt:usage", "ode23_tspans_events: a tspan matrix must be n x m (one row per packet), got %d x %d",
+                                      (int)tm, (int)tn);
+                nt = (int)tn;
+            } else {                                   /* the shared vector as every packet's row */
+                rows = (double*)mxCalloc(n * (size_t)nt > 0 ? n * (size_t)nt : 1, sizeof(double));
+                for (int j = 0; j < nt; j++)
+                    for (size_t i = 0; i < n; i++) rows[(size_t)j * n + i] = tsp[j];
+                tsp = rows;
+            }
+        }
         /* ev: nev x 4, columns [kind level direction terminal] */
         int nev = (int)mxGetM(prhs[6]), cap = (int)mxGetScalar(prhs[7]);
-        if (mxGetN(prhs[6]) != 4) mexErrMsgIdAndTxt("swrt:usage", "ode23_events: ev must be nev x 4 = [kind level direction terminal]");
-        if (nev < 1 || nev > SWRT_MAX_EVENTS) mexErrMsgIdAndTxt("swrt:usage", "ode23_events: 1 to %d events", SWRT_MAX_EVENTS);
+        if (mxGetN(prhs[6]) != 4) mexErrMsgIdAndTxt("swrt:usage", "%s: ev must be nev x 4 = [kind level direction terminal]", cmd);
+        if (nev < 1 || nev > SWRT_MAX_EVENTS) mexErrMsgIdAndTxt("swrt:usage", "%s: 1 to %d events", cmd, SWRT_MAX_EVENTS);
         const double* e = mxGetPr(prhs[6]);
         swrt_event ev[SWRT_MAX_EVENTS];
         for (int j = 0; j < nev; j++) {
@@ -357,9 +377,10 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (nlhs > 5) { plhs[5] = mxCreateDoubleMatrix((size_t)n, 4 * nc, mxREAL); ye = mxGetPr(plhs[5]); }
         if (nlhs > 6) ie = (int32_t*)mxCalloc(n * nc > 0 ? n * nc : 1, sizeof(int32_t));
         if (nlhs > 7) ne = (int32_t*)mxCalloc(n > 0 ? n : 1, sizeof(int32_t));
-        if (swrt_ode23_packets_events(h, mxGetPr(prhs[2]), nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), ev, nev,
-                                      cap, Y, ps, t_end, te, ye, ie, ne, st))
-            fail(h, cmd);
+        int rc = (spans ? swrt_ode23_packets_tspans_events : swrt_ode23_packets_events)(
+            h, tsp, nt, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), mxGetScalar(prhs[5]), ev, nev, cap, Y, ps, t_end, te, ye, ie, ne, st);
+        if (rows) mxFree(rows);
+        if (rc) fail(h, cmd);
         plhs[0] = mxCreateDoubleMatrix(1, 7, mxREAL);
         for (int i = 0; i < 7; i++) mxGetPr(plhs[0])[i] = (double)st[i];
         if (ps) {

@@ -566,16 +566,27 @@ __device__ __forceinline__ double spacing(double t) {          // np.spacing(abs
     t = fabs(t);
     return __dsub_rn(nextafter(t, __longlong_as_double(0x7ff0000000000000LL)), t);
 }
+// tdir*t: the time in integration order (t forward, -t backward, both exact), so that one set of comparisons and one
+// bracket serve both directions.  Without SPANS every solve is forward and this is t itself.
+template <bool SPANS> __device__ __forceinline__ double ev_key(bool fwd, double t) {
+    if constexpr (SPANS) return fwd ? t : -t;
+    else return t;
+}
 // the crossing of event j inside the step, g(t0) = vL and g(tnew) = vR of opposite signs: Illinois regula falsi on the
-// interpolant (DESIGN.md section 11).  Returns te; g at p(te) is 0 or has vR's sign.
-__device__ double ev_locate(const EvStep& q, int kind, double level, double f, double gH, double vL, double vR) {
+// interpolant over [tL, tR] = [t0, tnew] in integration order, so tR < tL backward (DESIGN.md section 11).  The backward
+// locator is the forward one mirrored (t -> -t gives te bit for bit up to sign).  Returns te; g at p(te) is 0 or has vR's
+// sign.
+template <bool SPANS>
+__device__ double ev_locate(const EvStep& q, bool fwd, int kind, double level, double f, double gH, double vL, double vR) {
     if (vR == 0.0) return q.tnew;
     double tL = q.t0, tR = q.tnew, gL = vL, gR = vR;
     const double tol = __dmul_rn(128.0, fmax(spacing(tL), spacing(tR))), half = __dmul_rn(0.5, tol);
     int moved = 0;                                               // the end that moved last: -1 left, +1 right
-    for (int it = 0; it < 64 && __dsub_rn(tR, tL) > tol; it++) {
+    // the forward bracket on tdir*t: tdir*(tR - tL) > tol, and tm kept half inside both ends
+    for (int it = 0; it < 64 && __dsub_rn(ev_key<SPANS>(fwd, tR), ev_key<SPANS>(fwd, tL)) > tol; it++) {
         double tm = __dsub_rn(tR, __dmul_rn(gR, __ddiv_rn(__dsub_rn(tR, tL), __dsub_rn(gR, gL))));
-        tm = py_min(py_max(tm, __dadd_rn(tL, half)), __dsub_rn(tR, half));
+        tm = ev_key<SPANS>(fwd, py_min(py_max(ev_key<SPANS>(fwd, tm), __dadd_rn(ev_key<SPANS>(fwd, tL), half)),
+                                       __dsub_rn(ev_key<SPANS>(fwd, tR), half)));
         double v[4];
         ev_point(q, tm, v);
         const double gm = ev_g(kind, level, f, gH, v);
@@ -592,11 +603,14 @@ __device__ double ev_locate(const EvStep& q, int kind, double level, double f, d
     }
     return tR;
 }
-// after packet i's accepted step (c.t = tnew): detect, locate and record its events in (te, ie) order.  Returns true on a
-// terminal stop, with its time and state in tstop / ystop; records after tstop are not kept.
+// after packet i's accepted step (c.t = tnew): detect, locate and record its events in order of encounter (ascending
+// tdir*te, then ie).  Returns true on a terminal stop, with its time and state in tstop / ystop; records after tstop are
+// not kept.  SPANS: the direction is the packet's own c.tdir, else forward.
+template <bool SPANS>
 __device__ __forceinline__ bool pkt_events(const Bs23Args& a, long long i, const Ode23Ctl& c, const Ode23Ev& ev, double& tstop,
                                            double ystop[4]) {
     const long long n = a.n;
+    const bool fwd = c.tdir > 0.0;
     EvStep q;
 #pragma unroll
     for (int k = 0; k < 4; k++) {
@@ -616,22 +630,28 @@ __device__ __forceinline__ bool pkt_events(const Bs23Args& a, long long i, const
         ev.vl[j * n + i] = vR;
         // vL != 0, no NaN, a sign change the direction allows (a zero at the left end is never an event)
         if ((vL < 0.0 && vR >= 0.0 && ev.dir[j] >= 0) || (vL > 0.0 && vR <= 0.0 && ev.dir[j] <= 0)) {
-            te[j] = ev_locate(q, ev.kind[j], ev.level[j], ev.f, ev.gH, vL, vR);
+            te[j] = ev_locate<SPANS>(q, fwd, ev.kind[j], ev.level[j], ev.f, ev.gH, vL, vR);
             fired |= 1u << j;
-            if (ev.term[j] && (!stop || te[j] < tstop)) { tstop = te[j]; stop = true; }
+            if (ev.term[j] && (!stop || ev_key<SPANS>(fwd, te[j]) < ev_key<SPANS>(fwd, tstop))) {
+                tstop = te[j];
+                stop = true;
+            }
         }
     }
     if (!fired) return false;
 #pragma unroll
     for (int j = 0; j < kMaxEvents; j++)
-        if (stop && te[j] > tstop) fired &= ~(1u << j);
+        if (stop && ev_key<SPANS>(fwd, te[j]) > ev_key<SPANS>(fwd, tstop)) fired &= ~(1u << j);
     int cnt = ev.ne[i];
-    while (fired) {                                              // the earliest (te, j) first
+    while (fired) {                                              // the first encountered (te, j) first
         int jm = -1;
         double tm = 0.0;
 #pragma unroll
         for (int j = 0; j < kMaxEvents; j++)
-            if (((fired >> j) & 1u) && (jm < 0 || te[j] < tm)) { jm = j; tm = te[j]; }
+            if (((fired >> j) & 1u) && (jm < 0 || ev_key<SPANS>(fwd, te[j]) < ev_key<SPANS>(fwd, tm))) {
+                jm = j;
+                tm = te[j];
+            }
         fired &= ~(1u << jm);
         if (cnt < ev.cap) {
             double v[4];
@@ -699,7 +719,7 @@ __global__ void ode23_pkt_begin_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, doubl
 // Block-reduced into the report pair of this round: the packets still unfinished and the attempts the slowest of them
 // needs; the other pair is cleared for the next round.  EV: the accepted step's events; a terminal one stops the packet
 // at its te (status 2) with that record's state, and only the dense rows up to te are written.  SPANS: the packet's own
-// tfinal, hmax, tdir and tspan row.
+// tfinal, hmax, tdir and tspan row; with EV the events follow that packet's direction.
 template <bool EV, bool SPANS>
 __global__ void __launch_bounds__(256) ode23_pkt_decide_kernel(Bs23Args a, Ode23Pkt s, Ode23Ctl c, double thr, int round, Ode23Ev ev,
                                                                Ode23Spans sp) {
@@ -716,9 +736,11 @@ __global__ void __launch_bounds__(256) ode23_pkt_decide_kernel(Bs23Args a, Ode23
             bool stop = false;
             double tstop = 0.0, ystop[4];
             if constexpr (EV) {
-                stop = pkt_events(a, i, c, ev, tstop, ystop);
+                stop = pkt_events<SPANS>(a, i, c, ev, tstop, ystop);
                 if (stop && c.ntspan > 2)
-                    while (c.nxt_end > c.nxt && c.tspan[c.nxt_end - 1] > tstop) c.nxt_end--;
+                    while (c.nxt_end > c.nxt &&
+                           ev_key<SPANS>(c.tdir > 0.0, c.tspan[c.nxt_end - 1]) > ev_key<SPANS>(c.tdir > 0.0, tstop))
+                        c.nxt_end--;
             }
             if (c.ntspan > 2) bs23_rows_at(a, i, c);
             bs23_accept_at(a, i);
@@ -819,7 +841,8 @@ void launch_ode23_pkt_begin(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ctl
                             const Ode23Spans* sp, cudaStream_t st) {
     if (a.n <= 0) return;
     const unsigned nb = nblk(a.n, 256);
-    if (ev) ode23_pkt_begin_kernel<true, false><<<nb, 256, 0, st>>>(a, s, k, thr, *ev, Ode23Spans{});
+    if (ev && sp) ode23_pkt_begin_kernel<true, true><<<nb, 256, 0, st>>>(a, s, k, thr, *ev, *sp);
+    else if (ev) ode23_pkt_begin_kernel<true, false><<<nb, 256, 0, st>>>(a, s, k, thr, *ev, Ode23Spans{});
     else if (sp) ode23_pkt_begin_kernel<false, true><<<nb, 256, 0, st>>>(a, s, k, thr, Ode23Ev{}, *sp);
     else ode23_pkt_begin_kernel<false, false><<<nb, 256, 0, st>>>(a, s, k, thr, Ode23Ev{}, Ode23Spans{});
 }
@@ -827,7 +850,8 @@ void launch_ode23_pkt_decide(const Bs23Args& a, const Ode23Pkt& s, const Ode23Ct
                              const Ode23Spans* sp, cudaStream_t st) {
     if (a.n <= 0) return;
     const unsigned nb = nblk(a.n, 256);
-    if (ev) ode23_pkt_decide_kernel<true, false><<<nb, 256, 0, st>>>(a, s, k, thr, round, *ev, Ode23Spans{});
+    if (ev && sp) ode23_pkt_decide_kernel<true, true><<<nb, 256, 0, st>>>(a, s, k, thr, round, *ev, *sp);
+    else if (ev) ode23_pkt_decide_kernel<true, false><<<nb, 256, 0, st>>>(a, s, k, thr, round, *ev, Ode23Spans{});
     else if (sp) ode23_pkt_decide_kernel<false, true><<<nb, 256, 0, st>>>(a, s, k, thr, round, Ode23Ev{}, *sp);
     else ode23_pkt_decide_kernel<false, false><<<nb, 256, 0, st>>>(a, s, k, thr, round, Ode23Ev{}, Ode23Spans{});
 }

@@ -126,6 +126,17 @@ class ShardedEnsemble:
             return ode23(self.engine, tspan, tmax, rtol, atol, per_packet=True, events=events, ev_cap=ev_cap)
         return ode23(self.engine, tspan, tmax, rtol, atol, reduce_max=self._allreduce_max)
 
+    def ode23_packets_tspans_events(self, tspan, tmax, events, rtol=1e-3, atol=1e-6, ev_cap=4):
+        """``Engine.ode23_packets_tspans_events`` on the local shard, with no collective: a 2-D ``tspan`` is the global
+        ``(ntspan, n_total)`` matrix and this rank solves its columns [lo, hi); a 1-D one is shared by every packet.  The
+        returned counts and event records are this rank's."""
+        tspan = np.asarray(tspan, dtype=np.float64)
+        if tspan.ndim == 2:
+            if tspan.shape[1] != self.n_total:
+                raise ValueError(f"ode23_packets_tspans_events: tspan must have n_total = {self.n_total} columns, got {tspan.shape}")
+            tspan = tspan[:, self.lo:self.hi]
+        return self.engine.ode23_packets_tspans_events(tspan, tmax, events, rtol, atol, ev_cap)
+
     def _allreduce_max(self, v):
         if self.dist is None or self.world == 1:
             return v

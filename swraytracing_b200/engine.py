@@ -79,6 +79,9 @@ SIGNATURES = {
     "swrt_ode23_packets_events": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, C.POINTER(_Event), C.c_int,
                                             C.c_int, _dp, C.POINTER(C.c_int32), _dp, _dp, _dp, C.POINTER(C.c_int32),
                                             C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
+    "swrt_ode23_packets_tspans_events": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_double, C.POINTER(_Event),
+                                                   C.c_int, C.c_int, _dp, C.POINTER(C.c_int32), _dp, _dp, _dp, C.POINTER(C.c_int32),
+                                                   C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
     "swrt_hist_omega_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_launch": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int, C.POINTER(C.c_void_p)]),
     "swrt_hist_omega_wait": (C.c_int, [C.c_void_p]),
@@ -390,7 +393,8 @@ class Engine:
         A 2-D ``tspan`` of shape ``(ntspan, n)`` gives every packet its own (swrt_ode23_packets_tspans): column ``i`` is
         packet ``i``'s tspan, so ``Y[j, :, i]`` is its state at ``tspan[j, i]``, as ``ode23(odefun, tspan(:, i), y0(:, i))``
         gives it.  Each column has its own direction (backward when it decreases); a constant column keeps its packet
-        where it is.  ``t`` is then the per-packet array ``tspan[-1]``.  Events need a 1-D ``tspan``."""
+        where it is.  ``t`` is then the per-packet array ``tspan[-1]``.  Events need a 1-D ``tspan`` here; with a
+        per-packet or decreasing ``tspan`` use ``ode23_packets_tspans_events``."""
         ts = _f64(tspan)
         if ts.ndim == 2:
             if events is not None:
@@ -399,6 +403,8 @@ class Engine:
                 raise ValueError(f"ode23_packets: a per-packet tspan must be (ntspan >= 2, n = {self.n}), got {ts.shape}")
         elif ts.ndim != 1:
             raise ValueError(f"ode23_packets: tspan must be 1-D (shared) or 2-D (ntspan, n), got shape {ts.shape}")
+        if events is not None:
+            return self._ode23_events(self.lib.swrt_ode23_packets_events, ts, tmax, rtol, atol, events, ev_cap)
         nt = ts.shape[0]
         dense = nt > 2
         Y = np.empty((nt, 4, self.n)) if dense else None
@@ -410,28 +416,56 @@ class Engine:
             self._check(self.lib.swrt_ode23_packets_tspans(self._h, _ptr(ts), int(nt), float(tmax or 0.0), float(rtol),
                                                            float(atol), _ptr(Y) if dense else None, pstat.ctypes.data_as(i32),
                                                            _ptr(t_end), st))
-        elif events is None:
+        else:
             st = (C.c_int64 * 5)()
             self._check(self.lib.swrt_ode23_packets(self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol),
                                                     _ptr(Y) if dense else None, pstat.ctypes.data_as(i32), _ptr(t_end), st))
-        else:
-            evs = [tuple(e) + (0, False)[len(e) - 2:] for e in events]      # direction 0, not terminal by default
-            arr = (_Event * max(len(evs), 1))(*[_Event(int(kind), int(d), int(term), 0, float(level)) for kind, level, d, term in evs])
-            cap = max(int(ev_cap), 0)
-            te, ye, ie = np.empty((cap, self.n)), np.empty((cap, 4, self.n)), np.empty((cap, self.n), dtype=np.int32)
-            ne = np.empty(self.n, dtype=np.int32)
-            st = (C.c_int64 * 7)()
-            self._check(self.lib.swrt_ode23_packets_events(
-                self._h, _ptr(ts), int(ts.size), float(tmax or 0.0), float(rtol), float(atol), arr, len(evs), int(ev_cap),
-                _ptr(Y) if dense else None, pstat.ctypes.data_as(i32), _ptr(t_end), _ptr(te), _ptr(ye), ie.ctypes.data_as(i32),
-                ne.ctypes.data_as(i32), st))
         out = {"nsteps": st[0], "nfailed": st[1], "nfevals": st[2], "t": ts[-1].copy() if ts.ndim == 2 else float(ts[-1]),
                "stopped": st[3], "host_waits": st[4],
                "steps": pstat[0].copy(), "rejected": pstat[1].copy(), "status": pstat[2].copy(), "t_end": t_end}
         if dense:
             out["Y"] = Y
-        if events is not None:
-            out.update(te=te, ye=ye, ie=ie, ne=ne, events=st[5], terminated=st[6])
+        return out
+
+    def ode23_packets_tspans_events(self, tspan, tmax, events, rtol=1e-3, atol=1e-6, ev_cap=4):
+        """``ode23`` with ``odeset('Events', ...)`` once per packet, every packet with its own tspan in either direction
+        (swrt_ode23_packets_tspans_events): ``for i = 1:n, ode23(odefun, tspan(:, i), y0(:, i), odeset('Events', ...))``.
+        ``tspan`` is ``(ntspan, n)`` (column ``i`` is packet ``i``'s, as in ``ode23_packets``) or 1-D, shared by every
+        packet in either direction.  ``events`` and ``ev_cap`` as in ``ode23_packets``; everything about them follows each
+        packet's direction of integration: rising means rising as the packet integrates (as t decreases when it goes
+        backward), records come in order of encounter, and a terminal event stops the packet at the first terminal
+        crossing it meets.  Returns ``ode23_packets(events=...)``'s dict with ``t`` the per-packet ``tspan[-1]``."""
+        ts = _f64(tspan)
+        if ts.ndim == 1 and ts.shape[0] >= 2:           # shared: the same row for every packet
+            ts = np.ascontiguousarray(np.broadcast_to(ts[:, None], (ts.shape[0], self.n)))
+        elif ts.ndim != 2 or ts.shape[0] < 2 or ts.shape[1] != self.n:
+            raise ValueError(f"ode23_packets_tspans_events: tspan must be (ntspan >= 2,) or (ntspan >= 2, n = {self.n}), "
+                             f"got shape {ts.shape}")
+        return self._ode23_events(self.lib.swrt_ode23_packets_tspans_events, ts, tmax, rtol, atol, events, ev_cap)
+
+    def _ode23_events(self, fn, ts, tmax, rtol, atol, events, ev_cap):
+        """the call and result dict of the per-packet solves with events; ts is 1-D (shared) or (ntspan, n)"""
+        nt = ts.shape[0]
+        dense = nt > 2
+        Y = np.empty((nt, 4, self.n)) if dense else None
+        pstat = np.empty((3, self.n), dtype=np.int32)          # the C side's n x 3 column-major block
+        t_end = np.empty(self.n)
+        i32 = C.POINTER(C.c_int32)
+        evs = [tuple(e) + (0, False)[len(e) - 2:] for e in events]      # direction 0, not terminal by default
+        arr = (_Event * max(len(evs), 1))(*[_Event(int(kind), int(d), int(term), 0, float(level)) for kind, level, d, term in evs])
+        cap = max(int(ev_cap), 0)
+        te, ye, ie = np.empty((cap, self.n)), np.empty((cap, 4, self.n)), np.empty((cap, self.n), dtype=np.int32)
+        ne = np.empty(self.n, dtype=np.int32)
+        st = (C.c_int64 * 7)()
+        self._check(fn(self._h, _ptr(ts), int(nt), float(tmax or 0.0), float(rtol), float(atol), arr, len(evs), int(ev_cap),
+                       _ptr(Y) if dense else None, pstat.ctypes.data_as(i32), _ptr(t_end), _ptr(te), _ptr(ye),
+                       ie.ctypes.data_as(i32), ne.ctypes.data_as(i32), st))
+        out = {"nsteps": st[0], "nfailed": st[1], "nfevals": st[2], "t": ts[-1].copy() if ts.ndim == 2 else float(ts[-1]),
+               "stopped": st[3], "host_waits": st[4],
+               "steps": pstat[0].copy(), "rejected": pstat[1].copy(), "status": pstat[2].copy(), "t_end": t_end}
+        if dense:
+            out["Y"] = Y
+        out.update(te=te, ye=ye, ie=ie, ne=ne, events=st[5], terminated=st[6])
         return out
 
     # -- diagnostics --
