@@ -356,10 +356,6 @@ __device__ __forceinline__ void leapfrog_kick(const double (&F)[NF], const SpecA
 // ATAB: 0 = x twiddles rotated in registers inside the k-loop; 1 = tabulated once per step in shared memory; 2 = tabulated
 // once per step in a per-CTA global scratch (L2-resident; grids whose table does not fit in shared memory), read back
 // with plain loads one unrolled body ahead -- in both table forms the k-loop holds no fp64 instruction but the DMMAs.
-// MODE SPEC_ANCHOR (K1 of the anchored leapfrog, DESIGN.md section 3e): a row is (occupied anchor, expansion order r) instead
-// of a packet.  A warp's 8 rows are 2 anchors x 4 orders of one parity (a.parity): r = 2*(row & 3) + parity, so that one
-// stack serves the CTA (even orders: the normal stack; odd orders: the S/D-swapped one).  The twiddle table carries
-// (kx/kmax)^r e^{i kx t_a}; the epilogue writes i^r/r! * the pass's accumulators as K2's B fragments instead of stage 2.
 template <int NPL, int G, int MT, int MODE, bool PSI, int ATAB>
 __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(const SpecArgs a) {
     static_assert(!ATAB || MT == 1, "the twiddle table is laid out for one m-tile per warp");
@@ -369,8 +365,6 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     constexpr int HALF_NT = NT / 2;
     constexpr int TILE_P = kConsumerWarps * 8 * MT;
     static_assert(NT % 2 == 0, "n-tiles are fetched in pairs");
-    constexpr bool ANC = MODE == SPEC_ANCHOR;
-    static_assert(!ANC || (PSI && MT == 1 && ATAB == 2), "the anchor contraction runs on psi-hat stacks with the global table");
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const PackGeom& g = a.g;
@@ -385,9 +379,7 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     double* sA;
     if constexpr (ATAB == 2) sA = a.twid + ((size_t)blockIdx.x * kConsumerWarps + warp) * g.ksteps * 32 + lane;
     else sA = reinterpret_cast<double*>(smem_raw + (size_t)nstages * chunk_bytes + 128) + (size_t)warp * g.ksteps * 32 + lane;
-    const long long nocc = ANC ? (long long)*a.anc_nocc : 0;
-    const long long nrows = ANC ? 4 * nocc : a.n;
-    const long long ntiles = (nrows + TILE_P - 1) / TILE_P;
+    const long long ntiles = (a.n + TILE_P - 1) / TILE_P;
     const int nevals = (MODE == SPEC_LEAPFROG) ? a.nsteps : 1;
     // SPEC_EVAL_DEV (swrt_ode23): the stack the host would pick for the controller's alpha; nothing to do once it is done
     const double* stack = a.stack;
@@ -478,17 +470,10 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
     for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         long long prow[MT];
         double px[MT], py[MT], pk[MT], pl[MT];
-        int anc_id = 0;                     // SPEC_ANCHOR: this row's anchor
 #pragma unroll
         for (int mt = 0; mt < MT; mt++) {
             long long r = tile * TILE_P + (long long)warp * 8 * MT + mt * 8 + quad_row;
             prow[mt] = r;
-            if constexpr (ANC) {
-                const long long slot = (r >> 2) < nocc ? (r >> 2) : nocc - 1;
-                anc_id = a.anc_list[slot];
-                px[mt] = py[mt] = pk[mt] = pl[mt] = 0.0;
-                continue;
-            }
             long long rc = r < a.n ? r : a.n - 1;
             if (MODE == SPEC_LEAPFROG) { px[mt] = a.x[rc]; py[mt] = a.y[rc]; pk[mt] = a.k[rc]; pl[mt] = a.l[rc]; }
             else { px[mt] = a.xin[rc]; py[mt] = a.yin[rc]; pk[mt] = 0; pl[mt] = 0; }
@@ -521,7 +506,7 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
             double F[MT][NF];
             double kyd[MT];                     // PSI: this lane's ky of group 0 in the current pass (as double)
 #pragma unroll
-            for (int mt = 0; mt < (ANC ? 0 : MT); mt++) {
+            for (int mt = 0; mt < MT; mt++) {
                 double s1, c1;
                 sincospi(reduced_turns(px[mt], a.dx, a.nxd, a.inv_nx), &s1, &c1);
                 double er = kx0 ? c1 : 1.0, ei = kx0 ? s1 : 0.0;
@@ -558,25 +543,7 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
                 kyd[mt] = (double)jq;
             }
 
-            if constexpr (ANC) {
-                // A element of this lane: (kx/kmax)^r * (cos | sin)(pi kx t_a), kx = 2s + kx0.  t_a = (id + 1/2) * anc_h is a
-                // dyadic rational with few bits, so kx * t_a is exact and sincospi gives each twiddle to the last bit or so.
-                const int r = 2 * (quad_row & 3) + a.parity;
-                const double ta = ((double)anc_id + 0.5) * a.anc_h;
-                for (int s = 0; s < g.ksteps; s++) {
-                    const int kx = 2 * s + kx0;
-                    double v = 0.0;
-                    if (kx <= g.kmax) {
-                        double sn, cs;
-                        sincospi((double)kx * ta, &sn, &cs);
-                        const double w = (double)kx / (double)g.kmax;
-                        double wr = 1.0;
-                        for (int i = 0; i < r; i++) wr *= w;
-                        v = wr * (odd ? sn : cs);
-                    }
-                    sA[s * 32] = v;
-                }
-            } else if constexpr (ATAB) {
+            if constexpr (ATAB) {
                 // the same two recurrences the in-loop rotation runs, tabulated once per step for all passes
                 double ap = ep0[0], aq = eq0[0], bp = ep1[0], bq = eq1[0];
                 for (int s = 0; s < g.ksteps; s += 2) {
@@ -660,33 +627,10 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
                     stage = nstage; phase = nphase;
                     ++ci;
                 }
-                if constexpr (ANC) {
-                    // K2's B fragments of this pass: H'_r = i^r / r! * H~_r.  Real column 2jq (re) and 2jq+1 (im) of n-tile t
-                    // go to the B lane (column * 4 + r % 4) of k-step r / 4, in the dense stack's [pass][kstep][tp][lane][2] order.
-                    if (prow[0] < nrows) {
-                        const int r = 2 * (quad_row & 3) + a.parity;
-                        double fact = 1.0;
-                        for (int i = 2; i <= r; i++) fact *= (double)i;
-                        double* blk = a.hexp + (size_t)anc_id * a.anc_block + (size_t)pass * 2 * NT * 32;
-                        const int ks = r >> 2, krow = r & 3;
+                // ---- stage 2: F_c += Gr*cos(ky ty) - Gi*sin(ky ty) for this lane's ky ----------
 #pragma unroll
-                        for (int t = 0; t < NT; t++) {
-                            const double re = acc[0][t][0] / fact, im = acc[0][t][1] / fact;
-                            const double hr = (r & 3) == 0 ? re : ((r & 3) == 1 ? -im : ((r & 3) == 2 ? -re : im));
-                            const double hi = (r & 3) == 0 ? im : ((r & 3) == 1 ? re : ((r & 3) == 2 ? -im : -re));
-                            double* dst = blk + ((size_t)(ks * HALF_NT + (t >> 1)) * 32) * 2 + (t & 1);
-                            dst[((2 * jq) * 4 + krow) * 2] = hr;
-                            dst[((2 * jq + 1) * 4 + krow) * 2] = hi;
-                        }
-                    }
-                } else {
-                    // ---- stage 2: F_c += Gr*cos(ky ty) - Gi*sin(ky ty) for this lane's ky ----------
-#pragma unroll
-                    for (int mt = 0; mt < MT; mt++) stage2_pass<NPL, G, PSI, NF>(acc[mt], ytw[mt], yrot[mt], kyd[mt], F[mt]);
-                }
+                for (int mt = 0; mt < MT; mt++) stage2_pass<NPL, G, PSI, NF>(acc[mt], ytw[mt], yrot[mt], kyd[mt], F[mt]);
             }
-            if constexpr (ANC) continue;
-            else {
             // ---- quad reduction: the 4 lanes of a quad hold 4 interleaved ky subsets ----------
 #pragma unroll
             for (int mt = 0; mt < MT; mt++) finish_planes<PSI, NPL, NF, MODE == SPEC_EVAL_DEV>(F[mt], a, ev);
@@ -706,7 +650,6 @@ __global__ void __launch_bounds__(kSpecThreads, kCtasPerSm) spectral_kernel(cons
                         }
                     }
                 }
-            }
             }
         }
         if (MODE == SPEC_LEAPFROG) {
@@ -783,11 +726,12 @@ cudaError_t launch_spectral(const SpecArgs& a, int mode, int mtiles, int num_sms
 }
 
 // ================================================================================================
-// anchored leapfrog (DESIGN.md section 3e): per sub-step  drift + key -> counting sort -> K1 (SPEC_ANCHOR) -> K2
+// anchored leapfrog (DESIGN.md section 3e): per sub-step  drift + key -> counting sort -> K1 (anchor_transform_kernel) -> K2
 // ================================================================================================
 // Anchor cells of 2^-m turns, m the smallest with (pi kmax 2^-m)^R / R! <= 2^-53 (the truncation bound of the expansion
-// relative to sum |B|).  Grids from 256^2 to 512^2: below, a cell holds too few packets to pay for its K1 rows (C2 at
-// 128^2 is at break-even); above, an anchor's H' block (npass * 12 KB) no longer fits two CTAs per SM.
+// relative to sum |B|).  Grids 256^2 and 512^2 (the transforms K1 is instantiated for): below, the dense kernel's cost per
+// packet is small enough that the anchored sub-step's fixed cost does not pay; above, an anchor's H' block (npass * 12 KB)
+// no longer fits two K2 CTAs per SM.
 int anchor_log2_cells(int nx) {
     if (nx < 256 || nx > 512 || (nx & (nx - 1))) return 0;
     const double kmax = nx / 2 - 1;
@@ -798,30 +742,234 @@ int anchor_log2_cells(int nx) {
     return 0;
 }
 
-cudaError_t launch_spectral_anchor(const SpecArgs& a, int max_rows, int num_sms, cudaStream_t st) {
-    if (a.g.npl != 3 || a.g.G != 8 || a.g.atab != 2 || !a.twid || !a.psi) return cudaErrorInvalidValue;
-    SpecArgs b = a;
-    b.n = max_rows;                   // grid sizing only: the kernel reads the row count from anc_nocc
-    return launch_inst2<3, 8, 1, SPEC_ANCHOR, true, 2>(b, num_sms, st);
-}
+// ------------------------------------------------------------------------------------------------
+// K1: the expansion blocks of every anchor cell by a fused fp64 FFT (anchor_transform_kernel)
+// ------------------------------------------------------------------------------------------------
+// For anchor cell c of N = 64 M cells (M = nx = 2 (kmax + 1)), order r < 8 and every stack column (plane, ky):
+//   H~_r(c) = sum_{kx=-kmax..kmax} (kx/kmax)^r C(kx) e^{i pi kx t_c},   t_c = (2c + 1) / N,
+// and K2 reads H'_r = i^r / r! * H~_r.  With c = 64 q + s the sum splits into a pre-twiddle and an M-point transform:
+//   H~_r(64 q + s) = sum_{k mod M} [ (kx/kmax)^r C(kx) e^{i pi kx (2s + 1) / N} ] e^{2 pi i k q / M},   kx = k or k - M,
+// the residue kmax + 1 being zero.  C(+-kx) = (S +- D) / 2 undoes the stack's fold (C(0) = S).  The transform is a
+// Stockham radix-8 FFT (last pass radix 4 at M = 256) in shared memory; pre-twiddles and FFT twiddles are sincospi of exact
+// dyadic arguments, so no error is carried across s or across passes.
+//
+// A work item is (pass, tp, ky column j, k-step ks, s): 8 transforms (2 n-tiles x the 4 orders r = 4 ks + 0..3) whose
+// outputs at q form one 128-byte line of K2's B layout in cell 64 q + s, hexp[c][pass][ks][tp][lane = col*4 + r%4][which].
+// Items run in (column, s) order and are split evenly over a persistent grid; a CTA re-reads the input columns only when
+// (pass, tp, j) changes.  Every cell is written whatever the occupancy, so H' depends on the flow and the sub-step only.
+constexpr int kAtThreads = 256;
+constexpr int kAtTr = 8;                // transforms per work item
+constexpr int kAtS = 64;                // N / M: pre-twiddle phases s
 
-// S/D-swapped stack for the odd expansion orders: in [[Sr Si],[-Di Dr]] the element (Er/Ei row, re/im column) is replaced
-// by the one of [[Dr Di],[-Si Sr]], which is the element of the partner lane (k row ^ 1, n column ^ 1), negated when
-// row and column parity differ.  Exact, so blending and swapping commute.
-__global__ void stack_swap_kernel(const double* __restrict__ in, double* __restrict__ out, size_t n) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const size_t stride = (size_t)gridDim.x * blockDim.x;
-    for (; i < n; i += stride) {
-        const int lane = (int)((i >> 1) & 31);
-        const bool same = (lane & 1) == ((lane >> 2) & 1);
-        const double v = in[i ^ (size_t)10];        // lane ^ 5
-        out[i] = same ? v : -v;
+__device__ __forceinline__ Cplx cadd(Cplx a, Cplx b) { return Cplx{a.re + b.re, a.im + b.im}; }
+__device__ __forceinline__ Cplx csub(Cplx a, Cplx b) { return Cplx{a.re - b.re, a.im - b.im}; }
+__device__ __forceinline__ Cplx cmul_i(Cplx a) { return Cplx{-a.im, a.re}; }
+
+// in-place DFT with the positive exponent, v_m <- sum_i v_i e^{2 pi i i m / R}
+__device__ __forceinline__ void dft4(Cplx& v0, Cplx& v1, Cplx& v2, Cplx& v3) {
+    const Cplx t0 = cadd(v0, v2), t1 = csub(v0, v2), t2 = cadd(v1, v3), t3 = cmul_i(csub(v1, v3));
+    v0 = cadd(t0, t2); v2 = csub(t0, t2); v1 = cadd(t1, t3); v3 = csub(t1, t3);
+}
+template <int R>
+__device__ __forceinline__ void dft(Cplx (&v)[R]) {
+    if constexpr (R == 4) {
+        dft4(v[0], v[1], v[2], v[3]);
+    } else {
+        static_assert(R == 8, "radix 4 or 8");
+        constexpr double h = 0.70710678118654752440;        // sqrt(1/2)
+        dft4(v[0], v[2], v[4], v[6]);
+        dft4(v[1], v[3], v[5], v[7]);
+        const Cplx o1{(v[3].re - v[3].im) * h, (v[3].re + v[3].im) * h};     // e^{i pi/4} O_1
+        const Cplx o2 = cmul_i(v[5]);                                         // e^{i pi/2} O_2
+        const Cplx o3{(-v[7].re - v[7].im) * h, (v[7].re - v[7].im) * h};    // e^{3 i pi/4} O_3
+        const Cplx e0 = v[0], e1 = v[2], e2 = v[4], e3 = v[6], o0 = v[1];
+        v[0] = cadd(e0, o0); v[4] = csub(e0, o0);
+        v[1] = cadd(e1, o1); v[5] = csub(e1, o1);
+        v[2] = cadd(e2, o2); v[6] = csub(e2, o2);
+        v[3] = cadd(e3, o3); v[7] = csub(e3, o3);
     }
 }
-void launch_stack_swap(const double* in, double* out, size_t n, cudaStream_t st) {
-    size_t nb = (n + 255) / 256;
-    if (nb > 148 * 16) nb = 148 * 16;
-    stack_swap_kernel<<<(unsigned)nb, 256, 0, st>>>(in, out, n);
+
+template <int M> struct AtSmem {
+    static constexpr int kPad = M + M / 8;                   // transform stride in the work buffer (padded, bank spread)
+    static constexpr size_t kBuf = (size_t)kAtTr * kPad;     // complex; also holds the 16-double output lines of M cells
+    static constexpr size_t kBytes = (kBuf + 2 * M + M + M) * sizeof(Cplx);    // buffer | input (2 n-tiles) | twiddles | pre-twiddles
+};
+__device__ __forceinline__ int at_pad(int k) { return k + (k >> 3); }
+
+// One Stockham pass of radix R over the 8 transforms of an item, stride L (the product of the earlier radices).
+// KIND 0: the first pass, input = weighted, pre-twiddled columns; 1: work buffer in place; 2: the last pass, writes
+// H' = i^r / r! * X into the output lines (q-major, 16 doubles per cell, XOR-swizzled by q).
+template <int M, int R, int L, int KIND>
+__device__ __forceinline__ void at_pass(Cplx* buf, const Cplx* xin, const Cplx* tw, const Cplx* pre, int ks, int kmax) {
+    constexpr int BPT = M / R;                                   // butterflies per transform
+    constexpr int CNT = kAtTr * BPT / kAtThreads;                 // per thread
+    static_assert(CNT >= 1 && kAtTr * BPT % kAtThreads == 0, "butterflies must tile the CTA");
+    constexpr int P = AtSmem<M>::kPad;
+    auto load = [&](int c, Cplx (&v)[R]) {
+        const int u = threadIdx.x + c * kAtThreads, tr = u / BPT, b = u % BPT;
+#pragma unroll
+        for (int i = 0; i < R; i++) {
+            const int k = b + i * BPT;
+            if constexpr (KIND == 0) {
+                const int kx = k < M / 2 ? k : k - M;
+                const double w = (double)kx / (double)kmax;
+                const int r = 4 * ks + (tr & 3);
+                double wr = 1.0;
+                for (int e = 0; e < r; e++) wr *= w;
+                const Cplx y = cmul(xin[(tr >> 2) * M + k], pre[k]);
+                v[i] = Cplx{wr * y.re, wr * y.im};
+            } else {
+                v[i] = buf[tr * P + at_pad(k)];
+            }
+            if constexpr (L > 1) {
+                if (i > 0) v[i] = cmul(v[i], tw[(i * (b % L)) * (M / (L * R))]);
+            }
+        }
+        dft<R>(v);
+    };
+    auto store = [&](int c, const Cplx (&v)[R]) {
+        const int u = threadIdx.x + c * kAtThreads, tr = u / BPT, b = u % BPT;
+        const int q0 = (b / L) * L * R + b % L;
+        if constexpr (KIND < 2) {
+#pragma unroll
+            for (int m = 0; m < R; m++) buf[tr * P + at_pad(q0 + m * L)] = v[m];
+        } else {
+            const int krow = tr & 3, r = 4 * ks + krow, which = tr >> 2;
+            double fact = 1.0;
+            for (int e = 2; e <= r; e++) fact *= (double)e;
+            double* line = reinterpret_cast<double*>(buf);
+#pragma unroll
+            for (int m = 0; m < R; m++) {
+                const int q = q0 + m * L;
+                const double re = v[m].re / fact, im = v[m].im / fact;
+                const double hr = krow == 0 ? re : (krow == 1 ? -im : (krow == 2 ? -re : im));
+                const double hi = krow == 0 ? im : (krow == 1 ? re : (krow == 2 ? -im : -re));
+                const int p = krow * 2 + which;                   // line position of the real part; imaginary at + 8
+                line[q * 16 + (p ^ (q & 15))] = hr;
+                line[q * 16 + ((p + 8) ^ (q & 15))] = hi;
+            }
+        }
+    };
+    if constexpr (KIND == 1) {
+        // thread group c touches only transforms [c * 8 / CNT, (c + 1) * 8 / CNT): in place one group at a time
+#pragma unroll
+        for (int c = 0; c < CNT; c++) {
+            Cplx v[R];
+            load(c, v);
+            __syncthreads();
+            store(c, v);
+        }
+    } else {
+        // the first pass reads the inputs, not the buffer; the last one writes lines that span every transform's region
+        Cplx v[CNT][R];
+#pragma unroll
+        for (int c = 0; c < CNT; c++) load(c, v[c]);
+        if constexpr (KIND == 2) __syncthreads();
+#pragma unroll
+        for (int c = 0; c < CNT; c++) store(c, v[c]);
+    }
+    __syncthreads();
+}
+
+template <int LOGM>
+__global__ void __launch_bounds__(kAtThreads, 2) anchor_transform_kernel(const SpecArgs a) {
+    constexpr int M = 1 << LOGM, N = kAtS * M;
+    constexpr int NT = 24, HALF_NT = NT / 2;                     // psi-hat stack: 3 planes x G = 8
+    constexpr size_t P = AtSmem<M>::kBuf;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    Cplx* buf = reinterpret_cast<Cplx*>(smem_raw);
+    Cplx* xin = buf + P;                     // [which][k]: the item's two input columns, unfolded, residues mod M
+    Cplx* tw = xin + 2 * M;                  // e^{2 pi i m / M}
+    Cplx* pre = tw + M;                      // e^{i pi kx (2s + 1) / N}
+    const int kmax = a.g.kmax;
+    const int ncols = a.g.npass * HALF_NT * 4 * 2;
+    const long long items = (long long)ncols * kAtS;
+    const long long lo = items * blockIdx.x / gridDim.x, hi = items * (blockIdx.x + 1) / gridDim.x;
+    for (int m = threadIdx.x; m < M; m += kAtThreads) {
+        double sn, cs;
+        sincospi((double)m * (2.0 / M), &sn, &cs);
+        tw[m] = Cplx{cs, sn};
+    }
+    int cached = -1;
+    for (long long it = lo; it < hi; it++) {
+        const int col = (int)(it / kAtS), s = (int)(it % kAtS);
+        const int ks = col & 1, j = (col >> 1) & 3, tp = (col >> 3) % HALF_NT, pass = (col >> 3) / HALF_NT;
+        if ((col >> 1) != cached) {          // unfold the stack's S/D columns of (pass, tp, j) for both n-tiles
+            cached = col >> 1;
+            for (int e = threadIdx.x; e < 2 * M; e += kAtThreads) {
+                const int which = e / M, kx = e % M;
+                if (kx > kmax) {
+                    if (kx == kmax + 1) xin[which * M + kx] = Cplx{0.0, 0.0};
+                    continue;
+                }
+                // lane = krow + 4 * ncol, krow = 2 (kx & 1) + part_k, ncol = 2 j + part_n: v[part_k][part_n]
+                const double* src = a.stack + ((size_t)(pass * a.g.ksteps + (kx >> 1)) * HALF_NT + tp) * 64 + which;
+                const int l0 = 2 * (kx & 1) + 8 * j;
+                const double v00 = src[(l0) * 2], v01 = src[(l0 + 4) * 2], v10 = src[(l0 + 1) * 2], v11 = src[(l0 + 5) * 2];
+                // S = (v00, v01), D = (v11, -v10)
+                if (kx == 0) {
+                    xin[which * M] = Cplx{v00, v01};
+                } else {
+                    xin[which * M + kx] = Cplx{0.5 * (v00 + v11), 0.5 * (v01 - v10)};
+                    xin[which * M + M - kx] = Cplx{0.5 * (v00 - v11), 0.5 * (v01 + v10)};
+                }
+            }
+        }
+        for (int k = threadIdx.x; k < M; k += kAtThreads) {
+            const int kx = k < M / 2 ? k : k - M;
+            double sn, cs;
+            sincospi((double)(kx * (2 * s + 1)) * (1.0 / N), &sn, &cs);
+            pre[k] = Cplx{cs, sn};
+        }
+        __syncthreads();                     // inputs ready; the previous item's lines have been written out
+        at_pass<M, 8, 1, 0>(buf, xin, tw, pre, ks, kmax);
+        if constexpr (LOGM == 9) {
+            at_pass<M, 8, 8, 1>(buf, xin, tw, pre, ks, kmax);
+            at_pass<M, 8, 64, 2>(buf, xin, tw, pre, ks, kmax);
+        } else {
+            static_assert(LOGM == 8, "M = 256 or 512");
+            at_pass<M, 8, 8, 1>(buf, xin, tw, pre, ks, kmax);
+            at_pass<M, 4, 64, 2>(buf, xin, tw, pre, ks, kmax);
+        }
+        // the M output lines of this item: 128 contiguous bytes in each cell 64 q + s
+        const double* line = reinterpret_cast<const double*>(buf);
+        double* dst = a.hexp + (size_t)s * a.anc_block + ((size_t)(pass * 2 + ks) * HALF_NT + tp) * 64 + j * 16;
+        for (int e = threadIdx.x; e < M * 16; e += kAtThreads) {
+            const int q = e >> 4, p = e & 15;
+            dst[(size_t)q * kAtS * a.anc_block + p] = line[q * 16 + (p ^ (q & 15))];
+        }
+    }
+}
+
+double anchor_transform_flops(const PackGeom& g) {
+    // per transform point: complex product by the pre-twiddle (6) and the order weight (2) in the first pass, 1/r! (2) in
+    // the last; per radix-8 butterfly 56 (two 4-point DFTs of 16, the e^{i pi/4} rotations 8, the combination 16), per
+    // radix-4 one 16; a complex twiddle (6) on all but the first input of every butterfly after the first pass
+    const int M = g.nx;
+    const double bf8 = 56.0 + 7 * 6.0, bf4 = 16.0 + 3 * 6.0;
+    double per = 10.0 * M + 56.0 * (M / 8) + bf8 * (M / 8) + (M == 512 ? bf8 * (M / 8) : bf4 * (M / 4));
+    return per * (double)g.npass * g.NT * 4 * kAnchorOrders * kAtS;
+}
+
+cudaError_t launch_anchor_transform(const SpecArgs& a, int nanchors, int num_sms, cudaStream_t st) {
+    if (a.g.npl != 3 || a.g.G != 8 || !a.psi || 2 * (a.g.kmax + 1) != a.g.nx || nanchors != kAtS * a.g.nx)
+        return cudaErrorInvalidValue;
+    auto run = [&](auto kern, size_t smem) {
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        int per_sm = 0;
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kAtThreads, smem);
+        if (e != cudaSuccess) return e;
+        if (per_sm < 1) per_sm = 1;
+        const long long items = (long long)a.g.npass * 12 * 4 * 2 * kAtS;
+        const long long grid = (long long)num_sms * per_sm < items ? (long long)num_sms * per_sm : items;
+        kern<<<(unsigned)grid, kAtThreads, smem, st>>>(a);
+        return cudaGetLastError();
+    };
+    if (a.g.nx == 512) return run(anchor_transform_kernel<9>, AtSmem<512>::kBytes);
+    if (a.g.nx == 256) return run(anchor_transform_kernel<8>, AtSmem<256>::kBytes);
+    return cudaErrorInvalidValue;
 }
 
 // first half drift (the dense kernel's arithmetic) and the anchor key; rank = position inside the anchor (atomic order:
@@ -849,36 +997,31 @@ void launch_anchor_key(double* x, double* y, const double* k, const double* l, l
                                                                   key, rank);
 }
 
-// exclusive scan of the anchor counts and the compacted list of occupied anchors (one CTA; at most 2^15 anchors)
+// exclusive scan of the anchor counts (one CTA; at most 2^15 anchors)
 __global__ void __launch_bounds__(1024) anchor_scan_kernel(const unsigned long long* __restrict__ cnt, unsigned long long* __restrict__ off,
-                                                           int* __restrict__ occ, int* __restrict__ nocc, int nanchors) {
+                                                           int nanchors) {
     __shared__ unsigned long long sc[1024];
-    __shared__ int so[1024];
     const int t = threadIdx.x;
     const int per = (nanchors + 1023) / 1024;
     const int lo = t * per, hi = (lo + per < nanchors) ? lo + per : nanchors;
-    unsigned long long c = 0; int o = 0;
-    for (int i = lo; i < hi; i++) { c += cnt[i]; o += cnt[i] != 0; }
-    sc[t] = c; so[t] = o;
+    unsigned long long c = 0;
+    for (int i = lo; i < hi; i++) c += cnt[i];
+    sc[t] = c;
     __syncthreads();
     for (int d = 1; d < 1024; d <<= 1) {
         const unsigned long long vc = t >= d ? sc[t - d] : 0;
-        const int vo = t >= d ? so[t - d] : 0;
         __syncthreads();
-        sc[t] += vc; so[t] += vo;
+        sc[t] += vc;
         __syncthreads();
     }
     unsigned long long base = t ? sc[t - 1] : 0;
-    int ob = t ? so[t - 1] : 0;
     for (int i = lo; i < hi; i++) {
         off[i] = base;
         base += cnt[i];
-        if (cnt[i]) occ[ob++] = i;
     }
-    if (t == 1023) *nocc = so[1023];
 }
-void launch_anchor_scan(const unsigned long long* cnt, unsigned long long* off, int* occ, int* nocc, int nanchors, cudaStream_t st) {
-    anchor_scan_kernel<<<1, 1024, 0, st>>>(cnt, off, occ, nocc, nanchors);
+void launch_anchor_scan(const unsigned long long* cnt, unsigned long long* off, int nanchors, cudaStream_t st) {
+    anchor_scan_kernel<<<1, 1024, 0, st>>>(cnt, off, nanchors);
 }
 
 __global__ void anchor_scatter_kernel(const int* __restrict__ key, const unsigned long long* __restrict__ rank,

@@ -114,14 +114,13 @@ struct swrt_handle {
     double* twid = nullptr; size_t twid_cap = 0;          // global twiddle-table scratch of the dense kernel (atab == 2)
     int twiddle_pref = 0;                                 // swrt_set_tuning bits 3-4
     double* arena_h = nullptr; size_t arena_h_cap = 0;      // NUFFT (u,v,H,0) grids
-    // anchored leapfrog (DESIGN.md section 3e): per-packet sort keys, per-anchor counts / offsets / occupied list, the H'
-    // blocks of every anchor and the S/D-swapped stacks of the current run
+    // anchored leapfrog (DESIGN.md section 3e): per-packet sort keys, per-anchor counts / offsets and the H' blocks of
+    // every anchor
     int64_t anc_cap = 0;
     int* anc_key = nullptr; unsigned long long* anc_rank = nullptr; long long* anc_perm = nullptr;
     int anc_n = 0;
-    unsigned long long *anc_cnt = nullptr, *anc_off = nullptr; int *anc_occ = nullptr, *anc_nocc = nullptr;
+    unsigned long long *anc_cnt = nullptr, *anc_off = nullptr;
     double* anc_hexp = nullptr; size_t anc_hexp_cap = 0;
-    double* anc_swap = nullptr; size_t anc_swap_cap = 0;
     // host staging of swrt_step_host / swrt_set_packets / swrt_get_packets (pinned ring + copy streams)
     struct Stager* stager = nullptr;
     // multi-device handle (swrt_params.ngpu > 1): one single-device child per GPU, contiguous packet shards
@@ -719,8 +718,8 @@ int swrt_destroy(swrt_handle* h) {
     dfree(h->grid_tmp);
     for (auto& st : h->stacks) { dfree(st.slot[0]); dfree(st.slot[1]); dfree(st.blend); }
     dfree(h->anc_key); dfree(h->anc_rank); dfree(h->anc_perm);
-    dfree(h->anc_cnt); dfree(h->anc_off); dfree(h->anc_occ); dfree(h->anc_nocc);
-    dfree(h->anc_hexp); dfree(h->anc_swap);
+    dfree(h->anc_cnt); dfree(h->anc_off);
+    dfree(h->anc_hexp);
     for (auto& p : h->e) dfree(p);
     dfree(h->xs); dfree(h->ys); dfree(h->ax); dfree(h->ay); dfree(h->om); dfree(h->Om);
     dfree(h->diag_dev); dfree(h->edges_dev); dfree(h->counts_dev); dfree(h->bs_norm_dev);
@@ -1013,7 +1012,6 @@ struct RunOps {
     int scheme = 0, m = 0;
     bool xka = false, composed = false;
     bool anchored = false;                // SPECTRAL leapfrog through K1 + K2 (run_anchored)
-    const double* stack_sw = nullptr;     // anchored: the S/D-swapped stacks, laid out like sa.stack
     double dt = 0, alpha0 = 0, dalpha = 0;
     int j0 = 0, mt = 1;
     SpecArgs sa{};
@@ -1030,7 +1028,7 @@ static int ensure_arena(swrt_handle* h, double*& p, size_t& cap, size_t doubles)
     return SWRT_OK;
 }
 
-// The SPECTRAL leapfrog on a psi-hat flow runs anchored (K1 per occupied anchor, K2 per packet) on the grids
+// The SPECTRAL leapfrog on a psi-hat flow runs anchored (K1 per anchor cell, K2 per packet) on the grids
 // anchor_log2_cells accepts; the choice depends on the grid, the scheme and the flow form only, never on the packet count,
 // so that a packet's result is the same in every ensemble it is part of.
 static bool anchored_leapfrog(const swrt_handle* h, int scheme, double alpha0, double dalpha) {
@@ -1048,12 +1046,10 @@ static int ensure_anchor(swrt_handle* h, int64_t n, int nanc, size_t hexp_double
         h->anc_cap = n;
     }
     if (nanc != h->anc_n) {
-        dfree(h->anc_cnt); dfree(h->anc_off); dfree(h->anc_occ); dfree(h->anc_nocc);
+        dfree(h->anc_cnt); dfree(h->anc_off);
         h->anc_n = 0;
         CU(h, cudaMalloc(&h->anc_cnt, (size_t)nanc * sizeof(unsigned long long)));
         CU(h, cudaMalloc(&h->anc_off, (size_t)nanc * sizeof(unsigned long long)));
-        CU(h, cudaMalloc(&h->anc_occ, (size_t)nanc * sizeof(int)));
-        CU(h, cudaMalloc(&h->anc_nocc, sizeof(int)));
         h->anc_n = nanc;
     }
     return ensure_arena(h, h->anc_hexp, h->anc_hexp_cap, hexp_doubles);
@@ -1072,7 +1068,7 @@ static int prepare_run(swrt_handle* h, int scheme, double dt, double alpha0, dou
     if (mode == SWRT_MODE_SPECTRAL && scheme == SWRT_SCHEME_LEAPFROG) {
         SpecArgs& a = r.sa;
         r.anchored = anchored_leapfrog(h, scheme, alpha_first, dalpha);
-        r.mt = r.anchored ? 1 : pick_mtiles(h, h->n);          // K1 is the one-m-tile contraction
+        r.mt = r.anchored ? 1 : pick_mtiles(h, h->n);          // K1 reads the one-m-tile stack
         const bool psi = use_psi(h, td ? 0.5 : alpha_first);
         const int sub = psi ? SUB_PSI3 : SUB_SIX;
         if (!td) {
@@ -1092,14 +1088,6 @@ static int prepare_run(swrt_handle* h, int scheme, double dt, double alpha0, dou
         a.x = h->x; a.y = h->y; a.k = h->k; a.l = h->l;
         fill_spec_geom(h, a);
         a.f2 = h->p.f * h->p.f; a.gH = h->p.gH; a.dt = dt; a.nsteps = m;
-        if (r.anchored) {       // odd expansion orders contract the S/D-swapped stacks (one per step of a time-dependent run)
-            const size_t nd = (size_t)(a.nstack > 1 ? a.nstack : 1) * a.g.total_doubles;
-            if ((rc = ensure_arena(h, h->anc_swap, h->anc_swap_cap, nd))) return rc;
-            launch_stack_swap(a.stack, h->anc_swap, nd, h->stream);
-            h->launches++;
-            CU(h, cudaGetLastError());
-            r.stack_sw = h->anc_swap;
-        }
         return SWRT_OK;
     }
     if (mode == SWRT_MODE_NUFFT && (scheme == SWRT_SCHEME_LEAPFROG || !h->unfused_rk4)) {
@@ -1228,41 +1216,36 @@ static int run_composed_rk4(swrt_handle* h, const RunOps& r) {
     return SWRT_OK;
 }
 
-// anchored leapfrog over packets [lo, lo+cnt), per step j: first half drift + anchor key, counting sort by anchor, K1 on
-// the even and on the odd expansion orders of every occupied anchor, K2 (expansion, stage 2, kick, second half drift).
-// No host synchronisation: the row count of K1 stays on the device.
+// anchored leapfrog over packets [lo, lo+cnt), per step j: first half drift + anchor key, counting sort by anchor, K1 (the
+// expansion blocks of every anchor cell from step j's stack), K2 (expansion, stage 2, kick, second half drift).
+// No host synchronisation.
 static int run_anchored(swrt_handle* h, const RunOps& r, int64_t lo, int64_t cnt) {
     const int mlog = anchor_log2_cells(h->p.nx);
     const int nanc = 1 << mlog;                        // anchor cells of 2^-mlog turns
     SpecArgs a = r.sa;
     a.n = cnt; a.x += lo; a.y += lo; a.k += lo; a.l += lo;
-    a.g.atab = 2;                                      // K1 writes its (kx/kmax)^r-weighted table to the per-CTA scratch
     a.anc_block = (size_t)a.g.npass * 2 * a.g.NT * 32;
     a.anc_h = std::ldexp(1.0, 1 - mlog);               // cell width in reduced_turns' t (one period = 2)
     a.zscale = M_PI * (double)a.g.kmax;
     int rc;
     if ((rc = ensure_anchor(h, cnt, nanc, (size_t)nanc * a.anc_block))) return rc;
-    if ((rc = ensure_twid(h, a.g, &a.twid))) return rc;
-    a.anc_list = h->anc_occ; a.anc_nocc = h->anc_nocc; a.anc_cnt = h->anc_cnt; a.anc_off = h->anc_off;
+    a.anc_cnt = h->anc_cnt; a.anc_off = h->anc_off;
     a.anc_perm = h->anc_perm; a.hexp = h->anc_hexp;
     const double inv_h = std::ldexp(1.0, mlog - 1);
     for (int j = 0; j < r.m; j++) {
         CU(h, cudaMemsetAsync(h->anc_cnt, 0, (size_t)nanc * sizeof(unsigned long long), h->stream));
         launch_anchor_key(a.x, a.y, a.k, a.l, cnt, a.dx, a.nxd, a.inv_nx, a.f2, a.gH, a.dt, inv_h, nanc, h->anc_cnt, h->anc_key,
                           h->anc_rank, h->stream);
-        launch_anchor_scan(h->anc_cnt, h->anc_off, h->anc_occ, h->anc_nocc, nanc, h->stream);
+        launch_anchor_scan(h->anc_cnt, h->anc_off, nanc, h->stream);
         launch_anchor_scatter(h->anc_key, h->anc_rank, h->anc_off, h->anc_perm, cnt, h->stream);
         CU(h, cudaGetLastError());
         const size_t so = a.nstack > 1 ? (size_t)j * a.g.total_doubles : 0;
         SpecArgs k1 = a;
-        k1.nstack = 1; k1.nsteps = 1;
-        k1.stack = r.sa.stack + so; k1.parity = 0;
-        CU(h, launch_spectral_anchor(k1, 4 * nanc, h->num_sms, h->stream));
-        k1.stack = r.stack_sw + so; k1.parity = 1;
-        CU(h, launch_spectral_anchor(k1, 4 * nanc, h->num_sms, h->stream));
+        k1.stack = r.sa.stack + so;
+        CU(h, launch_anchor_transform(k1, nanc, h->num_sms, h->stream));
         a.ev = j;
         CU(h, launch_anchored_step(a, nanc, h->stream));
-        h->launches += 6;
+        h->launches += 5;
     }
     h->last_nlaunch++;       // one packet-stepping run, as one dense-kernel launch is; swrt_launch_count has every kernel
     return SWRT_OK;
@@ -1932,12 +1915,10 @@ double swrt_work_per_eval(const swrt_handle* h, int nplanes) {
     if (h->p.mode == SWRT_MODE_SPECTRAL) {
         if (nplanes == 3 && anchor_log2_cells(h->p.nx) > 0 && h->n > 0) {
             // the anchored leapfrog on a psi-hat flow: K2 runs 2 k-steps (R = 8 orders) per packet over the padded columns,
-            // K1 runs R rows of the padded dense contraction per occupied anchor (at most min(n, anchors) of them)
+            // K1 the fp64 flops of its transforms (every anchor cell, whatever the occupancy), spread over the packets
             const PackGeom g = make_geom(h->p.nx, 3, kSubsetIds[SUB_PSI3], 1, h->twiddle_pref);
-            const double cols = (double)g.npass * g.NT * 8, nanc = std::ldexp(1.0, anchor_log2_cells(h->p.nx));
-            const double k1_row = 2.0 * (4.0 * g.ksteps) * cols, k2_packet = 2.0 * kAnchorOrders * cols;
-            const double occ = (double)h->n < nanc ? (double)h->n : nanc;
-            return k2_packet + kAnchorOrders * occ * k1_row / (double)h->n;
+            const double cols = (double)g.npass * g.NT * 8, k2_packet = 2.0 * kAnchorOrders * cols;
+            return k2_packet + anchor_transform_flops(g) / (double)h->n;
         }
         // executed DMMA flops per packet per evaluation: (kx>=0 count) * (ky count) * planes * 8
         // flops per folded complex MAC ... = 2 * nplanes * nx^2 for the unpadded problem

@@ -195,36 +195,35 @@ struct SpecArgs {
                             //   time-dependent flow pre-blended at al_j for every step of the launch); 0/1 = one stack
     double* twid;           // atab == 2: per-CTA twiddle scratch, gridDim.x * 8 warps * ksteps * 32 doubles
     unsigned long long* trace;   // developer timeline buffer (only read when built with -DSWRT_TRACE)
-    // anchored leapfrog (DESIGN.md section 3e).  SPEC_ANCHOR contracts rows (occupied anchor, expansion order) instead of
-    // packets; anchored_step_kernel expands the result to the packets of each anchor and steps them.
-    const int* anc_list;                  // occupied anchor ids, compacted (SPEC_ANCHOR)
-    const int* anc_nocc;                  // device: number of occupied anchors; SPEC_ANCHOR rows = 4 * nocc
+    // anchored leapfrog (DESIGN.md section 3e).  anchor_transform_kernel writes the expansion blocks of every anchor cell;
+    // anchored_step_kernel expands them to the packets of each anchor and steps them.
     const unsigned long long* anc_cnt;    // packets per anchor id
     const unsigned long long* anc_off;    // first entry of each anchor in anc_perm
     const long long* anc_perm;            // packet indices grouped by anchor
     double* hexp;                         // H' blocks (K2's B fragments), anc_block doubles per anchor id
     size_t anc_block;                     // npass * 2 k-steps * NT * 32
-    int parity;                           // SPEC_ANCHOR: 0 = even orders (normal stack), 1 = odd orders (S/D-swapped stack)
     double anc_h;                         // anchor cell width in the reduced coordinate t of reduced_turns (t in [0, 2))
     double zscale;                        // pi * kmax: z = zscale * (t - t_anchor)
     int ev;                               // anchored_step_kernel: sub-step index j of the run (mean-shear blend weight)
     Ode23Sel sel;                         // SPEC_EVAL_DEV: stack and alpha chosen from the ode23 controller
 };
 
-enum SpecMode { SPEC_EVAL = 0, SPEC_LEAPFROG = 1, SPEC_ANCHOR = 2, SPEC_EVAL_DEV = 3 };
+enum SpecMode { SPEC_EVAL = 0, SPEC_LEAPFROG = 1, SPEC_EVAL_DEV = 3 };
 
-// anchored leapfrog: expansion order, anchor geometry and the kernels around K1 (SPEC_ANCHOR) and K2
+// anchored leapfrog: expansion order, anchor geometry and its kernels (K1 = anchor_transform_kernel, K2 = anchored_step_kernel)
 constexpr int kAnchorOrders = 8;        // R: Taylor orders of e^{i kx delta} kept per anchor (two DMMA k-steps)
 constexpr int kAncWarps = 4;            // warps per CTA of anchored_step_kernel (two CTAs per SM)
 // anchor cell width in turns 2^-m for an nx grid, or 0 when this grid keeps the dense kernel
 int anchor_log2_cells(int nx);
-cudaError_t launch_spectral_anchor(const SpecArgs& a, int max_rows, int num_sms, cudaStream_t st);
+// H' blocks of all nanchors = 64 nx cells from the stack a.stack (one sub-step) into a.hexp
+cudaError_t launch_anchor_transform(const SpecArgs& a, int nanchors, int num_sms, cudaStream_t st);
+// fp64 flops one launch of it executes (pre-twiddles and weights, butterflies, pass twiddles, output scaling)
+double anchor_transform_flops(const PackGeom& g);
 cudaError_t launch_anchored_step(const SpecArgs& a, int nanchors, cudaStream_t st);
-void launch_stack_swap(const double* in, double* out, size_t n, cudaStream_t st);
 void launch_anchor_key(double* x, double* y, const double* k, const double* l, long long n, double dx, double nxd, double inv_nx,
                        double f2, double gH, double dt, double inv_h, int nanchors, unsigned long long* cnt, int* key,
                        unsigned long long* rank, cudaStream_t st);
-void launch_anchor_scan(const unsigned long long* cnt, unsigned long long* off, int* occ, int* nocc, int nanchors, cudaStream_t st);
+void launch_anchor_scan(const unsigned long long* cnt, unsigned long long* off, int nanchors, cudaStream_t st);
 void launch_anchor_scatter(const int* key, const unsigned long long* rank, const unsigned long long* off, long long* perm, long long n,
                            cudaStream_t st);
 

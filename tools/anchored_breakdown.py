@@ -1,10 +1,10 @@
-"""Per-kernel time of the anchored SPECTRAL leapfrog: drift + key, sort (scan + scatter), K1 (the anchor contraction,
-spectral_kernel<...,SPEC_ANCHOR=2,...>), K2 (anchored_step_kernel), from torch.profiler's CUDA activity records.
+"""Per-kernel time of the anchored SPECTRAL leapfrog: drift + key, sort (scan + scatter), K1 (the expansion blocks of every
+anchor cell, anchor_transform_kernel), K2 (anchored_step_kernel), from torch.profiler's CUDA activity records.
 
     python tools/anchored_breakdown.py [--out DIR]
 
-Shapes: C4 (512^2 two-frame, 16,777,216 packets, 2 sub-steps per step) and 65,536 packets at 512^2 (the regime below
-~8 packets per anchor where K1 costs more than the dense kernel would).  The whole step is also timed with CUDA events
+Shapes: C4 (512^2 two-frame, 16,777,216 packets, 2 sub-steps per step) and 65,536 packets at 512^2 (two packets per
+anchor cell: K1 costs the same whatever the packet count).  The whole step is also timed with CUDA events
 (L2 not flushed; median of 5).  Prints one JSON object per shape and writes them to DIR/anchored_breakdown.json.
 """
 import argparse
@@ -22,12 +22,12 @@ def classify(name):
         return "drift_key"
     if "anchor_scan_kernel" in name or "anchor_scatter_kernel" in name:
         return "sort"
-    if "spectral_kernel" in name:
+    if "anchor_transform_kernel" in name:
         return "K1"
     if "anchored_step_kernel" in name:
         return "K2"
-    if "stack_swap_kernel" in name or "axpby" in name:
-        return "stack_blend_swap"
+    if "axpby" in name:
+        return "stack_blend"
     return "other"
 
 
