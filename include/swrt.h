@@ -301,6 +301,36 @@ int swrt_packet_quantity(swrt_handle* h, int q, double alpha, double* out /* n *
  * swrt_packet_quantity.                                                                                            */
 int swrt_hist2(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
                double alpha, uint64_t* counts, int accumulate);
+/* per-packet weights for swrt_weight_scale / swrt_hist2_sums; a is the packets' wave action (1 when swrt_set_packets was
+ * given a NULL a), every product rounded on its own                                                               */
+#define SWRT_W_ACTION     0  /* a */
+#define SWRT_W_ENERGY     1  /* omega*a, omega bit-identical to swrt_omega's (needs no flow) */
+#define SWRT_W_PSEUDO_K   2  /* k*a */
+#define SWRT_W_PSEUDO_L   3  /* l*a */
+#define SWRT_MAX_WEIGHTS  4
+/* scale_exp[v] = E, the least integer with |w| < 2^E for every finite weight w[v] of the ensemble (0 when all are zero
+ * or non-finite); a multi-device handle MAX-all-reduces it over its devices.  alpha is the flow time of omega.
+ * SWRT_ERR_ARG: nw outside 1..SWRT_MAX_WEIGHTS, an unknown kind, a null pointer.                                    */
+int swrt_weight_scale(swrt_handle* h, const int32_t* w, int nw, double alpha, int32_t* scale_exp /* nw */);
+/* Per-bin sums of nw weight kinds w[0..nw) over swrt_hist2's bins, as fixed-point integers that every sharding and
+ * packet order sums to the same bits.  Each weight becomes q = rint(w * 2^(95-E)) (|q| <= 2^95, E = scale_exp[v], or
+ * swrt_weight_scale's when scale_exp is NULL); its three 32-bit digits (signed like w) are added to int64 counters.
+ * The sum is Sum(q) * 2^(E-95) rounded once to the nearest double (swrt_fixed_sums_to_double): exactly rounded when
+ * all weights are within 2^42 of the largest (|w| >= 2^(E-43): q is w scaled, no rounding), else fixed-point to
+ * 2^(E-95), each smaller weight off by at most 2^(E-96).
+ * Binning, refusals and the bin rule are swrt_hist2's.  sums[(v*(nye-1) + j)*(nxe-1) + i] (may be NULL);
+ * counts (may be NULL) = swrt_hist2's; acc (may be NULL) = acc[4*b + c], b the sums index: c = 0, 1, 2 the digit
+ * counters of 2^0, 2^32, 2^64 and c = 3 the weights that were non-finite or >= 2^E in magnitude (such a bin's sum is
+ * NaN).  A multi-device handle MAX-all-reduces the exponents and SUM-all-reduces acc and counts.  SWRT_ERR_ARG, with the
+ * handle usable: swrt_hist2's refusals, nw outside 1..SWRT_MAX_WEIGHTS, an unknown kind, a scale_exp outside
+ * -1073..1024, more than 2^31 - 1 packets (the counters' bound); SWRT_ERR_STATE as in swrt_packet_quantity.          */
+int swrt_hist2_sums(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
+                    double alpha, const int32_t* w, int nw, const int32_t* scale_exp, double* sums, uint64_t* counts,
+                    int64_t* acc);
+/* sums[v*nbins + b] = (acc[4*(v*nbins + b)] + acc[..+1]*2^32 + acc[..+2]*2^64) * 2^(scale_exp[v] - 95), rounded once to
+ * the nearest double (ties to even; overflow to +-inf, subnormal results rounded at 2^-1074); NaN where acc[..+3] != 0.
+ * Host only, needs no device: the final step of swrt_hist2_sums, and of a caller who all-reduces acc itself.         */
+int swrt_fixed_sums_to_double(const int64_t* acc, int64_t nbins, int nw, const int32_t* scale_exp, double* sums);
 
 /* ---- spectral <-> grid kit on the device (setup, not hot path) ----------------------------- */
 /* fk = g2k(fg) (g2k.m:5-9) and fg = k2g(fk) (k2g.m:5-6, fulspec.m:10-19), column-major.         */

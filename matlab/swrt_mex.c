@@ -423,6 +423,26 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         plhs[0] = mxCreateDoubleMatrix((size_t)nxe - 1, (size_t)nye - 1, mxREAL);
         for (size_t i = 0; i < nb; i++) mxGetPr(plhs[0])[i] = (double)c[i];
         mxFree(c);
+    } else if (!strcmp(cmd, "hist2_sums")) {          /* [S, N] = (h, qx, xedges, qy, yedges, wkinds [, alpha]) */
+        /* S(i, j + (v-1)*(nye-1)): kind wkinds(v) summed over bin (i, j), i.e. reshape(S, nxe-1, nye-1, []) is the
+         * (nxe-1) x (nye-1) x nw array; N as in 'hist2' */
+        need(nrhs, 7, "'hist2_sums', h, qx, xedges, qy, yedges, wkinds [, alpha]");
+        int nxe = (int)mxGetNumberOfElements(prhs[3]), nye = (int)mxGetNumberOfElements(prhs[5]);
+        int nw = (int)mxGetNumberOfElements(prhs[6]);
+        if (nxe < 2 || nye < 2) mexErrMsgIdAndTxt("swrt:usage", "hist2_sums: at least two edges on each axis");
+        if (nw < 1 || nw > SWRT_MAX_WEIGHTS) mexErrMsgIdAndTxt("swrt:usage", "hist2_sums: 1 to %d weight kinds", SWRT_MAX_WEIGHTS);
+        int32_t wk[SWRT_MAX_WEIGHTS];
+        for (int v = 0; v < nw; v++) wk[v] = (int32_t)mxGetPr(prhs[6])[v];
+        size_t nb = (size_t)(nxe - 1) * (size_t)(nye - 1);
+        uint64_t* c = nlhs > 1 ? (uint64_t*)mxCalloc(nb, sizeof(uint64_t)) : NULL;
+        plhs[0] = mxCreateDoubleMatrix((size_t)nxe - 1, (size_t)(nye - 1) * (size_t)nw, mxREAL);
+        if (swrt_hist2_sums(h, (int)mxGetScalar(prhs[2]), mxGetPr(prhs[3]), nxe, (int)mxGetScalar(prhs[4]), mxGetPr(prhs[5]), nye,
+                            sc(prhs, nrhs, 7, 0.0), wk, nw, NULL, mxGetPr(plhs[0]), c, NULL)) fail(h, cmd);
+        if (nlhs > 1) {
+            plhs[1] = mxCreateDoubleMatrix((size_t)nxe - 1, (size_t)nye - 1, mxREAL);
+            for (size_t i = 0; i < nb; i++) mxGetPr(plhs[1])[i] = (double)c[i];
+            mxFree(c);
+        }
     } else if (!strcmp(cmd, "packet_quantity")) {     /* q = (h, qkind [, alpha]) */
         need(nrhs, 3, "'packet_quantity', h, qkind [, alpha]");
         if (swrt_packet_quantity(h, (int)mxGetScalar(prhs[2]), sc(prhs, nrhs, 3, 0.0), vec(&plhs[0], n))) fail(h, cmd);

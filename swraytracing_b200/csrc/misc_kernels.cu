@@ -253,6 +253,116 @@ __global__ void __launch_bounds__(1024) hist2_kernel(long long n, int qx, int qy
     }
 }
 
+// ---- swrt_weight_scale / swrt_hist2_sums ----------------------------------------------------------------------------
+__device__ __forceinline__ double packet_weight(int kind, const PktQ& p, const double* a, long long i) {
+    const double ai = a[i];
+    switch (kind) {
+        case SWRT_W_ACTION: return ai;
+        case SWRT_W_ENERGY: return __dmul_rn(p.om[i], ai);
+        case SWRT_W_PSEUDO_K: return __dmul_rn(p.k[i], ai);
+        default: return __dmul_rn(p.l[i], ai);
+    }
+}
+// the largest finite |w| of each kind -> its frexp exponent E (max |w| < 2^E), biased: a block reduction, then one
+// atomicMax per kind
+__global__ void __launch_bounds__(256) weight_scale_kernel(long long n, WeightKinds w, PktQ p, const double* __restrict__ a,
+                                                           int* __restrict__ exp_dev) {
+    __shared__ int se[SWRT_MAX_WEIGHTS];
+    if (threadIdx.x < SWRT_MAX_WEIGHTS) se[threadIdx.x] = 0;
+    __syncthreads();
+    double m[SWRT_MAX_WEIGHTS] = {0.0, 0.0, 0.0, 0.0};
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+#pragma unroll
+        for (int v = 0; v < SWRT_MAX_WEIGHTS; v++) {
+            if (v >= w.n) break;
+            const double x = fabs(packet_weight(w.kind[v], p, a, i));
+            if (x <= 1.7976931348623157e308) m[v] = fmax(m[v], x);         // finite only (NaN compares false)
+        }
+    }
+#pragma unroll
+    for (int v = 0; v < SWRT_MAX_WEIGHTS; v++) {
+        if (v >= w.n) break;
+        int e = 0;
+        if (m[v] > 0.0) { frexp(m[v], &e); e += kScaleBias; }
+        e = __reduce_max_sync(0xffffffffu, e);
+        if ((threadIdx.x & 31) == 0 && e) atomicMax(&se[v], e);
+    }
+    __syncthreads();
+    if (threadIdx.x < w.n && se[threadIdx.x]) atomicMax(&exp_dev[threadIdx.x], se[threadIdx.x]);
+}
+// 2^s for -1022 <= s <= 1023
+__device__ __forceinline__ double pow2(int s) { return __longlong_as_double((long long)(s + 1023) << 52); }
+// Per-bin fixed-point sums.  The loop and the bin of a packet are hist2_kernel's.  Each weight w of a binned packet
+// becomes |q| = rint(|w| 2^(95-E)) < 2^95 (the scaling, by two powers of two so that each stays a normal number, is
+// exact; rint is the one rounding) and three 32-bit digits of |q|, split by exact fp64 operations and signed like w.  The
+// lanes of a warp that share a bin (__match_any_sync) add their digits as signed 16-bit halves with one redux each
+// (32 lanes * 2^16 fits an int), and the lowest of them adds the digit sums (< 2^37 in magnitude) to the bin's int64
+// counters.  A weight that is not finite or not below 2^E counts in the bin's fourth counter instead.
+__global__ void __launch_bounds__(1024) hist2_sums_kernel(long long n, int qx, int qy, PktQ p, const double* __restrict__ a,
+                                                         WeightKinds w, const int* __restrict__ exp_dev,
+                                                         const double* __restrict__ edges, int nxe, int nye,
+                                                         long long* __restrict__ acc, unsigned long long* __restrict__ counts) {
+    extern __shared__ unsigned char hs[];
+    double* ex = reinterpret_cast<double*>(hs);
+    double* ey = ex + nxe;
+    const int nbx = nxe - 1, nby = nye - 1;
+    const long long nb = (long long)nbx * nby;
+    for (int i = threadIdx.x; i < nxe + nye; i += blockDim.x) ex[i] = edges[i];
+    double f1[SWRT_MAX_WEIGHTS], f2[SWRT_MAX_WEIGHTS];
+#pragma unroll
+    for (int v = 0; v < SWRT_MAX_WEIGHTS; v++) {
+        const int be = v < w.n ? exp_dev[v] : 0;
+        const int s = 95 - (be ? be - kScaleBias : 0), s1 = s >> 1;     // -1073 <= E <= 1024: both halves are normal
+        f1[v] = pow2(s1); f2[v] = pow2(s - s1);
+    }
+    __syncthreads();
+    const double xlo = ex[0], xhi = ex[nbx], ylo = ey[0], yhi = ey[nby];
+    const int lane = threadIdx.x & 31;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long i0 = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); i0 < n; i0 += stride) {
+        const long long i = i0 + lane;
+        int bin = -1;
+        if (i < n) {
+            const double vx = packet_quantity(qx, p, i), vy = packet_quantity(qy, p, i);
+            if (vx >= xlo && vx <= xhi && vy >= ylo && vy <= yhi)             // also drops NaN
+                bin = bin_index(ex, nbx, vx) + bin_index(ey, nby, vy) * nbx;
+        }
+        const unsigned peers = __match_any_sync(0xffffffffu, bin);
+        if (bin < 0) continue;
+        const bool leader = lane == __ffs(peers) - 1;
+        if (leader && counts) atomicAdd(&counts[bin], (unsigned long long)__popc(peers));
+#pragma unroll
+        for (int v = 0; v < SWRT_MAX_WEIGHTS; v++) {
+            if (v >= w.n) break;
+            const double wt = packet_weight(w.kind[v], p, a, i);
+            const double qd = __dmul_rn(__dmul_rn(fabs(wt), f1[v]), f2[v]);
+            const bool bad = !(qd < 0x1p95);                                    // NaN, inf, or |w| >= 2^E
+            int piece[6] = {0, 0, 0, 0, 0, 0};
+            if (!bad) {
+                const double q = rint(qd);
+                const double h2 = floor(__dmul_rn(q, 0x1p-64));
+                const double r = __dsub_rn(q, __dmul_rn(h2, 0x1p64));
+                const double h1 = floor(__dmul_rn(r, 0x1p-32));
+                const double h0 = __dsub_rn(r, __dmul_rn(h1, 0x1p32));
+                const unsigned d[3] = {(unsigned)h0, (unsigned)h1, (unsigned)h2};
+                const int sg = wt < 0.0 ? -1 : 1;
+#pragma unroll
+                for (int c = 0; c < 3; c++) { piece[2 * c] = sg * (int)(d[c] & 0xffffu); piece[2 * c + 1] = sg * (int)(d[c] >> 16); }
+            }
+            long long* cell = acc + 4 * ((long long)v * nb + bin);
+#pragma unroll
+            for (int c = 0; c < 3; c++) {
+                const long long s = (long long)__reduce_add_sync(peers, piece[2 * c]) +
+                                    (long long)__reduce_add_sync(peers, piece[2 * c + 1]) * 65536;
+                if (leader && s) atomicAdd(reinterpret_cast<unsigned long long*>(cell + c), (unsigned long long)s);
+            }
+            const int nbad = __reduce_add_sync(peers, bad ? 1 : 0);
+            if (leader && nbad) atomicAdd(reinterpret_cast<unsigned long long*>(cell + 3), (unsigned long long)nbad);
+        }
+    }
+}
+
 // partial sums per block, then one block reduces the partials in a fixed order (deterministic)
 constexpr int kDiagBlocks = 296;
 __global__ void __launch_bounds__(256) diag_partial_kernel(long long n, const double* __restrict__ x,
@@ -910,6 +1020,31 @@ cudaError_t launch_hist2(long long n, int qx, int qy, const PktQ& p, const doubl
     unsigned nb = (unsigned)(per_sm > 0 ? per_sm : 1) * (unsigned)nsm;
     if (nb > nblk(n, 1024)) nb = nblk(n, 1024);
     kern<<<nb, 1024, bytes, st>>>(n, qx, qy, p, edges_dev, nxe, nye, counts_dev);
+    return cudaGetLastError();
+}
+void launch_weight_scale(long long n, const WeightKinds& w, const PktQ& p, const double* a, int* exp_dev, cudaStream_t st) {
+    if (n <= 0) return;
+    unsigned nb = nblk(n, 256);
+    if (nb > 148 * 8) nb = 148 * 8;
+    weight_scale_kernel<<<nb, 256, 0, st>>>(n, w, p, a, exp_dev);
+}
+cudaError_t launch_hist2_sums(long long n, int qx, int qy, const PktQ& p, const double* a, const WeightKinds& w,
+                              const int* exp_dev, const double* edges_dev, int nxe, int nye, long long* acc_dev,
+                              unsigned long long* counts_dev, cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    int dev = 0, nsm = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return e;
+    // global counters only: the digits and non-finite count take 32 bytes per (bin, kind), so a private copy per CTA fits
+    // shared memory only below ~7,000 bin-kinds, smaller than the spectra people plot
+    const size_t bytes = (size_t)(nxe + nye) * 8;
+    if ((e = cudaFuncSetAttribute(hist2_sums_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes)) != cudaSuccess) return e;
+    int per_sm = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, hist2_sums_kernel, 1024, bytes)) != cudaSuccess) return e;
+    unsigned nb = (unsigned)(per_sm > 0 ? per_sm : 1) * (unsigned)nsm;
+    if (nb > nblk(n, 1024)) nb = nblk(n, 1024);
+    hist2_sums_kernel<<<nb, 1024, bytes, st>>>(n, qx, qy, p, a, w, exp_dev, edges_dev, nxe, nye, acc_dev, counts_dev);
     return cudaGetLastError();
 }
 void launch_diag(long long n, const double* x, const double* y, const double* k, const double* l, const double* a,

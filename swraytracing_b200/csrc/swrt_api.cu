@@ -102,6 +102,9 @@ struct swrt_handle {
     double* h2_edges_dev = nullptr; int h2_edges_cap = 0;
     std::vector<double> h2_edges_host; int h2_nxe = 0;
     unsigned long long* h2_counts_dev = nullptr; int64_t h2_counts_cap = 0;
+    // swrt_weight_scale / swrt_hist2_sums: the biased scale exponents (kScaleBias) and their host image, the digit counters
+    int* ws_exp_dev = nullptr; int ws_exp_host[SWRT_MAX_WEIGHTS] = {};
+    long long* h2s_acc_dev = nullptr; int64_t h2s_acc_cap = 0;
     // instrumentation
     int64_t launches = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, hist_ev = nullptr;
@@ -159,6 +162,9 @@ int grp_ideal_omega_hist(swrt_handle* g, double alpha, int64_t npts, const doubl
                          const double* kvy, int nangles, double omega0, const double* edges, int nedges, uint64_t* counts);
 int grp_hist2(swrt_handle* g, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye, double alpha,
               uint64_t* counts, int accumulate);
+int grp_weight_scale(swrt_handle* g, const WeightKinds& wk, double alpha, int32_t* scale_exp);
+int grp_hist2_sums(swrt_handle* g, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye, double alpha,
+                   const WeightKinds& wk, const int32_t* scale_exp, double* sums, uint64_t* counts, int64_t* acc);
 int up(swrt_handle* g, swrt_handle* c, int rc);
 inline double* at(double* p, int64_t lo) { return p ? p + lo : nullptr; }
 void stager_free(swrt_handle* h);
@@ -723,7 +729,7 @@ int swrt_destroy(swrt_handle* h) {
     for (auto& p : h->e) dfree(p);
     dfree(h->xs); dfree(h->ys); dfree(h->ax); dfree(h->ay); dfree(h->om); dfree(h->Om);
     dfree(h->diag_dev); dfree(h->edges_dev); dfree(h->counts_dev); dfree(h->bs_norm_dev);
-    dfree(h->h2_edges_dev); dfree(h->h2_counts_dev);
+    dfree(h->h2_edges_dev); dfree(h->h2_counts_dev); dfree(h->ws_exp_dev); dfree(h->h2s_acc_dev);
     for (auto& p : h->bs_yt) dfree(p);
     for (auto& row : h->bs_f) for (auto& p : row) dfree(p);
     dfree(h->ode_ctl);
@@ -1587,10 +1593,11 @@ int swrt_ideal_omega_hist(swrt_handle* h, double alpha, int64_t npts, const doub
 
 // ---- swrt_packet_quantity / swrt_hist2 ----
 static bool valid_quantity(int q) { return q >= SWRT_Q_XMOD && q <= SWRT_Q_OMEGA_ABS; }
-// the packet arrays of the quantities qa, qb; om / Om computed first when one of them is a frequency
-static int quantity_inputs(swrt_handle* h, int qa, int qb, double alpha, PktQ& p) {
+// the packet arrays of the quantities qa, qb; om / Om computed first when one of them is a frequency (om also when
+// omega_too: the energy weight)
+static int quantity_inputs(swrt_handle* h, int qa, int qb, double alpha, PktQ& p, bool omega_too = false) {
     const bool need_abs = qa == SWRT_Q_OMEGA_ABS || qb == SWRT_Q_OMEGA_ABS;
-    if (need_abs || qa == SWRT_Q_OMEGA || qb == SWRT_Q_OMEGA) {
+    if (need_abs || omega_too || qa == SWRT_Q_OMEGA || qb == SWRT_Q_OMEGA) {
         int rc = compute_omega(h, alpha, need_abs);
         if (rc) return rc;
     }
@@ -1629,12 +1636,8 @@ static int hist2_args(swrt_handle* h, int qx, const double* xedges, int nxe, int
     }
     return SWRT_OK;
 }
-// the histogram into h2_counts_dev (queued, no host wait); the arguments have been checked
-static int hist2_to_device(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
-                           double alpha) {
-    int rc;
-    PktQ p;
-    if ((rc = quantity_inputs(h, qx, qy, alpha, p))) return rc;
+// h2_edges_dev holding xedges then yedges, and room for the u64 counts in h2_counts_dev (queued, no host wait)
+static int hist2_buffers(swrt_handle* h, const double* xedges, int nxe, const double* yedges, int nye) {
     const int ne = nxe + nye;
     const int64_t nb = (int64_t)(nxe - 1) * (nye - 1);
     if (ne > h->h2_edges_cap) {
@@ -1654,6 +1657,16 @@ static int hist2_to_device(swrt_handle* h, int qx, const double* xedges, int nxe
         h->h2_nxe = nxe;
         CU(h, cudaMemcpyAsync(h->h2_edges_dev, h->h2_edges_host.data(), (size_t)ne * 8, cudaMemcpyHostToDevice, h->stream));
     }
+    return SWRT_OK;
+}
+// the histogram into h2_counts_dev (queued, no host wait); the arguments have been checked
+static int hist2_to_device(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
+                           double alpha) {
+    int rc;
+    PktQ p;
+    if ((rc = quantity_inputs(h, qx, qy, alpha, p))) return rc;
+    if ((rc = hist2_buffers(h, xedges, nxe, yedges, nye))) return rc;
+    const int64_t nb = (int64_t)(nxe - 1) * (nye - 1);
     CU(h, cudaMemsetAsync(h->h2_counts_dev, 0, (size_t)nb * 8, h->stream));
     CU(h, launch_hist2(h->n, qx, qy, p, h->h2_edges_dev, nxe, nye, h->h2_counts_dev, h->stream));
     h->launches++;
@@ -1675,6 +1688,153 @@ int swrt_hist2(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, co
     CU(h, cudaStreamSynchronize(h->stream));
     CU(h, cudaGetLastError());
     for (size_t i = 0; i < nb; i++) counts[i] = accumulate ? counts[i] + tmp[i] : tmp[i];
+    return SWRT_OK;
+}
+
+// ---- swrt_weight_scale / swrt_hist2_sums ----
+static int weight_args(swrt_handle* h, const int32_t* w, int nw, WeightKinds& wk) {
+    REQUIRE(h, w, SWRT_ERR_ARG, "null weight kinds");
+    REQUIRE(h, nw >= 1 && nw <= SWRT_MAX_WEIGHTS, SWRT_ERR_ARG, "nw = %d outside 1..%d", nw, SWRT_MAX_WEIGHTS);
+    wk = WeightKinds{nw, {0, 0, 0, 0}};
+    for (int v = 0; v < nw; v++) {
+        REQUIRE(h, w[v] >= SWRT_W_ACTION && w[v] <= SWRT_W_PSEUDO_L, SWRT_ERR_ARG, "unknown weight kind %d", (int)w[v]);
+        wk.kind[v] = w[v];
+    }
+    return SWRT_OK;
+}
+static bool needs_omega(const WeightKinds& wk) {
+    for (int v = 0; v < wk.n; v++) if (wk.kind[v] == SWRT_W_ENERGY) return true;
+    return false;
+}
+static int32_t unbias_exp(int be) { return be ? be - kScaleBias : 0; }
+// the inputs of the quantities qx, qy and of the weights, then each kind's biased scale exponent into ws_exp_dev: the
+// caller's (given) or computed by the scale kernel (queued, no host wait)
+static int weight_scale_to_device(swrt_handle* h, int qx, int qy, double alpha, const WeightKinds& wk, const int32_t* given) {
+    PktQ p;
+    int rc = quantity_inputs(h, qx, qy, alpha, p, needs_omega(wk));
+    if (rc) return rc;
+    if (!h->ws_exp_dev) CU(h, cudaMalloc(&h->ws_exp_dev, SWRT_MAX_WEIGHTS * sizeof(int)));
+    if (given) {
+        for (int v = 0; v < wk.n; v++) h->ws_exp_host[v] = given[v] + kScaleBias;
+        CU(h, cudaMemcpyAsync(h->ws_exp_dev, h->ws_exp_host, wk.n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+        return SWRT_OK;
+    }
+    CU(h, cudaMemsetAsync(h->ws_exp_dev, 0, SWRT_MAX_WEIGHTS * sizeof(int), h->stream));
+    launch_weight_scale(h->n, wk, p, h->a, h->ws_exp_dev, h->stream);
+    h->launches++;
+    return SWRT_OK;
+}
+// the digit counters (and, want_counts, the u64 counts) into h2s_acc_dev / h2_counts_dev after weight_scale_to_device
+// (queued, no host wait)
+static int hist2_sums_to_device(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
+                                const WeightKinds& wk, bool want_counts) {
+    int rc = hist2_buffers(h, xedges, nxe, yedges, nye);
+    if (rc) return rc;
+    const int64_t nb = (int64_t)(nxe - 1) * (nye - 1), nacc = 4 * nb * wk.n;
+    if (nacc > h->h2s_acc_cap) {
+        dfree(h->h2s_acc_dev); h->h2s_acc_cap = 0;
+        CU(h, cudaMalloc(&h->h2s_acc_dev, (size_t)nacc * 8));
+        h->h2s_acc_cap = nacc;
+    }
+    CU(h, cudaMemsetAsync(h->h2s_acc_dev, 0, (size_t)nacc * 8, h->stream));
+    if (want_counts) CU(h, cudaMemsetAsync(h->h2_counts_dev, 0, (size_t)nb * 8, h->stream));
+    const PktQ p{h->x, h->y, h->k, h->l, h->om, h->Om, h->p.L};          // om / Om filled by weight_scale_to_device
+    CU(h, launch_hist2_sums(h->n, qx, qy, p, h->a, wk, h->ws_exp_dev, h->h2_edges_dev, nxe, nye, h->h2s_acc_dev,
+                            want_counts ? h->h2_counts_dev : nullptr, h->stream));
+    h->launches++;
+    return SWRT_OK;
+}
+// c's exponents, accumulators and counts to the host, then the sums (err: the handle that reports a failure)
+static int hist2_sums_finish(swrt_handle* err, swrt_handle* c, int64_t nb, int nw, double* sums, uint64_t* counts, int64_t* acc) {
+    std::vector<int64_t> tmp;
+    if (!acc) { tmp.resize((size_t)(4 * nb * nw)); acc = tmp.data(); }
+    int be[SWRT_MAX_WEIGHTS] = {};
+    CU(err, cudaSetDevice(c->p.device));
+    CU(err, cudaMemcpyAsync(be, c->ws_exp_dev, nw * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CU(err, cudaMemcpyAsync(acc, c->h2s_acc_dev, (size_t)(4 * nb * nw) * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (counts) CU(err, cudaMemcpyAsync(counts, c->h2_counts_dev, (size_t)nb * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(err, cudaStreamSynchronize(c->stream));
+    CU(err, cudaGetLastError());
+    int32_t E[SWRT_MAX_WEIGHTS];
+    for (int v = 0; v < nw; v++) E[v] = unbias_exp(be[v]);
+    return sums ? swrt_fixed_sums_to_double(acc, nb, nw, E, sums) : SWRT_OK;
+}
+
+int swrt_weight_scale(swrt_handle* h, const int32_t* w, int nw, double alpha, int32_t* scale_exp) {
+    if (!h) return SWRT_ERR_ARG;
+    WeightKinds wk;
+    int rc = weight_args(h, w, nw, wk);
+    if (rc) return rc;
+    REQUIRE(h, scale_exp, SWRT_ERR_ARG, "null scale_exp");
+    GROUP(h, grp_weight_scale(h, wk, alpha, scale_exp));
+    CU(h, cudaSetDevice(h->p.device));
+    if ((rc = weight_scale_to_device(h, SWRT_Q_K, SWRT_Q_K, alpha, wk, nullptr))) return rc;
+    CU(h, cudaMemcpyAsync(h->ws_exp_host, h->ws_exp_dev, nw * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(h, cudaStreamSynchronize(h->stream));
+    CU(h, cudaGetLastError());
+    for (int v = 0; v < nw; v++) scale_exp[v] = unbias_exp(h->ws_exp_host[v]);
+    return SWRT_OK;
+}
+
+int swrt_hist2_sums(swrt_handle* h, int qx, const double* xedges, int nxe, int qy, const double* yedges, int nye,
+                    double alpha, const int32_t* w, int nw, const int32_t* scale_exp, double* sums, uint64_t* counts,
+                    int64_t* acc) {
+    if (!h) return SWRT_ERR_ARG;
+    int rc = hist2_args(h, qx, xedges, nxe, qy, yedges, nye);
+    if (rc) return rc;
+    WeightKinds wk;
+    if ((rc = weight_args(h, w, nw, wk))) return rc;
+    for (int v = 0; scale_exp && v < nw; v++)
+        REQUIRE(h, scale_exp[v] >= -1073 && scale_exp[v] <= 1024, SWRT_ERR_ARG, "scale_exp[%d] = %d outside -1073..1024", v, (int)scale_exp[v]);
+    REQUIRE(h, h->n <= INT32_MAX, SWRT_ERR_ARG, "%lld packets: the digit counters hold at most 2^31 - 1", (long long)h->n);
+    GROUP(h, grp_hist2_sums(h, qx, xedges, nxe, qy, yedges, nye, alpha, wk, scale_exp, sums, counts, acc));
+    CU(h, cudaSetDevice(h->p.device));
+    if ((rc = weight_scale_to_device(h, qx, qy, alpha, wk, scale_exp))) return rc;
+    if ((rc = hist2_sums_to_device(h, qx, xedges, nxe, qy, yedges, nye, wk, counts != nullptr))) return rc;
+    return hist2_sums_finish(h, h, (int64_t)(nxe - 1) * (nye - 1), nw, sums, counts, acc);
+}
+
+// one bin: (c[0] + c[1] 2^32 + c[2] 2^64) 2^(E-95) rounded once to the nearest double, NaN when c[3] != 0
+static double fixed_to_double(const int64_t* c, int32_t E) {
+    if (c[3] != 0) return NAN;
+    using u128 = unsigned __int128;
+    using i128 = __int128;
+    const i128 t = (i128)c[1] * ((i128)1 << 32) + c[0];                // |t| < 2^96
+    const i128 hi = (i128)c[2] + (t >> 64);                               // S = hi 2^64 + lo, 0 <= lo < 2^64
+    const uint64_t lo = (uint64_t)t;
+    const bool neg = hi < 0;
+    u128 m = ((u128)hi << 64) | lo;                                       // S mod 2^128 ...
+    if (neg) m = -m;                                                      // ... and |S| < 2^128
+    if (m == 0) return 0.0;
+    const uint64_t mh = (uint64_t)(m >> 64);
+    const int bits = mh ? 128 - __builtin_clzll(mh) : 64 - __builtin_clzll((uint64_t)m);
+    const int64_t e0 = (int64_t)E - 95;                                   // the weight of m's bit 0
+    const int64_t lead = e0 + bits - 1;
+    if (lead > 1023) return neg ? -HUGE_VAL : HUGE_VAL;
+    const int64_t qexp = std::max<int64_t>(lead - 52, -1074);            // the quantum of the result's binade
+    uint64_t r;
+    int64_t rexp = qexp;
+    if (qexp <= e0) {
+        r = (uint64_t)m;                                                  // at most 53 bits: exact
+        rexp = e0;
+    } else {
+        const int64_t sh = qexp - e0;
+        if (sh > 128) {
+            r = 0;                                                        // m < 2^128 <= half a quantum
+        } else {
+            r = sh == 128 ? 0 : (uint64_t)(m >> sh);
+            const u128 rem = sh == 128 ? m : m & (((u128)1 << sh) - 1), half = (u128)1 << (sh - 1);
+            if (rem > half || (rem == half && (r & 1))) r++;              // ties to even
+        }
+    }
+    const double v = std::ldexp((double)r, (int)rexp);                   // r <= 2^53: exact, or +inf past DBL_MAX
+    return neg ? -v : v;
+}
+
+int swrt_fixed_sums_to_double(const int64_t* acc, int64_t nbins, int nw, const int32_t* scale_exp, double* sums) {
+    if (nbins < 0 || nw < 0 || (nbins > 0 && nw > 0 && (!acc || !scale_exp || !sums))) return SWRT_ERR_ARG;
+    for (int v = 0; v < nw; v++)
+        for (int64_t b = 0; b < nbins; b++) sums[v * nbins + b] = fixed_to_double(acc + 4 * (v * nbins + b), scale_exp[v]);
     return SWRT_OK;
 }
 

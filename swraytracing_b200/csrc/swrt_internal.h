@@ -312,6 +312,18 @@ void launch_packet_quantity(long long n, int q, const PktQ& p, double* out, cuda
 // Per-CTA shared-memory counters when they fit the opt-in shared memory, else global atomics.  Returns the launch error.
 cudaError_t launch_hist2(long long n, int qx, int qy, const PktQ& p, const double* edges_dev, int nxe, int nye,
                          unsigned long long* counts_dev, cudaStream_t st);
+// swrt_weight_scale / swrt_hist2_sums: the weight kinds SWRT_W_* of one call, computed from PktQ's k, l, om and a.  The
+// scale exponents live on the device as E + kScaleBias (0: no finite non-zero weight, E = 0) so that a zeroed word is the
+// identity of the int32 MAX the kernel and a multi-device all-reduce apply.
+struct WeightKinds { int n; int kind[4]; };            // 4 = SWRT_MAX_WEIGHTS
+constexpr int kScaleBias = 1100;
+// atomicMax of every kind's biased exponent into exp_dev[0..nw) (zeroed by the caller)
+void launch_weight_scale(long long n, const WeightKinds& w, const PktQ& p, const double* a, int* exp_dev, cudaStream_t st);
+// the fixed-point digits of each kind's weights, per bin of (qx, qy), added to acc_dev (4 int64 per (bin, kind), layout of
+// swrt_hist2_sums' acc) with the exponents exp_dev; counts_dev (may be null) gets swrt_hist2's counts.  Global atomics only.
+cudaError_t launch_hist2_sums(long long n, int qx, int qy, const PktQ& p, const double* a, const WeightKinds& w,
+                              const int* exp_dev, const double* edges_dev, int nxe, int nye, long long* acc_dev,
+                              unsigned long long* counts_dev, cudaStream_t st);
 void launch_diag(long long n, const double* x, const double* y, const double* k, const double* l, const double* a,
                  const double* omega, const double* Omega_abs, double* out8_dev, cudaStream_t st);
 void launch_fill(double* p, double v, long long n, cudaStream_t st);

@@ -178,6 +178,24 @@ class ShardedEnsemble:
         local = np.asarray(self.engine.hist2(qx, xedges, qy, yedges, alpha))
         return self._allreduce_sum(local.astype(np.int64)).astype(np.uint64)
 
+    def hist2_sums(self, qx, xedges, qy, yedges, weights, alpha=0.0):
+        """``Engine.hist2_sums`` over all shards, bit-identical under any world size: every rank's scale exponents
+        MAX-all-reduced, each rank's int64 accumulators with those exponents SUM-all-reduced, then rounded once on the host
+        (``fixed_sums_to_double``).  Returns ``(sums, counts)``."""
+        from .engine import fixed_sums_to_double
+        e = np.asarray(self.engine.weight_scale(weights, alpha), dtype=np.int32)
+        if self.dist is not None and self.world > 1:
+            import torch
+            t = torch.from_numpy(e.copy())
+            if self.device is not None:
+                t = t.to(self.device)
+            self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
+            e = t.cpu().numpy()
+        _, counts, acc = self.engine.hist2_sums(qx, xedges, qy, yedges, weights, alpha, scale_exp=e, return_acc=True)
+        acc = self._allreduce_sum(np.ascontiguousarray(acc))
+        counts = self._allreduce_sum(np.asarray(counts).astype(np.int64)).astype(np.uint64)
+        return fixed_sums_to_double(acc, e), counts
+
     def hist_pipeline(self, edges, kind=0):
         return HistPipeline(self, edges, kind)
 

@@ -21,6 +21,8 @@ FLAG_RHS_GH = 1
 EVENT_X, EVENT_Y, EVENT_K, EVENT_L, EVENT_KMAG, EVENT_OMEGA = 0, 1, 2, 3, 4, 5
 MAX_EVENTS = 8
 Q_XMOD, Q_YMOD, Q_K, Q_L, Q_KMAG, Q_THETA, Q_OMEGA, Q_OMEGA_ABS = 0, 1, 2, 3, 4, 5, 6, 7
+W_ACTION, W_ENERGY, W_PSEUDO_K, W_PSEUDO_L = 0, 1, 2, 3
+MAX_WEIGHTS = 4
 
 _dp = C.POINTER(C.c_double)
 
@@ -91,6 +93,10 @@ SIGNATURES = {
     "swrt_omega": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp]),
     "swrt_packet_quantity": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp]),
     "swrt_hist2": (C.c_int, [C.c_void_p, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_double, C.POINTER(C.c_uint64), C.c_int]),
+    "swrt_weight_scale": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_double, C.POINTER(C.c_int32)]),
+    "swrt_hist2_sums": (C.c_int, [C.c_void_p, C.c_int, _dp, C.c_int, C.c_int, _dp, C.c_int, C.c_double, C.POINTER(C.c_int32),
+                                  C.c_int, C.POINTER(C.c_int32), _dp, C.POINTER(C.c_uint64), C.POINTER(C.c_int64)]),
+    "swrt_fixed_sums_to_double": (C.c_int, [C.POINTER(C.c_int64), C.c_int64, C.c_int, C.POINTER(C.c_int32), _dp]),
     "swrt_g2k": (C.c_int, [C.c_int, _dp, C.c_int, _dp, _dp]),
     "swrt_k2g": (C.c_int, [C.c_int, _dp, _dp, C.c_int, _dp]),
     "swrt_qg_create": (C.c_int, [C.c_int, C.c_int] + [C.c_double] * 8 + [_dp, _dp, C.POINTER(C.c_void_p)]),
@@ -189,6 +195,39 @@ def _f64(a):
 
 def _ptr(a):
     return a.ctypes.data_as(_dp) if a is not None else None
+
+
+def _i32p(a):
+    return a.ctypes.data_as(C.POINTER(C.c_int32)) if a is not None else None
+
+
+def _weight_kinds(weights):
+    """one W_* kind or a sequence of 1..MAX_WEIGHTS of them -> int32 array (checked before any library call)"""
+    w = np.atleast_1d(np.asarray(weights))
+    if w.ndim != 1 or not 1 <= w.size <= MAX_WEIGHTS or not np.issubdtype(w.dtype, np.integer):
+        raise ValueError(f"weights must be 1..{MAX_WEIGHTS} of W_ACTION, W_ENERGY, W_PSEUDO_K, W_PSEUDO_L, got {weights!r}")
+    if not np.all((w >= W_ACTION) & (w <= W_PSEUDO_L)):
+        raise ValueError(f"unknown weight kind in {weights!r}")
+    return np.ascontiguousarray(w, dtype=np.int32)
+
+
+def fixed_sums_to_double(acc, scale_exp):
+    """swrt_fixed_sums_to_double on the host (no device): ``acc`` int64 of shape ``(nw, nbx, nby, 4)`` as
+    ``Engine.hist2_sums(..., return_acc=True)`` returns it (or a sum of such arrays), ``scale_exp`` the nw exponents
+    -> the ``(nw, nbx, nby)`` sums, each rounded once"""
+    acc = np.asarray(acc)
+    if acc.dtype != np.int64 or acc.ndim != 4 or acc.shape[3] != 4:
+        raise ValueError(f"acc must be an int64 array of shape (nw, nbx, nby, 4), got {acc.dtype} {acc.shape}")
+    nw, nbx, nby, _ = acc.shape
+    e = np.ascontiguousarray(np.atleast_1d(scale_exp), dtype=np.int32)
+    if e.shape != (nw,):
+        raise ValueError(f"scale_exp must hold {nw} exponents, got {e.shape}")
+    raw = np.ascontiguousarray(acc.transpose(0, 2, 1, 3))                  # C: acc[4*((v*nby + j)*nbx + i) + c]
+    out = np.empty((nw, nby, nbx))
+    rc = load_library().swrt_fixed_sums_to_double(raw.ctypes.data_as(C.POINTER(C.c_int64)), nbx * nby, nw, _i32p(e), _ptr(out))
+    if rc != 0:
+        raise SwrtError(rc, "swrt_fixed_sums_to_double")
+    return out.transpose(0, 2, 1)
 
 
 def _colmajor(a):
@@ -537,6 +576,39 @@ class Engine:
             counts[...] = buf
             return counts
         return buf
+
+    def weight_scale(self, weights, alpha=0.0):
+        """swrt_weight_scale: for each kind in ``weights`` (``W_ACTION``, ``W_ENERGY``, ``W_PSEUDO_K``, ``W_PSEUDO_L``) the least
+        E with |w| < 2^E over every finite weight of the ensemble (0 when there is none); int32 array"""
+        w = _weight_kinds(weights)
+        out = np.zeros(w.size, dtype=np.int32)
+        self._check(self.lib.swrt_weight_scale(self._h, _i32p(w), w.size, float(alpha), _i32p(out)))
+        return out
+
+    def hist2_sums(self, qx, xedges, qy, yedges, weights, alpha=0.0, scale_exp=None, return_acc=False):
+        """per-bin sums of packet weights over ``hist2``'s bins (swrt_hist2_sums): ``(sums, counts)``, sums float64 of shape
+        ``(nw, nxe-1, nye-1)`` (``sums[v, i, j]``: kind ``weights[v]`` summed over bin (i, j)), counts as ``hist2``
+        returns them.  Each sum is the fixed-point total of the weights scaled by 2^(95-E), rounded once: exactly rounded
+        when all weights are within 2^42 of the largest, else fixed-point to 2^(E-95); NaN where a binned packet's weight
+        is not finite.  ``scale_exp``: the nw exponents E to use (default: ``weight_scale``'s).  ``return_acc``: also the
+        int64 accumulators, shape ``(nw, nxe-1, nye-1, 4)`` (three digit counters and the non-finite count), which
+        ``fixed_sums_to_double`` finishes."""
+        w = _weight_kinds(weights)
+        xe, ye = _f64(xedges).ravel(), _f64(yedges).ravel()
+        nbx, nby = max(xe.size - 1, 0), max(ye.size - 1, 0)
+        e = None
+        if scale_exp is not None:
+            e = np.ascontiguousarray(np.atleast_1d(scale_exp), dtype=np.int32)
+            if e.shape != (w.size,):
+                raise ValueError(f"hist2_sums: scale_exp must hold {w.size} exponents, got {e.shape}")
+        sums = np.empty((w.size, nby, nbx))                      # C: sums[(v*nby + j)*nbx + i]
+        counts = np.empty((nby, nbx), dtype=np.uint64)
+        acc = np.empty((w.size, nby, nbx, 4), dtype=np.int64) if return_acc else None
+        self._check(self.lib.swrt_hist2_sums(self._h, int(qx), _ptr(xe), xe.size, int(qy), _ptr(ye), ye.size, float(alpha),
+                                             _i32p(w), w.size, _i32p(e), _ptr(sums), counts.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                             acc.ctypes.data_as(C.POINTER(C.c_int64)) if return_acc else None))
+        out = (sums.transpose(0, 2, 1), counts.T)
+        return out + (acc.transpose(0, 2, 1, 3),) if return_acc else out
 
     # -- instrumentation --
     def launch_count(self, reset=False):
