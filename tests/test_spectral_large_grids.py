@@ -150,17 +150,18 @@ def test_eval_every_twiddle_home_and_seven_planes(nx, name):
 LEAPFROG_SIZES = [8, 10, 192, 256, 512, 1024]
 
 
-def leapfrog_errors(nx, name, form):
-    """(one step, 8 two-frame sub-steps) against CO.leapfrog_spectral, relative to the increment"""
+def leapfrog_errors(nx, name, form, m=8, make=None):
+    """(one step, m two-frame sub-steps at alpha_j = (j + 1/2)/m) against CO.leapfrog_spectral, relative to the
+    increment; ``make(w, form, two)`` builds the engine (default: this file's dense-mode ``engine``)"""
     w, (x, y, k, l) = sample(name, nx, 40)
-    with engine(w, form, two=True) as e:
-        assert e.contracted_planes() == (3 if form == "psi" else 6)
+    with (make or engine)(w, form, two=True) as e:
+        if make is None:
+            assert e.contracted_planes() == (3 if form == "psi" else 6)
         e.set_packets(x, y, k, l)
         e.step(S.SCHEME_LEAPFROG, w.dt, 1)
         got1 = e.get_packets()
         xs, ys, ks, ls = (v[-25:] for v in (x, y, k, l))          # 16 random + the edge positions
-        m = 8
-        a0, da = 1.0 / 16, 1.0 / 8
+        a0, da = 0.5 / m, 1.0 / m
         e.set_packets(xs, ys, ks, ls)
         e.step(S.SCHEME_LEAPFROG, w.dt / m, m, a0, da)           # pre-blended stacks, one per sub-step
         gotm = e.get_packets()
@@ -190,9 +191,9 @@ RK4_CASES = [("rk4_packet", "psi"), ("rk4_packet", "planes"), ("rk4_packet", "tw
              ("rk4_xka", "two-frame")]
 
 
-def rk4_error(nx, scheme, flow):
-    """2 fused steps against step_packet / step_packet_xka with exact-sum fields; wave action as in
-    test_spectral_fused_rk4_equals_the_composed_launches"""
+def rk4_error(nx, scheme, flow, make=None, unfused=False):
+    """2 fused steps (the composed launches with ``unfused``) against step_packet / step_packet_xka with exact-sum
+    fields; wave action as in test_spectral_fused_rk4_equals_the_composed_launches"""
     xka = scheme == "rk4_xka"
     two = flow == "two-frame"
     w, (x, y, k, l) = sample("C4" if two else "C5", nx, 55)
@@ -200,7 +201,9 @@ def rk4_error(nx, scheme, flow):
     seven = xka or flow == "planes"
     m = 2
     a0, da = (0.5 / m, 1.0 / m) if two else (0.0, 0.0)
-    with engine(w, "seven" if seven else "psi", two=two) as e:
+    with (make or engine)(w, "seven" if seven else "psi", two=two) as e:
+        if unfused:
+            e.set_tuning(unfused_rk4=True)
         e.set_packets(x, y, k, l, a)
         e.step(S.SCHEME_RK4_XKA if xka else S.SCHEME_RK4_PACKET, w.dt, m, a0, da)
         got = e.get_packets(with_a=True)
@@ -235,15 +238,32 @@ def ray_ode(w, n, two):
     return O.generate_raytracing_ode(None, None, n, w.f, w.Cg, T_ODE if two else np.inf, w.dx, eval6=eval6)
 
 
-def ode23_errors(nx, form, two):
-    """Engine.ode23 over [0, T], a 7-entry dense tspan forward and backward, and Engine.ode23_packets on 8 packets,
-    against the oracle's ode23; the step counts must be identical"""
+def c3_packets(nx):
     w, pk = sample("C3", nx, 7)
-    pk = np.stack(pk)
+    return w, np.stack(pk)
+
+
+def mixed_tspans(n, nt=5, seed=3):
+    """per-packet tspans: forward [T - t, T], backward [t, 0] and zero-length rows, in turn"""
+    rs = np.random.RandomState(seed)
+    T = rs.uniform(0.5, 1.0, n) * T_ODE
+    ts = np.empty((nt, n))
+    for i in range(n):
+        ts[:, i] = (np.linspace(T_ODE - T[i], T_ODE, nt), np.linspace(T[i], 0.0, nt), np.full(nt, T[i]))[i % 3]
+    return ts
+
+
+def ode23_errors(nx, form, two, make=None, packets=c3_packets, tspans=False):
+    """Engine.ode23 over [0, T], a 7-entry dense tspan forward and backward, and Engine.ode23_packets on every other
+    packet (with ``tspans`` also on mixed_tspans, one tspan per packet), against the oracle's ode23; the step counts
+    must be identical"""
+    w, pk = packets(nx)
     n = pk.shape[1]
     tmax = T_ODE if two else None
     errs = {}
-    with engine(w, form, two=two) as e:
+    sub = pk[:, ::2]
+    ts2 = mixed_tspans(sub.shape[1])
+    with (make or engine)(w, form, two=two) as e:
         for key, tspan in (("final", [0.0, T_ODE]), ("dense", T_ODE * np.linspace(0, 1, 7)),
                            ("backward", T_ODE * np.linspace(1, 0, 7))):
             e.set_packets(*pk)
@@ -256,17 +276,30 @@ def ode23_errors(nx, form, two):
             else:
                 assert np.array_equal(st["Y"][0], pk)
                 errs[key] = max(rel_increment_err(st["Y"][j], yref[j].reshape(4, n), pk) for j in range(1, 7))
-        sub = pk[:, ::2]
         e.set_packets(*sub)
         st = e.ode23_packets([0.0, T_ODE], tmax)
         got = np.stack(e.get_packets())
-    ref = []
+        if tspans:
+            e.set_packets(*sub)
+            st2 = e.ode23_packets(ts2, tmax)
+            got2 = np.stack(e.get_packets())
+    ref, ref2 = [], []
     for i in range(sub.shape[1]):
         yi, si = B.ode23(ray_ode(w, 1, two), [0.0, T_ODE], sub[:, i])
         ref.append(yi)
         assert (st["steps"][i], st["rejected"][i]) == (si["nsteps"], si["nfailed"]), i
+        if tspans:
+            Yi, si = B.ode23(ray_ode(w, 1, two), ts2[:, i], sub[:, i])
+            ref2.append(Yi)
+            assert (st2["steps"][i], st2["rejected"][i]) == (si["nsteps"], si["nfailed"]), ("tspans", i)
     assert np.all(st["status"] == 0)
     errs["packets"] = rel_increment_err(got, np.stack(ref, axis=1), sub)
+    if tspans:
+        assert np.all(st2["status"] == 0)
+        Y2 = np.stack(ref2, axis=2)                               # (nt, 4, n)
+        assert np.array_equal(st2["Y"][0], sub) and np.array_equal(got2[:, 2::3], sub[:, 2::3])
+        errs["tspans"] = max(rel_increment_err(st2["Y"][j], Y2[j], sub) for j in range(1, ts2.shape[0]))
+        errs["tspans final"] = rel_increment_err(got2, Y2[-1], sub)
     return errs
 
 
@@ -278,15 +311,19 @@ def test_ode23_256(form, two):
     assert max(errs.values()) < TOL_SUBSTEPS, errs
 
 
-@pytest.mark.gpu
-def test_ode23_512_steady():
-    w, pk = sample("C3", 512, 7)
-    pk = np.stack(pk)
-    with engine(w, "psi") as e:
+def ode23_steady_error(nx, make=None, packets=c3_packets):
+    """one coupled steady solve over [0, T] on a psi-hat flow against the oracle: identical counts, error of the increment"""
+    w, pk = packets(nx)
+    with (make or engine)(w, "psi") as e:
         e.set_packets(*pk)
         st = e.ode23([0.0, T_ODE], None)
         got = np.stack(e.get_packets())
     yref, sref = B.ode23(ray_ode(w, pk.shape[1], False), [0.0, T_ODE], pk.ravel())
     assert (st["nsteps"], st["nfailed"], st["nfevals"]) == (sref["nsteps"], sref["nfailed"], sref["nfevals"])
-    err = rel_increment_err(got, yref.reshape(4, -1), pk)
+    return rel_increment_err(got, yref.reshape(4, -1), pk)
+
+
+@pytest.mark.gpu
+def test_ode23_512_steady():
+    err = ode23_steady_error(512)
     assert err < TOL_SUBSTEPS, err
